@@ -65,7 +65,36 @@ def parse_args():
     ap.add_argument("--full-upload", action="store_true",
                     help="e2e legs upload the whole frame every step instead of the search windows of the active targets (cfg.upload_window)")
     ap.add_argument("--cpu-sample-frames", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path returned for its last step as DIR/<name>.npy (float32): per "
+                         "stream (rank 0's streams) and target success, status, score and bbox, and (b200 arm) the NV12 frame with the "
+                         "box drawn into it. "
+                         "The reference arm's frame is left out: its HUD prints the measured FPS")
     return ap.parse_args()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(directory, outputs):
+    """Each array as `directory`/<name>.npy in float32, 64 MB in all.  An array larger than what is left of that is stored as a fixed
+    sample: the elements at the sorted flat positions np.random.default_rng(0).choice(size, n, replace=False), the same in every run."""
+    os.makedirs(directory, exist_ok=True)
+    left = DUMP_BYTES
+    for name, a in sorted(outputs.items(), key=lambda kv: np.asarray(kv[1]).size):
+        a = np.asarray(a, dtype=np.float32)
+        left -= 4096  # .npy header
+        if a.nbytes > left:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, left // a.itemsize, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(directory, name + ".npy"), a)
+        left -= a.nbytes
+
+
+def result_outputs(results):
+    """results[stream][target] = (success, status, score, bbox) -> the arrays of --dump-outputs."""
+    return {"success": [[r[0] for r in rs] for rs in results], "status": [[r[1] for r in rs] for rs in results],
+            "score": [[r[2] for r in rs] for rs in results], "bbox": [[r[3] for r in rs] for rs in results]}
 
 
 def dist_env():
@@ -237,6 +266,9 @@ def run_reference(args):
         p.step(ring[(args.warmup + i) % len(ring)].copy())
     dt = time.perf_counter() - t0
     fps = args.steps / dt
+    if args.dump_outputs:
+        rc, ok, score, bb = p.last
+        dump_outputs(args.dump_outputs, result_outputs([[(ok, rc, score, bb)]]))
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": fps, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
         "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -452,6 +484,9 @@ def run_b200(args):
     sampler = ClockSampler(local_rank)
     sampler.start()
     leg_dev = timed(streams, "device", K, Wm)
+    if args.dump_outputs and rank == 0:   # the headline leg's last step: the handles' results and the frame its overlay was drawn into
+        dumped = result_outputs([[(r.success, r.status, r.score, r.bbox) for r in s.trk._results()] for s in streams])
+        dumped["frame_nv12"] = torch.stack([s.dev[(Wm + K - 1) % s.dev_frames] for s in streams]).cpu().numpy()
     for s in streams:
         s.reset()
     lat_dev = run_leg(streams, "device_sync", min(K, 200), 0, want_lat=True)  # per-frame latency of the synchronous device-resident call
@@ -775,6 +810,8 @@ def run_b200(args):
                 out["trajectory_check"] = {"frames": len(cpu_traj), "boxes_equal": same, "max_dscore": dmax,
                                            "what": "GPU (synchronous update, clean frames) vs CPU oracle on the first frames of the workload"}
                 assert dmax <= 1e-3 and same >= 0.97 * len(cpu_traj), out["trajectory_check"]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumped)
         print(json.dumps(out))
     if world > 1:
         dist.barrier()

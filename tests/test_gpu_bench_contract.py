@@ -53,13 +53,25 @@ def test_reference_arm_line(built):
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["value"] == d["value"]
 
 
-def test_both_arms_print_the_same_config_keys(built):
-    """The driver compares the two arms' `config`: same keys, and the same values for the workload-defining ones."""
+def test_both_arms_print_the_same_config_keys(built, tmp_path):
+    """The driver compares the two arms' `config`: same keys, and the same values for the workload-defining ones.  Both arms' last
+    timed step tracked the same frame: their --dump-outputs results agree (|dscore| <= 1e-3, boxes within a floor tie)."""
     sys.path.insert(0, ROOT)
     import bench
     import argparse
+
+    import numpy as np
     a = argparse.Namespace(model="tiny", streams_per_gpu=1, gpus=1, ring=0, steps=40, warmup=5)
     assert set(bench.config_dict(a)) >= {"workload", "resolution", "format", "targets", "model", "streams_per_gpu", "weights", "call", "l2"}
-    g = _run("--steps", "12", "--warmup", "3", "--no-cpu-baseline", "--no-extras")
-    r = _run("--impl", "reference", "--steps", "12", "--warmup", "3")
+    g = _run("--steps", "12", "--warmup", "3", "--no-cpu-baseline", "--no-extras", "--dump-outputs", str(tmp_path / "g"))
+    r = _run("--impl", "reference", "--steps", "12", "--warmup", "3", "--dump-outputs", str(tmp_path / "r"))
     assert g["config"] == r["config"]
+    res = {"success", "status", "score", "bbox"}
+    assert {p.stem for p in (tmp_path / "g").iterdir()} == res | {"frame_nv12"} and {p.stem for p in (tmp_path / "r").iterdir()} == res
+    dg, dr = ({k: np.load(tmp_path / arm / f"{k}.npy") for k in res} for arm in ("g", "r"))
+    assert all(dg[k].dtype == np.float32 and dg[k].shape == dr[k].shape for k in res)
+    assert dg["success"][0, 0] == dr["success"][0, 0] == 1 and dg["status"][0, 0] == dr["status"][0, 0] == 0
+    assert abs(dg["score"] - dr["score"]).max() <= 1e-3 and abs(dg["bbox"] - dr["bbox"]).max() <= 1, (dg, dr)
+    fr = np.load(tmp_path / "g" / "frame_nv12.npy")
+    assert fr.dtype == np.float32 and fr.shape == (1, 1920 * 1080 * 3 // 2) and fr.min() >= 0 and fr.max() <= 255
+    assert np.array_equal(fr, np.round(fr))
