@@ -383,6 +383,36 @@ __device__ __forceinline__ void tmem_ld_32x8(uint32_t taddr, float (&v)[8]) {
 }
 __device__ __forceinline__ void tmem_ld_cols(uint32_t taddr, float (&v)[16]) { tmem_ld_32x16(taddr, v); }
 __device__ __forceinline__ void tmem_ld_cols(uint32_t taddr, float (&v)[8]) { tmem_ld_32x8(taddr, v); }
+
+// ---- M = 64 accumulators (cta_group::1): row 16 q + i sits in lane 32 q + i, i < 16 — the first 16 lanes of every lane quarter.
+// The 16x32bx2 shapes address those 16 lanes from a whole warp: thread l < 16 accesses lane l of the warp's quarter at columns
+// taddr .., thread l >= 16 lane l - 16 at columns taddr + OFF .. (OFF: immediate, in 32-bit columns).
+__device__ __forceinline__ void tmem_ld_16x2_x8_issue(uint32_t taddr, uint32_t (&r)[8]) {  // OFF = 8
+    asm volatile("tcgen05.ld.sync.aligned.16x32bx2.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8], 8;"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+                 : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[8]) {
+    asm volatile("tcgen05.wait::ld.sync.aligned;" : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7])::"memory");
+}
+__device__ __forceinline__ void tmem_ld_16x2(uint32_t taddr, float (&v)[8]) {  // OFF = 8
+    uint32_t r[8];
+    tmem_ld_16x2_x8_issue(taddr, r);
+    tmem_ld_wait(r);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
+}
+__device__ __forceinline__ void tmem_ld_16x2(uint32_t taddr, float (&v)[4]) {  // OFF = 4
+    uint32_t r[4];
+    asm volatile("tcgen05.ld.sync.aligned.16x32bx2.x4.b32 {%0, %1, %2, %3}, [%4], 4;" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(taddr));
+    asm volatile("tcgen05.wait::ld.sync.aligned;" : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3])::"memory");
+#pragma unroll
+    for (int i = 0; i < 4; ++i) v[i] = __uint_as_float(r[i]);
+}
+__device__ __forceinline__ void tmem_st_16x2_x4(uint32_t taddr, const uint32_t (&r)[4]) {  // OFF = 4
+    asm volatile("tcgen05.st.sync.aligned.16x32bx2.x4.b32 [%0], 4, {%1, %2, %3, %4};" ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3])
+                 : "memory");
+}
 __device__ __forceinline__ float ex2_approx(float x) {
     float y;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));

@@ -380,6 +380,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
         t->chain_mlp = t->fuse_ln && D <= 192 && !getenv("VT_B200_NO_CHAIN");
         if (t->chain_mlp) VT_TRY(cudaMalloc(&t->Pbuf, sizeof(float) * (Hd / 64) * B * kNTok * D));
         t->att_chain_ok = t->chain_mlp && t->fuse_ln && D / t->heads == 64 && (int)(Hd / 64) >= t->heads && t->nsplit && !getenv("VT_B200_NO_ATT_CHAIN");
+        t->att_q64 = !getenv("VT_B200_ATT_Q128");
         t->split_k = t->chain_mlp && Hd / 64 >= 4 && (C == 64 || C == 128) && !getenv("VT_B200_NO_SPLITK");
         if (t->split_k) {
             VT_TRY(cudaMalloc(&t->Phead, sizeof(float) * 9 * B * kNTx * C));

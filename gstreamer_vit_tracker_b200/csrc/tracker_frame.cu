@@ -139,12 +139,14 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool recor
                 VT_LAUNCH(tc_gemm_as_launch(p.qkv, M, ns, s, pdl, t->sm_count));
             else
                 VT_LAUNCH(tc_gemm_launch(p.qkv, M, ns, s, pdl, spread));
-            // Latency mode: the proj GEMM is folded into the attention kernel (per-head partial products, D / 64 replicas per tile) and
-            // reduce_ln adds the heads + bias + residual and applies LN2 — one kernel and one dependency edge less per block.
-            const bool att_chain = spread && t->att_chain_ok && n * t->heads * 3 * (D / kAttChainW) <= kSpreadCtas;
+            // Latency mode: the proj GEMM is folded into the attention kernel (per-head partial products, D / kAttChainW replicas per
+            // tile) and reduce_ln adds the heads + bias + residual and applies LN2 — one kernel and one dependency edge less per block.
+            // 64-row query tiles (5 per sequence) when that grid still fits one wave: each CTA computes half the exponentials.
+            const bool att_q64 = spread && t->att_chain_ok && t->att_q64 && n * t->heads * 5 * (D / kAttChainW) <= kSpreadCtas;
+            const bool att_chain = att_q64 || (spread && t->att_chain_ok && n * t->heads * 3 * (D / kAttChainW) <= kSpreadCtas);
             if (t->tc_attention)
                 VT_LAUNCH(tc_attention_launch(att_chain ? p.att : t->plan_att, n, t->heads, ns, t->d_tc_err, s, pdl, t->d_trace,
-                                              att_chain ? VT_ATT_CHAIN : (spread ? VT_ATT_DUP : VT_ATT_PLAIN)));
+                                              att_q64 ? VT_ATT_CHAIN_Q64 : att_chain ? VT_ATT_CHAIN : (spread ? VT_ATT_DUP : VT_ATT_PLAIN)));
             else
                 VT_LAUNCH(launch_attention(t->QKV, nullptr, t->att_hi, LO(t->att_lo), n, D, t->heads, s));
             if (att_chain) {

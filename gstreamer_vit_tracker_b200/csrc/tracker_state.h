@@ -162,6 +162,7 @@ struct vt_tracker {
         TcAttentionPlan att;  // plan_att + this block's W_proj maps (chained form)
     };
     bool att_chain_ok = false;  // the chained attention form is available (VT_B200_NO_ATT_CHAIN disables)
+    bool att_q64 = true;        // ... on 64-row query tiles where the grid fits one wave (VT_B200_ATT_Q128: always 128-row tiles)
     std::vector<BlockPlans> plans;
 
     std::map<int, cudaGraphExec_t> graphs;

@@ -365,6 +365,7 @@ bool tc_gemm_as_mlp_supported(const TcGemmPlan& p, int nsplit);
 cudaError_t tc_gemm_as_mlp_launch(const TcGemmPlan& p, int M, cudaStream_t s, bool pdl, int sm_count, int* planes, const TcGemmPlan* fc2 = nullptr);
 struct TcAttentionPlan {      // kernel parameter block (__grid_constant__)
     CUtensorMap mQhi, mQlo, mKhi, mKlo, mVhi, mVlo;
+    CUtensorMap mQ64hi, mQ64lo;      // Q in boxes of 64 rows (VT_ATT_CHAIN_Q64)
     CUtensorMap mW2hi, mW2lo;        // chained form: W_proj [D][D], boxes of 64 x 64
     __nv_bfloat16 *out_hi, *out_lo;  // [B][320][D]: the proj GEMM's A operand
     float* p2;                       // chained form: fp32 partial proj products, plane h = head h: [heads][batch][320][D]
@@ -377,8 +378,9 @@ bool tc_attention_plan_init(TcAttentionPlan* p, const __nv_bfloat16* Qhi, const 
 bool tc_attention_plan_chain(TcAttentionPlan* p, const __nv_bfloat16* Whi, const __nv_bfloat16* Wlo, float* P2, int64_t plane_elems);
 cudaError_t tc_attention_setup();
 // form: plain; DUP = two replicas per tile storing the hi / lo output tiles; CHAIN = proj folded in (D / 64 replicas per tile, each
-// stores one 64-column slice of the head's partial proj product; needs tc_attention_plan_chain) — the latter two are "spread" forms
-enum { VT_ATT_PLAIN = 0, VT_ATT_DUP = 1, VT_ATT_CHAIN = 2 };
+// stores one kAttChainW-column slice of the head's partial proj product; needs tc_attention_plan_chain); CHAIN_Q64 = CHAIN on 64-row query
+// tiles (M = 64 UMMAs: five tiles instead of 128 + 128 + 64, half the exponentials per CTA) — the latter three are "spread" forms
+enum { VT_ATT_PLAIN = 0, VT_ATT_DUP = 1, VT_ATT_CHAIN = 2, VT_ATT_CHAIN_Q64 = 3 };
 constexpr int kAttChainW = 32;  // columns of the partial proj product per replica CTA of the chained form (32 or 64)
 cudaError_t tc_attention_launch(const TcAttentionPlan& p, int B, int heads, int nsplit, int* err, cudaStream_t s, bool pdl,
                                 unsigned long long* trace = nullptr, int form = VT_ATT_PLAIN);
