@@ -253,7 +253,6 @@ constexpr int kMlpABytes = kAsMaxKb * 2 * kTileABytes;
 constexpr int kMlpSmemTotal = kMlpABytes + kMlpStages * kMlpStageBytes + 1024;
 constexpr uint32_t kMlpColH = 256, kMlpColAcc2 = 320;
 static_assert(kTcBM * kMaxAsChainN * 4 <= kMlpABytes + kMlpStages * kMlpStageBytes, "the partial tile is staged over the dead operand buffers");
-static_assert(6 * kTcBM * 64 * 4 <= kMlpABytes + kMlpStages * kMlpStageBytes, "fused reduce: 2 received + X + LN hi/lo + 2 outgoing blocks");
 
 __device__ __forceinline__ void mlp_group(int g, int n, bool& is_w2, int& chunk) {
     if (g == 0) is_w2 = false, chunk = 0;
@@ -262,21 +261,9 @@ __device__ __forceinline__ void mlp_group(int g, int n, bool& is_w2, int& chunk)
     else is_w2 = true, chunk = (g >> 1) - 1;
 }
 
-// FUSE: the nb2 = N2 / 64 CTAs of a row tile form a cluster and reduce their partial products among themselves — CTA r owns output
-// columns [64 r, 64 r + 64): the other CTAs push their partial columns for it straight from registers into its (dead) operand buffers
-// with st.async (the stores signal its mbarrier), it adds bias + residual + the partials in rank order (the order reduce_ln_kernel
-// uses: X is bit-identical to the plane form), exchanges LayerNorm statistics with its peers (as gemm_tc.cu's fused LayerNorm) and
-// stores the fp32 X tile and the bf16 (hi, lo) LayerNorm tile of the next GEMM.  No partial planes, no reduce kernel, one dependency
-// edge less per block.  a2 = the FC2 plan's arguments (bias, X, LayerNorm parameters and outputs).
-constexpr int kMlpRecvBytes = kTcBM * 64 * 4;  // one sender's [128 rows][64 columns] fp32 block
-template <bool FUSE>
-__global__ void __launch_bounds__(kAsThreads, 1) gemm_as_mlp_kernel(const __grid_constant__ TcMaps mp, const TcGemmArgs a, const TcGemmArgs a2,
-                                                                   const int chunks_per_cta) {
+__global__ void __launch_bounds__(kAsThreads, 1) gemm_as_mlp_kernel(const __grid_constant__ TcMaps mp, const TcGemmArgs a, const int chunks_per_cta) {
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t a_bar[kAsMaxKb], full_bar[kMlpStages], empty_bar[kMlpStages], acc_full[2], acc_empty[2], h_full, h_free, acc2_full;
-    __shared__ __align__(8) uint64_t red_bar, ln_bar;
-    __shared__ float2 ln_loc[FUSE ? kTcColGroups : 1][FUSE ? kTcBM : 1];   // (sum, M2) of the 16 columns of thread (row, g)
-    __shared__ float2 ln_part[FUSE ? 8 : 1][FUSE ? kTcBM : 1];             // (sum, M2) of the 64 columns of every CTA of the cluster, per row
     __shared__ uint32_t tmem_base_s;
     __shared__ unsigned long long* trace_slot;
     constexpr int CPT = kAsChunk / kTcColGroups;
@@ -329,12 +316,6 @@ __global__ void __launch_bounds__(kAsThreads, 1) gemm_as_mlp_kernel(const __grid
             for (int s = 0; s < kMlpStages; ++s) mbar_init(&full_bar[s], 1), mbar_init(&empty_bar[s], 1);
             for (int b = 0; b < 2; ++b) mbar_init(&acc_full[b], 1), mbar_init(&acc_empty[b], kTcThreads / 32);
             mbar_init(&h_full, kTcThreads / 32), mbar_init(&h_free, 1), mbar_init(&acc2_full, 1);
-            if (FUSE) {  // armed now: peers only send after the cluster barrier below
-                mbar_init(&red_bar, 1), mbar_init(&ln_bar, 1);
-                fence_barrier_init();
-                mbar_arrive_expect_tx(&red_bar, (cluster_nctarank() - 1) * (uint32_t)kMlpRecvBytes);
-                mbar_arrive_expect_tx(&ln_bar, cluster_nctarank() * kTcBM * (uint32_t)sizeof(float2));
-            }
             fence_barrier_init();
         }
         __syncwarp();
@@ -476,7 +457,6 @@ __global__ void __launch_bounds__(kAsThreads, 1) gemm_as_mlp_kernel(const __grid
         ok &= mbar_wait(&acc2_full, 0);
         tcgen05_fence_after();
         if (e == 0) tr.mark(5);
-        if (!FUSE) {
         const int cols_per = N2 / kTcColGroups, sw = row & 7;
         for (int c = g * cols_per; c < (g + 1) * cols_per; c += 16) {
             float pv[16];
@@ -491,143 +471,6 @@ __global__ void __launch_bounds__(kAsThreads, 1) gemm_as_mlp_kernel(const __grid
         for (int cb = 0; cb < N2 / 32; ++cb)
             tile_to_global<128>(smem + cb * (kTcBM * 128), a.p, (int64_t)cb * 128, tr_rows, 0, 0, blockIdx.x, e);
         if (e == 0) tr.mark(7);
-        }
-    }
-    if (FUSE) {
-        // every CTA of the cluster is past its MMAs (the epilogue warps arrive after acc2_full): operand buffers are dead everywhere
-        cluster_arrive_release();
-        cluster_wait_acquire();
-        const int e = tid - 64, ew = e >> 5;
-        const int quarter = warp & 3, row = quarter * 32 + lane, g = ew >> 2, sw = row & 7;
-        const uint32_t lane_base = tmem + ((uint32_t)(quarter * 32) << 16);
-        const uint32_t rank = cluster_ctarank(), nct = cluster_nctarank();
-        uint8_t* recv = smem;                                   // [nct - 1][128 rows][256 B], 16-byte chunks XOR-swizzled by row & 7
-        uint8_t* sC = smem + 2 * kMlpRecvBytes;                 // fp32 X tile: two boxes of [128 rows][128 B]
-        uint8_t* sLnHi = sC + kMlpRecvBytes, *sLnLo = sLnHi + kTcBM * 128;
-        uint8_t* sOut = sLnLo + kTcBM * 128;                     // outgoing blocks, one per peer, in the receiver's layout
-        float own[16];
-        if (warp >= 2) {
-            for (uint32_t b = 0; b < nct; ++b) {
-                float pv[16];
-                tmem_ld_32x16(lane_base + kMlpColAcc2 + 64 * b + 16 * g, pv);
-                if (b == rank) {
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) own[j] = pv[j];
-                } else {
-                    const uint32_t slot = rank < b ? rank : rank - 1;
-                    (void)slot;
-                    uint8_t* out = sOut + (b < rank ? b : b - 1) * kMlpRecvBytes + row * 256;  // staged locally, then ONE bulk copy per peer
-#pragma unroll
-                    for (int q = 0; q < 4; ++q)
-                        *reinterpret_cast<float4*>(out + (((4 * g + q) ^ sw) << 4)) = make_float4(pv[4 * q], pv[4 * q + 1], pv[4 * q + 2], pv[4 * q + 3]);
-                }
-            }
-            // (per-thread remote stores — st.async or st.shared::cluster, 16 bytes each, 32 rows per warp instruction — took ~10 us for the
-            // 64 KB a CTA sends: the exchange goes through the bulk-copy engine instead)
-            fence_proxy_async_smem();
-            asm volatile("bar.sync 1, %0;" ::"n"(kTcThreads) : "memory");
-            if (e == 0) {
-                for (uint32_t b = 0; b < nct; ++b) {
-                    if (b == rank) continue;
-                    const uint32_t slot_in = rank < b ? rank : rank - 1;
-                    dsmem_bulk_copy(cluster_map_shared(smem_u32(recv + slot_in * kMlpRecvBytes), b), smem_u32(sOut + (b < rank ? b : b - 1) * kMlpRecvBytes),
-                                    (uint32_t)kMlpRecvBytes, cluster_map_shared(smem_u32(&red_bar), b));
-                }
-            }
-            const TileRows tr_rows(m0, a.period, a.batch_off);
-            // bias + residual row while the partials travel: X is flat [rows][N2]
-            const int m = m0 + row, nc = 64 * (int)rank + 16 * g;
-            float v[16];
-#pragma unroll
-            for (int j = 0; j < 16; j += 4) {
-                const float4 b4 = a2.bias ? __ldg(reinterpret_cast<const float4*>(a2.bias + nc + j)) : make_float4(0.f, 0.f, 0.f, 0.f);
-                float4 x4 = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (m < a.M) x4 = __ldcg(reinterpret_cast<const float4*>(reinterpret_cast<const float*>(a2.c.base) + (int64_t)m * N2 + nc + j));
-                v[j] = x4.x + b4.x, v[j + 1] = x4.y + b4.y, v[j + 2] = x4.z + b4.z, v[j + 3] = x4.w + b4.w;
-            }
-            ok &= mbar_wait(&red_bar, 0);
-            for (uint32_t r = 0; r < nct; ++r) {  // partials in rank order (reduce_ln_kernel: plane order)
-                if (r == rank) {
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) v[j] += own[j];
-                } else {
-                    const uint8_t* src = recv + (r < rank ? r : r - 1) * kMlpRecvBytes + row * 256;
-#pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const float4 p4 = *reinterpret_cast<const float4*>(src + (((4 * g + q) ^ sw) << 4));
-                        v[4 * q] += p4.x, v[4 * q + 1] += p4.y, v[4 * q + 2] += p4.z, v[4 * q + 3] += p4.w;
-                    }
-                }
-            }
-            {   // row statistics of this thread's 16 columns
-                float sm = 0.f;
-#pragma unroll
-                for (int j = 0; j < 16; ++j) sm += v[j];
-                const float mu = sm * (1.f / 16);
-                float m2 = 0.f;
-#pragma unroll
-                for (int j = 0; j < 16; ++j) {
-                    const float d = v[j] - mu;
-                    m2 = fmaf(d, d, m2);
-                }
-                ln_loc[g][row] = make_float2(sm, m2);
-            }
-            // fp32 X tile staged as two [128 rows][128 B] boxes (swizzled), as in gemm_tc.cu
-            uint8_t* c_row = sC + ((g * 16) >> 5) * (kTcBM * 128) + row * 128;
-            const int c_chunk0 = ((g * 16) & 31) >> 2;
-#pragma unroll
-            for (int q = 0; q < 4; ++q)
-                *reinterpret_cast<float4*>(c_row + (((c_chunk0 + q) ^ sw) << 4)) = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
-            asm volatile("bar.sync 1, %0;" ::"n"(kTcThreads) : "memory");
-            if (g == 0) {  // (sum, M2) of this CTA's 64 columns of the row (Chan), pushed to every CTA of the cluster
-                float sm = 0.f;
-#pragma unroll
-                for (int q = 0; q < kTcColGroups; ++q) sm += ln_loc[q][row].x;
-                const float mu = sm * (1.f / 64);
-                float m2 = 0.f;
-#pragma unroll
-                for (int q = 0; q < kTcColGroups; ++q) {
-                    const float2 p = ln_loc[q][row];
-                    const float d = p.x * (1.f / 16) - mu;
-                    m2 += p.y + 16.f * d * d;
-                }
-                const uint32_t mine = smem_u32(&ln_part[rank][row]), bar = smem_u32(&ln_bar);
-                for (uint32_t r = 0; r < nct; ++r) st_async_cluster_f2(cluster_map_shared(mine, r), sm, m2, cluster_map_shared(bar, r));
-            }
-#pragma unroll
-            for (int bx = 0; bx < 2; ++bx)
-                tile_to_global<128>(sC + bx * (kTcBM * 128), a2.c, (int64_t)(64 * rank + 32 * bx) * 4, tr_rows, a2.c_row_off, 0, 0, e);
-            if (a2.ln_g) {
-                float gam[16], bet[16];
-#pragma unroll
-                for (int j = 0; j < 16; j += 4) {
-                    const float4 g4 = __ldg(reinterpret_cast<const float4*>(a2.ln_g + nc + j)), b4 = __ldg(reinterpret_cast<const float4*>(a2.ln_b + nc + j));
-                    gam[j] = g4.x, gam[j + 1] = g4.y, gam[j + 2] = g4.z, gam[j + 3] = g4.w;
-                    bet[j] = b4.x, bet[j + 1] = b4.y, bet[j + 2] = b4.z, bet[j + 3] = b4.w;
-                }
-                ok &= mbar_wait(&ln_bar, 0);
-                float tot = 0.f;
-                for (uint32_t r = 0; r < nct; ++r) tot += ln_part[r][row].x;
-                const float mean = tot / (float)N2;
-                float M2 = 0.f;
-                for (uint32_t r = 0; r < nct; ++r) {
-                    const float2 p = ln_part[r][row];
-                    const float d = p.x * (1.f / 64) - mean;
-                    M2 += p.y + 64.f * d * d;
-                }
-                const float rstd = 1.f / sqrtf(M2 / (float)N2 + 1e-6f);
-                float y[16];
-#pragma unroll
-                for (int j = 0; j < 16; ++j) y[j] = (v[j] - mean) * rstd * gam[j] + bet[j];
-                stage_split<16, false>(y, sLnHi, sLnLo, row, g, true);
-                asm volatile("bar.sync 1, %0;" ::"n"(kTcThreads) : "memory");
-                tile_to_global<128>(sLnHi, a2.ln_out[0], (int64_t)(64 * rank) * 2, tr_rows, a2.ln_row_off, 0, 0, e);
-                tile_to_global<128>(sLnLo, a2.ln_out[1], (int64_t)(64 * rank) * 2, tr_rows, a2.ln_row_off, 0, 0, e);
-            } else {
-                ok &= mbar_wait(&ln_bar, 0);  // (nobody leaves before every peer's statistics have landed in its shared memory)
-            }
-            if (e == 0) tr.mark(7);
-        }
     }
     if (!ok && a.err) atomicExch(a.err, 1);
     tcgen05_fence_before();
@@ -640,15 +483,14 @@ cudaError_t tc_gemm_as_setup() {
     cudaError_t e = cudaFuncSetAttribute(gemm_as_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, AsSmem<1>::kTotal);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_as_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, AsSmem<2>::kTotal);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_as_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, AsSmem<3>::kTotal);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_as_mlp_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMlpSmemTotal);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_as_mlp_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kMlpSmemTotal);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_as_mlp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kMlpSmemTotal);
     return e;
 }
 
-// The plan must be a plain 64-column-tile plan (tc_plan_init with bn = 64) whose epilogue is a bf16 (hi, lo) tile store or the QKV scatter.
+// The plan's epilogue must be a bf16 (hi, lo) tile store or the QKV scatter.
 bool tc_gemm_as_supported(const TcGemmPlan& p) {
     const TcGemmArgs& a = p.args;
-    return p.bn == 64 && a.K % kTcBK == 0 && a.K / kTcBK <= kAsMaxKb && a.N % kAsChunk == 0 && !a.conv_feat && !a.kb_per_split && !a.chain_n &&
+    return a.K % kTcBK == 0 && a.K / kTcBK <= kAsMaxKb && a.N % kAsChunk == 0 && !a.conv_feat && !a.kb_per_split && !a.chain_n &&
            !a.ln_g && !a.c_on && !a.residual && !a.pos && !a.relu && (a.o_mode == 1 || a.o_mode == 2) && (a.o_mode != 2 || (a.N / 3) % 64 == 0);
 }
 
@@ -667,30 +509,18 @@ int tc_gemm_as_split(int M, int n_chunks, int sm_count, int* per_cta) {
 // plan = an FC1 plan with tc_plan_chain applied (bf16x3 operands); writes *planes partial planes to the chain output
 bool tc_gemm_as_mlp_supported(const TcGemmPlan& p, int nsplit) {
     const TcGemmArgs& a = p.args;
-    return nsplit == 3 && p.bn == 64 && a.K % kTcBK == 0 && a.K / kTcBK <= kAsMaxKb && a.N % kAsChunk == 0 && !a.conv_feat && !a.kb_per_split &&
+    return nsplit == 3 && a.K % kTcBK == 0 && a.K / kTcBK <= kAsMaxKb && a.N % kAsChunk == 0 && !a.conv_feat && !a.kb_per_split &&
            a.chain_n > 0 && a.chain_n % 64 == 0 && a.chain_n <= kMaxAsChainN && !a.ln_g && !a.c_on && !a.residual && !a.pos && !a.relu && a.o_mode == 3;
 }
-// fc2 (optional): the FC2 plan of the block (bias, residual X, LayerNorm of the next GEMM).  When the split gives exactly N2 / 64 CTAs per
-// row tile they reduce their partials inside a cluster and *planes comes back 0: no reduce_ln_kernel launch is needed.
-cudaError_t tc_gemm_as_mlp_launch(const TcGemmPlan& p, int M, cudaStream_t s, bool pdl, int sm_count, int* planes, const TcGemmPlan* fc2) {
+cudaError_t tc_gemm_as_mlp_launch(const TcGemmPlan& p, int M, cudaStream_t s, bool pdl, int sm_count, int* planes) {
     if (!tc_gemm_as_mlp_supported(p, 3) || M <= 0) return cudaErrorInvalidValue;
     TcGemmArgs a = p.args;
     a.M = M;
-    a.chain_slices = 0, a.dup_hl = 0, a.dup_ln = 0, a.mcast = 0;
+    a.chain_slices = 0, a.dup_hl = 0, a.dup_ln = 0;
     int per_cta = 1;
-    const int sx = tc_gemm_as_split(M, a.N / kAsChunk, sm_count, &per_cta);
-    const dim3 grid(sx, (M + kTcBM - 1) / kTcBM, 1);
-    // Opt-in (VT_B200_AS_FUSE=1): measured SLOWER than partial planes + reduce_ln_kernel at 5120 rows (cfg4 ViT 684-705 us against 651 us;
-    // per-thread remote stores: 730 us) — a CTA moves its 64 KB through distributed shared memory at ~10 B/clk, the reduce kernel reads the
-    // planes from L2 on all SMs at once.  Kept as a tested alternative (profiles/r2_final.md).
-    const bool no_fuse = getenv("VT_B200_AS_FUSE") == nullptr;  // (read per launch = per graph capture)
-    if (fc2 && !no_fuse && sx == a.chain_n / 64 && sx >= 2 && sx <= 8 && fc2->args.c_on && fc2->args.residual && fc2->args.N == a.chain_n &&
-        fc2->args.period == a.period && static_cast<const void*>(fc2->args.c.base) != nullptr) {
-        *planes = 0;
-        return launch_ex(gemm_as_mlp_kernel<true>, grid, dim3(kAsThreads), kMlpSmemTotal, s, pdl, sx, p.maps, a, fc2->args, per_cta);
-    }
-    *planes = sx;
-    return launch_ex(gemm_as_mlp_kernel<false>, grid, dim3(kAsThreads), kMlpSmemTotal, s, pdl, 1, p.maps, a, a, per_cta);
+    *planes = tc_gemm_as_split(M, a.N / kAsChunk, sm_count, &per_cta);
+    const dim3 grid(*planes, (M + kTcBM - 1) / kTcBM, 1);
+    return launch_ex(gemm_as_mlp_kernel, grid, dim3(kAsThreads), kMlpSmemTotal, s, pdl, 1, p.maps, a, per_cta);
 }
 
 cudaError_t tc_gemm_as_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, int sm_count) {
@@ -698,7 +528,7 @@ cudaError_t tc_gemm_as_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream
     if (!tc_gemm_as_supported(p)) return cudaErrorInvalidValue;
     TcGemmArgs a = p.args;
     a.M = M;
-    a.chain_slices = 0, a.dup_hl = 0, a.dup_ln = 0, a.mcast = 0;
+    a.chain_slices = 0, a.dup_hl = 0, a.dup_ln = 0;
     int per_cta = 1;
     dim3 grid(tc_gemm_as_split(M, a.N / kAsChunk, sm_count, &per_cta), (M + kTcBM - 1) / kTcBM, 1);
     if (nsplit == 3) return launch_ex(gemm_as_kernel<3>, grid, dim3(kAsThreads), AsSmem<3>::kTotal, s, pdl, 1, p.maps, a, per_cta);

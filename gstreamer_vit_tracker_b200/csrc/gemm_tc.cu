@@ -29,6 +29,7 @@
 // a share of the epilogue output — a CTA stores at ~26 B/clk, which is what bounds the 32..96 KB epilogues: FC1 chain in three
 // 64-column slices (the GELU'd hidden tile then is a TMEM A operand), QKV scatter as hi / lo replicas, fused-LN GEMM as fp32 / LN-hi /
 // LN-lo replicas.  All forms are re-associations of the same sums (tests/test_gpu_tracker.py::test_kernel_forms_agree).
+// 128 x 32 tiles and TMA multicast of the activation tile across column-tile CTAs were measured without gain (DESIGN.md §7).
 // The 3x3 head convolution runs through the same kernel: its A operand is gathered by TMA from the [B,16,16,D] token grid with
 // shifted (possibly negative) coordinates; out-of-bounds elements are zero-filled by the TMA unit = zero padding of the conv.
 #include <stdlib.h>
@@ -42,19 +43,17 @@ namespace vt {
 
 constexpr int kTcStages = 3;
 constexpr int kMaxChainN = 192;                 // widest chained second GEMM (TMEM: 128 + N2 <= 512 columns)
-constexpr int kChainBN = 64;                    // the chained GEMM consumes a 64-column hidden tile
+constexpr int kTcBN = 64;                       // column-tile width; the chained GEMM consumes the 64-column hidden tile as its K
 
-// BN = 64: the default tile.  BN = 32 (VT_B200_TILE32): twice the CTAs, half the epilogue per CTA — measured without gain
-// (profiles/r1d_final.md), kept as an option for QKV, proj, patch embed and head conv.
-template <int NSPLIT, int BN>
+template <int NSPLIT>
 struct TcSmem {
     static constexpr int kParts = NSPLIT == 3 ? 2 : 1;  // NSPLIT: 1 = bf16, 2 = fp16 (single pass), 3 = bf16 hi + lo
-    static constexpr int kTileBBytes = BN * kTcBK * 2;   // 8 / 4 KB
-    static constexpr int kTileOBytes = kTcBM * BN * 2;   // 16 / 8 KB: one bf16 output tile, rows of 128 / 64 bytes
-    static constexpr int kTileCBytes = kTcBM * BN * 4;   // 32 / 16 KB: the fp32 tile as BN / 32 boxes of [128 rows][128 B]
+    static constexpr int kTileBBytes = kTcBN * kTcBK * 2;   // 8 KB
+    static constexpr int kTileOBytes = kTcBM * kTcBN * 2;   // 16 KB: one bf16 output tile, rows of 128 bytes
+    static constexpr int kTileCBytes = kTcBM * kTcBN * 4;   // 32 KB: the fp32 tile as two boxes of [128 rows][128 B]
     static constexpr int kStageBytes = kParts * (kTileABytes + kTileBBytes);
     // the ring is padded (bf16 mode) so that the chained GEMM's result tile fits behind the staged hidden tile
-    static constexpr int kRingMin = BN == kChainBN ? 2 * kTileOBytes + kTcBM * kMaxChainN * 4 : 4 * kTileOBytes;
+    static constexpr int kRingMin = 2 * kTileOBytes + kTcBM * kMaxChainN * 4;
     static constexpr int kPipeBytes = kTcStages * kStageBytes > kRingMin ? kTcStages * kStageBytes : kRingMin;
     // after the main loop the pipeline ring is dead and holds the staged output tiles
     static constexpr int kOffOhi = 0, kOffOlo = kTileOBytes, kOffLnHi = 2 * kTileOBytes, kOffLnLo = 3 * kTileOBytes;
@@ -62,7 +61,7 @@ struct TcSmem {
     // chained second GEMM (FC2 partial inside the FC1 kernel): its weight slice [N2 <= 192][64] per part lives where the fp32
     // tile would be, its fp32 result tile [128][N2] is staged in the dead ring behind the two hidden-tile parts
     static constexpr int kOffB2 = kPipeBytes, kB2PartBytes = kMaxChainN * 128, kOffP = 2 * kTileOBytes;
-    static constexpr int kTailBytes = (BN == kChainBN && kParts * kB2PartBytes > kTileCBytes) ? kParts * kB2PartBytes : kTileCBytes;
+    static constexpr int kTailBytes = kParts * kB2PartBytes > kTileCBytes ? kParts * kB2PartBytes : kTileCBytes;
     static constexpr int kTotal = kPipeBytes + kTailBytes + 1024;  // + alignment slack
     static_assert(4 * kTileOBytes <= kPipeBytes, "staging must fit in the dead pipeline ring");
 };
@@ -76,16 +75,17 @@ struct TcSmem {
 constexpr int kMaxLnCluster = 8;
 
 
-template <int NSPLIT, int BN>
+template <int NSPLIT>
 __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_constant__ TcMaps mp, const TcGemmArgs a) {
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t full_bar[kTcStages], empty_bar[kTcStages], accum_bar, resid_bar, b2_bar, accum2_bar, ln_bar;
     __shared__ uint32_t tmem_base_s;
     __shared__ float2 ln_loc[kTcColGroups][kTcBM];   // (sum, M2) of the CPT columns of thread (row, g)
-    __shared__ float2 ln_part[kMaxLnCluster][kTcBM];  // (sum, M2) of the BN columns of every CTA of the cluster, per row
+    __shared__ float2 ln_part[kMaxLnCluster][kTcBM];  // (sum, M2) of the 64 columns of every CTA of the cluster, per row
     __shared__ unsigned long long* trace_slot;
-    using SM = TcSmem<NSPLIT, BN>;
-    constexpr int CPT = BN / kTcColGroups;   // accumulator columns per thread: 16 / 8
+    using SM = TcSmem<NSPLIT>;
+    constexpr int BN = kTcBN;
+    constexpr int CPT = BN / kTcColGroups;   // 16 accumulator columns per thread
     constexpr int RB = BN * 2;               // bytes per row of a bf16 staging tile
     constexpr int kTileBBytes = SM::kTileBBytes, kTileOBytes = SM::kTileOBytes, kTileCBytes = SM::kTileCBytes;
     constexpr bool kLo = NSPLIT == 3, kF16 = NSPLIT == 2;
@@ -105,7 +105,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
     const int acc2_cols = (sliced && kLo) ? 2 * N2 : N2;              // sliced + bf16x3: hi*lo term in a second column half
     // dup_ln (spread form of a GEMM with fused LayerNorm): replica 0 stores the fp32 tile, replica 1 the LayerNorm hi tile, replica 2 the lo tile
     const bool do_ln = a.ln_g != nullptr && (!a.dup_ln || blockIdx.z > 0), do_c = a.c_on && (!a.dup_ln || blockIdx.z == 0);
-    const bool do_ln_any = a.ln_g != nullptr;
     const bool ln_hi = !a.dup_ln || blockIdx.z == 1, ln_lo = kLo && (!a.dup_ln || blockIdx.z == 2);
     // dup_hl (spread form of the QKV scatter): replica 0 stores the bf16 hi tiles, replica 1 the lo tiles
     const bool st_hi = !a.dup_hl || blockIdx.z == 0, st_lo = kLo && (!a.dup_hl || blockIdx.z == 1);
@@ -122,8 +121,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
     if (warp == 0 && elect_one_sync()) {  // (one thread; elect.sync lets the compiler issue the TMA instructions without election loops)
         tma_prefetch_desc(&mp.Ahi), tma_prefetch_desc(&mp.Bhi);
         if (kLo) tma_prefetch_desc(&mp.Alo), tma_prefetch_desc(&mp.Blo);
-        // multicast activation tiles: a stage is refilled in every CTA of the cluster at once, so it is released by all of them
-        for (int s = 0; s < kTcStages; ++s) mbar_init(&full_bar[s], 1), mbar_init(&empty_bar[s], a.mcast > 1 ? a.mcast : 1);
+        for (int s = 0; s < kTcStages; ++s) mbar_init(&full_bar[s], 1), mbar_init(&empty_bar[s], 1);
         mbar_init(&accum_bar, 1), mbar_init(&resid_bar, 1), mbar_init(&b2_bar, 1), mbar_init(&accum2_bar, 1), mbar_init(&ln_bar, 1);
         fence_barrier_init();
         // LayerNorm exchange: every CTA of the cluster (this one included) sends one float2 per row into ln_part of this CTA
@@ -158,9 +156,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
     __syncthreads();
     tcgen05_fence_after();
     const uint32_t tmem = tmem_base_s;
-    // cluster handshake ("this CTA is running, its barriers are initialised and armed"): peers may multicast activation tiles into
-    // its shared memory / push LayerNorm partials after the matching wait
-    const bool clustered = a.ln_g != nullptr || a.mcast > 1;
+    // cluster handshake ("this CTA is running, its barriers are initialised and armed"): peers may push LayerNorm partials into its
+    // shared memory after the matching wait
+    const bool clustered = a.ln_g != nullptr;
     if (clustered) cluster_arrive_release();
 
     pdl_wait();               // the activations (A, residual) are complete and visible from here on
@@ -186,14 +184,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
                     const int b = m0 / kNTx, y0 = (m0 % kNTx) / kMap;
                     tma_load_4d(st, &mp.Ahi, &full_bar[s], d0, tap % 3 - 1, y0 + tap / 3 - 1, b);
                     if (kLo) tma_load_4d(st + kTileABytes, &mp.Alo, &full_bar[s], d0, tap % 3 - 1, y0 + tap / 3 - 1, b);
-                } else if (a.mcast > 1) {
-                    // the a.mcast column-tile CTAs of this cluster share the activation tile: k-block kb is fetched once, by rank kb % mcast,
-                    // and multicast into everybody's stage (each CTA armed its own full barrier with the full stage byte count)
-                    if ((uint32_t)(kb % a.mcast) == cluster_ctarank()) {
-                        const uint16_t mask = (uint16_t)((1u << a.mcast) - 1);
-                        tma_load_2d_mcast(st, &mp.Ahi, &full_bar[s], (kb0 + kb) * kTcBK, m0, mask);
-                        if (kLo) tma_load_2d_mcast(st + kTileABytes, &mp.Alo, &full_bar[s], (kb0 + kb) * kTcBK, m0, mask);
-                    }
                 } else {
                     tma_load_2d(st, &mp.Ahi, &full_bar[s], (kb0 + kb) * kTcBK, m0);
                     if (kLo) tma_load_2d(st + kTileABytes, &mp.Alo, &full_bar[s], (kb0 + kb) * kTcBK, m0);
@@ -231,9 +221,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
                         umma_bf16(tmem, dAhi, dBhi, idesc, (kb | k) != 0);
                     }
                 }
-                // stage reusable once these MMAs have read it
-                if (a.mcast > 1) umma_commit_mcast(&empty_bar[s], (uint16_t)((1u << a.mcast) - 1));
-                else umma_commit(&empty_bar[s]);
+                umma_commit(&empty_bar[s]);  // stage reusable once these MMAs have read it
             }
             umma_commit(&accum_bar);
         }
@@ -249,7 +237,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
     int o_which = 0, o_h = 0, o_d = 0;
     if (a.o_mode == 2) {  // QKV: this CTA's 64 columns are one head of Q, K or V
         const int Dm = a.N / 3;
-        o_which = n0 / Dm, o_h = (n0 - o_which * Dm) / 64, o_d = (n0 - o_which * Dm) % 64;  // head_dim 64; BN = 32: half a head
+        o_which = n0 / Dm, o_h = (n0 - o_which * Dm) / 64, o_d = (n0 - o_which * Dm) % 64;  // head_dim 64
     }
     float bias_v[CPT];
     if (a.bias) {  // does not depend on the accumulator: fetch while the MMAs run
@@ -319,19 +307,17 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
         for (int q = 0; q < CPT / 4; ++q)
             *reinterpret_cast<float4*>(c_row + (((c_chunk0 + q) ^ sw) << 4)) = make_float4(v[4 * q], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
     }
-    // sliced chain with the 64-column tile: the hidden tile goes back into tensor memory as packed bf16 (thread (row, g) = K-step g: 8
-    // columns hi, 8 columns lo), so the chained UMMAs fetch only the weight slice from shared memory
-    const bool a_tmem = BN == kChainBN && sliced && kLo && a.o_mode == 3;
+    // sliced chain: the hidden tile goes back into tensor memory as packed bf16 (thread (row, g) = K-step g: 8 columns hi, 8 columns
+    // lo), so the chained UMMAs fetch only the weight slice from shared memory
+    const bool a_tmem = sliced && kLo && a.o_mode == 3;
     if (a_tmem) {
-        if constexpr (CPT == 16) {
-            uint32_t hi[8], lo[8];
+        uint32_t hi[8], lo[8];
 #pragma unroll
-            for (int j = 0; j < 16; j += 2) split2_bf16(v[j], v[j + 1], hi[j >> 1], lo[j >> 1]);
-            const uint32_t ta = tmem + ((uint32_t)((warp & 3) * 32) << 16) + kColA2 + g * 16;
-            tmem_st_32x8(ta, hi);
-            tmem_st_32x8(ta + 8, lo);
-            tmem_st_wait();
-        }
+        for (int j = 0; j < 16; j += 2) split2_bf16(v[j], v[j + 1], hi[j >> 1], lo[j >> 1]);
+        const uint32_t ta = tmem + ((uint32_t)((warp & 3) * 32) << 16) + kColA2 + g * 16;
+        tmem_st_32x8(ta, hi);
+        tmem_st_32x8(ta + 8, lo);
+        tmem_st_wait();
     } else if (a.o_mode) {  // (o_mode 3: staged only — the tile is the A operand of the chained GEMM)
         if (o_which < 2) {
             stage_split<CPT, kF16>(v, smem + SM::kOffOhi, smem + SM::kOffOlo, row, g, kLo);
@@ -394,7 +380,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
         }
     }
     if (tid == 0) tr.mark(7);
-    if (BN == kChainBN && a.chain_n) {
+    if (a.chain_n) {
         // ---- chained GEMM: P_j[128, N2] = hidden tile (just staged as a 128B-swizzled K-major A operand, bf16 hi / lo) x
         // W2[:, n0 .. n0 + 64)^T.  The hidden activations never travel to global memory; the N / 64 partial results P_j of one row
         // tile are summed in a fixed order by reduce_ln_kernel, which also applies bias, residual and the next LayerNorm.
@@ -407,7 +393,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
                 if (sliced && kLo) {  // H_hi x [W2_hi; W2_lo] as one UMMA of 2 N2 columns + H_lo x W2_hi (the epilogue adds the halves)
                     const uint32_t idesc2 = umma_idesc_bf16(kTcBM, N2), idesc2n = umma_idesc_bf16(kTcBM, 2 * N2);
 #pragma unroll
-                    for (int k = 0; k < kChainBN / 16; ++k) {
+                    for (int k = 0; k < BN / 16; ++k) {
                         const uint64_t dB = umma_desc_from_lo(b_lo + 2 * k);
                         umma_bf16_ta(tmem + kAcc1Cols, tmem + kColA2 + 16 * k, dB, idesc2n, k != 0);
                         umma_bf16_ta(tmem + kAcc1Cols, tmem + kColA2 + 16 * k + 8, dB, idesc2, 1);
@@ -415,7 +401,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
                 } else {
                     const uint32_t idesc2 = kF16 ? umma_idesc_f16(kTcBM, N2) : umma_idesc_bf16(kTcBM, N2);  // K = the 64 hidden columns of this CTA
 #pragma unroll
-                    for (int k = 0; k < kChainBN / 16; ++k) {
+                    for (int k = 0; k < BN / 16; ++k) {
                         const uint64_t dA = umma_desc_from_lo(a_lo + 2 * k), dB = umma_desc_from_lo(b_lo + 2 * k);
                         umma_bf16(tmem + kAcc1Cols, dA, dB, idesc2, k != 0);
                         if (kLo) {
@@ -491,9 +477,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
     __syncthreads();
     if (tid == 0) tr.mark(3);
     if (warp == 1) tmem_dealloc(tmem, tmem_cols);
-    // multicast without the LayerNorm exchange: peers still deliver stage-release arrivals to this CTA's barriers until their own main
-    // loops end, so nobody leaves before everybody's has (with the LayerNorm exchange every CTA has already waited for every peer's epilogue)
-    if (a.mcast > 1 && !do_ln_any) cluster_arrive_release(), cluster_wait_acquire();
 }
 
 // ---- host side ------------------------------------------------------------------------------------------------------
@@ -571,10 +554,6 @@ bool tc_resid_map(CUtensorMap* out, const float* base, uint64_t rows, uint64_t c
 
 // chained second GEMM of plan p: weights W2 [N2][K2] (K2 = N of the first GEMM), partial results P [N/64][batch][rows][N2] fp32
 bool tc_plan_chain(TcGemmPlan* p, const __nv_bfloat16* W2hi, const __nv_bfloat16* W2lo, int N2, float* P, uint64_t rows, uint64_t batch) {
-    if (p->bn != kChainBN) {
-        set_error("the chained GEMM needs the 64-column tile");
-        return false;
-    }
     if (N2 % 64 || N2 > kMaxChainN) {
         set_error("chained GEMM needs N2 %% 64 == 0 and N2 <= %d (N2=%d)", kMaxChainN, N2);
         return false;
@@ -583,20 +562,18 @@ bool tc_plan_chain(TcGemmPlan* p, const __nv_bfloat16* W2hi, const __nv_bfloat16
     const uint64_t dims[2] = {K2, (uint64_t)N2}, strides[1] = {K2 * 2};
     const uint32_t box[2] = {(uint32_t)kTcBK, 64};  // loaded as 64-row boxes (a CTA of the sliced form takes one of them)
     bool ok = tc_make_map(&p->maps.B2hi, W2hi, 2, dims, strides, box) && tc_make_map(&p->maps.B2lo, W2lo ? W2lo : W2hi, 2, dims, strides, box);
-    p->args.p = tc_out(P, 4, N2, rows, 1, batch, K2 / kChainBN);
+    p->args.p = tc_out(P, 4, N2, rows, 1, batch, K2 / kTcBN);
     p->args.chain_n = N2, p->args.o_mode = 3;
     return ok;
 }
 
 bool tc_plan_init(TcGemmPlan* p, const __nv_bfloat16* Ahi, const __nv_bfloat16* Alo, uint64_t a_rows, const __nv_bfloat16* Whi,
-                  const __nv_bfloat16* Wlo, int N, int K, int conv_feat, int conv_batch, int bn) {
+                  const __nv_bfloat16* Wlo, int N, int K, int conv_feat, int conv_batch) {
     memset(p, 0, sizeof(*p));
-    if ((bn != 32 && bn != 64) || N % bn || K % kTcBK || (conv_feat && conv_feat % kTcBK)) {
-        set_error("tcgen05 GEMM needs a 32- or 64-column tile, N %% tile == 0 and K %% 64 == 0 (N=%d K=%d tile=%d)", N, K, bn);
+    if (N % kTcBN || K % kTcBK || (conv_feat && conv_feat % kTcBK)) {
+        set_error("tcgen05 GEMM needs N %% 64 == 0 and K %% 64 == 0 (N=%d K=%d)", N, K);
         return false;
     }
-    p->bn = bn;
-    p->mcast_ok = getenv("VT_B200_MCAST") != nullptr;  // measured: no gain on one stream, -12 % with 16 streams (profiles/r1d_final.md)
     bool ok = true;
     if (conv_feat) {  // A = token grid [batch][16][16][feat]
         const uint64_t dims[4] = {(uint64_t)conv_feat, kMap, kMap, (uint64_t)conv_batch};
@@ -608,8 +585,8 @@ bool tc_plan_init(TcGemmPlan* p, const __nv_bfloat16* Ahi, const __nv_bfloat16* 
         ok &= tc_make_map_2d(&p->maps.Ahi, Ahi, a_rows, K, kTcBM);
         ok &= tc_make_map_2d(&p->maps.Alo, Alo ? Alo : Ahi, a_rows, K, kTcBM);
     }
-    ok &= tc_make_map_2d(&p->maps.Bhi, Whi, N, K, bn);
-    ok &= tc_make_map_2d(&p->maps.Blo, Wlo ? Wlo : Whi, N, K, bn);
+    ok &= tc_make_map_2d(&p->maps.Bhi, Whi, N, K, kTcBN);
+    ok &= tc_make_map_2d(&p->maps.Blo, Wlo ? Wlo : Whi, N, K, kTcBN);
     // unused output maps must still be valid descriptors (they are never dereferenced when their mode is off)
     p->maps.R = p->maps.B2hi = p->maps.B2lo = p->maps.Bhi;
     p->args.N = N, p->args.K = K, p->args.conv_feat = conv_feat;
@@ -618,20 +595,17 @@ bool tc_plan_init(TcGemmPlan* p, const __nv_bfloat16* Ahi, const __nv_bfloat16* 
 }
 
 cudaError_t tc_gemm_setup() {
-    cudaError_t e = cudaFuncSetAttribute(gemm_tc_kernel<1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<1, 64>::kTotal);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<3, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<3, 64>::kTotal);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<2, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<2, 64>::kTotal);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<1, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<1, 32>::kTotal);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<3, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<3, 32>::kTotal);
+    cudaError_t e = cudaFuncSetAttribute(gemm_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<1>::kTotal);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<3>::kTotal);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<2>::kTotal);
     return e;
 }
 
-cudaError_t tc_gemm_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, bool spread, bool mcast_ln) {
+cudaError_t tc_gemm_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, bool spread) {
     if (M <= 0) return cudaSuccess;
     TcGemmArgs a = p.args;
     a.M = M;
-    const int bn = p.bn;
-    dim3 grid(a.N / bn, (M + kTcBM - 1) / kTcBM, a.kb_per_split ? a.K / kTcBK / a.kb_per_split : 1);
+    dim3 grid(a.N / kTcBN, (M + kTcBM - 1) / kTcBM, a.kb_per_split ? a.K / kTcBK / a.kb_per_split : 1);
     a.chain_slices = 0, a.dup_hl = 0, a.dup_ln = 0;
     if (spread && !a.kb_per_split && nsplit == 3 && a.ln_g && a.c_on && !a.chain_n && !a.o_mode && grid.x * grid.y * 3 <= (unsigned)kSpreadCtas)
         a.dup_ln = 1, grid.z = 3;  // three replicas of every tile: fp32 tile / LayerNorm hi / LayerNorm lo
@@ -640,30 +614,12 @@ cudaError_t tc_gemm_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t 
         a.dup_hl = 1, grid.z = 2;  // two replicas of every tile, one stores the hi parts and one the lo parts (halves the per-CTA egress)
     // latency mode: replicate the FC1 tiles over idle SMs, each replica computes and stores one 64-column slice of the chained product
     if (spread && !a.kb_per_split && a.chain_n && a.chain_n % (3 * 64) == 0 && grid.x * grid.y * 3 <= (unsigned)kSpreadCtas) a.chain_slices = 3, grid.z = 3;
-    int cluster_x = 1;
-    if (a.ln_g) {
-        cluster_x = a.N / bn;
-        if (cluster_x > kMaxLnCluster) return cudaErrorInvalidValue;
-    } else if (p.mcast_ok) {  // column tiles of one row tile share the activation tile: clusters of 4 / 3 / 2 of them
-        for (int g : {4, 3, 2})
-            if ((a.N / bn) % g == 0) {
-                cluster_x = g;
-                break;
-            }
-    }
-    // multicast needs plain 2-D activation boxes; the ring is reused cluster-wide (empty barriers count every CTA of the cluster).
-    // mcast_ln (throughput mode): the LayerNorm cluster of proj / FC2 shares its activation tile — with many rows these GEMMs are bound
-    // by L2 -> SM traffic (FC2: 393 KB of activations + 196 KB of weights per 128 x 64 tile), which the multicast cuts by 45 %.
-    a.mcast = ((p.mcast_ok || (mcast_ln && a.ln_g)) && cluster_x > 1 && !a.conv_feat && !a.kb_per_split) ? cluster_x : 0;
-    if (!a.mcast && !a.ln_g) cluster_x = 1;
-    if (nsplit == 2 && bn != 64) return cudaErrorInvalidValue;  // the fp16 form exists for the 64-column tile only
-    if (bn == 64) {
-        if (nsplit == 2) return launch_ex(gemm_tc_kernel<2, 64>, grid, dim3(kTcThreads), TcSmem<2, 64>::kTotal, s, pdl, cluster_x, p.maps, a);
-        if (nsplit == 3) return launch_ex(gemm_tc_kernel<3, 64>, grid, dim3(kTcThreads), TcSmem<3, 64>::kTotal, s, pdl, cluster_x, p.maps, a);
-        return launch_ex(gemm_tc_kernel<1, 64>, grid, dim3(kTcThreads), TcSmem<1, 64>::kTotal, s, pdl, cluster_x, p.maps, a);
-    }
-    if (nsplit == 3) return launch_ex(gemm_tc_kernel<3, 32>, grid, dim3(kTcThreads), TcSmem<3, 32>::kTotal, s, pdl, cluster_x, p.maps, a);
-    return launch_ex(gemm_tc_kernel<1, 32>, grid, dim3(kTcThreads), TcSmem<1, 32>::kTotal, s, pdl, cluster_x, p.maps, a);
+    // fused LayerNorm: the N / 64 column tiles of a row tile form one cluster
+    const int cluster_x = a.ln_g ? a.N / kTcBN : 1;
+    if (cluster_x > kMaxLnCluster) return cudaErrorInvalidValue;
+    if (nsplit == 2) return launch_ex(gemm_tc_kernel<2>, grid, dim3(kTcThreads), TcSmem<2>::kTotal, s, pdl, cluster_x, p.maps, a);
+    if (nsplit == 3) return launch_ex(gemm_tc_kernel<3>, grid, dim3(kTcThreads), TcSmem<3>::kTotal, s, pdl, cluster_x, p.maps, a);
+    return launch_ex(gemm_tc_kernel<1>, grid, dim3(kTcThreads), TcSmem<1>::kTotal, s, pdl, cluster_x, p.maps, a);
 }
 
 // fp32 -> bf16 (hi, lo) split of a dense buffer
@@ -712,8 +668,7 @@ extern "C" vt_status vt_debug_gemm(int32_t device, int32_t M, int32_t N, int32_t
     VT_CUDA(launch_split_bf16(dA, Ahi, nsplit == 2 ? nullptr : Alo, na, 0)); VT_CUDA(launch_split_bf16(dW, Whi, nsplit == 2 ? nullptr : Wlo, nw, 0));
     TcGemmPlan plan;
     vt_status st = VT_OK;
-    const char* tile = getenv("VT_DBG_TILE");  // diagnostics knob: column-tile width 64 (default) or 32
-    if (!tc_plan_init(&plan, Ahi, Alo, M, Whi, Wlo, N, K, 0, 0, tile ? atoi(tile) : 64)) st = VT_ERR_CUDA;
+    if (!tc_plan_init(&plan, Ahi, Alo, M, Whi, Wlo, N, K, 0, 0)) st = VT_ERR_CUDA;
     if (st == VT_OK) {
         plan.args.bias = dB, plan.args.gelu = gelu, plan.args.err = dErr, plan.args.c_on = 1;
         // diagnostics knobs: VT_DBG_PERIOD = rows per target of the output addressing (M must be a multiple), VT_DBG_RESID = C += C0

@@ -1031,8 +1031,6 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
     r.status = VT_ERR_NOT_INIT, r.success = 0, r.score = 0.f, r.bbox[0] = r.bbox[1] = r.bbox[2] = r.bbox[3] = 0, r.best = 0;
     if (slot >= 0) r = res[slot];
     const bool pass = r.status == VT_OK && r.success && r.score > gate;
-    const int dbg_skip = draw_box >> 8;  // diagnostics (VT_B200_HUD_SKIP): 1 = no host pass, 2 = no device pass, 4 = no background dim
-    draw_box &= 0xff;
     if (draw_box && pass) {
         const int x = r.bbox[0], y = r.bbox[1], w = r.bbox[2], h = r.bbox[3];
         for (int p = 0; p < 2; ++p) {
@@ -1071,8 +1069,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
             }
             __syncthreads();
         }
-        if (bg_first && (dbg_skip & 4)) first = 1;
-        else if (bg_first) {  // ---- the background dim: word interior from registers (or the device frame), ragged edges bytewise
+        if (bg_first) {  // ---- the background dim: word interior from registers (or the device frame), ragged edges bytewise
             const unsigned factor = 255u - (unsigned)(uint8_t)s_cmd[0].a;
             const long long rows = bg.y1 - bg.y0;
             if (bg.x1 > bg.x0 && (size_t)bg.y1 * (size_t)W <= len) {
@@ -1124,7 +1121,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
         for (int p = 0; p < 2; ++p) {
             uint8_t* dst = p == 0 ? frame : host;
             if (!dst) break;
-            if ((p == 0 && ((dbg_skip & 2) || !do_dev)) || (p == 1 && ((dbg_skip & 1) || !do_host))) continue;
+            if ((p == 0 && !do_dev) || (p == 1 && !do_host)) continue;
             Surface s{dst, len, W, H, fmt};
             for (int i = first; i < n_hud; ++i) {
                 const OverlayCmdDev& c = s_cmd[i];

@@ -133,28 +133,11 @@ __device__ __forceinline__ uint32_t cluster_map_shared(uint32_t smem_addr, uint3
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(rank));
     return r;
 }
-__device__ __forceinline__ void st_shared_cluster_f2(uint32_t addr, float x, float y) {
-    asm volatile("st.shared::cluster.v2.f32 [%0], {%1, %2};" ::"r"(addr), "f"(x), "f"(y) : "memory");
-}
 // asynchronous store into a peer CTA's shared memory that signals the peer's mbarrier with the byte count (no cluster barrier needed:
 // the receiver waits for expect_tx bytes on its own mbarrier)
 __device__ __forceinline__ void st_async_cluster_f2(uint32_t remote_addr, float x, float y, uint32_t remote_mbar) {
     asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v2.f32 [%0], {%1, %2}, [%3];" ::"r"(remote_addr), "f"(x), "f"(y),
                  "r"(remote_mbar)
-                 : "memory");
-}
-__device__ __forceinline__ void st_async_cluster_f4(uint32_t remote_addr, float x, float y, float z, float w, uint32_t remote_mbar) {
-    asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.f32 [%0], {%1, %2, %3, %4}, [%5];" ::"r"(remote_addr), "f"(x), "f"(y),
-                 "f"(z), "f"(w), "r"(remote_mbar)
-                 : "memory");
-}
-__device__ __forceinline__ void st_shared_cluster_f4(uint32_t addr, float x, float y, float z, float w) {
-    asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(x), "f"(y), "f"(z), "f"(w) : "memory");
-}
-// bulk copy from this CTA's shared memory into a peer's (addresses of the peer: mapa), completion counted on the peer's mbarrier
-__device__ __forceinline__ void dsmem_bulk_copy(uint32_t remote_dst, uint32_t local_src, uint32_t bytes, uint32_t remote_mbar) {
-    asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(remote_dst), "r"(local_src),
-                 "r"(bytes), "r"(remote_mbar)
                  : "memory");
 }
 __device__ __forceinline__ void cluster_arrive_release() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
@@ -173,15 +156,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
     asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(smem_u32(smem_dst)),
                  "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
                  : "memory");
-}
-// One CTA of a cluster loads the box and the TMA unit delivers it — data and mbarrier complete_tx — to the same shared-memory offsets
-// of every CTA in cta_mask: the CTAs of a cluster that need the same activation tile fetch it from L2 once.
-__device__ __forceinline__ void tma_load_2d_mcast(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;" ::"r"(
-            smem_u32(smem_dst)),
-        "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(cta_mask)
-        : "memory");
 }
 __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2) {
     asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(smem_u32(smem_dst)),
@@ -280,13 +254,6 @@ __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.
 // Arrives on the mbarrier when all previously issued MMAs of this thread have completed (implies fence::before_thread_sync).
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// the same arrival delivered to the barrier at this shared-memory offset in every CTA of cta_mask (stages that a multicast load fills
-// in all CTAs of a cluster are released cluster-wide)
-__device__ __forceinline__ void umma_commit_mcast(uint64_t* bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-                 "h"(cta_mask)
-                 : "memory");
 }
 
 // TMEM -> registers: 32 lanes (this warp's quarter) x 32 consecutive fp32 columns; thread l gets lane 32*(warp%4)+l.

@@ -371,7 +371,6 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
         VT_TRY(tc_gemm_as_setup());
         VT_TRY(cudaDeviceGetAttribute(&t->sm_count, cudaDevAttrMultiProcessorCount, cfg->device));
         if (const char* e = getenv("VT_B200_AS_ROWS")) t->as_rows = atoi(e);
-        if (const char* e = getenv("VT_B200_TP_ROWS")) t->tp_rows = atoi(e);
         t->as_mlp = !getenv("VT_B200_NO_AS_MLP");
         t->fuse_ln = D / 64 <= 8 && !getenv("VT_B200_NO_FUSE_LN");
         t->pdl = !getenv("VT_B200_NO_PDL");
@@ -435,10 +434,6 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
         auto wlo = [&](const float* w) { return t->w_lo + (w - t->d_weights); };
         bool ok = true;
         const uint64_t rows = B * kNTok;
-        // Column-tile width of QKV / proj / patch / head.  128x32 tiles (VT_B200_TILE32=1: twice the CTAs, half the epilogue per CTA) were
-        // measured and bring nothing: the accumulator is ready at the same 2.05 us (the 96 KB A tile per CTA bounds it, not the UMMAs) and
-        // the 6-CTA LayerNorm cluster of proj is slower than the 3-CTA one (profiles/r1d_final.md).  FC1 needs the 64-column tile anyway.
-        const int bn_lat = getenv("VT_B200_TILE32") ? 32 : 64;
         // outputs of the GEMM epilogues (TcOut: dense [planes][targets][heads][rows][cols]) and the flat residual TMA source
         CUtensorMap mXres;
         ok &= tc_resid_map(&mXres, t->X, B * kNTok, D);
@@ -456,7 +451,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
             oQ[4] = tc_out_vt(t->vt_hi, kNTok, t->heads, Bi), oQ[5] = tc_out_vt(t->vt_lo, kNTok, t->heads, Bi);
         }
         // patch embed (search): A = patches [B*256, 768] -> X rows 64.. of every target, + pos_x
-        ok &= tc_plan_init(&t->plan_patch_x, t->px_hi, t->px_lo, B * kNTx, whi(t->patch_w), wlo(t->patch_w), (int)D, kPatchK, 0, 0, bn_lat);
+        ok &= tc_plan_init(&t->plan_patch_x, t->px_hi, t->px_lo, B * kNTx, whi(t->patch_w), wlo(t->patch_w), (int)D, kPatchK, 0, 0);
         {
             TcGemmArgs& a = t->plan_patch_x.args;
             a.bias = t->patch_b, a.pos = t->pos_x, a.pos_rows = kNTx;
@@ -480,7 +475,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
         for (int l = 0; l < t->depth && ok; ++l) {
             const BlockW& b = t->blk[l];
             vt_tracker::BlockPlans& p = t->plans[l];
-            ok &= tc_plan_init(&p.qkv, t->ln_hi, t->ln_lo, rows, whi(b.qkv_w), wlo(b.qkv_w), (int)(3 * D), (int)D, 0, 0, bn_lat);
+            ok &= tc_plan_init(&p.qkv, t->ln_hi, t->ln_lo, rows, whi(b.qkv_w), wlo(b.qkv_w), (int)(3 * D), (int)D, 0, 0);
             p.qkv.args.bias = b.qkv_b, p.qkv.args.period = kNTok;
             if (t->tc_attention) {
                 p.qkv.args.o_mode = 2;
@@ -488,8 +483,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
             } else {
                 p.qkv.args.c_on = 1, p.qkv.args.c = oQKV;
             }
-            ok &= tc_plan_init(&p.proj, t->att_hi, t->att_lo, rows, whi(b.proj_w), wlo(b.proj_w), (int)D, (int)D, 0, 0,
-                               D / bn_lat <= 8 ? bn_lat : 64);
+            ok &= tc_plan_init(&p.proj, t->att_hi, t->att_lo, rows, whi(b.proj_w), wlo(b.proj_w), (int)D, (int)D, 0, 0);
             p.proj.args.bias = b.proj_b, p.proj.args.period = kNTok, p.proj.args.residual = 1, p.proj.args.c_on = 1;
             p.proj.maps.R = mXres, p.proj.args.c = oX;
             if (t->fuse_ln) p.proj.args.ln_g = b.ln2_g, p.proj.args.ln_b = b.ln2_b, p.proj.args.ln_out[0] = oLn[0], p.proj.args.ln_out[1] = oLn[1];
@@ -514,7 +508,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
             }
         }
         // 3x3 head conv: A gathered by TMA from the [B,16,16,D] final-LN grid (zero fill = zero padding), weights [C][tap][D]
-        ok &= tc_plan_init(&t->plan_head, t->yf_hi, t->yf_lo, 0, whi(t->h1_w), wlo(t->h1_w), (int)C, (int)(9 * D), (int)D, (int)B, bn_lat);
+        ok &= tc_plan_init(&t->plan_head, t->yf_hi, t->yf_lo, 0, whi(t->h1_w), wlo(t->h1_w), (int)C, (int)(9 * D), (int)D, (int)B);
         t->plan_head.args.bias = t->h1_b, t->plan_head.args.relu = 1, t->plan_head.args.period = kNTx, t->plan_head.args.c_on = 1;
         t->plan_head.args.c = oH1;
         if (t->split_k) {  // one tap per slice -> fp32 partials [9][B][256][C]; bias, ReLU, 1x1 conv and decode in head_decode_kernel

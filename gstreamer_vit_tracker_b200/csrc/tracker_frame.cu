@@ -111,7 +111,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool recor
         // Many targets: the split-K forms of patch embed (4 K-slices) and head conv (one 3x3 tap per slice) are shaped for one target's
         // three row tiles; from 8 targets on they are 384 / 576 short CTAs (2.6 / 3.9 waves), so the slices are merged — 2 K-slices, 3 taps
         // per slice: a third of the partial planes, CTAs that run three times as many MMAs per prologue.
-        const bool merge_slices = t->split_k && n >= kUnchainTargets && !getenv("VT_B200_NO_MERGE_SLICES");
+        const bool merge_slices = t->split_k && n >= kUnchainTargets;
         int patch_np = 4;
         if (merge_slices) {
             TcGemmPlan pp = t->plan_patch_x;
@@ -134,7 +134,6 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool recor
             if (!fuse) VT_LAUNCH(launch_layernorm_split(t->X, D, b.ln1_g, b.ln1_b, t->ln_hi, LO(t->ln_lo), M, D, 1 << 30, 0, 0, s, pdl));
             // many rows (cfg4, stream groups): the A-stationary form — activation tile resident, epilogue of chunk i under the main loop of i + 1
             const bool as_form = t->as_rows > 0 && M >= t->as_rows;
-            const bool tp_mcast = t->tp_rows > 0 && M >= t->tp_rows;
             if (as_form && tc_gemm_as_supported(p.qkv))
                 VT_LAUNCH(tc_gemm_as_launch(p.qkv, M, ns, s, pdl, t->sm_count));
             else
@@ -156,7 +155,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool recor
                 r.ln_g = b.ln2_g, r.ln_b = b.ln2_b, r.ln_hi = t->ln_hi, r.ln_lo = LO(t->ln_lo), r.ln_rows = kNTok, r.ln_row_off = 0;
                 VT_LAUNCH(launch_reduce_ln(r, s, pdl));
             } else {
-                VT_LAUNCH(tc_gemm_launch(p.proj, M, ns, s, pdl && t->tc_attention, spread && !tp_mcast, tp_mcast));  // fused: + LN2
+                VT_LAUNCH(tc_gemm_launch(p.proj, M, ns, s, pdl && t->tc_attention, spread));  // fused: + LN2
             }
             if (!fuse) VT_LAUNCH(launch_layernorm_split(t->X, D, b.ln2_g, b.ln2_b, t->ln_hi, LO(t->ln_lo), M, D, 1 << 30, 0, 0, s, pdl));
             // Chained form (FC2 partial products inside the FC1 kernel, summed by reduce_ln): shortest critical path for a few targets.
@@ -168,7 +167,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool recor
             const bool chain = as_mlp || (t->chain_mlp && n < t->unchain_n);
             int planes = (int)(Hd / 64);
             if (as_mlp) {
-                VT_LAUNCH(tc_gemm_as_mlp_launch(p.fc1, M, s, pdl, t->sm_count, &planes, t->fuse_ln ? &p.fc2 : nullptr));
+                VT_LAUNCH(tc_gemm_as_mlp_launch(p.fc1, M, s, pdl, t->sm_count, &planes));
             } else if (chain) {
                 VT_LAUNCH(tc_gemm_launch(p.fc1, M, ns, s, pdl, spread));
             } else {
@@ -179,9 +178,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool recor
                 else
                     VT_LAUNCH(tc_gemm_launch(fc1, M, ns, s, pdl));
             }
-            if (chain && planes == 0) {
-                // (reduced inside the MLP kernel's clusters)
-            } else if (chain) {  // X += fc2_b + sum of the partials; LN1 of the next block / the final LN of the search rows
+            if (chain) {  // X += fc2_b + sum of the partials; LN1 of the next block / the final LN of the search rows
                 const bool last = l + 1 == t->depth;
                 ReduceLnArgs r{};
                 r.P = t->Pbuf, r.np = planes, r.p_stride = (int64_t)t->maxT * kNTok * D, r.bias = b.fc2_b, r.add = t->X, r.add_period = 0;
@@ -191,7 +188,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool recor
                 r.ln_rows = last ? kNTx : kNTok, r.ln_row_off = last ? -kNTz : 0;
                 VT_LAUNCH(launch_reduce_ln(r, s, pdl));
             } else {
-                VT_LAUNCH(tc_gemm_launch(p.fc2, M, ns, s, pdl, false, tp_mcast));  // fused: + LN1 of the next block / the final LN of the search rows
+                VT_LAUNCH(tc_gemm_launch(p.fc2, M, ns, s, pdl));  // fused: + LN1 of the next block / the final LN of the search rows
             }
             if (t->debug_capture)
                 VT_CUDA(cudaMemcpyAsync(t->d_dbg + (size_t)(l + 1) * t->maxT * kNTok * D, t->X, sizeof(float) * M * D, cudaMemcpyDeviceToDevice, s));
@@ -215,8 +212,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool recor
     if (t->cfg.box_overlay || t->hud_mode)  // box overlay and / or the frame's HUD list, pinned-frame mirror, ... and publishes the result block
         VT_LAUNCH(launch_box_overlay(t->frame_bytes, t->W, t->H, overlay_format(t->fmt), t->d_res, t->d_slots, n, t->cfg.overlay_gate, t->d_ctl,
                                      t->d_stamps + ST_OVL_END, s, t->pdl && !t->debug_capture, t->d_res, t->res_block_bytes,
-                                     t->cfg.box_overlay | (getenv("VT_B200_HUD_SKIP") ? atoi(getenv("VT_B200_HUD_SKIP")) << 8 : 0) |
-                                         ((t->hud_mode && !getenv("VT_B200_HUD_ONE_CTA")) ? 1 << 16 : 0)));
+                                     t->cfg.box_overlay | (t->hud_mode ? 1 << 16 : 0)));
     else  // results, stage stamps and the error flag -> the pinned host block of this frame's queue slot
         VT_LAUNCH(launch_publish(t->d_res, t->d_ctl, t->res_block_bytes, s, t->pdl && !t->debug_capture));
     return VT_OK;
@@ -518,10 +514,7 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
     if (!in_place) t->d_frame = t->d_frames[slot];  // the slot's own frame buffer: the other one may still be read by the frame in flight
     const bool lagging = t->q_count > 0;  // a frame is in flight: rect_mirror is one frame old, the windows are predictions
     UploadPlan plan;
-    // (the region a HUD list dims is read by the overlay kernel straight from the pinned host frame: it needs no upload of its own)
-    static const bool bg_from_host = getenv("VT_B200_HUD_BG_FROM_HOST") != nullptr;  // (measured slower: profiles/r2_final.md)
-    if (!in_place && !d_src)
-        plan_upload(t, len, host_frame != nullptr, lagging, (n_hud && !(bg_from_host && host_frame && t->hud_next_bg_leads)) ? t->hud_next_rmw : nullptr, plan);
+    if (!in_place && !d_src) plan_upload(t, len, host_frame != nullptr, lagging, n_hud ? t->hud_next_rmw : nullptr, plan);
     if (!in_place && !d_src && lagging) {
         // pipelined host frame: upload on the copy stream while the frame in flight computes; the main stream picks it up through an event
         vt_status st = do_upload(t, frame, len, plan, false, t->copy_stream);
@@ -765,9 +758,6 @@ vt_status tracker_set_hud(vt_tracker* t, const HudCmd* cmds, int n) {
             bytes += 1024;  // rect / crosshair / cursor / selection outlines
         }
     }
-    int n_bg = 0;
-    for (int i = 0; i < n; ++i) n_bg += cmds[i].cmd.kind == VT_OV_BACKGROUND;
-    t->hud_next_bg_leads = n_bg == 1 && cmds[0].cmd.kind == VT_OV_BACKGROUND && cmds[0].cond == VT_HUD_ALWAYS;
     t->hud_next_n = n, t->hud_next_bytes = bytes;
     memcpy(t->hud_next_rmw, rmw, sizeof(rmw));
     return VT_OK;

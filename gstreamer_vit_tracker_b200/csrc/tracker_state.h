@@ -115,8 +115,6 @@ struct vt_tracker {
     int hud_next_n = 0;
     int hud_next_rmw[4] = {0, 0, 0, 0};  // region the list reads before it writes (NV12 background dim): x0, y0, x1, y1; empty = none
     size_t hud_next_bytes = 0;            // pixels the list touches (device -> host accounting)
-    bool hud_next_bg_leads = false;       // the list's only background dim is its first, unconditional command: with a pinned frame the
-                                          // overlay kernel reads that region from the host frame and it needs no upload
     bool inflight_mirrored = false;
     float* d_maps = nullptr;
     OverlayCmdDev *d_cmds = nullptr, *h_cmds = nullptr;
@@ -149,8 +147,6 @@ struct vt_tracker {
     int sm_count = 148;         // SMs of the device (grid sizing of the throughput forms)
     int as_rows = 1024;         // rows (M) from which QKV / unchained FC1 run in the A-stationary throughput form (VT_B200_AS_ROWS; 0 = never)
     bool as_mlp = true;         // ... and the MLP as one chained A-stationary kernel + reduce (VT_B200_NO_AS_MLP disables: FC1 A-stationary, FC2 own GEMM)
-    int tp_rows = 0;            // rows from which proj / FC2 multicast their activation tile across the LayerNorm cluster (VT_B200_TP_ROWS; 0 =
-                                // never: measured without gain at 5120 rows, profiles/r2_final.md)
     bool counted = false;       // this handle is included in g_live_handles
     bool tc_attention = false;  // head_dim == 64
     TcAttentionPlan plan_att;

@@ -316,7 +316,6 @@ struct TcGemmArgs {
     int dup_ln;               // set at launch ("spread" form): replica 0 stores the fp32 tile, 1 the LayerNorm hi tile, 2 the lo tile
     int dup_hl;               // set at launch ("spread" form): replica z = 0 stores the bf16 hi tiles, z = 1 the lo tiles
     int chain_slices;         // set at launch ("spread" form): the chained product is computed in 3 column slices by 3 replicas of the tile
-    int mcast;                // set at launch: > 1 = the activation tile is multicast to this many column-tile CTAs of the cluster
     int kb_per_split;         // split-K: 64-wide k-blocks per blockIdx.z slice (0 = no split); the fp32 partial tile of slice z goes to
                               // plane z of c and bias / activations / residual must be off
     int chain_n;              // N2 of a chained second GEMM (0 = off): P[blockIdx.x] = tile x W2[:, n0..n0+64)^T -> p (plane blockIdx.x)
@@ -331,14 +330,12 @@ struct TcGemmArgs {
 struct TcMaps {               // kernel parameter block (__grid_constant__): the TMA load descriptors
     CUtensorMap Ahi, Alo, Bhi, Blo, R, B2hi, B2lo;
 };
-struct TcGemmPlan {
+struct TcGemmPlan {           // one GEMM on 128 x 64 output tiles
     TcMaps maps;
     TcGemmArgs args;
-    bool mcast_ok;            // TMA multicast of the activation tile across the column-tile CTAs of a cluster may be used
-    int bn;                   // column-tile width: 64 (throughput tile; required by the chained GEMM) or 32 (latency tile)
 };
 bool tc_plan_init(TcGemmPlan* p, const __nv_bfloat16* Ahi, const __nv_bfloat16* Alo, uint64_t a_rows, const __nv_bfloat16* Whi,
-                  const __nv_bfloat16* Wlo, int N, int K, int conv_feat, int conv_batch, int bn = 64);
+                  const __nv_bfloat16* Wlo, int N, int K, int conv_feat, int conv_batch);
 bool tc_plan_chain(TcGemmPlan* p, const __nv_bfloat16* W2hi, const __nv_bfloat16* W2lo, int N2, float* P, uint64_t rows, uint64_t batch);
 // dense outputs [planes][batch][heads][rows][cols] (elem_bytes 2 = bf16, 4 = fp32), V^T [batch][heads][64][tokens], and the flat fp32
 // residual source (TMA load)
@@ -349,7 +346,7 @@ cudaError_t tc_gemm_setup();
 // spread: latency mode — tiles are replicated over idle SMs so that each replica stores a share of the epilogue output (only when the
 // whole grid still fits in one wave of kSpreadCtas CTAs)
 constexpr int kSpreadCtas = 132;
-cudaError_t tc_gemm_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, bool spread = false, bool mcast_ln = false);
+cudaError_t tc_gemm_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, bool spread = false);
 // A-stationary throughput form (gemm_as.cu) of a plain 64-column-tile plan with K <= 192 whose epilogue is a bf16 (hi, lo) tile store or
 // the QKV scatter: one CTA per (128-row tile, range of 64-column chunks), the activation tile resident in shared memory, two TMEM
 // accumulators (main loop of chunk i + 1 under the epilogue of chunk i).  Bit-identical to tc_gemm_launch on the same plan.
@@ -360,9 +357,7 @@ cudaError_t tc_gemm_as_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream
 // tensor memory as the A operand of the chained product, which accumulates over all hidden chunks of the CTA; *planes partial planes
 // (CTAs per row tile) are written to the chain output for reduce_ln_kernel
 bool tc_gemm_as_mlp_supported(const TcGemmPlan& p, int nsplit);
-// fc2 (optional): with it, and N2 / 64 CTAs per row tile, the partials are reduced inside a cluster (bias, residual, LayerNorm fused):
-// *planes == 0 on return and no reduce_ln_kernel launch is needed
-cudaError_t tc_gemm_as_mlp_launch(const TcGemmPlan& p, int M, cudaStream_t s, bool pdl, int sm_count, int* planes, const TcGemmPlan* fc2 = nullptr);
+cudaError_t tc_gemm_as_mlp_launch(const TcGemmPlan& p, int M, cudaStream_t s, bool pdl, int sm_count, int* planes);
 struct TcAttentionPlan {      // kernel parameter block (__grid_constant__)
     CUtensorMap mQhi, mQlo, mKhi, mKlo, mVhi, mVlo;
     CUtensorMap mQ64hi, mQ64lo;      // Q in boxes of 64 rows (VT_ATT_CHAIN_Q64)
