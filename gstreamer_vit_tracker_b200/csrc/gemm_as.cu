@@ -494,12 +494,11 @@ bool tc_gemm_as_supported(const TcGemmPlan& p) {
            !a.ln_g && !a.c_on && !a.residual && !a.pos && !a.relu && (a.o_mode == 1 || a.o_mode == 2) && (a.o_mode != 2 || (a.N / 3) % 64 == 0);
 }
 
-// as many CTAs per row tile as fit in one wave, chunks dealt out evenly (the makespan is the largest share); returns CTAs per row tile
-int tc_gemm_as_split(int M, int n_chunks, int sm_count, int* per_cta) {
+// as many CTAs per row tile as fit in one wave (or `forced` > 0 of them), chunks dealt out evenly (the makespan is the largest share);
+// returns CTAs per row tile
+int tc_gemm_as_split(int M, int n_chunks, int sm_count, int forced, int* per_cta) {
     const int row_tiles = (M + kTcBM - 1) / kTcBM;
-    int smax = sm_count / row_tiles;
-    const int forced = getenv("VT_B200_AS_SPLIT") ? atoi(getenv("VT_B200_AS_SPLIT")) : 0;  // diagnostics / tests: CTAs per row tile
-    if (forced > 0) smax = forced;
+    int smax = forced > 0 ? forced : sm_count / row_tiles;
     if (smax < 1) smax = 1;
     if (smax > n_chunks) smax = n_chunks;
     *per_cta = (n_chunks + smax - 1) / smax;
@@ -512,25 +511,25 @@ bool tc_gemm_as_mlp_supported(const TcGemmPlan& p, int nsplit) {
     return nsplit == 3 && a.K % kTcBK == 0 && a.K / kTcBK <= kAsMaxKb && a.N % kAsChunk == 0 && !a.conv_feat && !a.kb_per_split &&
            a.chain_n > 0 && a.chain_n % 64 == 0 && a.chain_n <= kMaxAsChainN && !a.ln_g && !a.c_on && !a.residual && !a.pos && !a.relu && a.o_mode == 3;
 }
-cudaError_t tc_gemm_as_mlp_launch(const TcGemmPlan& p, int M, cudaStream_t s, bool pdl, int sm_count, int* planes) {
+cudaError_t tc_gemm_as_mlp_launch(const TcGemmPlan& p, int M, cudaStream_t s, bool pdl, int sm_count, int forced_split, int* planes) {
     if (!tc_gemm_as_mlp_supported(p, 3) || M <= 0) return cudaErrorInvalidValue;
     TcGemmArgs a = p.args;
     a.M = M;
     a.chain_slices = 0, a.dup_hl = 0, a.dup_ln = 0;
     int per_cta = 1;
-    *planes = tc_gemm_as_split(M, a.N / kAsChunk, sm_count, &per_cta);
+    *planes = tc_gemm_as_split(M, a.N / kAsChunk, sm_count, forced_split, &per_cta);
     const dim3 grid(*planes, (M + kTcBM - 1) / kTcBM, 1);
     return launch_ex(gemm_as_mlp_kernel, grid, dim3(kAsThreads), kMlpSmemTotal, s, pdl, 1, p.maps, a, per_cta);
 }
 
-cudaError_t tc_gemm_as_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, int sm_count) {
+cudaError_t tc_gemm_as_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, int sm_count, int forced_split) {
     if (M <= 0) return cudaSuccess;
     if (!tc_gemm_as_supported(p)) return cudaErrorInvalidValue;
     TcGemmArgs a = p.args;
     a.M = M;
     a.chain_slices = 0, a.dup_hl = 0, a.dup_ln = 0;
     int per_cta = 1;
-    dim3 grid(tc_gemm_as_split(M, a.N / kAsChunk, sm_count, &per_cta), (M + kTcBM - 1) / kTcBM, 1);
+    dim3 grid(tc_gemm_as_split(M, a.N / kAsChunk, sm_count, forced_split, &per_cta), (M + kTcBM - 1) / kTcBM, 1);
     if (nsplit == 3) return launch_ex(gemm_as_kernel<3>, grid, dim3(kAsThreads), AsSmem<3>::kTotal, s, pdl, 1, p.maps, a, per_cta);
     if (nsplit == 2) return launch_ex(gemm_as_kernel<2>, grid, dim3(kAsThreads), AsSmem<2>::kTotal, s, pdl, 1, p.maps, a, per_cta);
     return launch_ex(gemm_as_kernel<1>, grid, dim3(kAsThreads), AsSmem<1>::kTotal, s, pdl, 1, p.maps, a, per_cta);

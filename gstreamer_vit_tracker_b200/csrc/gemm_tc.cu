@@ -671,19 +671,7 @@ extern "C" vt_status vt_debug_gemm(int32_t device, int32_t M, int32_t N, int32_t
     if (!tc_plan_init(&plan, Ahi, Alo, M, Whi, Wlo, N, K, 0, 0)) st = VT_ERR_CUDA;
     if (st == VT_OK) {
         plan.args.bias = dB, plan.args.gelu = gelu, plan.args.err = dErr, plan.args.c_on = 1;
-        // diagnostics knobs: VT_DBG_PERIOD = rows per target of the output addressing (M must be a multiple), VT_DBG_RESID = C += C0
-        const char* per = getenv("VT_DBG_PERIOD");
-        const int period = per ? atoi(per) : 0;
-        if (period > 0 && M % period == 0) {
-            plan.args.period = period;
-            plan.args.c = tc_out(dC, 4, N, period, 1, M / period, 1);
-        } else {
-            plan.args.c = tc_out(dC, 4, N, M, 1, 1, 1);
-        }
-        if (getenv("VT_DBG_RESID")) {
-            plan.args.residual = 1;
-            if (!tc_resid_map(&plan.maps.R, dC, M, N)) st = VT_ERR_CUDA;
-        }
+        plan.args.c = tc_out(dC, 4, N, M, 1, 1, 1);
     }
     if (st == VT_OK) {
         cudaError_t e = tc_gemm_launch(plan, M, nsplit, 0, false);

@@ -496,8 +496,7 @@ vt_status vt_probe_frame(vt_context* c, uint8_t* frame, size_t len, const char* 
     const uint64_t num = c->frame_num++;
     const size_t need = c->cfg.format == VT_FMT_NV12 ? (size_t)c->frame_width * c->frame_height * 3 / 2
                                                      : (size_t)c->frame_width * c->frame_height * (c->cfg.format == VT_FMT_RGB24 ? 3 : 1);
-    static const bool two_step = getenv("VT_PROBE_TWO_STEP") != nullptr;  // diagnostics: force the pageable-frame path
-    const vt_status st = (!two_step && len >= need && vt::frame_is_pinned(frame)) ? probe_one_sync(c, frame, len, hud_override, nv12)
+    const vt_status st = (len >= need && vt::frame_is_pinned(frame)) ? probe_one_sync(c, frame, len, hud_override, nv12)
                                                                                 : probe_two_step(c, frame, len, hud_override, nv12);
     if (st != VT_OK) return st;
     probe_log(c, nv12, num);

@@ -209,8 +209,7 @@ cudaError_t launch_nv12_to_rgb(const uint8_t* d_nv12, size_t stride_in, uint8_t*
     const bool aligned = (width % 16 == 0) && (height % 2 == 0) && (height / 2 <= 65535) && (n_frames <= 65535) && (stride_in % 16 == 0) &&
                          (stride_out % 16 == 0) &&
                          ((reinterpret_cast<uintptr_t>(d_nv12) | reinterpret_cast<uintptr_t>(d_rgb)) % 16 == 0);
-    static const bool no_wide = getenv("VT_B200_CVT_NARROW") != nullptr;  // diagnostics: the 8-byte / two-row form
-    if (aligned && height % 4 == 0 && !no_wide) {
+    if (aligned && height % 4 == 0) {
         const int segs = (width + 511) / 512;
         const int wpb = segs < kCvt4Warps ? segs : kCvt4Warps;
         const dim3 grid((segs + wpb - 1) / wpb, height / 4, n_frames);  // one warp per 512-px x 4-row item
@@ -387,8 +386,7 @@ cudaError_t launch_yuy2_to_rgb(const uint8_t* d_yuy2, size_t stride_in, uint8_t*
     const bool aligned = (width % 8 == 0) && (height <= 65535) && (n_frames <= 65535) && (stride_in % 16 == 0) && (stride_out % 16 == 0) &&
                          ((size_t)width * 3 % 16 == 0) &&
                          ((reinterpret_cast<uintptr_t>(d_yuy2) | reinterpret_cast<uintptr_t>(d_rgb)) % 16 == 0);
-    static const bool no_wide = getenv("VT_B200_CVT_NARROW") != nullptr;  // diagnostics: the one-row / 16-byte form
-    if (aligned && width % 16 == 0 && !no_wide) {
+    if (aligned && width % 16 == 0) {
         const long long items = (long long)width * height / 16;  // flat 16-pixel items, 64 per warp
         const dim3 grid((unsigned)((items + 64 * kCvt4Warps - 1) / (64 * kCvt4Warps)), 1, n_frames);
         yuy2_to_rgb_vec2_kernel<<<grid, kCvt4Warps * 32, 0, s>>>(d_yuy2, stride_in, d_rgb, stride_out, width, height);
@@ -672,8 +670,7 @@ __global__ void __launch_bounds__(kRszThreads) resize_rgb_tile_kernel(const uint
 cudaError_t launch_resize_rgb_tab(const uint8_t* d_src, size_t stride_in, int sw, int sh, uint8_t* d_dst, size_t stride_out, int dw, int dh,
                                   int n_frames, const int4* d_xt, const int4* d_yt, cudaStream_t s, int max_src_rows) {
     if (sw <= 0 || sh <= 0 || dw <= 0 || dh <= 0 || n_frames <= 0) return cudaSuccess;
-    static const bool no_tile = getenv("VT_B200_RSZ_ROWWISE") != nullptr;  // diagnostics: the per-row form
-    if (max_src_rows > 0 && max_src_rows <= kRszSrcRows && !no_tile) {
+    if (max_src_rows > 0 && max_src_rows <= kRszSrcRows) {
         const dim3 grid((dw + kRszTilePx - 1) / kRszTilePx, (dh + kRszTileRows - 1) / kRszTileRows, n_frames);
         resize_rgb_tile_kernel<<<grid, kRszThreads, 0, s>>>(d_src, stride_in, sw, sh, d_dst, stride_out, dw, dh, d_xt, d_yt);
         return cudaGetLastError();

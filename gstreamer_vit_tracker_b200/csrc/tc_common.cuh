@@ -68,7 +68,7 @@ struct TraceRec {
         slot = shared_slot;
         if (threadIdx.x == 0) {
             unsigned long long* rec = nullptr;
-            // id bit 8 (VT_B200_TRACE_LASTX): trace the CTA with the LAST blockIdx.x instead of the first (e.g. a V^T tile of the QKV GEMM)
+            // id bit 8: trace the CTA with the LAST blockIdx.x instead of the first (e.g. a V^T tile of the QKV GEMM)
             const unsigned bx = (id & 0x100) ? gridDim.x - 1 : 0u;
             if (trace && blockIdx.x == bx && blockIdx.y == 0 && blockIdx.z == 0) {
                 const unsigned long long i = atomicAdd(trace, 1ull);

@@ -333,7 +333,7 @@ static vt_status overlay_impl(vt_tracker* t, uint8_t* frame, size_t len, const v
     vt_status st = build_cmds(t, cmds, n, spans);
     if (st != VT_OK) return st;
     if (n == 0) return VT_OK;
-    VT_CUDA(cudaEventRecord(t->ev[EV_DEC], t->stream));
+    VT_CUDA(cudaEventRecord(t->ev_ovl[0], t->stream));
     if (upload) {
         const size_t nb = std::min(len, t->frame_bytes);
         t->d_frame_is_last_host_frame = false;
@@ -351,7 +351,7 @@ static vt_status overlay_impl(vt_tracker* t, uint8_t* frame, size_t len, const v
         return VT_ERR_CUDA;
     }
     ++t->kernel_launches;
-    VT_CUDA(cudaEventRecord(t->ev[EV_OVL], t->stream));
+    VT_CUDA(cudaEventRecord(t->ev_ovl[1], t->stream));
     merge_spans(spans);
     bool staged = false;
     st = download_rows(t, frame, len, spans, &staged);
@@ -359,7 +359,7 @@ static vt_status overlay_impl(vt_tracker* t, uint8_t* frame, size_t len, const v
     VT_CUDA(cudaStreamSynchronize(t->stream));
     if (staged) unstage_rows(t, frame, len, spans);
     float ms = 0.f;
-    if (cudaEventElapsedTime(&ms, t->ev[EV_DEC], t->ev[EV_OVL]) == cudaSuccess) t->last[4] = ms;
+    if (cudaEventElapsedTime(&ms, t->ev_ovl[0], t->ev_ovl[1]) == cudaSuccess) t->last[4] = ms;
     else cudaGetLastError();
     return VT_OK;
 }

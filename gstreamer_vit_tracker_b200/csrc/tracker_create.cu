@@ -135,6 +135,31 @@ void bind_slot(vt_tracker* t, int slot) {
     t->h_tc_err = reinterpret_cast<int*>(t->h_stamps + ST_COUNT);
 }
 
+static void read_switches(vt_tracker* t) {
+    Switches& s = t->sw;
+    s.spread = !getenv("VT_B200_NO_SPREAD");
+    s.att_chain = !getenv("VT_B200_NO_ATT_CHAIN");
+    s.att_q64 = !getenv("VT_B200_ATT_Q128");
+    if (const char* e = getenv("VT_B200_UNCHAIN_N")) s.unchain_n = atoi(e);
+    if (const char* e = getenv("VT_B200_AS_ROWS")) s.as_rows = atoi(e);
+    s.as_mlp = !getenv("VT_B200_NO_AS_MLP");
+    if (const char* e = getenv("VT_B200_AS_SPLIT")) s.as_split = atoi(e);
+    s.trace = getenv("VT_B200_TRACE") != nullptr;
+    s.hostprof = getenv("VT_B200_HOSTPROF") != nullptr;
+    if (const char* e = getenv("VT_B200_WINDOW_SHRINK")) s.win_shrink = atoi(e) & ~1;
+}
+
+ShapeForms shape_forms(const vt_tracker* t) {
+    ShapeForms f;
+    const int D = t->D, Hd = t->hidden, C = t->head_ch;
+    f.fuse_ln = D / 64 <= 8;  // a LayerNorm cluster holds at most 8 column tiles
+    f.chain_mlp = f.fuse_ln && D <= 192;
+    f.tc_attention = D / t->heads == 64;
+    f.att_chain = f.chain_mlp && f.tc_attention && Hd / 64 >= t->heads;
+    f.split_k = f.chain_mlp && Hd / 64 >= 4 && (C == 64 || C == 128);
+    return f;
+}
+
 }  // namespace vt
 
 using namespace vt;
@@ -179,7 +204,7 @@ void vt_free_pinned(void* p) {
 
 void vt_tracker_destroy(vt_tracker* t) {
     if (!t) return;
-    if (t->hostprof && t->hp_n) {
+    if (t->sw.hostprof && t->hp_n) {
         const double n = (double)t->hp_n;
         fprintf(stderr, "[vt hostprof] frames %llu  submit: upload %.1f  graph launch %.1f  result copy+event %.1f | wait: stream sync %.1f  "
                         "err check+results %.1f  overlay rows %.1f  timing %.1f (us / frame)\n",
@@ -189,7 +214,7 @@ void vt_tracker_destroy(vt_tracker* t) {
     if (t->counted) registry_add(t->cfg.device, -1);
     if (t->stream) cudaStreamSynchronize(t->stream);
     for (auto& kv : t->graphs) cudaGraphExecDestroy(kv.second);
-    for (auto& e : t->ev)
+    for (auto& e : t->ev_ovl)
         if (e) cudaEventDestroy(e);
     if (t->d_rsz_taps) cudaFree(t->d_rsz_taps);
     if (t->d_fmt_in) cudaFree(t->d_fmt_in);
@@ -277,8 +302,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
                                                    : (size_t)t->W * t->H * 3;
     t->threshold = cfg->score_threshold > 0.f ? cfg->score_threshold : 0.20f;
     t->debug_capture = cfg->debug_capture;
-    t->hostprof = getenv("VT_B200_HOSTPROF") != nullptr;
-    if (const char* e = getenv("VT_B200_WINDOW_SHRINK")) t->win_shrink = atoi(e) & ~1;
+    read_switches(t);
     auto fail = [&](vt_status st) {
         vt_tracker_destroy(t);
         return st;
@@ -294,7 +318,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
         }                                                                                                        \
     } while (0)
     VT_TRY(cudaStreamCreateWithFlags(&t->stream, cudaStreamNonBlocking));
-    for (auto& e : t->ev) VT_TRY(cudaEventCreate(&e));
+    for (auto& e : t->ev_ovl) VT_TRY(cudaEventCreate(&e));
     const size_t D = t->D, Hd = t->hidden, C = t->head_ch, B = t->maxT;
     // A.4 normalisation LUT: (v/255 - mean_c)/std_c in double, rounded once to fp32 (channels in memory order)
     {
@@ -370,18 +394,10 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
         VT_TRY(tc_gemm_setup());
         VT_TRY(tc_gemm_as_setup());
         VT_TRY(cudaDeviceGetAttribute(&t->sm_count, cudaDevAttrMultiProcessorCount, cfg->device));
-        if (const char* e = getenv("VT_B200_AS_ROWS")) t->as_rows = atoi(e);
-        t->as_mlp = !getenv("VT_B200_NO_AS_MLP");
-        t->fuse_ln = D / 64 <= 8 && !getenv("VT_B200_NO_FUSE_LN");
-        t->pdl = !getenv("VT_B200_NO_PDL");
-        t->spread_ok = !getenv("VT_B200_NO_SPREAD");
-        if (const char* e = getenv("VT_B200_UNCHAIN_N")) t->unchain_n = atoi(e);
-        t->chain_mlp = t->fuse_ln && D <= 192 && !getenv("VT_B200_NO_CHAIN");
-        if (t->chain_mlp) VT_TRY(cudaMalloc(&t->Pbuf, sizeof(float) * (Hd / 64) * B * kNTok * D));
-        t->att_chain_ok = t->chain_mlp && t->fuse_ln && D / t->heads == 64 && (int)(Hd / 64) >= t->heads && t->nsplit && !getenv("VT_B200_NO_ATT_CHAIN");
-        t->att_q64 = !getenv("VT_B200_ATT_Q128");
-        t->split_k = t->chain_mlp && Hd / 64 >= 4 && (C == 64 || C == 128) && !getenv("VT_B200_NO_SPLITK");
-        if (t->split_k) {
+        const ShapeForms sf = shape_forms(t);
+        const size_t p_planes = std::max({sf.chain_mlp ? Hd / 64 : 0, sf.att_chain ? (size_t)t->heads : 0, sf.split_k ? (size_t)4 : 0});
+        if (p_planes) VT_TRY(cudaMalloc(&t->Pbuf, sizeof(float) * p_planes * B * kNTok * D));
+        if (sf.split_k) {
             VT_TRY(cudaMalloc(&t->Phead, sizeof(float) * 9 * B * kNTx * C));
             VT_TRY(cudaMalloc(&t->d_cand, sizeof(float) * B * 16 * 8));
             VT_TRY(cudaMalloc(&t->d_counters, sizeof(unsigned) * B));
@@ -420,8 +436,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
         VT_TRY(balloc(&t->att_hi, &t->att_lo, B * kNTok * D));
         VT_TRY(balloc(&t->hid_hi, &t->hid_lo, B * kNTok * Hd));
         VT_TRY(balloc(&t->yf_hi, &t->yf_lo, B * kNTx * D));
-        t->tc_attention = (D / t->heads == 64);
-        if (t->tc_attention) {
+        if (sf.tc_attention) {
             const size_t nq = B * t->heads * kNTok * 64;
             VT_TRY(balloc(&t->q_hi, &t->q_lo, nq));
             VT_TRY(balloc(&t->k_hi, &t->k_lo, nq));
@@ -445,7 +460,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
         const TcOut oH1 = tc_out(t->H1, 4, (int)C, kNTx, 1, Bi, 1), oZ = tc_out(t->Zemb, 4, Di, kNTz, 1, Bi, 1);
         const TcOut oQKV = tc_out(t->QKV, 4, 3 * Di, kNTok, 1, Bi, 1);
         TcOut oQ[6] = {};
-        if (t->tc_attention) {
+        if (sf.tc_attention) {
             oQ[0] = tc_out(t->q_hi, 2, 64, kNTok, t->heads, Bi, 1), oQ[1] = tc_out(t->q_lo, 2, 64, kNTok, t->heads, Bi, 1);
             oQ[2] = tc_out(t->k_hi, 2, 64, kNTok, t->heads, Bi, 1), oQ[3] = tc_out(t->k_lo, 2, 64, kNTok, t->heads, Bi, 1);
             oQ[4] = tc_out_vt(t->vt_hi, kNTok, t->heads, Bi), oQ[5] = tc_out_vt(t->vt_lo, kNTok, t->heads, Bi);
@@ -456,10 +471,10 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
             TcGemmArgs& a = t->plan_patch_x.args;
             a.bias = t->patch_b, a.pos = t->pos_x, a.pos_rows = kNTx;
             a.period = kNTx, a.c_on = 1, a.c_row_off = kNTz, a.c = oX;
-            if (t->split_k) {  // 4 x K = 192 slices -> fp32 partials [4][B][256][D]; bias, pos, LN1 happen in reduce_ln_kernel
+            if (sf.split_k) {  // 4 x K = 192 slices -> fp32 partials [4][B][256][D]; bias, pos, LN1 happen in reduce_ln_kernel
                 a.bias = nullptr, a.pos = nullptr, a.c_row_off = 0, a.kb_per_split = kPatchK / 64 / 4;
                 a.c = tc_out(t->Pbuf, 4, Di, kNTx, 1, Bi, 4);
-            } else if (t->fuse_ln) {  // LN1 of block 0 for the search rows, straight into the first QKV GEMM's A operand
+            } else if (sf.fuse_ln) {  // LN1 of block 0 for the search rows, straight into the first QKV GEMM's A operand
                 a.ln_g = t->blk[0].ln1_g, a.ln_b = t->blk[0].ln1_b, a.ln_row_off = kNTz;
                 a.ln_out[0] = oLn[0], a.ln_out[1] = oLn[1];
             }
@@ -477,7 +492,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
             vt_tracker::BlockPlans& p = t->plans[l];
             ok &= tc_plan_init(&p.qkv, t->ln_hi, t->ln_lo, rows, whi(b.qkv_w), wlo(b.qkv_w), (int)(3 * D), (int)D, 0, 0);
             p.qkv.args.bias = b.qkv_b, p.qkv.args.period = kNTok;
-            if (t->tc_attention) {
+            if (sf.tc_attention) {
                 p.qkv.args.o_mode = 2;
                 for (int i = 0; i < 6; ++i) p.qkv.args.o[i] = oQ[i];
             } else {
@@ -486,19 +501,19 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
             ok &= tc_plan_init(&p.proj, t->att_hi, t->att_lo, rows, whi(b.proj_w), wlo(b.proj_w), (int)D, (int)D, 0, 0);
             p.proj.args.bias = b.proj_b, p.proj.args.period = kNTok, p.proj.args.residual = 1, p.proj.args.c_on = 1;
             p.proj.maps.R = mXres, p.proj.args.c = oX;
-            if (t->fuse_ln) p.proj.args.ln_g = b.ln2_g, p.proj.args.ln_b = b.ln2_b, p.proj.args.ln_out[0] = oLn[0], p.proj.args.ln_out[1] = oLn[1];
+            if (sf.fuse_ln) p.proj.args.ln_g = b.ln2_g, p.proj.args.ln_b = b.ln2_b, p.proj.args.ln_out[0] = oLn[0], p.proj.args.ln_out[1] = oLn[1];
             ok &= tc_plan_init(&p.fc1, t->ln_hi, t->ln_lo, rows, whi(b.fc1_w), wlo(b.fc1_w), (int)Hd, (int)D, 0, 0);
             p.fc1.args.bias = b.fc1_b, p.fc1.args.gelu = 1, p.fc1.args.period = kNTok, p.fc1.args.o_mode = 1;
             p.fc1.args.o[0] = oHid[0], p.fc1.args.o[1] = oHid[1];
-            if (t->chain_mlp) ok &= tc_plan_chain(&p.fc1, whi(b.fc2_w), wlo(b.fc2_w), (int)D, t->Pbuf, kNTok, B);
-            if (t->att_chain_ok) {
+            if (sf.chain_mlp) ok &= tc_plan_chain(&p.fc1, whi(b.fc2_w), wlo(b.fc2_w), (int)D, t->Pbuf, kNTok, B);
+            if (sf.att_chain) {
                 p.att = t->plan_att;
                 ok &= tc_attention_plan_chain(&p.att, whi(b.proj_w), wlo(b.proj_w), t->Pbuf, (int64_t)B * kNTok * D);
             }
             ok &= tc_plan_init(&p.fc2, t->hid_hi, t->hid_lo, rows, whi(b.fc2_w), wlo(b.fc2_w), (int)D, (int)Hd, 0, 0);
             p.fc2.args.bias = b.fc2_b, p.fc2.args.period = kNTok, p.fc2.args.residual = 1, p.fc2.args.c_on = 1;
             p.fc2.maps.R = mXres, p.fc2.args.c = oX;
-            if (t->fuse_ln) {
+            if (sf.fuse_ln) {
                 TcGemmArgs& a = p.fc2.args;
                 if (l + 1 < t->depth) {
                     a.ln_g = t->blk[l + 1].ln1_g, a.ln_b = t->blk[l + 1].ln1_b, a.ln_out[0] = oLn[0], a.ln_out[1] = oLn[1];
@@ -511,14 +526,14 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
         ok &= tc_plan_init(&t->plan_head, t->yf_hi, t->yf_lo, 0, whi(t->h1_w), wlo(t->h1_w), (int)C, (int)(9 * D), (int)D, (int)B);
         t->plan_head.args.bias = t->h1_b, t->plan_head.args.relu = 1, t->plan_head.args.period = kNTx, t->plan_head.args.c_on = 1;
         t->plan_head.args.c = oH1;
-        if (t->split_k) {  // one tap per slice -> fp32 partials [9][B][256][C]; bias, ReLU, 1x1 conv and decode in head_decode_kernel
+        if (sf.split_k) {  // one tap per slice -> fp32 partials [9][B][256][C]; bias, ReLU, 1x1 conv and decode in head_decode_kernel
             t->plan_head.args.bias = nullptr, t->plan_head.args.relu = 0, t->plan_head.args.kb_per_split = (int)(D / 64);
             t->plan_head.args.c = tc_out(t->Phead, 4, (int)C, kNTx, 1, Bi, 9);
         }
         if (!ok) return fail(VT_ERR_CUDA);
         for (TcGemmPlan* p : {&t->plan_patch_x, &t->plan_patch_z, &t->plan_head}) p->args.err = t->d_tc_err;
         for (auto& p : t->plans) p.qkv.args.err = p.proj.args.err = p.fc1.args.err = p.fc2.args.err = t->d_tc_err;
-        if (getenv("VT_B200_TRACE")) {
+        if (t->sw.trace) {
             VT_TRY(cudaMalloc(&t->d_trace, tc::kTraceWords * 8));
             VT_TRY(cudaMemset(t->d_trace, 0, tc::kTraceWords * 8));
             t->plan_patch_x.args.trace = t->plan_head.args.trace = t->d_trace;
@@ -526,7 +541,6 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
             for (auto& p : t->plans) {
                 p.qkv.args.trace = p.proj.args.trace = p.fc1.args.trace = p.fc2.args.trace = t->d_trace;
                 p.qkv.args.trace_id = 2, p.proj.args.trace_id = 3, p.fc1.args.trace_id = 4, p.fc2.args.trace_id = 5;
-                if (getenv("VT_B200_TRACE_LASTX")) p.qkv.args.trace_id |= 0x100, p.fc1.args.trace_id |= 0x100;  // trace the last column tile
             }
         }
     }

@@ -44,10 +44,70 @@ static GemmArgs gemm_args(const float* A, int64_t lda, const float* W, const flo
     return g;
 }
 
+// The kernel forms of one forward, a function of the handle, n and spread (latency mode: few live handles on the GPU, run_forward):
+// the graph key (n, frame_valid, spread) determines them.
+constexpr int kAttSimt = -1;  // ForwardForms::att: launch_attention (else a VT_ATT_* form of tc_attention_launch)
+struct ForwardForms {
+    int patch_slices = 0;      // patch-embed K-slices summed by reduce_ln: 0 (unsplit), 4, or 2 (merged, from kUnchainTargets targets)
+    int head_planes = 0;       // head-conv partial planes summed by head_decode: 9, 3 (merged), or 0 (unsplit: H1 + decode_kernel)
+    bool ln_split = false;     // LayerNorm as separate layernorm_split kernels
+    bool qkv_as = false;       // QKV in the A-stationary form
+    int att = kAttSimt;
+    bool proj_in_att = false;  // proj folded into the attention kernel + reduce_ln, instead of the proj GEMM
+    bool mlp_chain = false;    // FC2 partial products inside the FC1 kernel + reduce_ln (else FC1 stores the hidden tile, FC2 GEMM)
+    bool mlp_as = false;       // FC1 (with the chained product: gemm_as_mlp_kernel) in the A-stationary form
+    bool spread = false;       // latency-mode replicas of the one-tile GEMMs (tc_gemm_launch picks them from the plan)
+    bool pdl = true;           // programmatic dependent launch along the chain (off under debug_capture)
+};
+
+// FC1 without the chained product: it stores the hidden tile for the FC2 GEMM
+static TcGemmPlan unchained_fc1(TcGemmPlan p) {
+    p.args.chain_n = 0, p.args.o_mode = 1;
+    return p;
+}
+
+static ForwardForms forward_forms(const vt_tracker* t, int n, bool spread) {
+    ForwardForms f;
+    f.pdl = !t->debug_capture;
+    if (!t->nsplit) return f;
+    const ShapeForms sf = shape_forms(t);
+    const vt_tracker::BlockPlans& p = t->plans[0];  // every block's plans have the same shape
+    const int M = n * kNTok, att_w = t->heads * (t->D / kAttChainW);
+    f.spread = spread;
+    // Many targets: the split-K forms of patch embed (4 K-slices) and head conv (one 3x3 tap per slice) are shaped for one target's
+    // three row tiles; from 8 targets on they are 384 / 576 short CTAs (2.6 / 3.9 waves), so the slices are merged — 2 K-slices, 3 taps
+    // per slice: a third of the partial planes, CTAs that run three times as many MMAs per prologue.
+    f.patch_slices = sf.split_k ? (n >= kUnchainTargets ? 2 : 4) : 0;
+    f.head_planes = sf.split_k ? (n >= kUnchainTargets ? 3 : 9) : 0;
+    f.ln_split = !sf.fuse_ln;
+    // many rows (cfg4, stream groups): the A-stationary form — activation tile resident, epilogue of chunk i under the main loop of i + 1
+    const bool as_form = t->sw.as_rows > 0 && M >= t->sw.as_rows;
+    f.qkv_as = as_form && tc_gemm_as_supported(p.qkv);
+    // Latency mode: the proj GEMM is folded into the attention kernel (per-head partial products, D / kAttChainW replicas per tile) and
+    // reduce_ln adds the heads + bias + residual and applies LN2 — one kernel and one dependency edge less per block.  64-row query
+    // tiles (5 per sequence) when that grid still fits one wave: each CTA computes half the exponentials.
+    if (sf.tc_attention) {
+        const bool chain = spread && sf.att_chain && t->sw.att_chain;
+        f.att = chain && t->sw.att_q64 && n * 5 * att_w <= kSpreadCtas ? VT_ATT_CHAIN_Q64
+                : chain && n * 3 * att_w <= kSpreadCtas            ? VT_ATT_CHAIN
+                : spread                                            ? VT_ATT_DUP
+                                                                    : VT_ATT_PLAIN;
+    }
+    f.proj_in_att = f.att == VT_ATT_CHAIN || f.att == VT_ATT_CHAIN_Q64;
+    // Chained form (FC2 partial products inside the FC1 kernel, summed by reduce_ln): shortest critical path for a few targets.
+    // From kUnchainTargets targets on the 12 fp32 partial planes per row tile cost more than the hidden round trip
+    // (cfg4, 16 targets: ViT stage 905 -> 819 us unchained), so FC1 writes the hidden tile and FC2 runs as its own GEMM.
+    // ... except in the A-stationary form, where a CTA accumulates the chained product over all of its hidden chunks (3 planes
+    // per row tile at 5120 rows, and no hidden round trip at all)
+    const bool as_mlp = as_form && sf.chain_mlp && t->sw.as_mlp && tc_gemm_as_mlp_supported(p.fc1, t->nsplit);
+    f.mlp_chain = as_mlp || (sf.chain_mlp && n < t->sw.unchain_n);
+    f.mlp_as = f.mlp_chain ? as_mlp : as_form && tc_gemm_as_supported(unchained_fc1(p.fc1));
+    return f;
+}
+
 // Enqueues crop -> ViT -> decode (-> box overlay) for the n active targets on t->stream.
-static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool record_events, bool capturing, bool spread) {
+static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const ForwardForms& f) {
     const int D = t->D, Hd = t->hidden, C = t->head_ch;
-    (void)record_events, (void)capturing;  // stage times come from device stamps (ST_*), not from event nodes
     cudaStream_t s = t->stream;
     FrameDesc fd{t->d_frame, t->W, t->H, t->fmt, t->frame_valid, t->d_ctl, t->cfg.pad_plus1};
     auto LO = [&](__nv_bfloat16* p) { return t->f16 ? nullptr : p; };  // fp16 mode: "hi only" (see vt_internal.h: operand_bits)
@@ -55,13 +115,12 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool recor
                                       LO(t->px_lo), s, t->d_stamps + ST_PRE));
     {
         dim3 grid((kNTz * D + 255) / 256, n);
-        const bool f = t->fuse_ln;
-        VT_LAUNCH(launch_ex(gather_template_kernel, grid, dim3(256), 0, s, t->pdl && !t->debug_capture, 1, t->X, (const float*)t->Zemb,
-                            (const int32_t*)t->d_slots, D, f ? (uint32_t*)t->ln_hi : nullptr, (uint32_t*)LO(t->ln_lo), (const uint32_t*)t->zln_hi,
-                            (const uint32_t*)t->zln_lo, t->d_stamps + ST_VIT));
+        const bool ln = t->nsplit && !f.ln_split;  // LN1 of block 0 for the template rows (the search rows get it after the patch embed)
+        VT_LAUNCH(launch_ex(gather_template_kernel, grid, dim3(256), 0, s, f.pdl, 1, t->X, (const float*)t->Zemb, (const int32_t*)t->d_slots, D,
+                            ln ? (uint32_t*)t->ln_hi : nullptr, (uint32_t*)LO(t->ln_lo), (const uint32_t*)t->zln_hi, (const uint32_t*)t->zln_lo,
+                            t->d_stamps + ST_VIT));
     }
     const int M = n * kNTok;
-    int head_np = 9;
     if (t->nsplit == 0) {
         // ---------------- fp32 CUDA-core path ----------------
         {
@@ -107,78 +166,48 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool recor
     } else {
         // ---------------- tensor-core path: tcgen05 GEMMs fed by TMA, bf16 (x3 split) operands, fp32 TMEM accumulators ----------------
         const int ns = t->nsplit;
-        const bool pdl = t->pdl && !t->debug_capture, fuse = t->fuse_ln;
-        // Many targets: the split-K forms of patch embed (4 K-slices) and head conv (one 3x3 tap per slice) are shaped for one target's
-        // three row tiles; from 8 targets on they are 384 / 576 short CTAs (2.6 / 3.9 waves), so the slices are merged — 2 K-slices, 3 taps
-        // per slice: a third of the partial planes, CTAs that run three times as many MMAs per prologue.
-        const bool merge_slices = t->split_k && n >= kUnchainTargets;
-        int patch_np = 4;
-        if (merge_slices) {
-            TcGemmPlan pp = t->plan_patch_x;
-            pp.args.kb_per_split = kPatchK / 64 / 2, patch_np = 2;
-            VT_LAUNCH(tc_gemm_launch(pp, n * kNTx, ns, s, pdl));
-        } else {
-            VT_LAUNCH(tc_gemm_launch(t->plan_patch_x, n * kNTx, ns, s, pdl));  // fused: + LN1 of block 0 for the search rows
-        }
-        if (t->split_k) {  // X[64.., :] = pos_x + patch_b + sum of the K-slices; LN1 of block 0
+        TcGemmPlan pp = t->plan_patch_x;
+        if (f.patch_slices) pp.args.kb_per_split = kPatchK / 64 / f.patch_slices;
+        VT_LAUNCH(tc_gemm_launch(pp, n * kNTx, ns, s, f.pdl));  // unsplit: + LN1 of block 0 for the search rows (fused)
+        if (f.patch_slices) {  // X[64.., :] = pos_x + patch_b + sum of the K-slices; LN1 of block 0
             ReduceLnArgs r{};
-            r.P = t->Pbuf, r.np = patch_np, r.p_stride = (int64_t)t->maxT * kNTx * D, r.bias = t->patch_b, r.add = t->pos_x, r.add_period = kNTx;
+            r.P = t->Pbuf, r.np = f.patch_slices, r.p_stride = (int64_t)t->maxT * kNTx * D, r.bias = t->patch_b, r.add = t->pos_x, r.add_period = kNTx;
             r.X = t->X, r.M = n * kNTx, r.D = D, r.period = kNTx, r.x_rows = kNTok, r.x_row_off = kNTz;
             r.ln_g = t->blk[0].ln1_g, r.ln_b = t->blk[0].ln1_b, r.ln_hi = t->ln_hi, r.ln_lo = LO(t->ln_lo), r.ln_rows = kNTok, r.ln_row_off = kNTz;
-            VT_LAUNCH(launch_reduce_ln(r, s, pdl));
+            VT_LAUNCH(launch_reduce_ln(r, s, f.pdl));
         }
         if (t->debug_capture) VT_CUDA(cudaMemcpyAsync(t->d_dbg, t->X, sizeof(float) * M * D, cudaMemcpyDeviceToDevice, s));
         for (int l = 0; l < t->depth; ++l) {
             const BlockW& b = t->blk[l];
             const vt_tracker::BlockPlans& p = t->plans[l];
-            if (!fuse) VT_LAUNCH(launch_layernorm_split(t->X, D, b.ln1_g, b.ln1_b, t->ln_hi, LO(t->ln_lo), M, D, 1 << 30, 0, 0, s, pdl));
-            // many rows (cfg4, stream groups): the A-stationary form — activation tile resident, epilogue of chunk i under the main loop of i + 1
-            const bool as_form = t->as_rows > 0 && M >= t->as_rows;
-            if (as_form && tc_gemm_as_supported(p.qkv))
-                VT_LAUNCH(tc_gemm_as_launch(p.qkv, M, ns, s, pdl, t->sm_count));
+            if (f.ln_split) VT_LAUNCH(launch_layernorm_split(t->X, D, b.ln1_g, b.ln1_b, t->ln_hi, LO(t->ln_lo), M, D, 1 << 30, 0, 0, s, f.pdl));
+            if (f.qkv_as)
+                VT_LAUNCH(tc_gemm_as_launch(p.qkv, M, ns, s, f.pdl, t->sm_count, t->sw.as_split));
             else
-                VT_LAUNCH(tc_gemm_launch(p.qkv, M, ns, s, pdl, spread));
-            // Latency mode: the proj GEMM is folded into the attention kernel (per-head partial products, D / kAttChainW replicas per
-            // tile) and reduce_ln adds the heads + bias + residual and applies LN2 — one kernel and one dependency edge less per block.
-            // 64-row query tiles (5 per sequence) when that grid still fits one wave: each CTA computes half the exponentials.
-            const bool att_q64 = spread && t->att_chain_ok && t->att_q64 && n * t->heads * 5 * (D / kAttChainW) <= kSpreadCtas;
-            const bool att_chain = att_q64 || (spread && t->att_chain_ok && n * t->heads * 3 * (D / kAttChainW) <= kSpreadCtas);
-            if (t->tc_attention)
-                VT_LAUNCH(tc_attention_launch(att_chain ? p.att : t->plan_att, n, t->heads, ns, t->d_tc_err, s, pdl, t->d_trace,
-                                              att_q64 ? VT_ATT_CHAIN_Q64 : att_chain ? VT_ATT_CHAIN : (spread ? VT_ATT_DUP : VT_ATT_PLAIN)));
-            else
+                VT_LAUNCH(tc_gemm_launch(p.qkv, M, ns, s, f.pdl, f.spread));
+            if (f.att == kAttSimt)
                 VT_LAUNCH(launch_attention(t->QKV, nullptr, t->att_hi, LO(t->att_lo), n, D, t->heads, s));
-            if (att_chain) {
+            else
+                VT_LAUNCH(tc_attention_launch(f.proj_in_att ? p.att : t->plan_att, n, t->heads, ns, t->d_tc_err, s, f.pdl, t->d_trace, f.att));
+            if (f.proj_in_att) {
                 ReduceLnArgs r{};
                 r.P = t->Pbuf, r.np = t->heads, r.p_stride = (int64_t)t->maxT * kNTok * D, r.bias = b.proj_b, r.add = t->X, r.add_period = 0;
                 r.X = t->X, r.M = M, r.D = D, r.period = kNTok, r.x_rows = kNTok, r.x_row_off = 0;
                 r.ln_g = b.ln2_g, r.ln_b = b.ln2_b, r.ln_hi = t->ln_hi, r.ln_lo = LO(t->ln_lo), r.ln_rows = kNTok, r.ln_row_off = 0;
-                VT_LAUNCH(launch_reduce_ln(r, s, pdl));
-            } else {
-                VT_LAUNCH(tc_gemm_launch(p.proj, M, ns, s, pdl && t->tc_attention, spread));  // fused: + LN2
+                VT_LAUNCH(launch_reduce_ln(r, s, f.pdl));
+            } else {  // fused: + LN2
+                VT_LAUNCH(tc_gemm_launch(p.proj, M, ns, s, f.pdl && f.att != kAttSimt, f.spread));
             }
-            if (!fuse) VT_LAUNCH(launch_layernorm_split(t->X, D, b.ln2_g, b.ln2_b, t->ln_hi, LO(t->ln_lo), M, D, 1 << 30, 0, 0, s, pdl));
-            // Chained form (FC2 partial products inside the FC1 kernel, summed by reduce_ln): shortest critical path for a few targets.
-            // From kUnchainTargets targets on the 12 fp32 partial planes per row tile cost more than the hidden round trip
-            // (cfg4, 16 targets: ViT stage 905 -> 819 us unchained), so FC1 writes the hidden tile and FC2 runs as its own GEMM.
-            // ... except in the A-stationary form, where a CTA accumulates the chained product over all of its hidden chunks (3 planes
-            // per row tile at 5120 rows, and no hidden round trip at all)
-            const bool as_mlp = as_form && t->chain_mlp && t->as_mlp && tc_gemm_as_mlp_supported(p.fc1, ns);
-            const bool chain = as_mlp || (t->chain_mlp && n < t->unchain_n);
-            int planes = (int)(Hd / 64);
-            if (as_mlp) {
-                VT_LAUNCH(tc_gemm_as_mlp_launch(p.fc1, M, s, pdl, t->sm_count, &planes));
-            } else if (chain) {
-                VT_LAUNCH(tc_gemm_launch(p.fc1, M, ns, s, pdl, spread));
-            } else {
-                TcGemmPlan fc1 = p.fc1;
-                fc1.args.chain_n = 0, fc1.args.o_mode = 1;
-                if (as_form && tc_gemm_as_supported(fc1))
-                    VT_LAUNCH(tc_gemm_as_launch(fc1, M, ns, s, pdl, t->sm_count));
-                else
-                    VT_LAUNCH(tc_gemm_launch(fc1, M, ns, s, pdl));
-            }
-            if (chain) {  // X += fc2_b + sum of the partials; LN1 of the next block / the final LN of the search rows
+            if (f.ln_split) VT_LAUNCH(launch_layernorm_split(t->X, D, b.ln2_g, b.ln2_b, t->ln_hi, LO(t->ln_lo), M, D, 1 << 30, 0, 0, s, f.pdl));
+            int planes = Hd / 64;
+            const TcGemmPlan fc1 = f.mlp_chain ? p.fc1 : unchained_fc1(p.fc1);
+            if (f.mlp_as && f.mlp_chain)
+                VT_LAUNCH(tc_gemm_as_mlp_launch(fc1, M, s, f.pdl, t->sm_count, t->sw.as_split, &planes));
+            else if (f.mlp_as)
+                VT_LAUNCH(tc_gemm_as_launch(fc1, M, ns, s, f.pdl, t->sm_count, t->sw.as_split));
+            else
+                VT_LAUNCH(tc_gemm_launch(fc1, M, ns, s, f.pdl, f.spread && f.mlp_chain));
+            if (f.mlp_chain) {  // X += fc2_b + sum of the partials; LN1 of the next block / the final LN of the search rows
                 const bool last = l + 1 == t->depth;
                 ReduceLnArgs r{};
                 r.P = t->Pbuf, r.np = planes, r.p_stride = (int64_t)t->maxT * kNTok * D, r.bias = b.fc2_b, r.add = t->X, r.add_period = 0;
@@ -186,35 +215,30 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, bool recor
                 r.ln_g = last ? t->lnf_g : t->blk[l + 1].ln1_g, r.ln_b = last ? t->lnf_b : t->blk[l + 1].ln1_b;
                 r.ln_hi = last ? t->yf_hi : t->ln_hi, r.ln_lo = LO(last ? t->yf_lo : t->ln_lo);
                 r.ln_rows = last ? kNTx : kNTok, r.ln_row_off = last ? -kNTz : 0;
-                VT_LAUNCH(launch_reduce_ln(r, s, pdl));
+                VT_LAUNCH(launch_reduce_ln(r, s, f.pdl));
             } else {
-                VT_LAUNCH(tc_gemm_launch(p.fc2, M, ns, s, pdl));  // fused: + LN1 of the next block / the final LN of the search rows
+                VT_LAUNCH(tc_gemm_launch(p.fc2, M, ns, s, f.pdl));  // fused: + LN1 of the next block / the final LN of the search rows
             }
             if (t->debug_capture)
                 VT_CUDA(cudaMemcpyAsync(t->d_dbg + (size_t)(l + 1) * t->maxT * kNTok * D, t->X, sizeof(float) * M * D, cudaMemcpyDeviceToDevice, s));
         }
-        if (!fuse) VT_LAUNCH(launch_layernorm_split(t->X, D, t->lnf_g, t->lnf_b, t->yf_hi, LO(t->yf_lo), n * kNTx, D, kNTx, kNTok, kNTz, s, pdl));
-        if (merge_slices) {
-            TcGemmPlan ph = t->plan_head;
-            ph.args.kb_per_split = 3 * (D / 64), head_np = 3;
-            VT_LAUNCH(tc_gemm_launch(ph, n * kNTx, ns, s, pdl));
-        } else {
-            VT_LAUNCH(tc_gemm_launch(t->plan_head, n * kNTx, ns, s, pdl));
-        }
+        if (f.ln_split) VT_LAUNCH(launch_layernorm_split(t->X, D, t->lnf_g, t->lnf_b, t->yf_hi, LO(t->yf_lo), n * kNTx, D, kNTx, kNTok, kNTz, s, f.pdl));
+        TcGemmPlan ph = t->plan_head;
+        if (f.head_planes) ph.args.kb_per_split = 9 * (D / 64) / f.head_planes;  // 3x3 taps per slice
+        VT_LAUNCH(tc_gemm_launch(ph, n * kNTx, ns, s, f.pdl));
     }
-    if (t->nsplit && t->split_k)
-        VT_LAUNCH(launch_head_decode(t->Phead, head_np, (int64_t)t->maxT * kNTx * C, C, t->h1_b, t->h2_w, t->h2_b, t->d_hann, t->d_state, t->d_slots, n,
-                                     t->threshold, t->d_res, t->d_maps, t->d_cand, t->d_counters, t->d_stamps, s, t->pdl && !t->debug_capture,
-                                     t->cfg.decode_window, t->d_tc_err));
+    if (f.head_planes)
+        VT_LAUNCH(launch_head_decode(t->Phead, f.head_planes, (int64_t)t->maxT * kNTx * C, C, t->h1_b, t->h2_w, t->h2_b, t->d_hann, t->d_state, t->d_slots,
+                                     n, t->threshold, t->d_res, t->d_maps, t->d_cand, t->d_counters, t->d_stamps, s, f.pdl, t->cfg.decode_window,
+                                     t->d_tc_err));
     else
         VT_LAUNCH(launch_decode(t->H1, C, t->h2_w, t->h2_b, t->d_hann, t->d_state, t->d_slots, n, t->threshold, t->d_res, t->d_maps, t->d_stamps, s,
                                 t->cfg.decode_window));
     if (t->cfg.box_overlay || t->hud_mode)  // box overlay and / or the frame's HUD list, pinned-frame mirror, ... and publishes the result block
         VT_LAUNCH(launch_box_overlay(t->frame_bytes, t->W, t->H, overlay_format(t->fmt), t->d_res, t->d_slots, n, t->cfg.overlay_gate, t->d_ctl,
-                                     t->d_stamps + ST_OVL_END, s, t->pdl && !t->debug_capture, t->d_res, t->res_block_bytes,
-                                     t->cfg.box_overlay | (t->hud_mode ? 1 << 16 : 0)));
+                                     t->d_stamps + ST_OVL_END, s, f.pdl, t->d_res, t->res_block_bytes, t->cfg.box_overlay | (t->hud_mode ? 1 << 16 : 0)));
     else  // results, stage stamps and the error flag -> the pinned host block of this frame's queue slot
-        VT_LAUNCH(launch_publish(t->d_res, t->d_ctl, t->res_block_bytes, s, t->pdl && !t->debug_capture));
+        VT_LAUNCH(launch_publish(t->d_res, t->d_ctl, t->res_block_bytes, s, f.pdl));
     return VT_OK;
 }
 
@@ -223,9 +247,10 @@ static vt_status run_forward(vt_tracker* t) {
     if (n == 0) return VT_OK;
     int launches = 0;
     const int dev = t->cfg.device;
-    const bool spread = t->spread_ok && dev >= 0 && dev < kMaxDevices && registry_total(dev) <= kSpreadMaxHandles;
+    const bool spread = t->sw.spread && dev >= 0 && dev < kMaxDevices && registry_total(dev) <= kSpreadMaxHandles;
+    const ForwardForms f = forward_forms(t, n, spread);
     if (!t->cfg.use_cuda_graph || t->debug_capture) {
-        vt_status st = enqueue_forward(t, n, launches, true, false, spread);
+        vt_status st = enqueue_forward(t, n, launches, f);
         t->kernel_launches += launches;
         t->kernels_per_frame = launches;
         return st;
@@ -235,7 +260,7 @@ static vt_status run_forward(vt_tracker* t) {
     if (it == t->graphs.end()) {
         cudaGraph_t graph = nullptr;
         VT_CUDA(cudaStreamBeginCapture(t->stream, cudaStreamCaptureModeThreadLocal));
-        vt_status st = enqueue_forward(t, n, launches, true, true, spread);
+        vt_status st = enqueue_forward(t, n, launches, f);
         cudaError_t e = cudaStreamEndCapture(t->stream, &graph);
         if (st != VT_OK) {
             if (graph) cudaGraphDestroy(graph);
@@ -305,8 +330,8 @@ static void plan_upload(vt_tracker* t, size_t len, bool pinned_host, bool laggin
             w[0] = w[1] = w[2] = w[3] = 0;  // the window misses the frame: the crop kernel flags it; nothing to read
             continue;
         }
-        if (t->win_shrink > 0 && w[2] - w[0] > 4 * t->win_shrink && w[3] - w[1] > 4 * t->win_shrink)
-            w[0] += t->win_shrink, w[1] += t->win_shrink, w[2] -= t->win_shrink, w[3] -= t->win_shrink;
+        const int sh = t->sw.win_shrink;  // diagnostics: windows too small on purpose exercise the crop kernel's pinned-frame fall-back
+        if (sh > 0 && w[2] - w[0] > 4 * sh && w[3] - w[1] > 4 * sh) w[0] += sh, w[1] += sh, w[2] -= sh, w[3] -= sh;
         bytes += (size_t)(w[2] - w[0]) * (w[3] - w[1]) * bpp2 / 2;
     }
     if (rmw && rmw[2] > rmw[0] && rmw[3] > rmw[1] && format_is_luma(t->fmt)) {
@@ -362,12 +387,6 @@ static vt_status do_upload(vt_tracker* t, const uint8_t* frame, size_t len, cons
         VT_CUDA(cudaMemcpyAsync(t->d_frame, t->h_stage, n, cudaMemcpyHostToDevice, stream));
     }
     return VT_OK;
-}
-
-// whole-frame upload (init, and the callers outside the per-frame path)
-vt_status upload_frame(vt_tracker* t, const uint8_t* frame, size_t len, bool allow_window, bool device_src, cudaStream_t stream) {
-    (void)allow_window;
-    return do_upload(t, frame, len, UploadPlan(), device_src, stream);
 }
 
 static void fill_results(vt_tracker* t, vt_result* results) {
@@ -471,14 +490,6 @@ static void collect_timing(vt_tracker* t) {
     ms[5] = wall > dev ? wall - dev : 0.f;  // results (and overlay rows) back in host memory + completion latency, host clock
     ms[6] = wall;
     if (t->active.empty()) ms[1] = ms[2] = ms[3] = ms[4] = 0.f;
-    if (getenv("VT_B200_STAMPDBG") && ovl) {  // diagnostics: overlay kernel prologue end / dependency satisfied / end, relative to the decode end
-        static double acc[3] = {0, 0, 0};
-        static int cnt = 0;
-        acc[0] += (double)((long long)st[6] - (long long)st[ST_DEC_END]), acc[1] += (double)((long long)st[7] - (long long)st[ST_DEC_END]);
-        acc[2] += (double)((long long)st[ST_OVL_END] - (long long)st[ST_DEC_END]);
-        if (++cnt % 50 == 0) fprintf(stderr, "[vt stampdbg] overlay vs decode end: prologue done %+.2f us, dependency satisfied %+.2f us, end %+.2f us\n",
-                                     acc[0] / cnt * 1e-3, acc[1] / cnt * 1e-3, acc[2] / cnt * 1e-3);
-    }
     memcpy(t->last, ms, sizeof(ms));
     t->r_h2d.push(ms[0]), t->r_pre.push(ms[1]), t->r_vit.push(ms[2]), t->r_dec.push(ms[3]), t->r_ovl.push(ms[4]), t->r_d2h.push(ms[5]),
         t->r_tot.push(ms[6]);
@@ -498,7 +509,7 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
         set_error("pageable host frames are staged through one buffer and cannot be pipelined: wait() first or use pinned frames");
         return VT_ERR_INVALID;
     }
-    const double hp0 = t->hostprof ? now_us() : 0;
+    const double hp0 = t->sw.hostprof ? now_us() : 0;
     const int slot = (t->q_head + t->q_count) % vt_tracker::kQueue;
     vt_tracker::Slot& q = t->q[slot];
     q.t_submit = std::chrono::steady_clock::now();
@@ -544,7 +555,7 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
         vt_status st = do_upload(t, frame, len, plan, false, nullptr);  // the host mirror of rect_last is exact: the search windows suffice
         if (st != VT_OK) return st;
     }
-    const double hp1 = t->hostprof ? now_us() : 0;
+    const double hp1 = t->sw.hostprof ? now_us() : 0;
     const bool ran = forward && !t->active.empty();
     if (ran) {
         vt_status st = run_forward(t);
@@ -558,12 +569,12 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
         }
         ++t->kernel_launches;
     }
-    const double hp2 = t->hostprof ? now_us() : 0;
+    const double hp2 = t->sw.hostprof ? now_us() : 0;
     // the result block reaches t->h_blk[slot] through the last kernel of the frame; nothing ran: copy it
     if (!ran && n_hud == 0) VT_CUDA(cudaMemcpyAsync(t->h_blk[slot], t->d_res, t->res_block_bytes, cudaMemcpyDeviceToHost, t->stream));
     VT_CUDA(cudaEventRecord(t->q_done[slot], t->stream));
     t->d2h_bytes += t->res_block_bytes;
-    if (t->hostprof) t->hp[0] += hp1 - hp0, t->hp[1] += hp2 - hp1, t->hp[2] += now_us() - hp2;
+    if (t->sw.hostprof) t->hp[0] += hp1 - hp0, t->hp[1] += hp2 - hp1, t->hp[2] += now_us() - hp2;
     ++t->q_count;
     t->in_flight = true;
     return VT_OK;
@@ -654,10 +665,10 @@ static vt_status wait_common(vt_tracker* t, vt_result* results) {
     t->in_flight = t->q_count > 0;
     t->t_submit = q.t_submit, t->inflight_frame = q.frame, t->inflight_mirrored = q.mirrored;
     const size_t len = q.len;
-    const double hp0 = t->hostprof ? now_us() : 0;
+    const double hp0 = t->sw.hostprof ? now_us() : 0;
     VT_CUDA(cudaEventSynchronize(t->q_done[slot]));
     bind_slot(t, slot);
-    const double hp1 = t->hostprof ? now_us() : 0;
+    const double hp1 = t->sw.hostprof ? now_us() : 0;
     if (*t->h_tc_err) {  // travels with the results; reset on the device for the next frame
         cudaMemsetAsync(t->d_tc_err, 0, sizeof(int), t->stream);
         *t->h_tc_err = 0;
@@ -665,7 +676,7 @@ static vt_status wait_common(vt_tracker* t, vt_result* results) {
         return VT_ERR_CUDA;
     }
     fill_results(t, results);
-    const double hp2 = t->hostprof ? now_us() : 0;
+    const double hp2 = t->sw.hostprof ? now_us() : 0;
     if (q.hud_bytes && t->inflight_mirrored) t->d2h_bytes += q.hud_bytes;  // HUD pixels mirrored into the pinned frame
     if (t->cfg.box_overlay && t->inflight_frame && t->inflight_mirrored) {
         // the overlay kernel wrote the box pixels straight into the caller's pinned frame: count them as device->host traffic
@@ -685,10 +696,10 @@ static vt_status wait_common(vt_tracker* t, vt_result* results) {
             if (staged) unstage_rows(t, t->inflight_frame, len, spans);
         }
     }
-    const double hp3 = t->hostprof ? now_us() : 0;
+    const double hp3 = t->sw.hostprof ? now_us() : 0;
     collect_timing(t);
     ++t->frames;
-    if (t->hostprof) t->hp[3] += hp1 - hp0, t->hp[4] += hp2 - hp1, t->hp[5] += hp3 - hp2, t->hp[6] += now_us() - hp3, ++t->hp_n;
+    if (t->sw.hostprof) t->hp[3] += hp1 - hp0, t->hp[4] += hp2 - hp1, t->hp[5] += hp3 - hp2, t->hp[6] += now_us() - hp3, ++t->hp_n;
     return VT_OK;
 }
 
@@ -794,7 +805,7 @@ vt_status vt_tracker_init(vt_tracker* t, int32_t target, const uint8_t* frame, s
             return VT_ERR_CROP_OUTSIDE;
         }
     }
-    vt_status st = upload_frame(t, frame, len);
+    vt_status st = do_upload(t, frame, len, UploadPlan(), false, nullptr);  // the whole frame
     if (st != VT_OK) return st;
     TargetState hs;
     memset(&hs, 0, sizeof(hs));

@@ -54,7 +54,21 @@ struct WeightSet {
 // follows the handle count.
 constexpr int kMaxDevices = 64, kSpreadMaxHandles = 2, kUnchainTargets = 8;
 
-enum { EV_START = 0, EV_H2D, EV_PRE, EV_VIT, EV_DEC, EV_OVL, EV_END, EV_COUNT };
+// Environment switches of a handle, read by read_switches at create (meaning and defaults: DESIGN.md §9).
+struct Switches {
+    bool spread = true, att_chain = true, att_q64 = true, as_mlp = true, trace = false, hostprof = false;
+    int unchain_n = kUnchainTargets, as_rows = 1024, as_split = 0, win_shrink = 0;
+};
+
+// The kernel forms the model shape allows on the tensor-core path (shape_forms): vt_tracker_create sizes the buffers and wires the
+// plans from them, forward_forms picks the forms of every forward among them.
+struct ShapeForms {
+    bool fuse_ln = false;       // LayerNorm fused into the producing GEMM's epilogue (else layernorm_split kernels)
+    bool chain_mlp = false;     // FC2 partial products inside the FC1 kernel + reduce_ln
+    bool tc_attention = false;  // tensor-core attention (else the SIMT attention kernel)
+    bool att_chain = false;     // proj folded into the attention kernel (per-head partials in Pbuf + reduce_ln)
+    bool split_k = false;       // patch embed and 3x3 head conv as split-K partials + reduce_ln / head_decode
+};
 
 }  // namespace vt
 
@@ -67,8 +81,8 @@ struct vt_tracker {
     size_t frame_bytes = 0;
     float threshold = 0.2f;
     cudaStream_t stream = nullptr;
-    cudaEvent_t ev[EV_COUNT] = {};
-    bool ev_valid = false;
+    cudaEvent_t ev_ovl[2] = {};  // around vt_overlay's kernel (overlay_ms)
+    Switches sw;
 
     // weights (one device allocation, shared between the handles of a device: WeightSet)
     std::shared_ptr<WeightSet> wset;
@@ -107,8 +121,6 @@ struct vt_tracker {
     FrameCtl* d_ctl = nullptr;         // per-frame control block (frame / host frame / result block addresses, valid windows, HUD list)
     // probe HUD (host_state.cpp): the frame's last kernel runs a per-frame command list; the list of the NEXT submit is staged in the
     // pinned block of that submit's queue slot by tracker_set_hud()
-    int win_shrink = 0;                // diagnostics (VT_B200_WINDOW_SHRINK=px at create): upload windows that are too small on purpose,
-                                       // so that the crop kernel's fall-back reads from the pinned host frame are exercised
     bool hud_mode = false;
     OverlayCmdDev* h_hud[2] = {nullptr, nullptr};
     OverlayCmdDev* d_hud[2] = {nullptr, nullptr};  // device copies of the lists (written by the stamp kernel from its parameter block)
@@ -135,20 +147,11 @@ struct vt_tracker {
                   *att_lo = nullptr, *hid_hi = nullptr, *hid_lo = nullptr, *yf_hi = nullptr, *yf_lo = nullptr;
     __nv_bfloat16 *q_hi = nullptr, *q_lo = nullptr, *k_hi = nullptr, *k_lo = nullptr, *vt_hi = nullptr, *vt_lo = nullptr;
     __nv_bfloat16 *zln_hi = nullptr, *zln_lo = nullptr;  // LN1 (block 0) of the template tokens, [B][64][D], computed at init
-    bool fuse_ln = false;       // LayerNorm fused into the producing GEMM's epilogue (cluster of D / 64 CTAs)
-    bool chain_mlp = false;     // FC2 partial products computed inside the FC1 kernel + reduce_ln_kernel (no hidden round trip)
-    float* Pbuf = nullptr;      // [hidden / 64][B][320][D] fp32 partial FC2 results (also the 4 split-K partials of the patch embed)
-    bool split_k = false;       // patch embed and 3x3 head conv as split-K partial GEMMs + reduce kernels
+    float* Pbuf = nullptr;      // [planes][B][320][D] fp32 partials: chained MLP (hidden / 64), chained attention (heads), patch-embed K-slices (4)
     float *Phead = nullptr, *d_cand = nullptr;  // [9 taps][B][256][head_ch] conv partials; [B][16][8] row candidates of the decode
     unsigned* d_counters = nullptr;
-    bool pdl = true;            // programmatic dependent launch along the kernel chain
-    bool spread_ok = true;      // latency-mode GEMM forms allowed (VT_B200_NO_SPREAD disables)
-    int unchain_n = kUnchainTargets;  // active targets from which the MLP runs unchained (VT_B200_UNCHAIN_N overrides)
     int sm_count = 148;         // SMs of the device (grid sizing of the throughput forms)
-    int as_rows = 1024;         // rows (M) from which QKV / unchained FC1 run in the A-stationary throughput form (VT_B200_AS_ROWS; 0 = never)
-    bool as_mlp = true;         // ... and the MLP as one chained A-stationary kernel + reduce (VT_B200_NO_AS_MLP disables: FC1 A-stationary, FC2 own GEMM)
     bool counted = false;       // this handle is included in g_live_handles
-    bool tc_attention = false;  // head_dim == 64
     TcAttentionPlan plan_att;
     int* d_tc_err = nullptr;
     unsigned long long* d_trace = nullptr;  // VT_B200_TRACE=1: device timeline of the chain (vt_tracker_debug_trace)
@@ -157,8 +160,6 @@ struct vt_tracker {
         TcGemmPlan qkv, proj, fc1, fc2;
         TcAttentionPlan att;  // plan_att + this block's W_proj maps (chained form)
     };
-    bool att_chain_ok = false;  // the chained attention form is available (VT_B200_NO_ATT_CHAIN disables)
-    bool att_q64 = true;        // ... on 64-row query tiles where the grid fits one wave (VT_B200_ATT_Q128: always 128-row tiles)
     std::vector<BlockPlans> plans;
 
     std::map<int, cudaGraphExec_t> graphs;
@@ -183,7 +184,6 @@ struct vt_tracker {
     std::chrono::steady_clock::time_point t_submit;
 
     // VT_B200_HOSTPROF=1: host-side wall time of the submit / wait phases, printed at destroy (diagnostics)
-    bool hostprof = false;
     double hp[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     uint64_t hp_n = 0;
 
@@ -198,8 +198,7 @@ bool is_pinned(const void* p);
 // vt_overlay_cmd -> device form (glyph rows resolved); VT_ERR_GLYPH for an unknown character in strict mode
 vt_status fill_cmd_dev(const vt_overlay_cmd& c, OverlayCmdDev& d);
 void bind_slot(vt_tracker* t, int slot);
-vt_status upload_frame(vt_tracker* t, const uint8_t* frame, size_t len, bool allow_window = false, bool device_src = false,
-                       cudaStream_t stream = nullptr);
+ShapeForms shape_forms(const vt_tracker* t);
 // rows of the frame touched by a rect / crosshair (reference clamping), span bookkeeping and the device -> host row copies
 bool rect_rows(int fmt, long long H, int y, int h, int th, long long& r0, long long& r1);
 bool cross_rows(long long H, int cy, int size, long long& r0, long long& r1);

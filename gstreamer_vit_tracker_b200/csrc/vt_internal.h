@@ -352,12 +352,13 @@ cudaError_t tc_gemm_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t 
 // accumulators (main loop of chunk i + 1 under the epilogue of chunk i).  Bit-identical to tc_gemm_launch on the same plan.
 cudaError_t tc_gemm_as_setup();
 bool tc_gemm_as_supported(const TcGemmPlan& p);
-cudaError_t tc_gemm_as_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, int sm_count);
+// forced_split > 0: that many CTAs per row tile instead of as many as fit one wave (VT_B200_AS_SPLIT)
+cudaError_t tc_gemm_as_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, int sm_count, int forced_split);
 // chained MLP in the A-stationary form (bf16x3): plan = an FC1 plan with tc_plan_chain applied; the GELU'd hidden tile goes back into
 // tensor memory as the A operand of the chained product, which accumulates over all hidden chunks of the CTA; *planes partial planes
 // (CTAs per row tile) are written to the chain output for reduce_ln_kernel
 bool tc_gemm_as_mlp_supported(const TcGemmPlan& p, int nsplit);
-cudaError_t tc_gemm_as_mlp_launch(const TcGemmPlan& p, int M, cudaStream_t s, bool pdl, int sm_count, int* planes);
+cudaError_t tc_gemm_as_mlp_launch(const TcGemmPlan& p, int M, cudaStream_t s, bool pdl, int sm_count, int forced_split, int* planes);
 struct TcAttentionPlan {      // kernel parameter block (__grid_constant__)
     CUtensorMap mQhi, mQlo, mKhi, mKlo, mVhi, mVlo;
     CUtensorMap mQ64hi, mQ64lo;      // Q in boxes of 64 rows (VT_ATT_CHAIN_Q64)

@@ -40,8 +40,7 @@ def main():
     dst = torch.empty((n, W * H * 3), dtype=torch.uint8, device="cuda")
     ms = timed(trk, lambda: trk.nv12_to_rgb_device(src.data_ptr(), W * H * 3 // 2, dst.data_ptr(), W * H * 3, n))
     by = n * (W * H * 3 // 2 + W * H * 3)
-    narrow = bool(os.environ.get("VT_B200_CVT_NARROW"))
-    out.append({"kernel": "nv12_to_rgb_vec_kernel" if narrow else "nv12_to_rgb_vec4_kernel", "frames": n, "resolution": "1920x1080", "bytes_per_launch": by, "ms_per_launch": ms,
+    out.append({"kernel": "nv12_to_rgb_vec4_kernel", "frames": n, "resolution": "1920x1080", "bytes_per_launch": by, "ms_per_launch": ms,
                 "achieved_gbs": by / ms / 1e6, "peak_gbs": hbm, "frac": by / ms / 1e6 / hbm})
     # YUY2 -> RGB, 256 x 640x512
     w, h, n2 = 640, 512, 256
@@ -49,7 +48,7 @@ def main():
     dst2 = torch.empty((n2, w * h * 3), dtype=torch.uint8, device="cuda")
     ms = timed(trk, lambda: trk.yuy2_to_rgb_device(src2.data_ptr(), w * h * 2, dst2.data_ptr(), w * h * 3, w, h, n2))
     by = n2 * (w * h * 2 + w * h * 3)
-    out.append({"kernel": "yuy2_to_rgb_vec_kernel" if narrow else "yuy2_to_rgb_vec2_kernel", "frames": n2, "resolution": "640x512", "bytes_per_launch": by, "ms_per_launch": ms,
+    out.append({"kernel": "yuy2_to_rgb_vec2_kernel", "frames": n2, "resolution": "640x512", "bytes_per_launch": by, "ms_per_launch": ms,
                 "achieved_gbs": by / ms / 1e6, "peak_gbs": hbm, "frac": by / ms / 1e6 / hbm})
     # RGB up-scale 640x512 -> 1280x1024, batch of 128 frames in one launch (126 MB in, 503 MB out)
     nb = 128
