@@ -52,6 +52,11 @@ class vt_overlay_cmd(C.Structure):
     ]
 
 
+class vt_surface(C.Structure):
+    """A pitched device frame: planes[0] = Y / RGB / gray, planes[1] = NV12 interleaved UV; pitch[i] = row pitch in bytes."""
+    _fields_ = [("planes", C.c_void_p * 2), ("pitch", C.c_size_t * 2)]
+
+
 class vt_timing(C.Structure):
     _fields_ = [
         ("fps", C.c_double), ("avg_conv_ms", C.c_double), ("avg_track_ms", C.c_double),
@@ -87,6 +92,10 @@ SYMBOLS = {
     "vt_tracker_submit_device": (C.c_int32, [_vp, _vp, C.c_size_t]),
     "vt_tracker_wait": (C.c_int32, [_vp, C.POINTER(vt_result)]),
     "vt_tracker_update_device": (C.c_int32, [_vp, _vp, C.c_size_t, C.POINTER(vt_result)]),
+    "vt_tracker_init_surface": (C.c_int32, [_vp, C.c_int32, C.POINTER(vt_surface), vt_bbox]),
+    "vt_tracker_update_surface": (C.c_int32, [_vp, C.POINTER(vt_surface), C.POINTER(vt_result)]),
+    "vt_tracker_submit_surface": (C.c_int32, [_vp, C.POINTER(vt_surface)]),
+    "vt_tracker_update_streams_surface": (C.c_int32, [_vp, C.POINTER(vt_surface), C.c_int32, C.POINTER(vt_result)]),
     "vt_tracker_run_streams_ring": (C.c_int32, [_vp, C.POINTER(C.c_void_p), C.c_int32, C.c_size_t, C.c_size_t, C.c_int32, C.c_int32, C.c_int32,
                                     C.POINTER(C.c_void_p), C.POINTER(vt_result), C.POINTER(C.c_double)]),
     "vt_tracker_update_streams": (C.c_int32, [_vp, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int32, C.POINTER(vt_result)]),

@@ -24,7 +24,7 @@ from typing import List, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib as L
-from ._lib import VtError, check, lib, vt_bbox, vt_config, vt_overlay_cmd, vt_result, vt_selection, vt_timing
+from ._lib import VtError, check, lib, vt_bbox, vt_config, vt_overlay_cmd, vt_result, vt_selection, vt_surface, vt_timing
 
 
 @dataclass(frozen=True)
@@ -92,6 +92,81 @@ def _ptr(a: np.ndarray) -> C.c_void_p:
     if not isinstance(a, np.ndarray) or a.dtype != np.uint8 or not a.flags["C_CONTIGUOUS"]:
         raise ValueError("frames are C-contiguous uint8 numpy arrays")
     return C.c_void_p(a.ctypes.data)
+
+
+Surface = Tuple[Sequence[int], Sequence[int]]  # ((plane 0 address, plane 1 address), (pitch 0, pitch 1)): device addresses, bytes
+
+
+def _surface(s: Surface) -> vt_surface:
+    planes, pitches = s
+    c = vt_surface()
+    for i in range(2):
+        c.planes[i] = int(planes[i]) if i < len(planes) and planes[i] else None
+        c.pitch[i] = int(pitches[i]) if i < len(pitches) else 0
+    return c
+
+
+class PitchedFrame:
+    """A packed frame laid out as a pitched device surface in torch buffers, like a decoder's output surface: rows `pitch` bytes apart
+    and, for NV12, the chroma plane `chroma_row` rows after the start of the Y plane (NVDEC: the surface height), or in an allocation
+    of its own (`separate_uv`).  Every byte outside the visible pixels (pitch padding, the gap between the planes) holds `fill`.
+    `surface` is the (planes, pitches) tuple the *_surface methods of VitTrack take."""
+
+    def __init__(self, width: int, height: int, fmt: str = "nv12", pitch: Optional[int] = None, chroma_row: Optional[int] = None,
+                 separate_uv: bool = False, fill: int = 0, device: int = 0):
+        import torch
+
+        self.width, self.height, self.fmt = width, height, fmt
+        self.row = width * (3 if fmt == "rgb24" else 1)
+        self.pitch = pitch if pitch is not None else self.row
+        if self.pitch < self.row:
+            raise ValueError("pitch is smaller than a row")
+        self.nv12 = fmt == "nv12"
+        self.uv_rows = (height + 1) // 2 if self.nv12 else 0
+        dev = torch.device("cuda", device)
+        if not self.nv12 or separate_uv:
+            self.buf = torch.full((height * self.pitch,), fill, dtype=torch.uint8, device=dev)
+            self.uv_buf = torch.full((self.uv_rows * self.pitch,), fill, dtype=torch.uint8, device=dev) if self.nv12 else None
+            self.uv_offset = 0
+        else:
+            crow = chroma_row if chroma_row is not None else height
+            if crow < height:
+                raise ValueError("the chroma plane overlaps the Y plane")
+            self.buf = torch.full(((crow + self.uv_rows) * self.pitch,), fill, dtype=torch.uint8, device=dev)
+            self.uv_buf, self.uv_offset = None, crow * self.pitch
+
+    def _planes(self):
+        y = self.buf[: self.height * self.pitch].view(self.height, self.pitch)[:, : self.row]
+        if not self.nv12:
+            return y, None
+        base = self.uv_buf if self.uv_buf is not None else self.buf[self.uv_offset:]
+        return y, base[: self.uv_rows * self.pitch].view(self.uv_rows, self.pitch)[:, : self.width]
+
+    def write(self, frame) -> None:
+        """Copies a packed frame (numpy array or torch tensor, host or device) into the visible pixels."""
+        import torch
+
+        f = torch.as_tensor(np.ascontiguousarray(frame) if isinstance(frame, np.ndarray) else frame).reshape(-1)
+        y, uv = self._planes()
+        n = self.height * self.row
+        y.copy_(f[:n].view(self.height, self.row))
+        if uv is not None:
+            uv.copy_(f[n: n + self.uv_rows * self.width].view(self.uv_rows, self.width))
+        torch.cuda.synchronize(self.buf.device)  # the tracker's stream does not order behind torch's
+
+    def read(self) -> np.ndarray:
+        """The visible pixels as a packed frame (host)."""
+        import torch
+
+        y, uv = self._planes()
+        return torch.cat([y.reshape(-1)] + ([uv.reshape(-1)] if uv is not None else [])).cpu().numpy()
+
+    @property
+    def surface(self) -> Surface:
+        if not self.nv12:
+            return (self.buf.data_ptr(), 0), (self.pitch, 0)
+        uv = self.uv_buf.data_ptr() if self.uv_buf is not None else self.buf.data_ptr() + self.uv_offset
+        return (self.buf.data_ptr(), uv), (self.pitch, self.pitch)
 
 
 def make_config(weights: str, width: int, height: int, fmt: str = "nv12", max_targets: int = 1, device: int = 0,
@@ -241,6 +316,29 @@ class VitTrack:
 
     def update_device(self, d_ptr: int, nbytes: int) -> List[TrackResult]:
         check(lib().vt_tracker_update_device(self._h, C.c_void_p(d_ptr), nbytes, self._res), "vt_tracker_update_device")
+        return self._results()
+
+    # -- pitched device surfaces (decoder output: NVDEC, NvBufSurface), tracked in place; PitchedFrame makes one in torch memory
+    def init_surface(self, surface: Surface, bbox: BBox, target: int = 0) -> None:
+        s = _surface(surface)
+        check(lib().vt_tracker_init_surface(self._h, target, C.byref(s), bbox._c()), "vt_tracker_init_surface")
+
+    def update_surface(self, surface: Surface) -> List[TrackResult]:
+        s = _surface(surface)
+        check(lib().vt_tracker_update_surface(self._h, C.byref(s), self._res), "vt_tracker_update_surface")
+        return self._results()
+
+    def submit_surface(self, surface: Surface) -> None:
+        """The caller keeps the surface's memory alive until the matching wait()."""
+        s = _surface(surface)
+        check(lib().vt_tracker_submit_surface(self._h, C.byref(s)), "vt_tracker_submit_surface")
+        self._inflight.append(None)
+
+    def update_streams_surface(self, surfaces: Sequence[Surface]) -> List[TrackResult]:
+        """Stream group on device surfaces: surfaces[i] is the current frame of the i-th active target's stream (see update_streams)."""
+        n = len(surfaces)
+        arr = (vt_surface * n)(*[_surface(s) for s in surfaces])
+        check(lib().vt_tracker_update_streams_surface(self._h, arr, n, self._res), "vt_tracker_update_streams_surface")
         return self._results()
 
     def run_ring(self, base_ptr: int, stride: int, frame_len: int, ring: int, first: int, n: int, mode: int, pristine_ptr: int = 0,

@@ -430,14 +430,13 @@ __device__ __forceinline__ Tap lin_tap(int i, int s, int d, bool clamp_frac) {
 }
 
 // Where the pixels of this frame live: the device frame inside the valid window (the part that was uploaded this frame), the
-// caller's pinned host frame (zero-copy loads over PCIe) outside of it.  With whole-frame uploads the window is the frame.
+// caller's pinned host frame (zero-copy loads over PCIe) outside of it.  With whole-frame uploads the window is the frame.  The device
+// frame may be a pitched surface (planes and pitches from the control block or the frame descriptor); the host frame is always packed.
 struct PixelSrc {
-    const uint8_t* dev;
-    const uint8_t* host;   // null: everything is on the device
-    int x0, y0, x1, y1;    // valid window of the device frame (even-aligned, so a pixel and its chroma pair sit on the same side)
-    __device__ __forceinline__ const uint8_t* at(int fx, int fy) const {
-        return (host && (fx < x0 || fx >= x1 || fy < y0 || fy >= y1)) ? host : dev;
-    }
+    const uint8_t *dev, *dev_uv;  // device planes: Y / RGB / gray, NV12 chroma
+    size_t pitch, uv_pitch;       // their row pitches
+    const uint8_t* host;          // null: everything is on the device
+    int x0, y0, x1, y1;           // valid window of the device frame (even-aligned, so a pixel and its chroma pair sit on the same side)
 };
 
 // RGB of the frame pixel (fx, fy); zero outside the frame (constant border of the crop).
@@ -446,17 +445,18 @@ __device__ __forceinline__ void frame_rgb(const FrameDesc& f, const PixelSrc& ps
     // pad_plus1 (App. A.7, older OpenCV): a crop that reaches the right / bottom edge pads one pixel more, i.e. the last column / row of
     // the frame reads as border; a crop that stays inside never addresses it, so the bound can move unconditionally
     if (!f.valid || fx < 0 || fy < 0 || fx >= f.width - f.pad_plus1 || fy >= f.height - f.pad_plus1) return;
-    const uint8_t* data = ps.at(fx, fy);
+    const bool host = ps.host && (fx < ps.x0 || fx >= ps.x1 || fy < ps.y0 || fy >= ps.y1);
+    const uint8_t* data = host ? ps.host : ps.dev;
     if (f.format == VT_FMT_RGB24) {
-        const uint8_t* p = data + ((size_t)fy * f.width + fx) * 3;
+        const uint8_t* p = data + (size_t)fy * (host ? (size_t)f.width * 3 : ps.pitch) + (size_t)fx * 3;
         r = p[0], g = p[1], b = p[2];
     } else if (f.format == VT_FMT_GRAY8) {
-        r = g = b = data[(size_t)fy * f.width + fx];
+        r = g = b = data[(size_t)fy * (host ? (size_t)f.width : ps.pitch) + fx];
     } else {
-        const size_t ysz = (size_t)f.width * f.height;
-        const int yv = data[(size_t)fy * f.width + fx];
-        const size_t uvi = ysz + (size_t)(fy >> 1) * f.width + (fx & ~1);
-        const Chroma c = chroma_terms(data[uvi], data[uvi + 1]);
+        const int yv = data[(size_t)fy * (host ? (size_t)f.width : ps.pitch) + fx];
+        const uint8_t* uv = host ? ps.host + (size_t)f.width * f.height : ps.dev_uv;
+        const size_t uvi = (size_t)(fy >> 1) * (host ? (size_t)f.width : ps.uv_pitch) + (fx & ~1);
+        const Chroma c = chroma_terms(uv[uvi], uv[uvi + 1]);
         yuv_px(yv, c, r, g, b);
     }
 }
@@ -469,10 +469,13 @@ __global__ void __launch_bounds__(256) crop_resize_norm_kernel(FrameDesc f, Targ
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // the template gather behind this kernel does not depend on it
     if (stamp && threadIdx.x == 0 && blockIdx.x == 0 && blockIdx.y == 0) *stamp = device_time_ns();
     const int bi = blockIdx.y;
-    PixelSrc ps{f.data, nullptr, 0, 0, f.width, f.height};
-    if (f.ctl) {  // per-frame control block: frame address, and which part of the device frame holds this frame's pixels
+    PixelSrc ps{f.data, f.uv, f.pitch[0], f.pitch[1], nullptr, 0, 0, f.width, f.height};
+    if (f.ctl) {  // per-frame control block: frame planes, and which part of the device frame holds this frame's pixels
         const bool own = bi < kMaxWin && f.ctl->frames[bi] != nullptr;  // stream group: this target has its own frame
         ps.dev = own ? f.ctl->frames[bi] : f.ctl->frame;
+        ps.dev_uv = own ? f.ctl->uvs[bi] : f.ctl->uv;
+        ps.pitch = own ? f.ctl->pitches[bi][0] : f.ctl->pitch[0];
+        ps.uv_pitch = own ? f.ctl->pitches[bi][1] : f.ctl->pitch[1];
         const int nw = f.ctl->n_win;
         if (nw >= 0) {
             ps.host = own ? f.ctl->host_frames[bi] : f.ctl->host_frame;
@@ -480,6 +483,9 @@ __global__ void __launch_bounds__(256) crop_resize_norm_kernel(FrameDesc f, Targ
             else ps.x1 = ps.y1 = 0;  // nothing of this target was uploaded
         }
     }
+    if (!ps.pitch) ps.pitch = (size_t)f.width * (f.format == VT_FMT_RGB24 ? 3 : 1);  // packed frame
+    if (!ps.dev_uv) ps.dev_uv = ps.dev + (size_t)f.width * f.height;
+    if (!ps.uv_pitch) ps.uv_pitch = (size_t)f.width;
     const int slot = slots[bi];
     TargetState* st = state + slot;
     const int bx = st->rect[0], by = st->rect[1], bw = st->rect[2], bh = st->rect[3];
@@ -701,14 +707,15 @@ __device__ __forceinline__ u64 umin64(u64 a, u64 b) { return a < b ? a : b; }
 
 struct Surface {
     uint8_t* d;
-    size_t len;
+    size_t len;            // bytes of the drawn plane (RGB writes are bounds-checked against it)
     int W, H, fmt;
+    size_t pitch;          // row pitch of the drawn plane in bytes (Y plane / RGB image)
 };
 // NV12: luma write (Y plane). RGB: bounds-checked colour write (src/drawing_rgb.rs:18-28).
-__device__ __forceinline__ void put_y(const Surface& s, u64 x, u64 y, uint8_t v) { s.d[y * (u64)s.W + x] = v; }
+__device__ __forceinline__ void put_y(const Surface& s, u64 x, u64 y, uint8_t v) { s.d[y * (u64)s.pitch + x] = v; }
 __device__ __forceinline__ void put_rgb(const Surface& s, int x, int y, uint8_t r, uint8_t g, uint8_t b) {
     if (x < 0 || y < 0 || x >= s.W || y >= s.H) return;
-    const size_t off = ((size_t)y * s.W + x) * 3;
+    const size_t off = (size_t)y * s.pitch + (size_t)x * 3;
     if (off + 2 < s.len) s.d[off] = r, s.d[off + 1] = g, s.d[off + 2] = b;
 }
 
@@ -800,7 +807,7 @@ __device__ void ov_background(const Surface& s, const OverlayCmdDev& c) {
         const u64 nx = x1 - x0, n = nx * (y1 - y0);
         const unsigned factor = 255u - (unsigned)(uint8_t)c.a;
         for (u64 i = threadIdx.x; i < n; i += blockDim.x) {
-            const u64 idx = (y0 + i / nx) * (u64)s.W + x0 + i % nx;
+            const u64 idx = (y0 + i / nx) * (u64)s.pitch + x0 + i % nx;
             s.d[idx] = (uint8_t)(((unsigned)s.d[idx] * factor) / 255u);
         }
     } else {  // src/drawing_rgb.rs:30-53: fill with 30
@@ -810,7 +817,7 @@ __device__ void ov_background(const Surface& s, const OverlayCmdDev& c) {
         const u64 rb = (xe - xs) * 3, n = rb * (ye - ys);
         for (u64 i = threadIdx.x; i < n; i += blockDim.x) {
             const u64 row = ys + i / rb;
-            const u64 off = (row * (u64)s.W + xs) * 3;
+            const u64 off = row * (u64)s.pitch + xs * 3;
             if (off + rb <= s.len) s.d[off + i % rb] = 30;
         }
     }
@@ -872,7 +879,7 @@ __device__ void ov_dispatch(const Surface& s, const OverlayCmdDev& c) {
 
 __global__ void __launch_bounds__(1024) overlay_kernel(uint8_t* frame, size_t len, int W, int H, int fmt,
                                                        const OverlayCmdDev* __restrict__ cmds, int n) {
-    Surface s{frame, len, W, H, fmt};
+    Surface s{frame, len, W, H, fmt, (size_t)W * (fmt == VT_FMT_RGB24 ? 3 : 1)};
     for (int i = 0; i < n; ++i) {
         ov_dispatch(s, cmds[i]);
         __syncthreads();
@@ -957,6 +964,11 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
     if (split && blockIdx.y == 1 && !host0) return;       // nothing to mirror into
     uint8_t* const frame = frame0;
     uint8_t* const host = host0;
+    // row pitch of the drawn plane: the caller's surface pitch for the device frame; the pinned host frame is packed.  (The HUD paths
+    // below address rows by W: HUD handles take packed frames only.)
+    const size_t row = (size_t)W * (fmt == VT_FMT_RGB24 ? 3 : 1);
+    const size_t fpitch0 = own ? ctl->pitches[blockIdx.x][0] : ctl->pitch[0];
+    const size_t fpitch = fpitch0 ? fpitch0 : row;
     const bool do_dev = !split || blockIdx.y == 0, do_host = host != nullptr && (!split || blockIdx.y == 1);
     int n_hud = blockIdx.x == 0 ? ctl->n_hud : 0;
     if (n_hud > kMaxCmds) n_hud = kMaxCmds;
@@ -1034,7 +1046,8 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
             uint8_t* dst = p == 0 ? frame : host;
             if (!dst) break;
             if ((p == 0 && !do_dev) || (p == 1 && !do_host)) continue;
-            Surface s{dst, len, W, H, fmt};
+            const size_t pitch = p == 0 ? fpitch : row;
+            Surface s{dst, pitch * H, W, H, fmt, pitch};
             if (fmt == VT_FMT_NV12) {
                 ov_rect_nv12(s, x, y, w, h, 3, 255);
                 __syncthreads();
@@ -1119,7 +1132,8 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
             uint8_t* dst = p == 0 ? frame : host;
             if (!dst) break;
             if ((p == 0 && !do_dev) || (p == 1 && !do_host)) continue;
-            Surface s{dst, len, W, H, fmt};
+            const size_t pitch = p == 0 ? fpitch : row;
+            Surface s{dst, pitch * H, W, H, fmt, pitch};
             for (int i = first; i < n_hud; ++i) {
                 const OverlayCmdDev& c = s_cmd[i];
                 if (c.kind < 0) continue;

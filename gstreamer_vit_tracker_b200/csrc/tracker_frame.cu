@@ -109,7 +109,7 @@ static ForwardForms forward_forms(const vt_tracker* t, int n, bool spread) {
 static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const ForwardForms& f) {
     const int D = t->D, Hd = t->hidden, C = t->head_ch;
     cudaStream_t s = t->stream;
-    FrameDesc fd{t->d_frame, t->W, t->H, t->fmt, t->frame_valid, t->d_ctl, t->cfg.pad_plus1};
+    FrameDesc fd{t->d_frame, nullptr, {0, 0}, t->W, t->H, t->fmt, t->frame_valid, t->d_ctl, t->cfg.pad_plus1};  // planes from d_ctl
     auto LO = [&](__nv_bfloat16* p) { return t->f16 ? nullptr : p; };  // fp16 mode: "hi only" (see vt_internal.h: operand_bits)
     VT_LAUNCH(launch_crop_resize_norm(fd, t->d_state, t->d_slots, n, 4, kSearch, t->d_lut, t->patches_x, (size_t)kNTx * kPatchK, t->px_hi,
                                       LO(t->px_lo), s, t->d_stamps + ST_PRE));
@@ -499,12 +499,66 @@ static inline double now_us() {
     return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
 
-static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_src, size_t len, bool forward = true) {
+// A full-length packed device frame d as a surface: {d, d + W * H}, {W, W} (RGB24 / GRAY8: one plane)
+static vt_surface packed_surface(const vt_tracker* t, const uint8_t* d) {
+    const bool nv12 = t->fmt == VT_FMT_NV12;
+    vt_surface s;
+    s.planes[0] = const_cast<uint8_t*>(d), s.planes[1] = nv12 ? const_cast<uint8_t*>(d) + (size_t)t->W * t->H : nullptr;
+    s.pitch[0] = (size_t)t->W * (t->fmt == VT_FMT_RGB24 ? 3 : 1), s.pitch[1] = nv12 ? (size_t)t->W : 0;
+    return s;
+}
+
+// The caller's surface (include/vt_tracker.h: vt_surface): every plane of the format present, a pitch that holds a row, and device (or
+// managed) memory of the handle's GPU.  `i` >= 0 names the surface of a stream group in the message.
+static vt_status check_surface(const vt_tracker* t, const vt_surface* s, const char* where, int i) {
+    if (!s) {
+        set_error("%s: surface %d is null", where, i);
+        return VT_ERR_INVALID;
+    }
+    const int np = t->fmt == VT_FMT_NV12 ? 2 : 1;
+    for (int p = 0; p < np; ++p) {
+        const size_t row = (size_t)t->W * (t->fmt == VT_FMT_RGB24 ? 3 : 1);
+        if (!s->planes[p]) {
+            set_error("%s: surface %d: plane %d is null", where, i, p);
+            return VT_ERR_INVALID;
+        }
+        if (s->pitch[p] < row) {
+            set_error("%s: surface %d: pitch[%d] = %zu is smaller than the plane's row (%zu bytes)", where, i, p, s->pitch[p], row);
+            return VT_ERR_INVALID;
+        }
+        cudaPointerAttributes a;
+        const cudaError_t e = cudaPointerGetAttributes(&a, s->planes[p]);
+        if (e != cudaSuccess) cudaGetLastError();  // (not a sticky error: clear it)
+        if (e != cudaSuccess || (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != t->cfg.device) {
+            set_error("%s: surface %d: plane %d is not device memory of GPU %d", where, i, p, t->cfg.device);
+            return VT_ERR_INVALID;
+        }
+    }
+    return VT_OK;
+}
+
+// Checks shared by the surface entry points: a probe (HUD) handle draws its command lists with packed-row addressing, and a synchronous
+// call finds no frame in flight.
+static vt_status surface_call(vt_tracker* t, const char* where, bool sync) {
+    if (t->hud_mode) {
+        set_error("%s: a probe (HUD) handle takes packed frames only", where);
+        return VT_ERR_INVALID;
+    }
+    if (sync && t->q_count) {
+        set_error("%s: frames are in flight (submit/wait); drain them first", where);
+        return VT_ERR_INVALID;
+    }
+    VT_CUDA(cudaSetDevice(t->cfg.device));
+    return VT_OK;
+}
+
+// surf: a pitched device surface tracked in place (frame / d_src unused)
+static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_src, size_t len, bool forward = true, const vt_surface* surf = nullptr) {
     if (t->q_count >= vt_tracker::kQueue) {
         set_error("%d frames are already in flight on this handle", t->q_count);
         return VT_ERR_INVALID;
     }
-    const bool pinned = d_src || is_pinned(frame);
+    const bool pinned = d_src || surf || is_pinned(frame);
     if (t->q_count > 0 && (!pinned || t->q[t->q_head].pageable)) {
         set_error("pageable host frames are staged through one buffer and cannot be pipelined: wait() first or use pinned frames");
         return VT_ERR_INVALID;
@@ -513,15 +567,18 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
     const int slot = (t->q_head + t->q_count) % vt_tracker::kQueue;
     vt_tracker::Slot& q = t->q[slot];
     q.t_submit = std::chrono::steady_clock::now();
-    q.frame = d_src ? nullptr : frame, q.len = len, q.pageable = !pinned;
+    q.frame = d_src || surf ? nullptr : frame, q.len = len, q.pageable = !pinned;
     // the caller's pinned frame is device-mapped under UVA: zero-copy target of the overlay mirror, fall-back source of the crop kernel
-    uint8_t* const host_frame = (frame && !d_src && pinned && len >= t->frame_bytes) ? frame : nullptr;
+    uint8_t* const host_frame = (frame && !d_src && !surf && pinned && len >= t->frame_bytes) ? frame : nullptr;
     // this frame's HUD list (staged by tracker_set_hud in this slot's pinned block)
     const int n_hud = t->hud_mode ? t->hud_next_n : 0;
     q.hud_bytes = n_hud ? t->hud_next_bytes : 0;
     q.mirrored = host_frame && (t->cfg.box_overlay || n_hud > 0);
-    // device-resident frame: track (and draw the box) straight in the caller's device memory — no device->device copy
-    const bool in_place = d_src && len >= t->frame_bytes;
+    // device-resident frame: track (and draw the box) straight in the caller's device memory — no device->device copy.  A full-length
+    // packed device frame is a surface like any other.
+    vt_surface packed;
+    if (!surf && d_src && len >= t->frame_bytes) packed = packed_surface(t, d_src), surf = &packed;
+    const bool in_place = surf != nullptr;
     if (!in_place) t->d_frame = t->d_frames[slot];  // the slot's own frame buffer: the other one may still be read by the frame in flight
     const bool lagging = t->q_count > 0;  // a frame is in flight: rect_mirror is one frame old, the windows are predictions
     UploadPlan plan;
@@ -535,7 +592,11 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
     }
     FrameCtl ctl;
     memset(&ctl, 0, sizeof(ctl));
-    ctl.frame = in_place ? d_src : t->d_frame, ctl.host_frame = host_frame, ctl.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
+    ctl.frame = in_place ? surf->planes[0] : t->d_frame, ctl.host_frame = host_frame, ctl.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
+    if (in_place) {
+        const bool nv12 = t->fmt == VT_FMT_NV12;
+        ctl.uv = nv12 ? surf->planes[1] : nullptr, ctl.pitch[0] = surf->pitch[0], ctl.pitch[1] = nv12 ? surf->pitch[1] : 0;
+    }
     ctl.hud = n_hud ? t->h_hud[slot] : nullptr, ctl.n_hud = n_hud;
     const bool hud_inline = n_hud > 0 && n_hud <= kHudInline && t->d_hud[slot] != nullptr;
     if (hud_inline) ctl.hud = t->d_hud[slot];
@@ -583,30 +644,42 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
 // Stream group: the n active targets of the handle are n independent video streams (one target each, same geometry), stepped together
 // through ONE batched forward (M = 320 n rows: from 1024 rows on the GEMMs run in their throughput forms).  frames[i] is the pinned
 // host frame of the i-th active target; each target's search window is uploaded into that target's own device frame and the box overlay
-// is mirrored into that target's host frame.  Synchronous (rect_mirror is exact: the windows are the real search windows).
-static vt_status submit_streams(vt_tracker* t, uint8_t* const* frames, const size_t* lens, int n) {
+// is mirrored into that target's host frame.  Or surfs[i] (frames / lens unused) is the i-th target's device surface, read and drawn
+// into in place.  Synchronous (rect_mirror is exact: the windows are the real search windows).
+static vt_status submit_streams(vt_tracker* t, uint8_t* const* frames, const size_t* lens, const vt_surface* surfs, int n) {
+    const char* where = surfs ? "vt_tracker_update_streams_surface" : "vt_tracker_update_streams";
     if (t->q_count > 0 || t->hud_mode) {
-        set_error("vt_tracker_update_streams: frames are in flight on this handle, or it is a probe (HUD) handle");
+        set_error("%s: frames are in flight on this handle, or it is a probe (HUD) handle", where);
         return VT_ERR_INVALID;
     }
     if (n != (int)t->active.size() || n <= 0 || n > kMaxWin) {
-        set_error("vt_tracker_update_streams: %d frames for %d active targets (one frame per active target, at most %d)", n, (int)t->active.size(), kMaxWin);
+        set_error("%s: %d frames for %d active targets (one frame per active target, at most %d)", where, n, (int)t->active.size(), kMaxWin);
         return VT_ERR_INVALID;
     }
-    for (int i = 0; i < n; ++i)
-        if (!frames[i] || lens[i] < t->frame_bytes || !is_pinned(frames[i])) {
-            set_error("vt_tracker_update_streams: frame %d must be a full frame in pinned host memory (vt_alloc_pinned)", i);
+    for (int i = 0; i < n; ++i) {
+        if (surfs) {
+            const vt_status st = check_surface(t, &surfs[i], where, i);
+            if (st != VT_OK) return st;
+        } else if (!frames[i] || lens[i] < t->frame_bytes || !is_pinned(frames[i])) {
+            set_error("%s: frame %d must be a full frame in pinned host memory (vt_alloc_pinned)", where, i);
             return VT_ERR_INVALID;
         }
+    }
     const int slot = t->q_head;
     vt_tracker::Slot& q = t->q[slot];
     q.t_submit = std::chrono::steady_clock::now();
-    q.frame = frames[0], q.len = lens[0], q.pageable = false, q.hud_bytes = 0, q.mirrored = true;
+    q.frame = surfs ? nullptr : frames[0], q.len = surfs ? 0 : lens[0], q.pageable = false, q.hud_bytes = 0, q.mirrored = !surfs;
     FrameCtl ctl;
     memset(&ctl, 0, sizeof(ctl));
     const bool windows = t->cfg.upload_window && !(t->W % 2) && !((t->H % 2) && t->fmt == VT_FMT_NV12);
     const size_t W = (size_t)t->W;
     for (int i = 0; i < n; ++i) {
+        if (surfs) {  // in place: nothing to upload, the whole surface holds the frame
+            const bool nv12 = t->fmt == VT_FMT_NV12;
+            ctl.frames[i] = surfs[i].planes[0], ctl.uvs[i] = nv12 ? surfs[i].planes[1] : nullptr;
+            ctl.pitches[i][0] = surfs[i].pitch[0], ctl.pitches[i][1] = nv12 ? surfs[i].pitch[1] : 0;
+            continue;
+        }
         if (!t->d_sframes[i]) {
             VT_CUDA(cudaMalloc(&t->d_sframes[i], t->frame_bytes + 256));
             VT_CUDA(cudaMemsetAsync(t->d_sframes[i], 0, t->frame_bytes + 256, t->stream));
@@ -639,8 +712,9 @@ static vt_status submit_streams(vt_tracker* t, uint8_t* const* frames, const siz
         }
         ctl.frames[i] = dst, ctl.host_frames[i] = frames[i];
     }
-    ctl.frame = t->d_sframes[0], ctl.host_frame = frames[0], ctl.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
-    ctl.n_win = n;
+    ctl.frame = ctl.frames[0], ctl.uv = ctl.uvs[0], ctl.pitch[0] = ctl.pitches[0][0], ctl.pitch[1] = ctl.pitches[0][1];
+    ctl.host_frame = ctl.host_frames[0], ctl.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
+    ctl.n_win = surfs ? -1 : n;
     t->frame_valid = 1, t->d_frame_is_last_host_frame = false;
     VT_CUDA(launch_stamp(t->d_stamps + ST_SUBMIT, t->d_ctl, ctl, t->stream));
     ++t->kernel_launches;
@@ -774,39 +848,26 @@ vt_status tracker_set_hud(vt_tracker* t, const HudCmd* cmds, int n) {
     return VT_OK;
 }
 
-}  // namespace vt
-
-using namespace vt;
-
-extern "C" {
-
-vt_status vt_tracker_init(vt_tracker* t, int32_t target, const uint8_t* frame, size_t len, vt_bbox box) {
-    if (!t || !frame || target < 0 || target >= t->maxT) {
-        set_error("vt_tracker_init: invalid argument");
-        return VT_ERR_INVALID;
+// The template window must intersect the frame (cv2 raises an ROI assertion otherwise, App. A.1)
+static vt_status check_template_window(const vt_tracker* t, vt_bbox box, const char* where) {
+    if (box.width <= 0 || box.height <= 0) {
+        set_error("%s: empty box", where);
+        return VT_ERR_CROP_OUTSIDE;
     }
-    if (t->in_flight) {
-        set_error("vt_tracker_init: a frame is in flight");
-        return VT_ERR_INVALID;
+    const int c = (int)ceil(sqrt((double)((long long)box.width * box.height)) * 2.0);
+    const int x1 = box.x + (box.width - c) / 2, y1 = box.y + (box.height - c) / 2;
+    const int pp = t->cfg.pad_plus1;
+    const int pl = std::max(0, -x1), pt = std::max(0, -y1), pr = std::max(x1 + c - t->W + pp, 0), pb = std::max(y1 + c - t->H + pp, 0);
+    if (c - pl - pr <= 0 || c - pt - pb <= 0) {
+        set_error("%s: template window lies outside the frame", where);
+        return VT_ERR_CROP_OUTSIDE;
     }
-    VT_CUDA(cudaSetDevice(t->cfg.device));
-    // the template window must intersect the frame (cv2 raises an ROI assertion otherwise, App. A.1)
-    {
-        if (box.width <= 0 || box.height <= 0) {
-            set_error("vt_tracker_init: empty box");
-            return VT_ERR_CROP_OUTSIDE;
-        }
-        const int c = (int)ceil(sqrt((double)((long long)box.width * box.height)) * 2.0);
-        const int x1 = box.x + (box.width - c) / 2, y1 = box.y + (box.height - c) / 2;
-        const int pp = t->cfg.pad_plus1;
-        const int pl = std::max(0, -x1), pt = std::max(0, -y1), pr = std::max(x1 + c - t->W + pp, 0), pb = std::max(y1 + c - t->H + pp, 0);
-        if (c - pl - pr <= 0 || c - pt - pb <= 0) {
-            set_error("vt_tracker_init: template window lies outside the frame");
-            return VT_ERR_CROP_OUTSIDE;
-        }
-    }
-    vt_status st = do_upload(t, frame, len, UploadPlan(), false, nullptr);  // the whole frame
-    if (st != VT_OK) return st;
+    return VT_OK;
+}
+
+// The template pass of vt_tracker_init[_surface] on the device frame fd: template crop -> patch embed (+ LN1 of block 0) of `target`,
+// which then joins the active targets with rect_last = box.
+static vt_status init_template(vt_tracker* t, int32_t target, vt_bbox box, const FrameDesc& fd) {
     TargetState hs;
     memset(&hs, 0, sizeof(hs));
     hs.rect[0] = box.x, hs.rect[1] = box.y, hs.rect[2] = box.width, hs.rect[3] = box.height, hs.active = 1;
@@ -814,7 +875,6 @@ vt_status vt_tracker_init(vt_tracker* t, int32_t target, const uint8_t* frame, s
     VT_CUDA(cudaMemcpyAsync(t->d_state + target, &hs, sizeof(hs), cudaMemcpyHostToDevice, t->stream));
     // d_slots is reused as a one-element list for the template pass, then restored
     VT_CUDA(cudaMemcpyAsync(t->d_slots, &slot, sizeof(slot), cudaMemcpyHostToDevice, t->stream));
-    FrameDesc fd{t->d_frame, t->W, t->H, t->fmt, t->frame_valid, nullptr, t->cfg.pad_plus1};
     int launches = 0;
     VT_LAUNCH(launch_crop_resize_norm(fd, t->d_state, t->d_slots, 1, 2, kTemplate, t->d_lut, t->patches_z, (size_t)kNTz * kPatchK, t->pz_hi,
                                       t->f16 ? nullptr : t->pz_lo, t->stream));
@@ -839,6 +899,47 @@ vt_status vt_tracker_init(vt_tracker* t, int32_t target, const uint8_t* frame, s
     }
     t->rect_mirror[target] = box;
     return sync_slots(t);
+}
+
+}  // namespace vt
+
+using namespace vt;
+
+extern "C" {
+
+vt_status vt_tracker_init(vt_tracker* t, int32_t target, const uint8_t* frame, size_t len, vt_bbox box) {
+    if (!t || !frame || target < 0 || target >= t->maxT) {
+        set_error("vt_tracker_init: invalid argument");
+        return VT_ERR_INVALID;
+    }
+    if (t->in_flight) {
+        set_error("vt_tracker_init: a frame is in flight");
+        return VT_ERR_INVALID;
+    }
+    VT_CUDA(cudaSetDevice(t->cfg.device));
+    vt_status st = check_template_window(t, box, "vt_tracker_init");
+    if (st != VT_OK) return st;
+    st = do_upload(t, frame, len, UploadPlan(), false, nullptr);  // the whole frame
+    if (st != VT_OK) return st;
+    return init_template(t, target, box, FrameDesc{t->d_frame, nullptr, {0, 0}, t->W, t->H, t->fmt, t->frame_valid, nullptr, t->cfg.pad_plus1});
+}
+
+vt_status vt_tracker_init_surface(vt_tracker* t, int32_t target, const vt_surface* s, vt_bbox box) {
+    if (!t || !s || target < 0 || target >= t->maxT) {
+        set_error("vt_tracker_init_surface: invalid argument");
+        return VT_ERR_INVALID;
+    }
+    if (t->in_flight) {
+        set_error("vt_tracker_init_surface: a frame is in flight");
+        return VT_ERR_INVALID;
+    }
+    vt_status st = surface_call(t, "vt_tracker_init_surface", true);
+    if (st == VT_OK) st = check_surface(t, s, "vt_tracker_init_surface", 0);
+    if (st == VT_OK) st = check_template_window(t, box, "vt_tracker_init_surface");
+    if (st != VT_OK) return st;
+    const bool nv12 = t->fmt == VT_FMT_NV12;
+    return init_template(t, target, box, FrameDesc{s->planes[0], nv12 ? s->planes[1] : nullptr, {s->pitch[0], nv12 ? s->pitch[1] : 0}, t->W, t->H,
+                                                   t->fmt, 1, nullptr, t->cfg.pad_plus1});
 }
 
 vt_status vt_tracker_drop(vt_tracker* t, int32_t target) {
@@ -895,7 +996,7 @@ vt_status vt_tracker_update(vt_tracker* t, uint8_t* frame, size_t len, vt_result
 vt_status vt_tracker_update_streams(vt_tracker* t, uint8_t* const* frames, const size_t* lens, int32_t n, vt_result* results) {
     if (!t || !frames || !lens) return VT_ERR_INVALID;
     VT_CUDA(cudaSetDevice(t->cfg.device));
-    vt_status st = submit_streams(t, frames, lens, n);
+    vt_status st = submit_streams(t, frames, lens, nullptr, n);
     if (st != VT_OK) return st;
     return wait_common(t, results);
 }
@@ -908,6 +1009,31 @@ vt_status vt_tracker_update_device(vt_tracker* t, uint8_t* d_frame, size_t len, 
         return VT_ERR_INVALID;
     }
     vt_status st = submit_common(t, nullptr, d_frame, len);
+    if (st != VT_OK) return st;
+    return wait_common(t, results);
+}
+
+vt_status vt_tracker_update_surface(vt_tracker* t, const vt_surface* s, vt_result* results) {
+    if (!t || !s) return VT_ERR_INVALID;
+    vt_status st = surface_call(t, "vt_tracker_update_surface", true);
+    if (st == VT_OK) st = check_surface(t, s, "vt_tracker_update_surface", 0);
+    if (st == VT_OK) st = submit_common(t, nullptr, nullptr, 0, true, s);
+    if (st != VT_OK) return st;
+    return wait_common(t, results);
+}
+
+vt_status vt_tracker_submit_surface(vt_tracker* t, const vt_surface* s) {
+    if (!t || !s) return VT_ERR_INVALID;
+    vt_status st = surface_call(t, "vt_tracker_submit_surface", false);
+    if (st == VT_OK) st = check_surface(t, s, "vt_tracker_submit_surface", 0);
+    if (st != VT_OK) return st;
+    return submit_common(t, nullptr, nullptr, 0, true, s);
+}
+
+vt_status vt_tracker_update_streams_surface(vt_tracker* t, const vt_surface* surfaces, int32_t n, vt_result* results) {
+    if (!t || !surfaces) return VT_ERR_INVALID;
+    VT_CUDA(cudaSetDevice(t->cfg.device));
+    vt_status st = submit_streams(t, nullptr, nullptr, surfaces, n);
     if (st != VT_OK) return st;
     return wait_common(t, results);
 }
@@ -979,7 +1105,7 @@ vt_status vt_tracker_run_streams_ring(vt_tracker* t, uint8_t* const* rings, int3
         const size_t off = (size_t)((first + i) % ring) * stride;
         for (int k = 0; k < n_streams; ++k) fr[k] = rings[k] + off, lens[k] = frame_len;
         const auto t0 = std::chrono::steady_clock::now();
-        st = submit_streams(t, fr, lens, n_streams);
+        st = submit_streams(t, fr, lens, nullptr, n_streams);
         if (st == VT_OK) st = wait_common(t, res.data());
         if (latency_us) latency_us[i] = std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - t0).count();
         if (st == VT_OK && pristine && t->cfg.box_overlay)  // undo what the box overlays drew: the rings are replayed on clean frames

@@ -124,6 +124,8 @@ struct OverlayCmdDev;
 constexpr int kMaxWin = 16;
 struct FrameCtl {
     const uint8_t* frame;      // device frame this step reads: the handle's own buffer, or the caller's device frame tracked in place
+    const uint8_t* uv;         // NV12 chroma plane of `frame`; null: packed behind the Y plane (frame + W * H)
+    size_t pitch[2];           // row pitch of `frame` / `uv` in bytes (pitched device surfaces); 0: packed rows
     uint8_t* host_frame;       // the caller's PINNED host frame (device-mapped under UVA) or null: zero-copy target of the overlay mirror
                                // and the crop kernel's fall-back source for pixels outside the uploaded windows
     uint32_t* hblk;            // pinned host result block of the frame's queue slot
@@ -133,6 +135,8 @@ struct FrameCtl {
     int32_t win[kMaxWin][4];   // x0, y0, x1, y1 (exclusive), even-aligned
     // stream groups (vt_tracker_update_streams): active target i reads — and is drawn into — its OWN frame; null = `frame` / `host_frame`
     const uint8_t* frames[kMaxWin];
+    const uint8_t* uvs[kMaxWin];          // chroma plane and row pitches of frames[i], as `uv` / `pitch` of `frame`
+    size_t pitches[kMaxWin][2];
     uint8_t* host_frames[kMaxWin];
     int32_t bg_on_device;      // the region a leading HUD background dim reads was uploaded with the windows: read it from the device frame
     int32_t bg_ready;          // set by the host-pass CTA of the overlay kernel once its copy of that region is in registers (reset per frame)
@@ -147,7 +151,9 @@ cudaError_t launch_publish(const void* d_blk, const FrameCtl* d_ctl, size_t byte
 
 // ---- pixel kernels (pixel.cu) ------------------------------------------------------------------
 struct FrameDesc {
-    const uint8_t* data;   // device pointer, tightly packed
+    const uint8_t* data;   // device pointer: the frame (plane 0: Y / RGB / gray)
+    const uint8_t* uv;     // NV12 chroma plane; null: packed behind the Y plane (data + W * H)
+    size_t pitch[2];       // row pitch of data / uv in bytes; 0: packed rows
     int32_t width, height;
     int32_t format;        // vt_format
     int32_t valid;         // 0: buffer was short -> black image (src/nv12_convert.rs:48-50)

@@ -159,6 +159,25 @@ vt_status vt_tracker_update_streams(vt_tracker* t, uint8_t* const* frames, const
  * probe (src/pipeline.rs:90-100,165-168) on a device surface. */
 vt_status vt_tracker_update_device(vt_tracker* t, uint8_t* d_frame, size_t len, vt_result* results);
 
+/* A frame in device memory on the handle's GPU, in the handle's format, with any row pitch (decoder surfaces: NVDEC, NvBufSurface).
+ * NV12: planes[0] = Y (H rows), planes[1] = interleaved UV ((H+1)/2 rows); RGB24 / GRAY8: planes[0] only, planes[1] ignored.
+ * pitch[i] >= the plane's row bytes (W for Y / UV / GRAY8, 3W for RGB24); planes may be separate allocations and need no alignment.
+ * A tightly packed frame d is the surface {d, d + W*H}, {W, W} (RGB24: {d, NULL}, {3W, 0}).
+ *
+ * The surface entry points below are additive (VT_ABI_VERSION stays 2): each behaves like the entry point it names, except that the
+ * frame is a surface.  The tracker reads the surface in place (nothing is copied), and with cfg.box_overlay draws the box into it: into
+ * planes[0] (the Y plane for NV12 / GRAY8, the image for RGB24) with the reference's clamping, so nothing is written into the pitch
+ * padding or the UV plane.  The surface must stay valid until the call returns (submit: until the matching wait()).
+ * VT_ERR_INVALID (and vt_last_error()) for a NULL surface or plane, a pitch below the plane's row bytes, a plane that is not device or
+ * managed memory of cfg.device, a probe (HUD) handle, and — synchronous calls — frames in flight. */
+typedef struct { uint8_t* planes[2]; size_t pitch[2]; } vt_surface;
+vt_status vt_tracker_init_surface(vt_tracker* t, int32_t target, const vt_surface* s, vt_bbox box);  /* ≙ vt_tracker_init */
+vt_status vt_tracker_update_surface(vt_tracker* t, const vt_surface* s, vt_result* results);         /* ≙ vt_tracker_update_device */
+vt_status vt_tracker_submit_surface(vt_tracker* t, const vt_surface* s);                             /* ≙ vt_tracker_submit_device; then wait() */
+/* ≙ vt_tracker_update_streams: surfaces[i] belongs to the i-th active target (n = the number of active targets, at most 16); each stream's
+ * box is drawn into its own surface.  Streams may have different pitches and plane offsets. */
+vt_status vt_tracker_update_streams_surface(vt_tracker* t, const vt_surface* surfaces, int32_t n, vt_result* results);
+
 /* The per-buffer loop of a streaming thread, run natively (≙ the GStreamer streaming thread invoking the probe once per buffer,
  * src/pipeline.rs:65-67): n frames of a ring (`ring` frames of frame_len bytes, `stride` bytes apart, starting at index `first`,
  * wrapping) go through this handle.  `frames` is host memory for the HOST modes (pinned for pipelining) and device memory for the
