@@ -94,6 +94,14 @@ def _ptr(a: np.ndarray) -> C.c_void_p:
     return C.c_void_p(a.ctypes.data)
 
 
+FORMATS = {"nv12": L.VT_FMT_NV12, "rgb24": L.VT_FMT_RGB24, "gray8": L.VT_FMT_GRAY8, "yuy2": L.VT_FMT_YUY2}
+
+
+def row_bytes(fmt: str, width: int) -> int:
+    """Bytes of one packed row of plane 0 (the Y plane, the RGB / gray image, the packed YUY2 words: 4 * ceil(width / 2))."""
+    return 4 * ((width + 1) // 2) if fmt == "yuy2" else width * (3 if fmt == "rgb24" else 1)
+
+
 Surface = Tuple[Sequence[int], Sequence[int]]  # ((plane 0 address, plane 1 address), (pitch 0, pitch 1)): device addresses, bytes
 
 
@@ -117,7 +125,7 @@ class PitchedFrame:
         import torch
 
         self.width, self.height, self.fmt = width, height, fmt
-        self.row = width * (3 if fmt == "rgb24" else 1)
+        self.row = row_bytes(fmt, width)
         self.pitch = pitch if pitch is not None else self.row
         if self.pitch < self.row:
             raise ValueError("pitch is smaller than a row")
@@ -182,7 +190,7 @@ def make_config(weights: str, width: int, height: int, fmt: str = "nv12", max_ta
         weights = _import_onnx_cached(weights)
     cfg.weights_path = weights.encode()
     cfg.device = device
-    cfg.format = {"nv12": L.VT_FMT_NV12, "rgb24": L.VT_FMT_RGB24, "gray8": L.VT_FMT_GRAY8}[fmt]
+    cfg.format = FORMATS[fmt]
     cfg.width, cfg.height, cfg.max_targets = width, height, max_targets
     cfg.score_threshold = score_threshold
     cfg.gemm_mode = gemm_mode

@@ -488,14 +488,13 @@ vt_status vt_context_run_ring(vt_context* c, uint8_t* frames, size_t stride, siz
 vt_status vt_probe_frame(vt_context* c, uint8_t* frame, size_t len, const char* const* hud_override) {
     if (!c || !c->tracker || !frame) return VT_ERR_INVALID;
     vt_tracker* t = c->tracker;
-    const bool nv12 = vt::format_is_luma(c->cfg.format);  // GRAY8 frames take the luma-plane HUD of src/pipeline.rs:125-174
+    const bool nv12 = vt::format_is_luma(c->cfg.format);  // GRAY8 / YUY2 frames take the luma-plane HUD of src/pipeline.rs:125-174
     // interval timing, src/pipeline.rs:69-79
     const auto now = std::chrono::steady_clock::now();
     if (c->have_last) vt_timing_add_interval(t, (uint64_t)std::chrono::duration_cast<std::chrono::microseconds>(now - c->last_time).count());
     c->last_time = now, c->have_last = true;
     const uint64_t num = c->frame_num++;
-    const size_t need = c->cfg.format == VT_FMT_NV12 ? (size_t)c->frame_width * c->frame_height * 3 / 2
-                                                     : (size_t)c->frame_width * c->frame_height * (c->cfg.format == VT_FMT_RGB24 ? 3 : 1);
+    const size_t need = vt::fmt_valid_bytes(c->cfg.format, c->frame_width, c->frame_height);
     const vt_status st = (len >= need && vt::frame_is_pinned(frame)) ? probe_one_sync(c, frame, len, hud_override, nv12)
                                                                                 : probe_two_step(c, frame, len, hud_override, nv12);
     if (st != VT_OK) return st;

@@ -437,7 +437,15 @@ struct PixelSrc {
     size_t pitch, uv_pitch;       // their row pitches
     const uint8_t* host;          // null: everything is on the device
     int x0, y0, x1, y1;           // valid window of the device frame (even-aligned, so a pixel and its chroma pair sit on the same side)
+    bool dev_words, host_words;   // YUY2: the plane's pixel-pair words are 4-byte aligned (base and pitch), one 32-bit load each
 };
+
+// the Y0 U Y1 V word of pixel fx in a YUY2 row: one 32-bit load when aligned, else four byte loads (surfaces may have any pitch)
+__device__ __forceinline__ uint32_t yuy2_word(const uint8_t* row, int fx, bool aligned) {
+    const uint8_t* q = row + 4 * (fx >> 1);
+    if (aligned) return *reinterpret_cast<const uint32_t*>(q);
+    return (uint32_t)q[0] | ((uint32_t)q[1] << 8) | ((uint32_t)q[2] << 16) | ((uint32_t)q[3] << 24);
+}
 
 // RGB of the frame pixel (fx, fy); zero outside the frame (constant border of the crop).
 __device__ __forceinline__ void frame_rgb(const FrameDesc& f, const PixelSrc& ps, int fx, int fy, int& r, int& g, int& b) {
@@ -452,6 +460,11 @@ __device__ __forceinline__ void frame_rgb(const FrameDesc& f, const PixelSrc& ps
         r = p[0], g = p[1], b = p[2];
     } else if (f.format == VT_FMT_GRAY8) {
         r = g = b = data[(size_t)fy * (host ? (size_t)f.width : ps.pitch) + fx];
+    } else if (f.format == VT_FMT_YUY2) {
+        const uint32_t w = yuy2_word(data + (size_t)fy * (host ? fmt_row_bytes(VT_FMT_YUY2, f.width) : ps.pitch), fx,
+                                     host ? ps.host_words : ps.dev_words);
+        const Chroma c = chroma_terms((int)((w >> 8) & 0xff), (int)(w >> 24));
+        yuv_px((int)((w >> ((fx & 1) * 16)) & 0xff), c, r, g, b);
     } else {
         const int yv = data[(size_t)fy * (host ? (size_t)f.width : ps.pitch) + fx];
         const uint8_t* uv = host ? ps.host + (size_t)f.width * f.height : ps.dev_uv;
@@ -483,9 +496,11 @@ __global__ void __launch_bounds__(256) crop_resize_norm_kernel(FrameDesc f, Targ
             else ps.x1 = ps.y1 = 0;  // nothing of this target was uploaded
         }
     }
-    if (!ps.pitch) ps.pitch = (size_t)f.width * (f.format == VT_FMT_RGB24 ? 3 : 1);  // packed frame
+    if (!ps.pitch) ps.pitch = fmt_row_bytes(f.format, f.width);  // packed frame
     if (!ps.dev_uv) ps.dev_uv = ps.dev + (size_t)f.width * f.height;
     if (!ps.uv_pitch) ps.uv_pitch = (size_t)f.width;
+    ps.dev_words = ((reinterpret_cast<uintptr_t>(ps.dev) | ps.pitch) & 3) == 0;
+    ps.host_words = (reinterpret_cast<uintptr_t>(ps.host) & 3) == 0;  // (packed YUY2 rows are whole words)
     const int slot = slots[bi];
     TargetState* st = state + slot;
     const int bx = st->rect[0], by = st->rect[1], bw = st->rect[2], bh = st->rect[3];
@@ -710,9 +725,13 @@ struct Surface {
     size_t len;            // bytes of the drawn plane (RGB writes are bounds-checked against it)
     int W, H, fmt;
     size_t pitch;          // row pitch of the drawn plane in bytes (Y plane / RGB image)
+    int step;              // luma formats: bytes between the Y samples of a row (1; YUY2: 2, the chroma bytes in between are never written)
 };
+__device__ __forceinline__ Surface make_surface(uint8_t* d, size_t len, int W, int H, int fmt, size_t pitch) {
+    return Surface{d, len, W, H, overlay_format(fmt), pitch, fmt_px_step(fmt)};
+}
 // NV12: luma write (Y plane). RGB: bounds-checked colour write (src/drawing_rgb.rs:18-28).
-__device__ __forceinline__ void put_y(const Surface& s, u64 x, u64 y, uint8_t v) { s.d[y * (u64)s.pitch + x] = v; }
+__device__ __forceinline__ void put_y(const Surface& s, u64 x, u64 y, uint8_t v) { s.d[y * (u64)s.pitch + x * (u64)s.step] = v; }
 __device__ __forceinline__ void put_rgb(const Surface& s, int x, int y, uint8_t r, uint8_t g, uint8_t b) {
     if (x < 0 || y < 0 || x >= s.W || y >= s.H) return;
     const size_t off = (size_t)y * s.pitch + (size_t)x * 3;
@@ -807,7 +826,7 @@ __device__ void ov_background(const Surface& s, const OverlayCmdDev& c) {
         const u64 nx = x1 - x0, n = nx * (y1 - y0);
         const unsigned factor = 255u - (unsigned)(uint8_t)c.a;
         for (u64 i = threadIdx.x; i < n; i += blockDim.x) {
-            const u64 idx = (y0 + i / nx) * (u64)s.pitch + x0 + i % nx;
+            const u64 idx = (y0 + i / nx) * (u64)s.pitch + (x0 + i % nx) * (u64)s.step;
             s.d[idx] = (uint8_t)(((unsigned)s.d[idx] * factor) / 255u);
         }
     } else {  // src/drawing_rgb.rs:30-53: fill with 30
@@ -879,7 +898,7 @@ __device__ void ov_dispatch(const Surface& s, const OverlayCmdDev& c) {
 
 __global__ void __launch_bounds__(1024) overlay_kernel(uint8_t* frame, size_t len, int W, int H, int fmt,
                                                        const OverlayCmdDev* __restrict__ cmds, int n) {
-    Surface s{frame, len, W, H, fmt, (size_t)W * (fmt == VT_FMT_RGB24 ? 3 : 1)};
+    const Surface s = make_surface(frame, len, W, H, fmt, fmt_row_bytes(fmt, W));
     for (int i = 0; i < n; ++i) {
         ov_dispatch(s, cmds[i]);
         __syncthreads();
@@ -926,25 +945,29 @@ __device__ void hud_score_glyphs(OverlayCmdDev& c, float score) {  // "score: " 
 constexpr int kOvThreads = 512;
 constexpr int kBgEdge = 2;    // ragged-edge bytes per thread held in registers (rows x <= 6 columns)
 constexpr int kBgWords = 20;  // words per thread held in registers: 512 x 20 x 4 = 40 KB >= the 400 x 80 HUD block
+// Pixels are addressed as row * y + step * x (step: the Y sample step of the format, 1 or 2); a word holds 4 / step pixels, and of a
+// YUY2 word only bytes 0 and 2 (Y0, Y1) are dimmed.
 struct BgRegion {
     long long x0, y0, x1, y1;  // clipped pixel rectangle (usize arithmetic of the reference), empty when x1 <= x0
-    long long ax0, ax1;        // 4-byte aligned interior of a row: [ax0, ax1), ax0 >= x0, ax1 <= x1
+    long long ax0, ax1;        // word-aligned interior of a row in pixels: [ax0, ax1), ax0 >= x0, ax1 <= x1
     int wpr;                   // words per row
-    bool vec;                  // rows are word addressable (W % 4 == 0)
+    bool vec;                  // rows are word addressable (row bytes % 4 == 0)
 };
-__device__ BgRegion bg_region(const OverlayCmdDev& c, int W, int H) {
+__device__ BgRegion bg_region(const OverlayCmdDev& c, int W, int H, size_t row, int step) {
     BgRegion g;
     const u64 x0 = (u64)c.x, y0 = (u64)c.y;
     const u64 x1 = umin64(x0 + (u64)c.w, (u64)W), y1 = umin64(y0 + (u64)c.h, (u64)H);
     g.x0 = (long long)x0, g.y0 = (long long)y0, g.x1 = x1 > x0 && y1 > y0 ? (long long)x1 : (long long)x0, g.y1 = (long long)y1;
-    g.vec = (W % 4) == 0;
-    g.ax0 = (g.x0 + 3) & ~3LL, g.ax1 = g.x1 & ~3LL;
-    g.wpr = g.vec && g.ax1 > g.ax0 ? (int)((g.ax1 - g.ax0) >> 2) : 0;
+    g.vec = (row % 4) == 0;
+    const long long ppw = 4 / step;  // pixels per word
+    g.ax0 = (g.x0 + ppw - 1) & ~(ppw - 1), g.ax1 = g.x1 & ~(ppw - 1);
+    g.wpr = g.vec && g.ax1 > g.ax0 ? (int)((g.ax1 - g.ax0) / ppw) : 0;
     return g;
 }
-__device__ __forceinline__ uint32_t dim4(uint32_t v, unsigned factor) {
-    return ((v & 0xff) * factor / 255u) | ((((v >> 8) & 0xff) * factor / 255u) << 8) | ((((v >> 16) & 0xff) * factor / 255u) << 16) |
-           (((v >> 24) * factor / 255u) << 24);
+__device__ __forceinline__ uint32_t dim4(uint32_t v, unsigned factor, int step) {
+    const uint32_t d = ((v & 0xff) * factor / 255u) | ((((v >> 8) & 0xff) * factor / 255u) << 8) |
+                       ((((v >> 16) & 0xff) * factor / 255u) << 16) | (((v >> 24) * factor / 255u) << 24);
+    return step == 2 ? (d & 0x00ff00ffu) | (v & 0xff00ff00u) : d;
 }
 
 __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int W, int H, int fmt, const DeviceResult* __restrict__ res,
@@ -965,8 +988,9 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
     uint8_t* const frame = frame0;
     uint8_t* const host = host0;
     // row pitch of the drawn plane: the caller's surface pitch for the device frame; the pinned host frame is packed.  (The HUD paths
-    // below address rows by W: HUD handles take packed frames only.)
-    const size_t row = (size_t)W * (fmt == VT_FMT_RGB24 ? 3 : 1);
+    // below address packed rows: HUD handles take packed frames only.)  fmt is the frame's format: drawn with the overlay semantics of ofmt
+    const size_t row = fmt_row_bytes(fmt, W);
+    const int ofmt = overlay_format(fmt), step = fmt_px_step(fmt);
     const size_t fpitch0 = own ? ctl->pitches[blockIdx.x][0] : ctl->pitch[0];
     const size_t fpitch = fpitch0 ? fpitch0 : row;
     const bool do_dev = !split || blockIdx.y == 0, do_host = host != nullptr && (!split || blockIdx.y == 1);
@@ -979,25 +1003,25 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
         __syncthreads();
     }
     // the luma background dim, if it leads the list unconditionally (the probe's HUD): prefetch its pixels from the host frame now
-    const bool bg_first = n_hud > 0 && fmt == VT_FMT_NV12 && s_cmd[0].kind == VT_OV_BACKGROUND && s_cmd[0].cond == VT_HUD_ALWAYS;
+    const bool bg_first = n_hud > 0 && ofmt == VT_FMT_NV12 && s_cmd[0].kind == VT_OV_BACKGROUND && s_cmd[0].cond == VT_HUD_ALWAYS;
     BgRegion bg{0, 0, 0, 0, 0, 0, 0, false};
     uint32_t bgw[kBgWords];
     uint8_t bge[kBgEdge];
     bool bg_pre = false, bg_edge_pre = false;
     if (bg_first) {
-        bg = bg_region(s_cmd[0], W, H);
+        bg = bg_region(s_cmd[0], W, H, row, step);
         const long long rows = bg.y1 - bg.y0;
         if (((reinterpret_cast<uintptr_t>(host) | reinterpret_cast<uintptr_t>(frame)) & 3) != 0) bg.wpr = 0;  // bytewise
         // source of the region: the device frame when it was uploaded with the windows (a copy-engine transfer ahead of the graph; an L2 hit
         // here), else the pinned host frame (PCIe reads: ~12 us for the 260 x 90 block, on the critical path of a short frame)
         const uint8_t* bsrc = (host && !ctl->bg_on_device) ? host : frame;
-        bg_pre = (host || ctl->bg_on_device) && bg.wpr > 0 && rows * bg.wpr <= (long long)kBgWords * kOvThreads && (size_t)bg.y1 * (size_t)W <= len;
+        bg_pre = (host || ctl->bg_on_device) && bg.wpr > 0 && rows * bg.wpr <= (long long)kBgWords * kOvThreads && (size_t)bg.y1 * row <= len;
         if (bg_pre) {
             const int total = (int)rows * bg.wpr;
 #pragma unroll
             for (int k = 0; k < kBgWords; ++k) {
                 const int i = threadIdx.x + k * kOvThreads;
-                if (i < total) bgw[k] = *reinterpret_cast<const volatile uint32_t*>(bsrc + (size_t)(bg.y0 + i / bg.wpr) * W + bg.ax0 + 4 * (i % bg.wpr));
+                if (i < total) bgw[k] = *reinterpret_cast<const volatile uint32_t*>(bsrc + (size_t)(bg.y0 + i / bg.wpr) * row + bg.ax0 * step + 4 * (i % bg.wpr));
             }
             // ... and the columns outside the word interior (<= 3 + 3 per row), so that nothing of the region is read after the dependency
             // wait: with two CTAs per target the other CTA dims the device frame's copy of the region after its own wait
@@ -1010,7 +1034,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
                     if (i < rows * ec) {
                         const uint32_t rq = (uint32_t)i / (uint32_t)ec;
                         const long long yy = bg.y0 + rq, kk = i - (long long)rq * ec, xx = kk < eh ? bg.x0 + kk : bg.ax1 + (kk - eh);
-                        bge[k] = *reinterpret_cast<const volatile uint8_t*>(bsrc + (size_t)yy * W + (size_t)xx);
+                        bge[k] = *reinterpret_cast<const volatile uint8_t*>(bsrc + (size_t)yy * row + (size_t)xx * step);
                     }
                 }
             }
@@ -1047,8 +1071,8 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
             if (!dst) break;
             if ((p == 0 && !do_dev) || (p == 1 && !do_host)) continue;
             const size_t pitch = p == 0 ? fpitch : row;
-            Surface s{dst, pitch * H, W, H, fmt, pitch};
-            if (fmt == VT_FMT_NV12) {
+            const Surface s = make_surface(dst, pitch * H, W, H, fmt, pitch);
+            if (ofmt == VT_FMT_NV12) {
                 ov_rect_nv12(s, x, y, w, h, 3, 255);
                 __syncthreads();
                 ov_crosshair_nv12(s, x + w / 2, y + h / 2, 15, 255);
@@ -1082,7 +1106,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
         if (bg_first) {  // ---- the background dim: word interior from registers (or the device frame), ragged edges bytewise
             const unsigned factor = 255u - (unsigned)(uint8_t)s_cmd[0].a;
             const long long rows = bg.y1 - bg.y0;
-            if (bg.x1 > bg.x0 && (size_t)bg.y1 * (size_t)W <= len) {
+            if (bg.x1 > bg.x0 && (size_t)bg.y1 * row <= len) {
                 if (bg.wpr > 0) {
                     const long long total = rows * bg.wpr;
                     for (long long base = 0; base < total; base += (long long)kBgWords * kOvThreads) {
@@ -1095,7 +1119,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
                                 const long long i = base + threadIdx.x + (long long)k * kOvThreads;
                                 if (i < total) {
                                     const uint32_t rr = (uint32_t)i / (uint32_t)bg.wpr, cc = (uint32_t)i - rr * (uint32_t)bg.wpr;
-                                    bgw[k] = *reinterpret_cast<const uint32_t*>(src + (size_t)(bg.y0 + rr) * W + bg.ax0 + 4 * cc);
+                                    bgw[k] = *reinterpret_cast<const uint32_t*>(src + (size_t)(bg.y0 + rr) * row + bg.ax0 * step + 4 * cc);
                                 }
                             }
                         }
@@ -1104,8 +1128,8 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
                             const long long i = base + threadIdx.x + (long long)k * kOvThreads;
                             if (i < total) {
                                 const uint32_t rr = (uint32_t)i / (uint32_t)bg.wpr, cc = (uint32_t)i - rr * (uint32_t)bg.wpr;
-                                const size_t o = (size_t)(bg.y0 + rr) * W + bg.ax0 + 4 * cc;
-                                const uint32_t d = dim4(bgw[k], factor);
+                                const size_t o = (size_t)(bg.y0 + rr) * row + bg.ax0 * step + 4 * cc;
+                                const uint32_t d = dim4(bgw[k], factor, step);
                                 if (do_dev) *reinterpret_cast<uint32_t*>(frame + o) = d;
                                 if (do_host) *reinterpret_cast<uint32_t*>(host + o) = d;
                             }
@@ -1118,7 +1142,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
                 for (long long i = threadIdx.x, kk = 0; i < rows * ec; i += blockDim.x, ++kk) {
                     const uint32_t rq = (uint32_t)i / (uint32_t)ec;  // (rows * ec < 2^31)
                     const long long yy = bg.y0 + rq, k = i - (long long)rq * ec, xx = k < eh ? bg.x0 + k : bg.ax1 + (k - eh);
-                    const size_t o = (size_t)yy * W + (size_t)xx;
+                    const size_t o = (size_t)yy * row + (size_t)xx * step;
                     const unsigned v = (bg_edge_pre && bg.wpr > 0) ? (unsigned)bge[kk < kBgEdge ? kk : 0] : (unsigned)(edge_host ? host[o] : frame[o]);
                     const uint8_t d = (uint8_t)((v * factor) / 255u);
                     if (do_dev) frame[o] = d;
@@ -1133,16 +1157,16 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
             if (!dst) break;
             if ((p == 0 && !do_dev) || (p == 1 && !do_host)) continue;
             const size_t pitch = p == 0 ? fpitch : row;
-            Surface s{dst, pitch * H, W, H, fmt, pitch};
+            const Surface s = make_surface(dst, pitch * H, W, H, fmt, pitch);
             for (int i = first; i < n_hud; ++i) {
                 const OverlayCmdDev& c = s_cmd[i];
                 if (c.kind < 0) continue;
-                if (p == 1 && c.kind == VT_OV_BACKGROUND && fmt == VT_FMT_NV12 && !split) {  // (split: this CTA dims the host pixels itself)
+                if (p == 1 && c.kind == VT_OV_BACKGROUND && ofmt == VT_FMT_NV12 && !split) {  // (split: this CTA dims the host pixels itself)
                     // a dim that does not lead the list: the host copy takes the final pixels of the region from the device frame (the
                     // later commands of this pass re-draw what lies on top of it)
-                    const BgRegion g = bg_region(c, W, H);
+                    const BgRegion g = bg_region(c, W, H, row, step);
                     for (long long j = threadIdx.x; j < (g.y1 - g.y0) * (g.x1 - g.x0); j += blockDim.x) {
-                        const size_t o = (size_t)(g.y0 + j / (g.x1 - g.x0)) * W + (size_t)(g.x0 + j % (g.x1 - g.x0));
+                        const size_t o = (size_t)(g.y0 + j / (g.x1 - g.x0)) * row + (size_t)(g.x0 + j % (g.x1 - g.x0)) * step;
                         if (o < len) host[o] = frame[o];
                     }
                 } else {

@@ -324,9 +324,9 @@ static vt_status build_cmds(vt_tracker* t, const vt_overlay_cmd* cmds, int n, st
 static vt_status overlay_impl(vt_tracker* t, uint8_t* frame, size_t len, const vt_overlay_cmd* cmds, int32_t n, bool upload) {
     if (!t || !frame || (n > 0 && !cmds) || t->in_flight) return VT_ERR_INVALID;
     VT_CUDA(cudaSetDevice(t->cfg.device));
-    const size_t need = format_is_luma(t->fmt) ? (size_t)t->W * t->H : 0;
+    const size_t need = format_is_luma(t->fmt) ? fmt_row_bytes(t->fmt, t->W) * t->H : 0;
     if (len < need) {
-        set_error("vt_overlay: frame shorter than its Y plane");
+        set_error("vt_overlay: frame shorter than its Y plane (YUY2: than the packed frame)");
         return VT_ERR_INVALID;
     }
     std::vector<std::pair<int, int>> spans;
@@ -345,7 +345,7 @@ static vt_status overlay_impl(vt_tracker* t, uint8_t* frame, size_t len, const v
         }
     }
     VT_CUDA(cudaMemcpyAsync(t->d_cmds, t->h_cmds, sizeof(OverlayCmdDev) * n, cudaMemcpyHostToDevice, t->stream));
-    cudaError_t e = launch_overlay(t->d_frame, std::min(len, t->frame_bytes), t->W, t->H, overlay_format(t->fmt), t->d_cmds, n, t->stream);
+    cudaError_t e = launch_overlay(t->d_frame, std::min(len, t->frame_bytes), t->W, t->H, t->fmt, t->d_cmds, n, t->stream);
     if (e != cudaSuccess) {
         set_error("overlay launch failed: %s", cudaGetErrorString(e));
         return VT_ERR_CUDA;

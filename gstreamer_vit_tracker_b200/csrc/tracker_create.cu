@@ -273,7 +273,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
     }
     const vt_config* cfg = &cfg_full;
     if (!cfg->weights_path || cfg->width <= 0 || cfg->height <= 0 || cfg->max_targets <= 0 || cfg->max_targets > 64 ||
-        (cfg->format != VT_FMT_NV12 && cfg->format != VT_FMT_RGB24 && cfg->format != VT_FMT_GRAY8)) {
+        (cfg->format != VT_FMT_NV12 && cfg->format != VT_FMT_RGB24 && cfg->format != VT_FMT_GRAY8 && cfg->format != VT_FMT_YUY2)) {
         set_error("vt_tracker_create: invalid configuration");
         return VT_ERR_INVALID;
     }
@@ -297,9 +297,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
     t->cfg = *cfg;
     t->cfg.weights_path = nullptr;
     t->W = cfg->width, t->H = cfg->height, t->fmt = cfg->format, t->maxT = cfg->max_targets;
-    t->frame_bytes = cfg->format == VT_FMT_NV12    ? (size_t)t->W * t->H + (size_t)((t->H + 1) / 2) * t->W + (t->W & 1)
-                     : cfg->format == VT_FMT_GRAY8 ? (size_t)t->W * t->H
-                                                   : (size_t)t->W * t->H * 3;
+    t->frame_bytes = fmt_frame_bytes(t->fmt, t->W, t->H);
     t->threshold = cfg->score_threshold > 0.f ? cfg->score_threshold : 0.20f;
     t->debug_capture = cfg->debug_capture;
     read_switches(t);

@@ -235,7 +235,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const Forw
         VT_LAUNCH(launch_decode(t->H1, C, t->h2_w, t->h2_b, t->d_hann, t->d_state, t->d_slots, n, t->threshold, t->d_res, t->d_maps, t->d_stamps, s,
                                 t->cfg.decode_window));
     if (t->cfg.box_overlay || t->hud_mode)  // box overlay and / or the frame's HUD list, pinned-frame mirror, ... and publishes the result block
-        VT_LAUNCH(launch_box_overlay(t->frame_bytes, t->W, t->H, overlay_format(t->fmt), t->d_res, t->d_slots, n, t->cfg.overlay_gate, t->d_ctl,
+        VT_LAUNCH(launch_box_overlay(t->frame_bytes, t->W, t->H, t->fmt, t->d_res, t->d_slots, n, t->cfg.overlay_gate, t->d_ctl,
                                      t->d_stamps + ST_OVL_END, s, f.pdl, t->d_res, t->res_block_bytes, t->cfg.box_overlay | (t->hud_mode ? 1 << 16 : 0)));
     else  // results, stage stamps and the error flag -> the pinned host block of this frame's queue slot
         VT_LAUNCH(launch_publish(t->d_res, t->d_ctl, t->res_block_bytes, s, f.pdl));
@@ -315,13 +315,42 @@ struct UploadPlan {
     int rmw[4] = {0, 0, 0, 0};
     size_t bytes = 0;
 };
+// Window uploads need windows whose pixels carry their own chroma: even x0 (NV12 chroma pairs, YUY2 words) and, for NV12, even y0.
+// YUY2 takes any W and H: a window that ends on an odd last column copies that column's whole word, and chroma is per row.
+static bool windows_allowed(const vt_tracker* t) {
+    return t->fmt == VT_FMT_YUY2 || (!(t->W % 2) && !((t->H % 2) && t->fmt == VT_FMT_NV12));
+}
+// bytes of plane 0 that hold the pixels [x0, x1) x [y0, y1) of a packed frame (YUY2: whole words)
+static size_t plane0_bytes(const vt_tracker* t, int x0, int y0, int x1, int y1) {
+    size_t o0, o1;
+    fmt_col_span(t->fmt, x0, x1, &o0, &o1);
+    return (o1 - o0) * (size_t)(y1 - y0);
+}
+// bytes of the window w = (x0, y0, x1, y1): plane 0 and, for NV12, the chroma rows under it
+static size_t window_bytes(const vt_tracker* t, const int* w) {
+    return plane0_bytes(t, w[0], w[1], w[2], w[3]) + (t->fmt == VT_FMT_NV12 ? (size_t)(w[2] - w[0]) * ((w[3] - w[1]) / 2) : 0);
+}
+// one 2D copy of the window w of a packed frame out of plane 0 (+ one of the NV12 chroma rows under it when `chroma`)
+static vt_status copy_window(const vt_tracker* t, uint8_t* dst, const uint8_t* src, const int* w, bool chroma, cudaMemcpyKind kind,
+                             cudaStream_t stream) {
+    const size_t row = fmt_row_bytes(t->fmt, t->W), rows = (size_t)(w[3] - w[1]);
+    size_t o0, o1;
+    fmt_col_span(t->fmt, w[0], w[2], &o0, &o1);
+    const size_t o = (size_t)w[1] * row + o0;
+    VT_CUDA(cudaMemcpy2DAsync(dst + o, row, src + o, row, o1 - o0, rows, kind, stream));
+    if (chroma && t->fmt == VT_FMT_NV12) {
+        const size_t W = (size_t)t->W, uvo = W * t->H + (size_t)(w[1] / 2) * W + w[0];
+        VT_CUDA(cudaMemcpy2DAsync(dst + uvo, W, src + uvo, W, (size_t)(w[2] - w[0]), rows / 2, kind, stream));
+    }
+    return VT_OK;
+}
+
 static void plan_upload(vt_tracker* t, size_t len, bool pinned_host, bool lagging, const int* rmw, UploadPlan& p) {
     p = UploadPlan();
-    const bool valid = (t->fmt == VT_FMT_NV12) ? (len >= (size_t)t->W * t->H * 3 / 2) : (len >= t->frame_bytes);
-    if (!t->cfg.upload_window || !pinned_host || !valid || len < t->frame_bytes || (int)t->active.size() > kMaxWin || (t->W % 2) ||
-        ((t->H % 2) && t->fmt == VT_FMT_NV12) || (t->active.empty() && !t->hud_mode))
+    const bool valid = len >= fmt_valid_bytes(t->fmt, t->W, t->H);
+    if (!t->cfg.upload_window || !pinned_host || !valid || len < t->frame_bytes || (int)t->active.size() > kMaxWin || !windows_allowed(t) ||
+        (t->active.empty() && !t->hud_mode))
         return;
-    const size_t bpp2 = t->fmt == VT_FMT_NV12 ? 3 : (t->fmt == VT_FMT_GRAY8 ? 2 : 6);  // bytes per pixel x 2
     size_t bytes = 0;
     int k = 0;
     for (int s : t->active) {
@@ -332,12 +361,12 @@ static void plan_upload(vt_tracker* t, size_t len, bool pinned_host, bool laggin
         }
         const int sh = t->sw.win_shrink;  // diagnostics: windows too small on purpose exercise the crop kernel's pinned-frame fall-back
         if (sh > 0 && w[2] - w[0] > 4 * sh && w[3] - w[1] > 4 * sh) w[0] += sh, w[1] += sh, w[2] -= sh, w[3] -= sh;
-        bytes += (size_t)(w[2] - w[0]) * (w[3] - w[1]) * bpp2 / 2;
+        bytes += window_bytes(t, w);
     }
     if (rmw && rmw[2] > rmw[0] && rmw[3] > rmw[1] && format_is_luma(t->fmt)) {
         p.has_rmw = true;
         p.rmw[0] = std::max(rmw[0], 0), p.rmw[1] = std::max(rmw[1], 0), p.rmw[2] = std::min(rmw[2], t->W), p.rmw[3] = std::min(rmw[3], t->H);
-        if (p.rmw[2] > p.rmw[0] && p.rmw[3] > p.rmw[1]) bytes += (size_t)(p.rmw[2] - p.rmw[0]) * (p.rmw[3] - p.rmw[1]);
+        if (p.rmw[2] > p.rmw[0] && p.rmw[3] > p.rmw[1]) bytes += plane0_bytes(t, p.rmw[0], p.rmw[1], p.rmw[2], p.rmw[3]);
         else p.has_rmw = false;
     }
     if (bytes * 2 > t->frame_bytes) return;  // not worth the extra copies
@@ -347,31 +376,20 @@ static void plan_upload(vt_tracker* t, size_t len, bool pinned_host, bool laggin
 static vt_status do_upload(vt_tracker* t, const uint8_t* frame, size_t len, const UploadPlan& p, bool device_src, cudaStream_t stream) {
     if (!stream) stream = t->stream;
     size_t n = std::min(len, t->frame_bytes);
-    t->frame_valid = (t->fmt == VT_FMT_NV12) ? (len >= (size_t)t->W * t->H * 3 / 2) : (len >= t->frame_bytes);
+    t->frame_valid = len >= fmt_valid_bytes(t->fmt, t->W, t->H);
     if (!t->frame_valid && t->fmt == VT_FMT_NV12) n = 0;  // src/nv12_convert.rs:48-50 -> black image
     if (n == 0) return VT_OK;
     const cudaMemcpyKind kind = device_src ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
     if (!p.whole) {
-        const size_t W = (size_t)t->W;
         for (int i = 0; i < p.n_win; ++i) {
             const int* w = p.win[i];
-            const size_t cols = (size_t)(w[2] - w[0]), rows = (size_t)(w[3] - w[1]);
-            if (!cols || !rows) continue;
-            if (t->fmt == VT_FMT_GRAY8) {
-                const size_t o = (size_t)w[1] * W + w[0];
-                VT_CUDA(cudaMemcpy2DAsync(t->d_frame + o, W, frame + o, W, cols, rows, kind, stream));
-            } else if (t->fmt == VT_FMT_NV12) {
-                const size_t yo = (size_t)w[1] * W + w[0], uvo = W * t->H + (size_t)(w[1] / 2) * W + w[0];
-                VT_CUDA(cudaMemcpy2DAsync(t->d_frame + yo, W, frame + yo, W, cols, rows, kind, stream));
-                VT_CUDA(cudaMemcpy2DAsync(t->d_frame + uvo, W, frame + uvo, W, cols, rows / 2, kind, stream));
-            } else {
-                const size_t pitch = W * 3, o = (size_t)w[1] * pitch + (size_t)w[0] * 3;
-                VT_CUDA(cudaMemcpy2DAsync(t->d_frame + o, pitch, frame + o, pitch, cols * 3, rows, kind, stream));
-            }
+            if (w[2] == w[0] || w[3] == w[1]) continue;
+            vt_status st = copy_window(t, t->d_frame, frame, w, true, kind, stream);
+            if (st != VT_OK) return st;
         }
-        if (p.has_rmw) {  // luma plane only (the NV12 / GRAY8 background dim reads and writes Y)
-            const size_t o = (size_t)p.rmw[1] * W + p.rmw[0];
-            VT_CUDA(cudaMemcpy2DAsync(t->d_frame + o, W, frame + o, W, (size_t)(p.rmw[2] - p.rmw[0]), (size_t)(p.rmw[3] - p.rmw[1]), kind, stream));
+        if (p.has_rmw) {  // plane 0 only (the luma background dim reads and writes Y)
+            vt_status st = copy_window(t, t->d_frame, frame, p.rmw, false, kind, stream);
+            if (st != VT_OK) return st;
         }
         if (!device_src) t->h2d_bytes += p.bytes;
         t->d_frame_is_last_host_frame = false;  // only windows of the frame are on the device
@@ -453,7 +471,7 @@ void merge_spans(std::vector<std::pair<int, int>>& spans) {
 
 // device -> host copy of whole rows [r0, r1] of the drawable plane (Y plane for NV12, the image for RGB24)
 vt_status download_rows(vt_tracker* t, uint8_t* frame, size_t len, const std::vector<std::pair<int, int>>& spans, bool* staged) {
-    const size_t pitch = (size_t)t->W * (format_is_luma(t->fmt) ? 1 : 3);
+    const size_t pitch = fmt_row_bytes(t->fmt, t->W);
     const bool pinned = is_pinned(frame);
     *staged = !pinned;
     for (auto& sp : spans) {
@@ -467,7 +485,7 @@ vt_status download_rows(vt_tracker* t, uint8_t* frame, size_t len, const std::ve
     return VT_OK;
 }
 void unstage_rows(vt_tracker* t, uint8_t* frame, size_t len, const std::vector<std::pair<int, int>>& spans) {
-    const size_t pitch = (size_t)t->W * (format_is_luma(t->fmt) ? 1 : 3);
+    const size_t pitch = fmt_row_bytes(t->fmt, t->W);
     for (auto& sp : spans) {
         const size_t off = (size_t)sp.first * pitch;
         size_t n = (size_t)(sp.second - sp.first + 1) * pitch;
@@ -504,7 +522,7 @@ static vt_surface packed_surface(const vt_tracker* t, const uint8_t* d) {
     const bool nv12 = t->fmt == VT_FMT_NV12;
     vt_surface s;
     s.planes[0] = const_cast<uint8_t*>(d), s.planes[1] = nv12 ? const_cast<uint8_t*>(d) + (size_t)t->W * t->H : nullptr;
-    s.pitch[0] = (size_t)t->W * (t->fmt == VT_FMT_RGB24 ? 3 : 1), s.pitch[1] = nv12 ? (size_t)t->W : 0;
+    s.pitch[0] = fmt_row_bytes(t->fmt, t->W), s.pitch[1] = nv12 ? (size_t)t->W : 0;
     return s;
 }
 
@@ -517,7 +535,7 @@ static vt_status check_surface(const vt_tracker* t, const vt_surface* s, const c
     }
     const int np = t->fmt == VT_FMT_NV12 ? 2 : 1;
     for (int p = 0; p < np; ++p) {
-        const size_t row = (size_t)t->W * (t->fmt == VT_FMT_RGB24 ? 3 : 1);
+        const size_t row = fmt_row_bytes(t->fmt, t->W);  // (NV12: the chroma rows are W bytes as well)
         if (!s->planes[p]) {
             set_error("%s: surface %d: plane %d is null", where, i, p);
             return VT_ERR_INVALID;
@@ -622,7 +640,7 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
         vt_status st = run_forward(t);
         if (st != VT_OK) return st;
     } else if (n_hud > 0) {  // no tracker runs on this frame (SELECT / LOST states of the probe): HUD list + publish only
-        cudaError_t e = launch_box_overlay(t->frame_bytes, t->W, t->H, overlay_format(t->fmt), t->d_res, t->d_slots, 0, t->cfg.overlay_gate, t->d_ctl,
+        cudaError_t e = launch_box_overlay(t->frame_bytes, t->W, t->H, t->fmt, t->d_res, t->d_slots, 0, t->cfg.overlay_gate, t->d_ctl,
                                            t->d_stamps + ST_OVL_END, t->stream, false, t->d_res, t->res_block_bytes, 0);
         if (e != cudaSuccess) {
             set_error("overlay launch failed: %s", cudaGetErrorString(e));
@@ -671,8 +689,7 @@ static vt_status submit_streams(vt_tracker* t, uint8_t* const* frames, const siz
     q.frame = surfs ? nullptr : frames[0], q.len = surfs ? 0 : lens[0], q.pageable = false, q.hud_bytes = 0, q.mirrored = !surfs;
     FrameCtl ctl;
     memset(&ctl, 0, sizeof(ctl));
-    const bool windows = t->cfg.upload_window && !(t->W % 2) && !((t->H % 2) && t->fmt == VT_FMT_NV12);
-    const size_t W = (size_t)t->W;
+    const bool windows = t->cfg.upload_window && windows_allowed(t);
     for (int i = 0; i < n; ++i) {
         if (surfs) {  // in place: nothing to upload, the whole surface holds the frame
             const bool nv12 = t->fmt == VT_FMT_NV12;
@@ -692,21 +709,9 @@ static vt_status submit_streams(vt_tracker* t, uint8_t* const* frames, const siz
             t->h2d_bytes += t->frame_bytes;
             w[0] = w[1] = 0, w[2] = t->W, w[3] = t->H;
         } else if (search_window(t, t->rect_mirror[t->active[i]], 0, w[0], w[1], w[2], w[3])) {
-            const size_t cols = (size_t)(w[2] - w[0]), rows = (size_t)(w[3] - w[1]);
-            if (t->fmt == VT_FMT_GRAY8) {
-                const size_t o = (size_t)w[1] * W + w[0];
-                VT_CUDA(cudaMemcpy2DAsync(dst + o, W, src + o, W, cols, rows, cudaMemcpyHostToDevice, t->stream));
-                t->h2d_bytes += cols * rows;
-            } else if (t->fmt == VT_FMT_NV12) {
-                const size_t yo = (size_t)w[1] * W + w[0], uvo = W * t->H + (size_t)(w[1] / 2) * W + w[0];
-                VT_CUDA(cudaMemcpy2DAsync(dst + yo, W, src + yo, W, cols, rows, cudaMemcpyHostToDevice, t->stream));
-                VT_CUDA(cudaMemcpy2DAsync(dst + uvo, W, src + uvo, W, cols, rows / 2, cudaMemcpyHostToDevice, t->stream));
-                t->h2d_bytes += cols * rows * 3 / 2;
-            } else {
-                const size_t pitch = W * 3, o = (size_t)w[1] * pitch + (size_t)w[0] * 3;
-                VT_CUDA(cudaMemcpy2DAsync(dst + o, pitch, src + o, pitch, cols * 3, rows, cudaMemcpyHostToDevice, t->stream));
-                t->h2d_bytes += cols * rows * 3;
-            }
+            vt_status st = copy_window(t, dst, src, w, true, cudaMemcpyHostToDevice, t->stream);
+            if (st != VT_OK) return st;
+            t->h2d_bytes += window_bytes(t, w);
         } else {
             w[0] = w[1] = w[2] = w[3] = 0;  // the window misses the frame: the crop kernel flags it
         }
@@ -778,14 +783,17 @@ static vt_status wait_common(vt_tracker* t, vt_result* results) {
 }
 
 // ---- ring replay support ----------------------------------------------------------------------------------------------------------
-// [x0, x1) x [y0, y1) of the drawable plane (Y plane / luma for NV12 and GRAY8, the RGB image otherwise), clipped to the frame
+// [x0, x1) x [y0, y1) of the drawable plane (Y plane / luma for NV12 and GRAY8, the RGB image for RGB24, the whole pixel-pair words
+// for YUY2), clipped to the frame
 void restore_rect_region(uint8_t* frame, const uint8_t* clean, int fmt, int W, int H, long long x0, long long y0, long long x1, long long y1) {
     x0 = std::max(x0, 0LL), y0 = std::max(y0, 0LL), x1 = std::min<long long>(x1, W), y1 = std::min<long long>(y1, H);
     if (x1 <= x0 || y1 <= y0) return;
-    const size_t bpp = format_is_luma(fmt) ? 1 : 3, pitch = (size_t)W * bpp;
+    const size_t pitch = fmt_row_bytes(fmt, W);
+    size_t o0, o1;
+    fmt_col_span(fmt, x0, x1, &o0, &o1);
     for (long long y = y0; y < y1; ++y) {
-        const size_t o = (size_t)y * pitch + (size_t)x0 * bpp;
-        memcpy(frame + o, clean + o, (size_t)(x1 - x0) * bpp);
+        const size_t o = (size_t)y * pitch + o0;
+        memcpy(frame + o, clean + o, o1 - o0);
     }
 }
 // a box overlay touches the box outline (inclusive x..x+w, y..y+h in the luma formats) and a +-15 px crosshair at its centre

@@ -28,9 +28,31 @@ void set_error(const char* fmt, ...);
 // caller's vt_config (any struct_size the ABI ever had) -> the library's full struct with defaults for what the caller's header lacks
 vt_status resolve_config(const vt_config* in, vt_config* out);
 
-// GRAY8 frames are a bare luma plane: drawn on with the NV12 (Y plane) overlay semantics
-inline int overlay_format(int fmt) { return fmt == VT_FMT_GRAY8 ? VT_FMT_NV12 : fmt; }
-inline bool format_is_luma(int fmt) { return fmt == VT_FMT_NV12 || fmt == VT_FMT_GRAY8; }
+// GRAY8 frames are a bare luma plane and YUY2 frames carry one Y sample per pixel: both are drawn on with the NV12 (Y plane)
+// overlay semantics
+__host__ __device__ inline int overlay_format(int fmt) { return fmt == VT_FMT_GRAY8 || fmt == VT_FMT_YUY2 ? VT_FMT_NV12 : fmt; }
+__host__ __device__ inline bool format_is_luma(int fmt) { return fmt == VT_FMT_NV12 || fmt == VT_FMT_GRAY8 || fmt == VT_FMT_YUY2; }
+
+// ---- plane geometry of a format: every site that addresses plane 0 (Y / RGB / gray / packed YUY2) goes through these ----------
+// bytes between horizontally adjacent pixels of plane 0: the RGB triple, the Y sample (YUY2: Y0 U Y1 V, every second byte)
+__host__ __device__ inline int fmt_px_step(int fmt) { return fmt == VT_FMT_RGB24 ? 3 : fmt == VT_FMT_YUY2 ? 2 : 1; }
+// bytes of one packed row of plane 0 (YUY2: whole pixel-pair words, 4 * ceil(W / 2): odd widths pad the last word)
+__host__ __device__ inline size_t fmt_row_bytes(int fmt, int W) {
+    return fmt == VT_FMT_YUY2 ? (size_t)4 * (size_t)((W + 1) / 2) : (size_t)W * (size_t)fmt_px_step(fmt);
+}
+// bytes of a packed frame, every plane
+__host__ __device__ inline size_t fmt_frame_bytes(int fmt, int W, int H) {
+    return fmt == VT_FMT_NV12 ? (size_t)W * H + (size_t)((H + 1) / 2) * W + (W & 1) : fmt_row_bytes(fmt, W) * (size_t)H;
+}
+// the shortest buffer that is a frame; anything shorter is an all-black image (NV12: src/nv12_convert.rs:48-50)
+__host__ __device__ inline size_t fmt_valid_bytes(int fmt, int W, int H) {
+    return fmt == VT_FMT_NV12 ? (size_t)W * H * 3 / 2 : fmt_frame_bytes(fmt, W, H);
+}
+// the bytes [*o0, *o1) of a plane-0 row that hold the pixels x0 .. x1 - 1 (YUY2: the whole words of those pixels)
+__host__ __device__ inline void fmt_col_span(int fmt, long long x0, long long x1, size_t* o0, size_t* o1) {
+    if (fmt == VT_FMT_YUY2) *o0 = (size_t)(2 * (x0 & ~1LL)), *o1 = (size_t)(4 * ((x1 + 1) / 2));
+    else *o0 = (size_t)(x0 * fmt_px_step(fmt)), *o1 = (size_t)(x1 * fmt_px_step(fmt));
+}
 
 #define VT_CUDA(call)                                                                              \
     do {                                                                                           \
@@ -198,6 +220,7 @@ struct OverlayCmdDev {     // device-side copy of vt_overlay_cmd with resolved g
 enum { VT_HUD_ALWAYS = 0, VT_HUD_IF_PASS = 1, VT_HUD_IF_FAIL = 2 };
 enum { VT_HUD_GIVEN = 0, VT_HUD_RESULT_RECT = 1, VT_HUD_RESULT_CROSS = 2, VT_HUD_SCORE_TEXT = 3 };
 constexpr int kHudDigitSlot = 37, kHudPercentSlot = 47;
+// (overlay kernels: `format` is the frame's vt_format; they draw with the semantics of overlay_format(format))
 cudaError_t launch_overlay(uint8_t* d_frame, size_t len, int width, int height, int format, const OverlayCmdDev* d_cmds, int n,
                            cudaStream_t s);
 // device-side box overlay straight from the decode result (rect thickness 3 + crosshair 15, src/pipeline.rs:165-168)

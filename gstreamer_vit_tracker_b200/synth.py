@@ -59,6 +59,27 @@ def rgb_to_nv12(rgb: np.ndarray) -> np.ndarray:
     return out
 
 
+def rgb_to_yuy2(rgb: np.ndarray) -> np.ndarray:
+    """BT.601 limited-range RGB(HWC u8) -> packed YUY2 bytes (words Y0 U Y1 V, rows of 4 * ceil(w/2) bytes, len = 4 * ceil(w/2) * h).
+
+    Any width and height.  Luma as rgb_to_nv12; chroma from the rounded mean of each horizontal pixel pair.  An odd width pads the
+    last word with a copy of the last pixel (its chroma is that pixel's own, Y1 = Y0).
+    """
+    h, w, _ = rgb.shape
+    p = rgb.astype(np.int32)
+    if w % 2:
+        p = np.concatenate([p, p[:, -1:]], axis=1)
+    r, g, b = p[..., 0], p[..., 1], p[..., 2]
+    y = np.clip(((66 * r + 129 * g + 25 * b + 128) >> 8) + 16, 0, 255)
+    m = (p[:, 0::2] + p[:, 1::2] + 1) >> 1
+    mr, mg, mb = m[..., 0], m[..., 1], m[..., 2]
+    u = np.clip(((-38 * mr - 74 * mg + 112 * mb + 128) >> 8) + 128, 0, 255)
+    v = np.clip(((112 * mr - 94 * mg - 18 * mb + 128) >> 8) + 128, 0, 255)
+    out = np.empty((h, p.shape[1] // 2, 4), dtype=np.uint8)
+    out[..., 0], out[..., 1], out[..., 2], out[..., 3] = y[:, 0::2], u, y[:, 1::2], v
+    return out.reshape(-1)
+
+
 def smooth_background(seed: int, w: int, h: int, cell: int = 32) -> np.ndarray:
     """Integer bilinear up-sampling of a coarse hash-noise grid plus 4-bit fine grain."""
     gh, gw = h // cell + 2, w // cell + 2

@@ -46,7 +46,11 @@ enum {
 
 /* VT_FMT_GRAY8: one byte per pixel (IR sensors; BASELINE config "IR/GRAY8 at 640x512"): the tracker sees r = g = b = gray and the
  * overlays follow the NV12 luma-plane semantics (src/nv12_convert.rs:172-343 write the Y plane only). */
-typedef enum { VT_FMT_NV12 = 0, VT_FMT_RGB24 = 1, VT_FMT_GRAY8 = 2 } vt_format;
+/* VT_FMT_YUY2: one plane of packed 4:2:2 words Y0 U Y1 V (most UVC / V4L2 cameras; the IR camera of src/pipeline_ir.rs:27-56), rows
+ * of 4 * ceil(W/2) bytes, so a packed frame is 4 * ceil(W/2) * H bytes; odd W and odd H are allowed.  The tracker sees exactly the RGB
+ * of vt_convert_yuy2_rgb (BT.601 integer arithmetic of src/nv12_convert.rs:24-30,124-126 on the pixel's word); the overlays follow the
+ * NV12 luma-plane semantics and write only the Y samples (byte 2x of row y), never the U / V bytes. */
+typedef enum { VT_FMT_NV12 = 0, VT_FMT_RGB24 = 1, VT_FMT_GRAY8 = 2, VT_FMT_YUY2 = 3 } vt_format;
 /* BF16X3 (default): bf16 hi + lo operands, three products per K-step, scores within ~1e-5 of the fp32 oracle.  BF16 / FP16: single-pass
  * operands, 17 % faster, score error ~1e-3 / ~3e-4 — opt-in (near-tie arg-max flips are possible at that error). */
 typedef enum { VT_GEMM_FP32_SIMT = 0, VT_GEMM_TCGEN05_BF16X3 = 1, VT_GEMM_TCGEN05_BF16 = 2, VT_GEMM_TCGEN05_FP16 = 3 } vt_gemm_mode;
@@ -160,14 +164,14 @@ vt_status vt_tracker_update_streams(vt_tracker* t, uint8_t* const* frames, const
 vt_status vt_tracker_update_device(vt_tracker* t, uint8_t* d_frame, size_t len, vt_result* results);
 
 /* A frame in device memory on the handle's GPU, in the handle's format, with any row pitch (decoder surfaces: NVDEC, NvBufSurface).
- * NV12: planes[0] = Y (H rows), planes[1] = interleaved UV ((H+1)/2 rows); RGB24 / GRAY8: planes[0] only, planes[1] ignored.
- * pitch[i] >= the plane's row bytes (W for Y / UV / GRAY8, 3W for RGB24); planes may be separate allocations and need no alignment.
- * A tightly packed frame d is the surface {d, d + W*H}, {W, W} (RGB24: {d, NULL}, {3W, 0}).
+ * NV12: planes[0] = Y (H rows), planes[1] = interleaved UV ((H+1)/2 rows); RGB24 / GRAY8 / YUY2: planes[0] only, planes[1] ignored.
+ * pitch[i] >= the plane's row bytes (W for Y / UV / GRAY8, 3W for RGB24, 4 * ceil(W/2) for YUY2); planes may be separate allocations
+ * and need no alignment.  A tightly packed frame d is the surface {d, d + W*H}, {W, W} (RGB24: {d, NULL}, {3W, 0}).
  *
  * The surface entry points below are additive (VT_ABI_VERSION stays 2): each behaves like the entry point it names, except that the
  * frame is a surface.  The tracker reads the surface in place (nothing is copied), and with cfg.box_overlay draws the box into it: into
- * planes[0] (the Y plane for NV12 / GRAY8, the image for RGB24) with the reference's clamping, so nothing is written into the pitch
- * padding or the UV plane.  The surface must stay valid until the call returns (submit: until the matching wait()).
+ * planes[0] (the Y plane for NV12 / GRAY8, the Y samples for YUY2, the image for RGB24) with the reference's clamping, so nothing is
+ * written into the pitch padding, the UV plane or the YUY2 chroma bytes.  The surface must stay valid until the call returns (submit: until the matching wait()).
  * VT_ERR_INVALID (and vt_last_error()) for a NULL surface or plane, a pitch below the plane's row bytes, a plane that is not device or
  * managed memory of cfg.device, a probe (HUD) handle, and — synchronous calls — frames in flight. */
 typedef struct { uint8_t* planes[2]; size_t pitch[2]; } vt_surface;
