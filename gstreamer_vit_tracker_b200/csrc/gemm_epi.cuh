@@ -54,10 +54,10 @@ __device__ __forceinline__ int swz(int row, int chunk) {
     return RB == 128 ? (chunk ^ (row & 7)) : (chunk ^ ((row >> 1) & 3));
 }
 
-// CPT (16 or 8) fp32 -> bf16 (hi, lo) into the staging tiles of a BN = 4 CPT column tile
-template <int CPT, bool F16>
+// CPT (16 or 8) fp32 -> bf16 (hi, lo) into the staging tiles: thread (row, g) holds columns CPT g .. of a tile with RB bytes per row
+// (RB = 8 CPT: four threads per row; RB = 128 with CPT = 8: eight threads per row, the 64-row tiles of gemm_tc_kernel)
+template <int CPT, bool F16, int RB = CPT * 8>
 __device__ __forceinline__ void stage_split(const float (&v)[CPT], uint8_t* tile_hi, uint8_t* tile_lo, int row, int g, bool with_lo) {
-    constexpr int RB = CPT * 8;  // bytes per tile row
     uint32_t hi[CPT / 2], lo[CPT / 2];
 #pragma unroll
     for (int j = 0; j < CPT; j += 2) split2_h<F16>(v[j], v[j + 1], hi[j >> 1], lo[j >> 1]);
@@ -87,13 +87,14 @@ struct TileRows {  // (row-in-target, target) of the two 64-row halves of a tile
         }
     }
 };
-// one [128 rows][RB bytes] swizzled tile; col_bytes = byte offset of the tile's first column inside a destination row
-template <int RB>
+// one [ROWS (128 or 64) rows][RB bytes] swizzled tile; col_bytes = byte offset of the tile's first column inside a destination row
+template <int RB, int ROWS = kTcBM>
 __device__ __forceinline__ void tile_to_global(const uint8_t* tile, const TcOut& o, int64_t col_bytes, const TileRows& r, int row_off, int head,
                                                int plane, int tid) {
     constexpr int CH = RB / 16, kRowsPerPass = kTcThreads / CH;  // 8 chunks, 64 rows per pass / 4 chunks, 128 rows in one pass
+    static_assert(ROWS % kRowsPerPass == 0, "whole passes");
 #pragma unroll
-    for (int i = 0; i < kTcBM / kRowsPerPass; ++i) {
+    for (int i = 0; i < ROWS / kRowsPerPass; ++i) {
         const int row = tid / CH + kRowsPerPass * i, ch = tid % CH, half = row >> 6;
         const int tt = r.t[half] + (row & 63) + row_off, b = r.b[half];
         if (tt >= 0 && tt < o.rows && b < o.batch) {
@@ -103,10 +104,11 @@ __device__ __forceinline__ void tile_to_global(const uint8_t* tile, const TcOut&
         }
     }
 }
-// V^T: two unswizzled [BN d][64 tokens] sub-tiles -> rows d_off.. of [targets][heads][64 d][tokens]; sub-tile k holds tokens t[k]..t[k]+63
-template <int BN>
+// V^T: SUBS (two, or one for a 64-row tile) unswizzled [BN d][64 tokens] sub-tiles -> rows d_off.. of [targets][heads][64 d][tokens];
+// sub-tile k holds tokens t[k]..t[k]+63
+template <int BN, int SUBS = 2>
 __device__ __forceinline__ void vt_tile_to_global(const uint8_t* tile, const TcOut& o, const TileRows& r, int head, int d_off, int tid) {
-    constexpr int kPasses = 2 * BN * 8 / kTcThreads;  // 2 sub-tiles x BN rows x 8 chunks over 512 threads
+    constexpr int kPasses = SUBS * BN * 8 / kTcThreads;  // SUBS sub-tiles x BN rows x 8 chunks over 512 threads
 #pragma unroll
     for (int i = 0; i < kPasses; ++i) {
         const int idx = tid + i * kTcThreads, sub = idx / (BN * 8), d = (idx >> 3) % BN, ch = idx & 7, b = r.b[sub];

@@ -29,6 +29,8 @@
 // a share of the epilogue output — a CTA stores at ~26 B/clk, which is what bounds the 32..96 KB epilogues: FC1 chain in three
 // 64-column slices (the GELU'd hidden tile then is a TMEM A operand), QKV scatter as hi / lo replicas, fused-LN GEMM as fp32 / LN-hi /
 // LN-lo replicas.  All forms are re-associations of the same sums (tests/test_gpu_tracker.py::test_kernel_forms_agree).
+// With one target the QKV scatter and the chained FC1 run on 64-row tiles (M = 64 UMMAs: five tiles of 320 rows instead of
+// 128 + 128 + 64, half the epilogue per CTA), the chained product in two slices of 96 columns (tests/test_gpu_gemm_q64.py).
 // 128 x 32 tiles and TMA multicast of the activation tile across column-tile CTAs were measured without gain (DESIGN.md §7).
 // The 3x3 head convolution runs through the same kernel: its A operand is gathered by TMA from the [B,16,16,D] token grid with
 // shifted (possibly negative) coordinates; out-of-bounds elements are zero-filled by the TMA unit = zero padding of the conv.
@@ -45,21 +47,25 @@ constexpr int kTcStages = 3;
 constexpr int kMaxChainN = 192;                 // widest chained second GEMM (TMEM: 128 + N2 <= 512 columns)
 constexpr int kTcBN = 64;                       // column-tile width; the chained GEMM consumes the 64-column hidden tile as its K
 
-template <int NSPLIT>
+// 64-row tiles (BM = 64, M = 64 UMMAs; bf16x3 only): the QKV scatter and the chained FC1 in two slices of kMaxChainN / 2 columns
+constexpr int kChainN64 = kMaxChainN / 2;
+
+template <int NSPLIT, int BM = kTcBM>
 struct TcSmem {
     static constexpr int kParts = NSPLIT == 3 ? 2 : 1;  // NSPLIT: 1 = bf16, 2 = fp16 (single pass), 3 = bf16 hi + lo
+    static constexpr int kTileABytes = BM * kTcBK * 2;  // 16 / 8 KB, one precision part
     static constexpr int kTileBBytes = kTcBN * kTcBK * 2;   // 8 KB
-    static constexpr int kTileOBytes = kTcBM * kTcBN * 2;   // 16 KB: one bf16 output tile, rows of 128 bytes
-    static constexpr int kTileCBytes = kTcBM * kTcBN * 4;   // 32 KB: the fp32 tile as two boxes of [128 rows][128 B]
+    static constexpr int kTileOBytes = BM * kTcBN * 2;      // 16 / 8 KB: one bf16 output tile, rows of 128 bytes
+    static constexpr int kTileCBytes = BM * kTcBN * 4;      // 32 / 16 KB: the fp32 tile as two boxes of [BM rows][128 B]
     static constexpr int kStageBytes = kParts * (kTileABytes + kTileBBytes);
     // the ring is padded (bf16 mode) so that the chained GEMM's result tile fits behind the staged hidden tile
-    static constexpr int kRingMin = 2 * kTileOBytes + kTcBM * kMaxChainN * 4;
+    static constexpr int kRingMin = 2 * kTileOBytes + BM * kMaxChainN * 4;
     static constexpr int kPipeBytes = kTcStages * kStageBytes > kRingMin ? kTcStages * kStageBytes : kRingMin;
     // after the main loop the pipeline ring is dead and holds the staged output tiles
     static constexpr int kOffOhi = 0, kOffOlo = kTileOBytes, kOffLnHi = 2 * kTileOBytes, kOffLnLo = 3 * kTileOBytes;
     static constexpr int kOffC = kPipeBytes;  // fp32 tile: residual in (TMA load during the main loop), C out, in place
     // chained second GEMM (FC2 partial inside the FC1 kernel): its weight slice [N2 <= 192][64] per part lives where the fp32
-    // tile would be, its fp32 result tile [128][N2] is staged in the dead ring behind the two hidden-tile parts
+    // tile would be, its fp32 result tile [BM][N2] is staged in the dead ring behind the two hidden-tile parts
     static constexpr int kOffB2 = kPipeBytes, kB2PartBytes = kMaxChainN * 128, kOffP = 2 * kTileOBytes;
     static constexpr int kTailBytes = kParts * kB2PartBytes > kTileCBytes ? kParts * kB2PartBytes : kTileCBytes;
     static constexpr int kTotal = kPipeBytes + kTailBytes + 1024;  // + alignment slack
@@ -75,42 +81,55 @@ struct TcSmem {
 constexpr int kMaxLnCluster = 8;
 
 
-template <int NSPLIT>
+// BM = 64 (tc_gemm_launch: q64): a 64-row tile with M = 64 UMMAs, for the QKV scatter (hi / lo replicas) and the sliced chained FC1
+// (hidden tile as a TMEM A operand) only.  Row 16 q + i of an M = 64 accumulator sits in TMEM lane 32 q + i (i < 16), so the 16 warps
+// split each row 8 ways (8 columns per thread) through the 16x32bx2 shapes; the fused-LN, split-K, residual, fp32-tile, bf16-tile,
+// conv and unsliced chained epilogues exist for BM = 128 only.
+template <int NSPLIT, int BM>
 __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_constant__ TcMaps mp, const TcGemmArgs a) {
+    static_assert(BM == kTcBM || (BM == 64 && NSPLIT == 3), "64-row tiles: bf16x3 only");
+    constexpr bool kQ64 = BM == 64;
     extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t full_bar[kTcStages], empty_bar[kTcStages], accum_bar, resid_bar, b2_bar, accum2_bar, ln_bar;
     __shared__ uint32_t tmem_base_s;
     __shared__ float2 ln_loc[kTcColGroups][kTcBM];   // (sum, M2) of the CPT columns of thread (row, g)
     __shared__ float2 ln_part[kMaxLnCluster][kTcBM];  // (sum, M2) of the 64 columns of every CTA of the cluster, per row
     __shared__ unsigned long long* trace_slot;
-    using SM = TcSmem<NSPLIT>;
+    using SM = TcSmem<NSPLIT, BM>;
     constexpr int BN = kTcBN;
-    constexpr int CPT = BN / kTcColGroups;   // 16 accumulator columns per thread
-    constexpr int RB = BN * 2;               // bytes per row of a bf16 staging tile
-    constexpr int kTileBBytes = SM::kTileBBytes, kTileOBytes = SM::kTileOBytes, kTileCBytes = SM::kTileCBytes;
+    constexpr int CPT = BN * BM / kTcThreads;  // accumulator columns per thread: 16 (4 threads per row) / 8 (8 threads per row)
+    constexpr int RB = BN * 2;                 // bytes per row of a bf16 staging tile
+    constexpr int kTileABytes = SM::kTileABytes, kTileBBytes = SM::kTileBBytes, kTileOBytes = SM::kTileOBytes, kTileCBytes = SM::kTileCBytes;
     constexpr bool kLo = NSPLIT == 3, kF16 = NSPLIT == 2;
+    const CUtensorMap &mAhi = kQ64 ? mp.Ahi64 : mp.Ahi, &mAlo = kQ64 ? mp.Alo64 : mp.Alo;
+    const CUtensorMap &mB2hi = kQ64 ? mp.B2hiHalf : mp.B2hi, &mB2lo = kQ64 ? mp.B2loHalf : mp.B2lo;
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int row = (warp & 3) * 32 + lane;   // accumulator row inside the tile = TMEM lane
-    const int g = warp >> 2;                  // column group: columns CPT g .. CPT g + CPT - 1 of the tile
-    const int n0 = blockIdx.x * BN, m0 = blockIdx.y * kTcBM;
+    // accumulator row inside the tile; warp w reads TMEM lane quarter w % 4 (BM = 128: row = lane; BM = 64: row 16 q + i in lane 32 q + i)
+    const int row = kQ64 ? (warp & 3) * 16 + (lane & 15) : (warp & 3) * 32 + lane;
+    // column group: columns CPT g .. CPT g + CPT - 1 of the tile (BM = 64: threads 16..31 take the 8 columns after those of threads 0..15)
+    const int g = kQ64 ? 2 * (warp >> 2) + (lane >> 4) : warp >> 2;
+    const uint32_t tq = (uint32_t)((warp & 3) * 32) << 16;  // TMEM lane quarter of the warp (address bits 16..)
+    const uint32_t wcol = kQ64 ? (warp >> 2) * 16 : g * CPT;  // first accumulator column a tcgen05.ld of the warp addresses
+    const int n0 = blockIdx.x * BN, m0 = blockIdx.y * BM;
     // split-K over blockIdx.z: this CTA contracts k-blocks [kb0, kb0 + num_kb) and stores its fp32 partial tile to C[.., z]
     const int num_kb = a.kb_per_split ? a.kb_per_split : a.K / kTcBK;
     const int kb0 = a.kb_per_split ? blockIdx.z * num_kb : 0;
     // "spread" form (latency mode, idle SMs available): blockIdx.z replicates the FC1 tile and replica z computes and stores columns
-    // [64 z, 64 z + 64) of the chained product — a CTA's egress (~26 B/clk/SM) is what bounds the 96 KB partial-tile epilogue.
-    const bool sliced = a.chain_slices > 1;
+    // [N2 z, N2 z + N2) of the chained product — a CTA's egress (~26 B/clk/SM) is what bounds the 96 KB partial-tile epilogue.
+    const bool sliced = a.chain_slices > 1;  // (BM = 64: two slices of kChainN64 columns)
     const int N2 = sliced ? a.chain_n / a.chain_slices : a.chain_n;   // chained columns of this CTA
     const int acc2_cols = (sliced && kLo) ? 2 * N2 : N2;              // sliced + bf16x3: hi*lo term in a second column half
     // dup_ln (spread form of a GEMM with fused LayerNorm): replica 0 stores the fp32 tile, replica 1 the LayerNorm hi tile, replica 2 the lo tile
-    const bool do_ln = a.ln_g != nullptr && (!a.dup_ln || blockIdx.z > 0), do_c = a.c_on && (!a.dup_ln || blockIdx.z == 0);
+    const bool do_ln = !kQ64 && a.ln_g != nullptr && (!a.dup_ln || blockIdx.z > 0), do_c = !kQ64 && a.c_on && (!a.dup_ln || blockIdx.z == 0);
     const bool ln_hi = !a.dup_ln || blockIdx.z == 1, ln_lo = kLo && (!a.dup_ln || blockIdx.z == 2);
     // dup_hl (spread form of the QKV scatter): replica 0 stores the bf16 hi tiles, replica 1 the lo tiles
     const bool st_hi = !a.dup_hl || blockIdx.z == 0, st_lo = kLo && (!a.dup_hl || blockIdx.z == 1);
     const int npre = num_kb < kTcStages ? num_kb : kTcStages;
     constexpr uint32_t kAcc1Cols = kLo ? 2 * BN : BN;  // bf16x3 keeps hi*lo in a second column half
-    constexpr uint32_t kColA2 = 256;  // sliced chain: the hidden tile as a packed bf16 A operand (columns 256..319)
+    // sliced chain: the hidden tile as a packed bf16 A operand, behind the chained accumulator (BM = 128: 2 x 64, BM = 64: 2 x 96 columns)
+    constexpr uint32_t kColA2 = kQ64 ? kAcc1Cols + 2 * kChainN64 : 256;
     const uint32_t tmem_need = a.chain_n == 0 ? kAcc1Cols : ((sliced && kLo) ? kColA2 + 64 : kAcc1Cols + acc2_cols);
     const uint32_t tmem_cols = tmem_need <= 32 ? 32 : (tmem_need <= 64 ? 64 : (tmem_need <= 128 ? 128 : (tmem_need <= 256 ? 256 : 512)));
     bool ok = true;
@@ -119,8 +138,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
 
     // ---- prologue: independent of the preceding kernel, overlaps its tail under PDL
     if (warp == 0 && elect_one_sync()) {  // (one thread; elect.sync lets the compiler issue the TMA instructions without election loops)
-        tma_prefetch_desc(&mp.Ahi), tma_prefetch_desc(&mp.Bhi);
-        if (kLo) tma_prefetch_desc(&mp.Alo), tma_prefetch_desc(&mp.Blo);
+        tma_prefetch_desc(&mAhi), tma_prefetch_desc(&mp.Bhi);
+        if (kLo) tma_prefetch_desc(&mAlo), tma_prefetch_desc(&mp.Blo);
         for (int s = 0; s < kTcStages; ++s) mbar_init(&full_bar[s], 1), mbar_init(&empty_bar[s], 1);
         mbar_init(&accum_bar, 1), mbar_init(&resid_bar, 1), mbar_init(&b2_bar, 1), mbar_init(&accum2_bar, 1), mbar_init(&ln_bar, 1);
         fence_barrier_init();
@@ -134,12 +153,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
             if (kLo) tma_load_2d(sb + kTileBBytes, &mp.Blo, &full_bar[kb], (kb0 + kb) * kTcBK, n0);
         }
         if (a.chain_n) {  // weight slice of the chained GEMM: W2[rows of this CTA][n0 .. n0 + 64), 64-row boxes per precision part
-            tma_prefetch_desc(&mp.B2hi);
+            tma_prefetch_desc(&mB2hi);
             mbar_arrive_expect_tx(&b2_bar, SM::kParts * N2 * 128);
-            if (sliced) {  // [W2_hi slice; W2_lo slice] adjacent: one N = 128 B operand
-                tma_load_2d(smem + SM::kOffB2, &mp.B2hi, &b2_bar, n0, blockIdx.z * N2);
-                if (kLo) tma_load_2d(smem + SM::kOffB2 + N2 * 128, &mp.B2lo, &b2_bar, n0, blockIdx.z * N2);
-            } else {
+            if (sliced) {  // [W2_hi slice; W2_lo slice] adjacent: one N = 2 N2 B operand
+                tma_load_2d(smem + SM::kOffB2, &mB2hi, &b2_bar, n0, blockIdx.z * N2);
+                if (kLo) tma_load_2d(smem + SM::kOffB2 + N2 * 128, &mB2lo, &b2_bar, n0, blockIdx.z * N2);
+            } else if (!kQ64) {
                 for (int r = 0; r < N2; r += 64) {
                     tma_load_2d(smem + SM::kOffB2 + r * 128, &mp.B2hi, &b2_bar, n0, r);
                     if (kLo) tma_load_2d(smem + SM::kOffB2 + SM::kB2PartBytes + r * 128, &mp.B2lo, &b2_bar, n0, r);
@@ -179,16 +198,16 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
                     tma_load_2d(sb, &mp.Bhi, &full_bar[s], (kb0 + kb) * kTcBK, n0);
                     if (kLo) tma_load_2d(sb + kTileBBytes, &mp.Blo, &full_bar[s], (kb0 + kb) * kTcBK, n0);
                 }
-                if (a.conv_feat) {  // 3x3 conv: K index = tap * feat + d; A rows are the 16x16 grid of one target
+                if (!kQ64 && a.conv_feat) {  // 3x3 conv: K index = tap * feat + d; A rows are the 16x16 grid of one target
                     const int chunks = a.conv_feat / kTcBK, tap = (kb0 + kb) / chunks, d0 = ((kb0 + kb) % chunks) * kTcBK;
                     const int b = m0 / kNTx, y0 = (m0 % kNTx) / kMap;
                     tma_load_4d(st, &mp.Ahi, &full_bar[s], d0, tap % 3 - 1, y0 + tap / 3 - 1, b);
                     if (kLo) tma_load_4d(st + kTileABytes, &mp.Alo, &full_bar[s], d0, tap % 3 - 1, y0 + tap / 3 - 1, b);
                 } else {
-                    tma_load_2d(st, &mp.Ahi, &full_bar[s], (kb0 + kb) * kTcBK, m0);
-                    if (kLo) tma_load_2d(st + kTileABytes, &mp.Alo, &full_bar[s], (kb0 + kb) * kTcBK, m0);
+                    tma_load_2d(st, &mAhi, &full_bar[s], (kb0 + kb) * kTcBK, m0);
+                    if (kLo) tma_load_2d(st + kTileABytes, &mAlo, &full_bar[s], (kb0 + kb) * kTcBK, m0);
                 }
-                if (kb == 0 && a.residual) {  // residual rows of this tile (flat [rows][N] fp32), two 128-byte-wide boxes
+                if (!kQ64 && kb == 0 && a.residual) {  // residual rows of this tile (flat [rows][N] fp32), two 128-byte-wide boxes
                     mbar_arrive_expect_tx(&resid_bar, kTileCBytes);
 #pragma unroll
                     for (int bx = 0; bx < BN / 32; ++bx) tma_load_2d(sC + bx * (kTcBM * 128), &mp.R, &resid_bar, n0 + 32 * bx, m0);
@@ -203,7 +222,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
         // accumulator columns [0, 64) (hi*hi) and [64, 128) (hi*lo), then A_lo x W_hi (N = 64) into [0, 64); the epilogue adds the
         // two halves.  (tools/probes/probe_umma.cu: an MMA with both operands in shared memory costs ~43 + N / 2 clk — the 4 KB A slice
         // is fetched before the math starts — so N = 128 + N = 64 (107 + 81 clk) beats three N = 64 MMAs (243 clk).)
-        constexpr uint32_t idesc = umma_idesc_h<kF16>(kTcBM, BN), idesc2n = umma_idesc_h<kF16>(kTcBM, 2 * BN);
+        constexpr uint32_t idesc = umma_idesc_h<kF16>(BM, BN), idesc2n = umma_idesc_h<kF16>(BM, 2 * BN);
         const uint32_t lo0 = umma_desc_lo(smem_u32(smem));
         if (elect_one_sync()) {
             for (int kb = 0; kb < num_kb; ++kb) {
@@ -231,7 +250,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
     // ---- epilogue: thread (row, g) owns 16 accumulator columns of its row
     const int m = m0 + row, nc = n0 + g * CPT;
     // this thread's CPT / 4 16-byte chunks of the fp32 tile: 32-column box (CPT g) / 32, first chunk ((CPT g) % 32) / 4, swizzled
-    uint8_t* c_row = sC + ((g * CPT) >> 5) * (kTcBM * 128) + row * 128;
+    uint8_t* c_row = sC + ((g * CPT) >> 5) * (BM * 128) + row * 128;
     const int c_chunk0 = ((g * CPT) & 31) >> 2, sw = row & 7;
     const TileRows tr_rows(m0, a.period, a.batch_off);
     int o_which = 0, o_h = 0, o_d = 0;
@@ -253,11 +272,15 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
     ok &= mbar_wait(&accum_bar, 0);
     tcgen05_fence_after();
     if (tid == 0) tr.mark(6);
+    auto ld_acc = [&](uint32_t col, float(&x)[CPT]) {  // this thread's CPT accumulator columns from the warp's column `col` on
+        if constexpr (kQ64) tmem_ld_16x2(tmem + tq + col, x);
+        else tmem_ld_cols(tmem + tq + col, x);
+    };
     float v[CPT];
-    tmem_ld_cols(tmem + ((uint32_t)((warp & 3) * 32) << 16) + g * CPT, v);
+    ld_acc(wcol, v);
     if (kLo) {
         float hl[CPT];
-        tmem_ld_cols(tmem + ((uint32_t)((warp & 3) * 32) << 16) + BN + g * CPT, hl);
+        ld_acc(BN + wcol, hl);
 #pragma unroll
         for (int j = 0; j < CPT; ++j) v[j] += hl[j];
     }
@@ -279,7 +302,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
             v[j] += p4.x, v[j + 1] += p4.y, v[j + 2] += p4.z, v[j + 3] += p4.w;
         }
     }
-    if (a.residual) {
+    if (!kQ64 && a.residual) {
         ok &= mbar_wait(&resid_bar, 0);
 #pragma unroll
         for (int q = 0; q < CPT / 4; ++q) {
@@ -310,18 +333,24 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
     // sliced chain: the hidden tile goes back into tensor memory as packed bf16 (thread (row, g) = K-step g: 8 columns hi, 8 columns
     // lo), so the chained UMMAs fetch only the weight slice from shared memory
     const bool a_tmem = sliced && kLo && a.o_mode == 3;
+    // (BM = 64: K-step warp / 4, threads 0..15 its elements 0..7 in columns +0..3 / +8..11, threads 16..31 elements 8..15 in +4..7 / +12..15)
     if (a_tmem) {
-        uint32_t hi[8], lo[8];
+        uint32_t hi[CPT / 2], lo[CPT / 2];
 #pragma unroll
-        for (int j = 0; j < 16; j += 2) split2_bf16(v[j], v[j + 1], hi[j >> 1], lo[j >> 1]);
-        const uint32_t ta = tmem + ((uint32_t)((warp & 3) * 32) << 16) + kColA2 + g * 16;
-        tmem_st_32x8(ta, hi);
-        tmem_st_32x8(ta + 8, lo);
+        for (int j = 0; j < CPT; j += 2) split2_bf16(v[j], v[j + 1], hi[j >> 1], lo[j >> 1]);
+        const uint32_t ta = tmem + tq + kColA2 + (wcol & ~15u);
+        if constexpr (kQ64) {
+            tmem_st_16x2_x4(ta, hi);
+            tmem_st_16x2_x4(ta + 8, lo);
+        } else {
+            tmem_st_32x8(ta, hi);
+            tmem_st_32x8(ta + 8, lo);
+        }
         tmem_st_wait();
     } else if (a.o_mode) {  // (o_mode 3: staged only — the tile is the A operand of the chained GEMM)
         if (o_which < 2) {
-            stage_split<CPT, kF16>(v, smem + SM::kOffOhi, smem + SM::kOffOlo, row, g, kLo);
-        } else {  // V^T: two unswizzled [BN d][64 tokens] sub-tiles; lanes are consecutive tokens -> 64-byte contiguous runs
+            stage_split<CPT, kF16, RB>(v, smem + SM::kOffOhi, smem + SM::kOffOlo, row, g, kLo);
+        } else {  // V^T: BM / 64 unswizzled [BN d][64 tokens] sub-tiles; lanes are consecutive tokens -> 64-byte contiguous runs
             const int sub = (row >> 6) * (BN * kHalfRows) + (g * CPT) * kHalfRows + (row & 63);
             __nv_bfloat16* th = reinterpret_cast<__nv_bfloat16*>(smem + SM::kOffOhi) + sub;
             __nv_bfloat16* tl = reinterpret_cast<__nv_bfloat16*>(smem + SM::kOffOlo) + sub;
@@ -343,7 +372,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
         else fence_proxy_async_smem();  // the staged tile is read by the tensor core (async proxy) in the chained GEMM
     }
     __syncthreads();
-    if (do_ln && g == 0) {  // one thread per row: (sum, M2) over the BN columns of this CTA (Chan), sent to every CTA of the cluster
+    if (!kQ64 && do_ln && g == 0) {  // one thread per row: (sum, M2) over the BN columns of this CTA (Chan), sent to every CTA of the cluster
         float s = 0.f;
 #pragma unroll
         for (int q = 0; q < kTcColGroups; ++q) s += ln_loc[q][row].x;
@@ -365,23 +394,23 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
     if (do_c) {  // split-K partials: plane = blockIdx.z
 #pragma unroll
         for (int bx = 0; bx < BN / 32; ++bx)
-            tile_to_global<128>(sC + bx * (kTcBM * 128), a.c, (int64_t)(n0 + 32 * bx) * 4, tr_rows, a.c_row_off, 0, a.kb_per_split ? blockIdx.z : 0, tid);
+            tile_to_global<128>(sC + bx * (BM * 128), a.c, (int64_t)(n0 + 32 * bx) * 4, tr_rows, a.c_row_off, 0, a.kb_per_split ? blockIdx.z : 0, tid);
     }
-    if (a.o_mode == 1) {
+    if (!kQ64 && a.o_mode == 1) {
         if (st_hi) tile_to_global<RB>(smem + SM::kOffOhi, a.o[0], (int64_t)n0 * 2, tr_rows, a.o_row_off, 0, 0, tid);
         if (st_lo) tile_to_global<RB>(smem + SM::kOffOlo, a.o[1], (int64_t)n0 * 2, tr_rows, a.o_row_off, 0, 0, tid);
     } else if (a.o_mode == 2) {  // Q / K: [B][heads][320][64]; V^T: [B][heads][64][320]
         if (o_which < 2) {
-            if (st_hi) tile_to_global<RB>(smem + SM::kOffOhi, a.o[2 * o_which], (int64_t)o_d * 2, tr_rows, 0, o_h, 0, tid);
-            if (st_lo) tile_to_global<RB>(smem + SM::kOffOlo, a.o[2 * o_which + 1], (int64_t)o_d * 2, tr_rows, 0, o_h, 0, tid);
+            if (st_hi) tile_to_global<RB, BM>(smem + SM::kOffOhi, a.o[2 * o_which], (int64_t)o_d * 2, tr_rows, 0, o_h, 0, tid);
+            if (st_lo) tile_to_global<RB, BM>(smem + SM::kOffOlo, a.o[2 * o_which + 1], (int64_t)o_d * 2, tr_rows, 0, o_h, 0, tid);
         } else {
-            if (st_hi) vt_tile_to_global<BN>(smem + SM::kOffOhi, a.o[4], tr_rows, o_h, o_d, tid);
-            if (st_lo) vt_tile_to_global<BN>(smem + SM::kOffOlo, a.o[5], tr_rows, o_h, o_d, tid);
+            if (st_hi) vt_tile_to_global<BN, BM / 64>(smem + SM::kOffOhi, a.o[4], tr_rows, o_h, o_d, tid);
+            if (st_lo) vt_tile_to_global<BN, BM / 64>(smem + SM::kOffOlo, a.o[5], tr_rows, o_h, o_d, tid);
         }
     }
     if (tid == 0) tr.mark(7);
     if (a.chain_n) {
-        // ---- chained GEMM: P_j[128, N2] = hidden tile (just staged as a 128B-swizzled K-major A operand, bf16 hi / lo) x
+        // ---- chained GEMM: P_j[BM, N2] = hidden tile (just staged as a 128B-swizzled K-major A operand, bf16 hi / lo) x
         // W2[:, n0 .. n0 + 64)^T.  The hidden activations never travel to global memory; the N / 64 partial results P_j of one row
         // tile are summed in a fixed order by reduce_ln_kernel, which also applies bias, residual and the next LayerNorm.
         if (warp == 1) {
@@ -390,8 +419,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
             const uint32_t a_lo = umma_desc_lo(smem_u32(smem + SM::kOffOhi)), b_lo = umma_desc_lo(smem_u32(smem + SM::kOffB2));
             constexpr uint32_t kLoA = kTileOBytes >> 4, kLoB = SM::kB2PartBytes >> 4;
             if (elect_one_sync()) {
-                if (sliced && kLo) {  // H_hi x [W2_hi; W2_lo] as one UMMA of 2 N2 columns + H_lo x W2_hi (the epilogue adds the halves)
-                    const uint32_t idesc2 = umma_idesc_bf16(kTcBM, N2), idesc2n = umma_idesc_bf16(kTcBM, 2 * N2);
+                if (kQ64 || (sliced && kLo)) {  // H_hi x [W2_hi; W2_lo] as one UMMA of 2 N2 columns + H_lo x W2_hi (the epilogue adds the halves)
+                    const uint32_t idesc2 = umma_idesc_bf16(BM, N2), idesc2n = umma_idesc_bf16(BM, 2 * N2);
 #pragma unroll
                     for (int k = 0; k < BN / 16; ++k) {
                         const uint64_t dB = umma_desc_from_lo(b_lo + 2 * k);
@@ -399,7 +428,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
                         umma_bf16_ta(tmem + kAcc1Cols, tmem + kColA2 + 16 * k + 8, dB, idesc2, 1);
                     }
                 } else {
-                    const uint32_t idesc2 = kF16 ? umma_idesc_f16(kTcBM, N2) : umma_idesc_bf16(kTcBM, N2);  // K = the 64 hidden columns of this CTA
+                    const uint32_t idesc2 = kF16 ? umma_idesc_f16(BM, N2) : umma_idesc_bf16(BM, N2);  // K = the 64 hidden columns of this CTA
 #pragma unroll
                     for (int k = 0; k < BN / 16; ++k) {
                         const uint64_t dA = umma_desc_from_lo(a_lo + 2 * k), dB = umma_desc_from_lo(b_lo + 2 * k);
@@ -417,30 +446,51 @@ __global__ void __launch_bounds__(kTcThreads, 1) gemm_tc_kernel(const __grid_con
         ok &= mbar_wait(&accum2_bar, 0);
         tcgen05_fence_after();
         if (tid == 0) tr.mark(5);
-        // thread (row, g) owns columns g * N2/4 .. of its row; fp32 tile staged as N2/32 boxes of [128 rows][128 B], swizzled
-        const int cols_per = N2 / kTcColGroups;
-        for (int c = g * cols_per; c < (g + 1) * cols_per; c += 16) {
-            float p[16];
-            tmem_ld_32x16(tmem + ((uint32_t)((warp & 3) * 32) << 16) + kAcc1Cols + c, p);
-            if (sliced && kLo) {
-                float hl[16];
-                tmem_ld_32x16(tmem + ((uint32_t)((warp & 3) * 32) << 16) + kAcc1Cols + N2 + c, hl);
+        // fp32 tile staged as N2/32 boxes of [BM rows][128 B], swizzled; stage4 = the 4 columns c.. of this thread's row
+        auto stage4 = [&](int c, float x0, float x1, float x2, float x3) {
+            *reinterpret_cast<float4*>(smem + SM::kOffP + (c >> 5) * (BM * 128) + row * 128 + ((((c & 31) >> 2) ^ sw) << 4)) = make_float4(x0, x1, x2, x3);
+        };
+        if constexpr (kQ64) {
+            // warp group w / 4 owns the 24 columns 24 (w / 4) .. of the N2 = 96: threads 0..15 columns +0..7 and +16..19, threads
+            // 16..31 +8..15 and +20..23; all four loads (hi*hi + lo*hi, hi*lo halves) in flight before the wait
+            constexpr int kW = kChainN64 / 4;
+            const uint32_t t2 = tmem + tq + kAcc1Cols + (warp >> 2) * kW;
+            uint32_t pa[8], pb[4], ha[8], hb[4];
+            tmem_ld_16x2_x8_issue(t2, pa), tmem_ld_16x2_x4_issue(t2 + 16, pb);
+            tmem_ld_16x2_x8_issue(t2 + kChainN64, ha), tmem_ld_16x2_x4_issue(t2 + kChainN64 + 16, hb);
+            tmem_ld_wait(pa), tmem_ld_wait(pb), tmem_ld_wait(ha), tmem_ld_wait(hb);
+            float p[12];
 #pragma unroll
-                for (int j = 0; j < 16; ++j) p[j] += hl[j];
+            for (int j = 0; j < 8; ++j) p[j] = __uint_as_float(pa[j]) + __uint_as_float(ha[j]);
+#pragma unroll
+            for (int j = 0; j < 4; ++j) p[8 + j] = __uint_as_float(pb[j]) + __uint_as_float(hb[j]);
+            const int c0 = (warp >> 2) * kW, h = lane >> 4;
+            stage4(c0 + 8 * h, p[0], p[1], p[2], p[3]);
+            stage4(c0 + 8 * h + 4, p[4], p[5], p[6], p[7]);
+            stage4(c0 + 16 + 4 * h, p[8], p[9], p[10], p[11]);
+        } else {
+            // thread (row, g) owns columns g * N2/4 .. of its row
+            const int cols_per = N2 / kTcColGroups;
+            for (int c = g * cols_per; c < (g + 1) * cols_per; c += 16) {
+                float p[16];
+                tmem_ld_32x16(tmem + tq + kAcc1Cols + c, p);
+                if (sliced && kLo) {
+                    float hl[16];
+                    tmem_ld_32x16(tmem + tq + kAcc1Cols + N2 + c, hl);
+#pragma unroll
+                    for (int j = 0; j < 16; ++j) p[j] += hl[j];
+                }
+#pragma unroll
+                for (int q = 0; q < 4; ++q) stage4(c + 4 * q, p[4 * q], p[4 * q + 1], p[4 * q + 2], p[4 * q + 3]);
             }
-            uint8_t* prow = smem + SM::kOffP + (c >> 5) * (kTcBM * 128) + row * 128;
-            const int ch0 = (c & 31) >> 2;
-#pragma unroll
-            for (int q = 0; q < 4; ++q)
-                *reinterpret_cast<float4*>(prow + (((ch0 + q) ^ sw) << 4)) = make_float4(p[4 * q], p[4 * q + 1], p[4 * q + 2], p[4 * q + 3]);
         }
         __syncthreads();
         if (tid == 0) tr.mark(4);
         for (int cb = 0; cb < N2 / 32; ++cb)  // P[j = blockIdx.x][target][row][32 cb ..]
-            tile_to_global<128>(smem + SM::kOffP + cb * (kTcBM * 128), a.p, (int64_t)cb * 128 + (sliced ? (int64_t)blockIdx.z * N2 * 4 : 0), tr_rows, 0, 0,
+            tile_to_global<128, BM>(smem + SM::kOffP + cb * (BM * 128), a.p, (int64_t)cb * 128 + (sliced ? (int64_t)blockIdx.z * N2 * 4 : 0), tr_rows, 0, 0,
                                 blockIdx.x, tid);
     }
-    if (do_ln) {  // ---- fused LayerNorm over the full row (N columns = cluster of N / BN CTAs)
+    if (!kQ64 && do_ln) {  // ---- fused LayerNorm over the full row (N columns = cluster of N / BN CTAs)
         const uint32_t nct = cluster_nctarank();
         float gam[CPT], bet[CPT];
 #pragma unroll
@@ -562,6 +612,8 @@ bool tc_plan_chain(TcGemmPlan* p, const __nv_bfloat16* W2hi, const __nv_bfloat16
     const uint64_t dims[2] = {K2, (uint64_t)N2}, strides[1] = {K2 * 2};
     const uint32_t box[2] = {(uint32_t)kTcBK, 64};  // loaded as 64-row boxes (a CTA of the sliced form takes one of them)
     bool ok = tc_make_map(&p->maps.B2hi, W2hi, 2, dims, strides, box) && tc_make_map(&p->maps.B2lo, W2lo ? W2lo : W2hi, 2, dims, strides, box);
+    const uint32_t box_half[2] = {(uint32_t)kTcBK, (uint32_t)N2 / 2};  // one slice of the two-slice form of the 64-row tiles
+    ok &= tc_make_map(&p->maps.B2hiHalf, W2hi, 2, dims, strides, box_half) && tc_make_map(&p->maps.B2loHalf, W2lo ? W2lo : W2hi, 2, dims, strides, box_half);
     p->args.p = tc_out(P, 4, N2, rows, 1, batch, K2 / kTcBN);
     p->args.chain_n = N2, p->args.o_mode = 3;
     return ok;
@@ -581,30 +633,47 @@ bool tc_plan_init(TcGemmPlan* p, const __nv_bfloat16* Ahi, const __nv_bfloat16* 
         const uint32_t box[4] = {(uint32_t)kTcBK, kMap, kTcBM / kMap, 1};
         ok &= tc_make_map(&p->maps.Ahi, Ahi, 4, dims, strides, box);
         ok &= tc_make_map(&p->maps.Alo, Alo ? Alo : Ahi, 4, dims, strides, box);
+        p->maps.Ahi64 = p->maps.Ahi, p->maps.Alo64 = p->maps.Alo;  // (no 64-row form)
     } else {
         ok &= tc_make_map_2d(&p->maps.Ahi, Ahi, a_rows, K, kTcBM);
         ok &= tc_make_map_2d(&p->maps.Alo, Alo ? Alo : Ahi, a_rows, K, kTcBM);
+        ok &= tc_make_map_2d(&p->maps.Ahi64, Ahi, a_rows, K, 64);
+        ok &= tc_make_map_2d(&p->maps.Alo64, Alo ? Alo : Ahi, a_rows, K, 64);
     }
     ok &= tc_make_map_2d(&p->maps.Bhi, Whi, N, K, kTcBN);
     ok &= tc_make_map_2d(&p->maps.Blo, Wlo ? Wlo : Whi, N, K, kTcBN);
     // unused output maps must still be valid descriptors (they are never dereferenced when their mode is off)
-    p->maps.R = p->maps.B2hi = p->maps.B2lo = p->maps.Bhi;
+    p->maps.R = p->maps.B2hi = p->maps.B2lo = p->maps.B2hiHalf = p->maps.B2loHalf = p->maps.Bhi;
     p->args.N = N, p->args.K = K, p->args.conv_feat = conv_feat;
     p->args.pos_rows = 1, p->args.period = 1 << 30;
     return ok;
 }
 
 cudaError_t tc_gemm_setup() {
-    cudaError_t e = cudaFuncSetAttribute(gemm_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<1>::kTotal);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<3>::kTotal);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<2>::kTotal);
+    cudaError_t e = cudaFuncSetAttribute(gemm_tc_kernel<1, kTcBM>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<1>::kTotal);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<3, kTcBM>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<3>::kTotal);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<2, kTcBM>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<2>::kTotal);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(gemm_tc_kernel<3, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem<3, 64>::kTotal);
     return e;
 }
 
-cudaError_t tc_gemm_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, bool spread) {
+// the epilogues the 64-row kernel has: the QKV scatter and the chained FC1 with the hidden tile in tensor memory (bf16x3, N2 = 192)
+bool tc_gemm_q64_supported(const TcGemmPlan& p, int nsplit) {
+    const TcGemmArgs& a = p.args;
+    if (nsplit != 3 || a.kb_per_split || a.conv_feat || a.ln_g || a.c_on || a.residual) return false;
+    return (a.o_mode == 2 && !a.chain_n) || (a.o_mode == 3 && a.chain_n == kMaxChainN);
+}
+
+cudaError_t tc_gemm_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, bool spread, bool q64) {
     if (M <= 0) return cudaSuccess;
     TcGemmArgs a = p.args;
     a.M = M;
+    if (q64) {  // two replicas of every 64-row tile: hi / lo stores of the QKV scatter, or two slices of the chained product
+        if (!spread || !tc_gemm_q64_supported(p, nsplit)) return cudaErrorInvalidValue;
+        a.chain_slices = a.chain_n ? 2 : 0, a.dup_hl = a.chain_n ? 0 : 1, a.dup_ln = 0;
+        const dim3 grid(a.N / kTcBN, (M + 63) / 64, 2);
+        return launch_ex(gemm_tc_kernel<3, 64>, grid, dim3(kTcThreads), TcSmem<3, 64>::kTotal, s, pdl, 1, p.maps, a);
+    }
     dim3 grid(a.N / kTcBN, (M + kTcBM - 1) / kTcBM, a.kb_per_split ? a.K / kTcBK / a.kb_per_split : 1);
     a.chain_slices = 0, a.dup_hl = 0, a.dup_ln = 0;
     if (spread && !a.kb_per_split && nsplit == 3 && a.ln_g && a.c_on && !a.chain_n && !a.o_mode && grid.x * grid.y * 3 <= (unsigned)kSpreadCtas)
@@ -617,9 +686,9 @@ cudaError_t tc_gemm_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t 
     // fused LayerNorm: the N / 64 column tiles of a row tile form one cluster
     const int cluster_x = a.ln_g ? a.N / kTcBN : 1;
     if (cluster_x > kMaxLnCluster) return cudaErrorInvalidValue;
-    if (nsplit == 2) return launch_ex(gemm_tc_kernel<2>, grid, dim3(kTcThreads), TcSmem<2>::kTotal, s, pdl, cluster_x, p.maps, a);
-    if (nsplit == 3) return launch_ex(gemm_tc_kernel<3>, grid, dim3(kTcThreads), TcSmem<3>::kTotal, s, pdl, cluster_x, p.maps, a);
-    return launch_ex(gemm_tc_kernel<1>, grid, dim3(kTcThreads), TcSmem<1>::kTotal, s, pdl, cluster_x, p.maps, a);
+    if (nsplit == 2) return launch_ex(gemm_tc_kernel<2, kTcBM>, grid, dim3(kTcThreads), TcSmem<2>::kTotal, s, pdl, cluster_x, p.maps, a);
+    if (nsplit == 3) return launch_ex(gemm_tc_kernel<3, kTcBM>, grid, dim3(kTcThreads), TcSmem<3>::kTotal, s, pdl, cluster_x, p.maps, a);
+    return launch_ex(gemm_tc_kernel<1, kTcBM>, grid, dim3(kTcThreads), TcSmem<1>::kTotal, s, pdl, cluster_x, p.maps, a);
 }
 
 // fp32 -> bf16 (hi, lo) split of a dense buffer

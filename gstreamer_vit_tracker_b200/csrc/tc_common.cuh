@@ -369,10 +369,16 @@ __device__ __forceinline__ void tmem_ld_16x2(uint32_t taddr, float (&v)[8]) {  /
 #pragma unroll
     for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
 }
+__device__ __forceinline__ void tmem_ld_16x2_x4_issue(uint32_t taddr, uint32_t (&r)[4]) {  // OFF = 4
+    asm volatile("tcgen05.ld.sync.aligned.16x32bx2.x4.b32 {%0, %1, %2, %3}, [%4], 4;" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[4]) {
+    asm volatile("tcgen05.wait::ld.sync.aligned;" : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3])::"memory");
+}
 __device__ __forceinline__ void tmem_ld_16x2(uint32_t taddr, float (&v)[4]) {  // OFF = 4
     uint32_t r[4];
-    asm volatile("tcgen05.ld.sync.aligned.16x32bx2.x4.b32 {%0, %1, %2, %3}, [%4], 4;" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3])::"memory");
+    tmem_ld_16x2_x4_issue(taddr, r);
+    tmem_ld_wait(r);
 #pragma unroll
     for (int i = 0; i < 4; ++i) v[i] = __uint_as_float(r[i]);
 }

@@ -140,6 +140,7 @@ static void read_switches(vt_tracker* t) {
     s.spread = !getenv("VT_B200_NO_SPREAD");
     s.att_chain = !getenv("VT_B200_NO_ATT_CHAIN");
     s.att_q64 = !getenv("VT_B200_ATT_Q128");
+    s.gemm_q64 = !getenv("VT_B200_GEMM_Q128");
     if (const char* e = getenv("VT_B200_UNCHAIN_N")) s.unchain_n = atoi(e);
     if (const char* e = getenv("VT_B200_AS_ROWS")) s.as_rows = atoi(e);
     s.as_mlp = !getenv("VT_B200_NO_AS_MLP");

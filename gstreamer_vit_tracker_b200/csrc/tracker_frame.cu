@@ -56,6 +56,7 @@ struct ForwardForms {
     bool proj_in_att = false;  // proj folded into the attention kernel + reduce_ln, instead of the proj GEMM
     bool mlp_chain = false;    // FC2 partial products inside the FC1 kernel + reduce_ln (else FC1 stores the hidden tile, FC2 GEMM)
     bool mlp_as = false;       // FC1 (with the chained product: gemm_as_mlp_kernel) in the A-stationary form
+    bool gemm_q64 = false;     // QKV and the chained FC1 on 64-row tiles (tc_gemm_launch q64)
     bool spread = false;       // latency-mode replicas of the one-tile GEMMs (tc_gemm_launch picks them from the plan)
     bool pdl = true;           // programmatic dependent launch along the chain (off under debug_capture)
 };
@@ -102,6 +103,12 @@ static ForwardForms forward_forms(const vt_tracker* t, int n, bool spread) {
     const bool as_mlp = as_form && sf.chain_mlp && t->sw.as_mlp && tc_gemm_as_mlp_supported(p.fc1, t->nsplit);
     f.mlp_chain = as_mlp || (sf.chain_mlp && n < t->sw.unchain_n);
     f.mlp_as = f.mlp_chain ? as_mlp : as_form && tc_gemm_as_supported(unchained_fc1(p.fc1));
+    // Latency mode: QKV and the chained FC1 on 64-row tiles (M = 64 UMMAs: five tiles instead of 128 + 128 + 64, half the epilogue per
+    // CTA) when both grids of two replicas per tile still fit one wave — one target
+    const int tiles64 = (M + 63) / 64;
+    f.gemm_q64 = spread && t->sw.gemm_q64 && !f.qkv_as && f.mlp_chain && !f.mlp_as && tc_gemm_q64_supported(p.qkv, t->nsplit) &&
+                 tc_gemm_q64_supported(p.fc1, t->nsplit) && (p.qkv.args.N / 64) * tiles64 * 2 <= kSpreadCtas &&
+                 (p.fc1.args.N / 64) * tiles64 * 2 <= kSpreadCtas;
     return f;
 }
 
@@ -184,7 +191,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const Forw
             if (f.qkv_as)
                 VT_LAUNCH(tc_gemm_as_launch(p.qkv, M, ns, s, f.pdl, t->sm_count, t->sw.as_split));
             else
-                VT_LAUNCH(tc_gemm_launch(p.qkv, M, ns, s, f.pdl, f.spread));
+                VT_LAUNCH(tc_gemm_launch(p.qkv, M, ns, s, f.pdl, f.spread, f.gemm_q64));
             if (f.att == kAttSimt)
                 VT_LAUNCH(launch_attention(t->QKV, nullptr, t->att_hi, LO(t->att_lo), n, D, t->heads, s));
             else
@@ -206,7 +213,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const Forw
             else if (f.mlp_as)
                 VT_LAUNCH(tc_gemm_as_launch(fc1, M, ns, s, f.pdl, t->sm_count, t->sw.as_split));
             else
-                VT_LAUNCH(tc_gemm_launch(fc1, M, ns, s, f.pdl, f.spread && f.mlp_chain));
+                VT_LAUNCH(tc_gemm_launch(fc1, M, ns, s, f.pdl, f.spread && f.mlp_chain, f.gemm_q64));
             if (f.mlp_chain) {  // X += fc2_b + sum of the partials; LN1 of the next block / the final LN of the search rows
                 const bool last = l + 1 == t->depth;
                 ReduceLnArgs r{};

@@ -56,7 +56,7 @@ constexpr int kMaxDevices = 64, kSpreadMaxHandles = 2, kUnchainTargets = 8;
 
 // Environment switches of a handle, read by read_switches at create (meaning and defaults: DESIGN.md §9).
 struct Switches {
-    bool spread = true, att_chain = true, att_q64 = true, as_mlp = true, trace = false, hostprof = false;
+    bool spread = true, att_chain = true, att_q64 = true, gemm_q64 = true, as_mlp = true, trace = false, hostprof = false;
     int unchain_n = kUnchainTargets, as_rows = 1024, as_split = 0, win_shrink = 0;
 };
 

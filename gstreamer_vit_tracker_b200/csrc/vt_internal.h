@@ -358,8 +358,9 @@ struct TcGemmArgs {
 };
 struct TcMaps {               // kernel parameter block (__grid_constant__): the TMA load descriptors
     CUtensorMap Ahi, Alo, Bhi, Blo, R, B2hi, B2lo;
+    CUtensorMap Ahi64, Alo64, B2hiHalf, B2loHalf;  // 64-row tiles (q64): A in boxes of 64 rows, W2 in boxes of N2 / 2 rows (one slice)
 };
-struct TcGemmPlan {           // one GEMM on 128 x 64 output tiles
+struct TcGemmPlan {           // one GEMM on 128 x 64 (or 64 x 64: q64) output tiles
     TcMaps maps;
     TcGemmArgs args;
 };
@@ -375,7 +376,10 @@ cudaError_t tc_gemm_setup();
 // spread: latency mode — tiles are replicated over idle SMs so that each replica stores a share of the epilogue output (only when the
 // whole grid still fits in one wave of kSpreadCtas CTAs)
 constexpr int kSpreadCtas = 132;
-cudaError_t tc_gemm_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, bool spread = false);
+// q64 (latency mode, bf16x3, plans that tc_gemm_q64_supported accepts): 64-row tiles with M = 64 UMMAs — the QKV scatter as hi / lo
+// replicas (2 CTAs per tile), the chained FC1 as two replicas of N2 / 2 chained columns each; any other plan is rejected
+cudaError_t tc_gemm_launch(const TcGemmPlan& p, int M, int nsplit, cudaStream_t s, bool pdl, bool spread = false, bool q64 = false);
+bool tc_gemm_q64_supported(const TcGemmPlan& p, int nsplit);
 // A-stationary throughput form (gemm_as.cu) of a plain 64-column-tile plan with K <= 192 whose epilogue is a bf16 (hi, lo) tile store or
 // the QKV scatter: one CTA per (128-row tile, range of 64-column chunks), the activation tile resident in shared memory, two TMEM
 // accumulators (main loop of chunk i + 1 under the epilogue of chunk i).  Bit-identical to tc_gemm_launch on the same plan.
