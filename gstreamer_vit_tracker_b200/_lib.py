@@ -57,6 +57,11 @@ class vt_surface(C.Structure):
     _fields_ = [("planes", C.c_void_p * 2), ("pitch", C.c_size_t * 2)]
 
 
+class vt_stream_geometry(C.Structure):
+    """The format and size of one target slot's frames in a stream group of mixed cameras (vt_tracker_set_stream_geometry)."""
+    _fields_ = [("format", C.c_int32), ("width", C.c_int32), ("height", C.c_int32), ("reserved", C.c_int32)]
+
+
 class vt_timing(C.Structure):
     _fields_ = [
         ("fps", C.c_double), ("avg_conv_ms", C.c_double), ("avg_track_ms", C.c_double),
@@ -99,6 +104,8 @@ SYMBOLS = {
     "vt_tracker_run_streams_ring": (C.c_int32, [_vp, C.POINTER(C.c_void_p), C.c_int32, C.c_size_t, C.c_size_t, C.c_int32, C.c_int32, C.c_int32,
                                     C.POINTER(C.c_void_p), C.POINTER(vt_result), C.POINTER(C.c_double)]),
     "vt_tracker_update_streams": (C.c_int32, [_vp, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.c_int32, C.POINTER(vt_result)]),
+    "vt_tracker_set_stream_geometry": (C.c_int32, [_vp, C.c_int32, C.POINTER(vt_stream_geometry)]),
+    "vt_tracker_get_stream_geometry": (C.c_int32, [_vp, C.c_int32, C.POINTER(vt_stream_geometry)]),
     "vt_tracker_run_ring": (C.c_int32, [_vp, _vp, C.c_size_t, C.c_size_t, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _vp, C.POINTER(vt_result),
                                         C.POINTER(C.c_double)]),
     "vt_context_run_ring": (C.c_int32, [_vp, _vp, C.c_size_t, C.c_size_t, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_char_p), _vp,

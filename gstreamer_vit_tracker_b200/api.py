@@ -24,7 +24,7 @@ from typing import List, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib as L
-from ._lib import VtError, check, lib, vt_bbox, vt_config, vt_overlay_cmd, vt_result, vt_selection, vt_surface, vt_timing
+from ._lib import VtError, check, lib, vt_bbox, vt_config, vt_overlay_cmd, vt_result, vt_selection, vt_stream_geometry, vt_surface, vt_timing
 
 
 @dataclass(frozen=True)
@@ -291,10 +291,30 @@ class VitTrack:
         check(lib().vt_tracker_update(self._h, _ptr(frame), frame.size, self._res), "vt_tracker_update")
         return self._results()
 
+    def set_stream_geometry(self, target: int, width: Optional[int] = None, height: Optional[int] = None, fmt: Optional[str] = None) -> None:
+        """Stream groups of mixed cameras (vt_tracker_set_stream_geometry): target slot `target` takes frames of `fmt` ("nv12", "rgb24",
+        "gray8", "yuy2") at width x height instead of the handle's geometry — init() on that slot and its stream in update_streams /
+        update_streams_surface / run_streams_ring.  Only a slot that is not initialised may change; no arguments: back to the handle's
+        geometry.  A handle with a slot of its own geometry takes frames through the stream-group calls only."""
+        if width is None and height is None and fmt is None:
+            check(lib().vt_tracker_set_stream_geometry(self._h, target, None), "vt_tracker_set_stream_geometry")
+            return
+        if width is None or height is None or fmt is None:
+            raise ValueError("set_stream_geometry takes width, height and fmt together (or none of them)")
+        g = vt_stream_geometry(FORMATS[fmt], int(width), int(height), 0)
+        check(lib().vt_tracker_set_stream_geometry(self._h, target, C.byref(g)), "vt_tracker_set_stream_geometry")
+
+    def get_stream_geometry(self, target: int) -> Tuple[int, int, str]:
+        """(width, height, fmt) of target slot `target`'s frames."""
+        g = vt_stream_geometry()
+        check(lib().vt_tracker_get_stream_geometry(self._h, target, C.byref(g)), "vt_tracker_get_stream_geometry")
+        return g.width, g.height, {v: k for k, v in FORMATS.items()}[g.format]
+
     def update_streams(self, frames: Sequence[np.ndarray]) -> List[TrackResult]:
         """Stream group (vt_tracker_update_streams): frames[i] — a full frame in pinned host memory (PinnedBuffer) — is the current
-        frame of the i-th active target's own video stream; all targets go through one batched forward, each stream's box overlay is
-        drawn into its own frame.  ≙ n TrackerContexts (src/pipeline.rs:55) stepped together."""
+        frame of the i-th active target's own video stream, of that target's geometry (set_stream_geometry); all targets go through one
+        batched forward, each stream's box overlay is drawn into its own frame.  ≙ n TrackerContexts (src/pipeline.rs:55) stepped
+        together."""
         n = len(frames)
         ptrs = (C.c_void_p * n)(*[_ptr(f).value for f in frames])
         lens = (C.c_size_t * n)(*[f.size for f in frames])
@@ -361,7 +381,8 @@ class VitTrack:
 
     def run_streams_ring(self, ring_ptrs: Sequence[int], stride: int, frame_len: int, ring: int, first: int, n: int,
                          pristine_ptrs: Optional[Sequence[int]] = None, want_latency: bool = False):
-        """n steps of a stream group in one native call (vt_tracker_run_streams_ring): ring_ptrs[i] = pinned host ring of stream i."""
+        """n steps of a stream group in one native call (vt_tracker_run_streams_ring): ring_ptrs[i] = pinned host ring of stream i.  With
+        streams of mixed geometries `frame_len` and `stride` cover the largest stream's frame."""
         k = len(ring_ptrs)
         rings = (C.c_void_p * k)(*ring_ptrs)
         clean = (C.c_void_p * k)(*pristine_ptrs) if pristine_ptrs is not None else None

@@ -431,13 +431,16 @@ __device__ __forceinline__ Tap lin_tap(int i, int s, int d, bool clamp_frac) {
 
 // Where the pixels of this frame live: the device frame inside the valid window (the part that was uploaded this frame), the
 // caller's pinned host frame (zero-copy loads over PCIe) outside of it.  With whole-frame uploads the window is the frame.  The device
-// frame may be a pitched surface (planes and pitches from the control block or the frame descriptor); the host frame is always packed.
+// frame may be a pitched surface (planes and pitches from the control block or the frame descriptor); the host frame is always packed,
+// and only exists beside a packed device frame of the same geometry (window uploads): it has the device frame's pitches and plane offset.
 struct PixelSrc {
     const uint8_t *dev, *dev_uv;  // device planes: Y / RGB / gray, NV12 chroma
     size_t pitch, uv_pitch;       // their row pitches
     const uint8_t* host;          // null: everything is on the device
     int x0, y0, x1, y1;           // valid window of the device frame (even-aligned, so a pixel and its chroma pair sit on the same side)
     bool dev_words, host_words;   // YUY2: the plane's pixel-pair words are 4-byte aligned (base and pitch), one 32-bit load each
+    int format;                   // vt_format of this target's frame
+    int xlim, ylim;               // pixels [0, xlim) x [0, ylim) are read, the rest is border (0 x 0 for a short frame)
 };
 
 // the Y0 U Y1 V word of pixel fx in a YUY2 row: one 32-bit load when aligned, else four byte loads (surfaces may have any pitch)
@@ -448,27 +451,24 @@ __device__ __forceinline__ uint32_t yuy2_word(const uint8_t* row, int fx, bool a
 }
 
 // RGB of the frame pixel (fx, fy); zero outside the frame (constant border of the crop).
-__device__ __forceinline__ void frame_rgb(const FrameDesc& f, const PixelSrc& ps, int fx, int fy, int& r, int& g, int& b) {
+__device__ __forceinline__ void frame_rgb(const PixelSrc& ps, int fx, int fy, int& r, int& g, int& b) {
     r = g = b = 0;
-    // pad_plus1 (App. A.7, older OpenCV): a crop that reaches the right / bottom edge pads one pixel more, i.e. the last column / row of
-    // the frame reads as border; a crop that stays inside never addresses it, so the bound can move unconditionally
-    if (!f.valid || fx < 0 || fy < 0 || fx >= f.width - f.pad_plus1 || fy >= f.height - f.pad_plus1) return;
+    if (fx < 0 || fy < 0 || fx >= ps.xlim || fy >= ps.ylim) return;
     const bool host = ps.host && (fx < ps.x0 || fx >= ps.x1 || fy < ps.y0 || fy >= ps.y1);
-    const uint8_t* data = host ? ps.host : ps.dev;
-    if (f.format == VT_FMT_RGB24) {
-        const uint8_t* p = data + (size_t)fy * (host ? (size_t)f.width * 3 : ps.pitch) + (size_t)fx * 3;
+    const uint8_t* data = host ? ps.host : ps.dev;  // (same pitches: see PixelSrc)
+    if (ps.format == VT_FMT_RGB24) {
+        const uint8_t* p = data + (size_t)fy * ps.pitch + (size_t)fx * 3;
         r = p[0], g = p[1], b = p[2];
-    } else if (f.format == VT_FMT_GRAY8) {
-        r = g = b = data[(size_t)fy * (host ? (size_t)f.width : ps.pitch) + fx];
-    } else if (f.format == VT_FMT_YUY2) {
-        const uint32_t w = yuy2_word(data + (size_t)fy * (host ? fmt_row_bytes(VT_FMT_YUY2, f.width) : ps.pitch), fx,
-                                     host ? ps.host_words : ps.dev_words);
+    } else if (ps.format == VT_FMT_GRAY8) {
+        r = g = b = data[(size_t)fy * ps.pitch + fx];
+    } else if (ps.format == VT_FMT_YUY2) {
+        const uint32_t w = yuy2_word(data + (size_t)fy * ps.pitch, fx, host ? ps.host_words : ps.dev_words);
         const Chroma c = chroma_terms((int)((w >> 8) & 0xff), (int)(w >> 24));
         yuv_px((int)((w >> ((fx & 1) * 16)) & 0xff), c, r, g, b);
     } else {
-        const int yv = data[(size_t)fy * (host ? (size_t)f.width : ps.pitch) + fx];
-        const uint8_t* uv = host ? ps.host + (size_t)f.width * f.height : ps.dev_uv;
-        const size_t uvi = (size_t)(fy >> 1) * (host ? (size_t)f.width : ps.uv_pitch) + (fx & ~1);
+        const int yv = data[(size_t)fy * ps.pitch + fx];
+        const uint8_t* uv = host ? ps.host + (ps.dev_uv - ps.dev) : ps.dev_uv;
+        const size_t uvi = (size_t)(fy >> 1) * ps.uv_pitch + (fx & ~1);
         const Chroma c = chroma_terms(uv[uvi], uv[uvi + 1]);
         yuv_px(yv, c, r, g, b);
     }
@@ -482,9 +482,13 @@ __global__ void __launch_bounds__(256) crop_resize_norm_kernel(FrameDesc f, Targ
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // the template gather behind this kernel does not depend on it
     if (stamp && threadIdx.x == 0 && blockIdx.x == 0 && blockIdx.y == 0) *stamp = device_time_ns();
     const int bi = blockIdx.y;
-    PixelSrc ps{f.data, f.uv, f.pitch[0], f.pitch[1], nullptr, 0, 0, f.width, f.height};
+    PixelSrc ps{f.data, f.uv, f.pitch[0], f.pitch[1], nullptr, 0, 0, f.width, f.height, false, false, f.format, 0, 0};
     if (f.ctl) {  // per-frame control block: frame planes, and which part of the device frame holds this frame's pixels
         const bool own = bi < kMaxWin && f.ctl->frames[bi] != nullptr;  // stream group: this target has its own frame
+        if (own) {  // ... of its own format and size (one target per blockIdx.y: the format branch varies between CTAs, never within one)
+            const int4 g = *reinterpret_cast<const int4*>(f.ctl->geom[bi]);
+            f.format = g.x, f.width = g.y, f.height = g.z, f.valid = g.w;
+        }
         ps.dev = own ? f.ctl->frames[bi] : f.ctl->frame;
         ps.dev_uv = own ? f.ctl->uvs[bi] : f.ctl->uv;
         ps.pitch = own ? f.ctl->pitches[bi][0] : f.ctl->pitch[0];
@@ -501,6 +505,10 @@ __global__ void __launch_bounds__(256) crop_resize_norm_kernel(FrameDesc f, Targ
     if (!ps.uv_pitch) ps.uv_pitch = (size_t)f.width;
     ps.dev_words = ((reinterpret_cast<uintptr_t>(ps.dev) | ps.pitch) & 3) == 0;
     ps.host_words = (reinterpret_cast<uintptr_t>(ps.host) & 3) == 0;  // (packed YUY2 rows are whole words)
+    ps.format = f.format;
+    // pad_plus1 (App. A.7, older OpenCV): a crop that reaches the right / bottom edge pads one pixel more, i.e. the last column / row of
+    // the frame reads as border; a crop that stays inside never addresses it, so the bound can move unconditionally
+    ps.xlim = f.valid ? f.width - f.pad_plus1 : 0, ps.ylim = f.valid ? f.height - f.pad_plus1 : 0;
     const int slot = slots[bi];
     TargetState* st = state + slot;
     const int bx = st->rect[0], by = st->rect[1], bw = st->rect[2], bh = st->rect[3];
@@ -523,10 +531,10 @@ __global__ void __launch_bounds__(256) crop_resize_norm_kernel(FrameDesc f, Targ
     const int cx0 = tx.ofs, cx1 = min(tx.ofs + 1, c - 1);
     const int cy0 = min(max(ty.ofs, 0), c - 1), cy1 = min(max(ty.ofs + 1, 0), c - 1);
     int p00[3], p01[3], p10[3], p11[3];
-    frame_rgb(f, ps, x1 + cx0, y1 + cy0, p00[0], p00[1], p00[2]);
-    frame_rgb(f, ps, x1 + cx1, y1 + cy0, p01[0], p01[1], p01[2]);
-    frame_rgb(f, ps, x1 + cx0, y1 + cy1, p10[0], p10[1], p10[2]);
-    frame_rgb(f, ps, x1 + cx1, y1 + cy1, p11[0], p11[1], p11[2]);
+    frame_rgb(ps, x1 + cx0, y1 + cy0, p00[0], p00[1], p00[2]);
+    frame_rgb(ps, x1 + cx1, y1 + cy0, p01[0], p01[1], p01[2]);
+    frame_rgb(ps, x1 + cx0, y1 + cy1, p10[0], p10[1], p10[2]);
+    frame_rgb(ps, x1 + cx1, y1 + cy1, p11[0], p11[1], p11[2]);
     const int nt = S >> 4;
     const int token = (dy >> 4) * nt + (dx >> 4);
     const size_t off = (size_t)bi * patches_stride + (size_t)token * kPatchK + (dy & 15) * 16 + (dx & 15);
@@ -979,6 +987,10 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
     // what it needs in one batch, and the HUD list comes out of pinned host memory, BEFORE the dependency wait: only the decode result
     // waits for the preceding kernel
     const bool own = blockIdx.x < (unsigned)kMaxWin && ctl->frames[blockIdx.x] != nullptr;  // stream group: block i draws into stream i's frame
+    if (own) {  // ... with stream i's format and size: nothing is written outside its plane 0
+        const int4 g = *reinterpret_cast<const int4*>(ctl->geom[blockIdx.x]);
+        fmt = g.x, W = g.y, H = g.z, len = fmt_frame_bytes(fmt, W, H);
+    }
     // HUD mode runs two CTAs per target (gridDim.y = 2): y = 0 draws on the device frame (and publishes), y = 1 on the pinned host frame —
     // the two passes over the command list (~8 us each on one CTA) run side by side
     const bool split = gridDim.y > 1;
@@ -1215,6 +1227,8 @@ __global__ void stamp_hud_kernel(unsigned long long* stamp, FrameCtl* dst, const
 cudaError_t launch_stamp(unsigned long long* stamp, FrameCtl* d_ctl, const FrameCtl& ctl, cudaStream_t s, const OverlayCmdDev* h_list, int n,
                          OverlayCmdDev* d_list) {
     static_assert(sizeof(FrameCtl) % 4 == 0 && sizeof(OverlayCmdDev) % 4 == 0, "word copy");
+    // stamp_hud_kernel's parameters (the control block by value next to the inline HUD list) stay within the 32764-byte parameter limit
+    static_assert(sizeof(FrameCtl) + sizeof(HudInline) + 4 * sizeof(void*) + sizeof(int) <= 32764, "stamp_hud_kernel parameter block");
     if (h_list && d_list && n > 0 && n <= kHudInline) {
         HudInline blk;
         memcpy(blk.c, h_list, sizeof(OverlayCmdDev) * (size_t)n);

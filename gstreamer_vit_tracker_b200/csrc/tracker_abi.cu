@@ -368,6 +368,7 @@ vt_status vt_overlay(vt_tracker* t, uint8_t* frame, size_t len, const vt_overlay
     return overlay_impl(t, frame, len, cmds, n, true);
 }
 vt_status vt_overlay_current(vt_tracker* t, uint8_t* frame, size_t len, const vt_overlay_cmd* cmds, int32_t n) {
+    if (t && check_uniform_geometry(t, "vt_overlay_current") != VT_OK) return VT_ERR_INVALID;
     if (t && t->cfg.upload_window) {
         set_error("vt_overlay_current needs the whole frame on the device: create the handle with upload_window = 0");
         return VT_ERR_INVALID;

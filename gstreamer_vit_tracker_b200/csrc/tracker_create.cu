@@ -273,8 +273,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
         if (rs != VT_OK) return rs;
     }
     const vt_config* cfg = &cfg_full;
-    if (!cfg->weights_path || cfg->width <= 0 || cfg->height <= 0 || cfg->max_targets <= 0 || cfg->max_targets > 64 ||
-        (cfg->format != VT_FMT_NV12 && cfg->format != VT_FMT_RGB24 && cfg->format != VT_FMT_GRAY8 && cfg->format != VT_FMT_YUY2)) {
+    if (!cfg->weights_path || cfg->max_targets <= 0 || cfg->max_targets > 64 || !geometry_ok(cfg->format, cfg->width, cfg->height)) {
         set_error("vt_tracker_create: invalid configuration");
         return VT_ERR_INVALID;
     }
@@ -545,6 +544,7 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
     }
     t->rect_mirror.assign(B, vt_bbox{0, 0, 0, 0});
     t->inited.assign(B, 0);
+    t->geom.assign(B, cfg_geom(t));
     VT_TRY(cudaStreamSynchronize(t->stream));
 #undef VT_TRY
     if (t->cfg.device >= 0 && t->cfg.device < kMaxDevices) {

@@ -298,14 +298,14 @@ static vt_status sync_slots(vt_tracker* t) {
 // Search window of a target in frame coordinates (App. A.1 with factor 4), grown by `margin_div` (0 = exact; d: by c / d on every side,
 // at least 16 px — used when the host's copy of rect_last lags by one frame), clipped to the frame and grown to even coordinates
 // (NV12 chroma pairs).  Returns false when the window misses the frame.
-static bool search_window(const vt_tracker* t, const vt_bbox& r, int margin_div, int& x0, int& y0, int& x1, int& y1) {
+static bool search_window(const StreamGeom& g, const vt_bbox& r, int margin_div, int& x0, int& y0, int& x1, int& y1) {
     if (r.width <= 0 || r.height <= 0) return false;
     const int c = (int)ceil(sqrt((double)(int)((long long)r.width * r.height)) * 4.0);
     const int m = margin_div > 0 ? std::max(16, c / margin_div) : 0;
     const long long wx = (long long)r.x + (r.width - c) / 2 - m, wy = (long long)r.y + (r.height - c) / 2 - m, e = (long long)c + 2 * m;
     x0 = (int)std::max(wx, 0LL) & ~1, y0 = (int)std::max(wy, 0LL) & ~1;
-    x1 = (int)std::min((std::min(wx + e, (long long)t->W) + 1) & ~1LL, (long long)t->W);
-    y1 = (int)std::min((std::min(wy + e, (long long)t->H) + 1) & ~1LL, (long long)t->H);
+    x1 = (int)std::min((std::min(wx + e, (long long)g.W) + 1) & ~1LL, (long long)g.W);
+    y1 = (int)std::min((std::min(wy + e, (long long)g.H) + 1) & ~1LL, (long long)g.H);
     return x1 > x0 && y1 > y0;
 }
 
@@ -324,29 +324,29 @@ struct UploadPlan {
 };
 // Window uploads need windows whose pixels carry their own chroma: even x0 (NV12 chroma pairs, YUY2 words) and, for NV12, even y0.
 // YUY2 takes any W and H: a window that ends on an odd last column copies that column's whole word, and chroma is per row.
-static bool windows_allowed(const vt_tracker* t) {
-    return t->fmt == VT_FMT_YUY2 || (!(t->W % 2) && !((t->H % 2) && t->fmt == VT_FMT_NV12));
+static bool windows_allowed(const StreamGeom& g) {
+    return g.fmt == VT_FMT_YUY2 || (!(g.W % 2) && !((g.H % 2) && g.fmt == VT_FMT_NV12));
 }
 // bytes of plane 0 that hold the pixels [x0, x1) x [y0, y1) of a packed frame (YUY2: whole words)
-static size_t plane0_bytes(const vt_tracker* t, int x0, int y0, int x1, int y1) {
+static size_t plane0_bytes(const StreamGeom& g, int x0, int y0, int x1, int y1) {
     size_t o0, o1;
-    fmt_col_span(t->fmt, x0, x1, &o0, &o1);
+    fmt_col_span(g.fmt, x0, x1, &o0, &o1);
     return (o1 - o0) * (size_t)(y1 - y0);
 }
 // bytes of the window w = (x0, y0, x1, y1): plane 0 and, for NV12, the chroma rows under it
-static size_t window_bytes(const vt_tracker* t, const int* w) {
-    return plane0_bytes(t, w[0], w[1], w[2], w[3]) + (t->fmt == VT_FMT_NV12 ? (size_t)(w[2] - w[0]) * ((w[3] - w[1]) / 2) : 0);
+static size_t window_bytes(const StreamGeom& g, const int* w) {
+    return plane0_bytes(g, w[0], w[1], w[2], w[3]) + (g.fmt == VT_FMT_NV12 ? (size_t)(w[2] - w[0]) * ((w[3] - w[1]) / 2) : 0);
 }
 // one 2D copy of the window w of a packed frame out of plane 0 (+ one of the NV12 chroma rows under it when `chroma`)
-static vt_status copy_window(const vt_tracker* t, uint8_t* dst, const uint8_t* src, const int* w, bool chroma, cudaMemcpyKind kind,
+static vt_status copy_window(const StreamGeom& g, uint8_t* dst, const uint8_t* src, const int* w, bool chroma, cudaMemcpyKind kind,
                              cudaStream_t stream) {
-    const size_t row = fmt_row_bytes(t->fmt, t->W), rows = (size_t)(w[3] - w[1]);
+    const size_t row = fmt_row_bytes(g.fmt, g.W), rows = (size_t)(w[3] - w[1]);
     size_t o0, o1;
-    fmt_col_span(t->fmt, w[0], w[2], &o0, &o1);
+    fmt_col_span(g.fmt, w[0], w[2], &o0, &o1);
     const size_t o = (size_t)w[1] * row + o0;
     VT_CUDA(cudaMemcpy2DAsync(dst + o, row, src + o, row, o1 - o0, rows, kind, stream));
-    if (chroma && t->fmt == VT_FMT_NV12) {
-        const size_t W = (size_t)t->W, uvo = W * t->H + (size_t)(w[1] / 2) * W + w[0];
+    if (chroma && g.fmt == VT_FMT_NV12) {
+        const size_t W = (size_t)g.W, uvo = W * g.H + (size_t)(w[1] / 2) * W + w[0];
         VT_CUDA(cudaMemcpy2DAsync(dst + uvo, W, src + uvo, W, (size_t)(w[2] - w[0]), rows / 2, kind, stream));
     }
     return VT_OK;
@@ -354,48 +354,52 @@ static vt_status copy_window(const vt_tracker* t, uint8_t* dst, const uint8_t* s
 
 static void plan_upload(vt_tracker* t, size_t len, bool pinned_host, bool lagging, const int* rmw, UploadPlan& p) {
     p = UploadPlan();
-    const bool valid = len >= fmt_valid_bytes(t->fmt, t->W, t->H);
-    if (!t->cfg.upload_window || !pinned_host || !valid || len < t->frame_bytes || (int)t->active.size() > kMaxWin || !windows_allowed(t) ||
+    const StreamGeom g = cfg_geom(t);  // (single-frame calls: a handle of uniform geometry)
+    const bool valid = len >= fmt_valid_bytes(g.fmt, g.W, g.H);
+    if (!t->cfg.upload_window || !pinned_host || !valid || len < t->frame_bytes || (int)t->active.size() > kMaxWin || !windows_allowed(g) ||
         (t->active.empty() && !t->hud_mode))
         return;
     size_t bytes = 0;
     int k = 0;
     for (int s : t->active) {
         int* w = p.win[k++];
-        if (!search_window(t, t->rect_mirror[s], lagging ? 8 : 0, w[0], w[1], w[2], w[3])) {
+        if (!search_window(g, t->rect_mirror[s], lagging ? 8 : 0, w[0], w[1], w[2], w[3])) {
             w[0] = w[1] = w[2] = w[3] = 0;  // the window misses the frame: the crop kernel flags it; nothing to read
             continue;
         }
         const int sh = t->sw.win_shrink;  // diagnostics: windows too small on purpose exercise the crop kernel's pinned-frame fall-back
         if (sh > 0 && w[2] - w[0] > 4 * sh && w[3] - w[1] > 4 * sh) w[0] += sh, w[1] += sh, w[2] -= sh, w[3] -= sh;
-        bytes += window_bytes(t, w);
+        bytes += window_bytes(g, w);
     }
     if (rmw && rmw[2] > rmw[0] && rmw[3] > rmw[1] && format_is_luma(t->fmt)) {
         p.has_rmw = true;
         p.rmw[0] = std::max(rmw[0], 0), p.rmw[1] = std::max(rmw[1], 0), p.rmw[2] = std::min(rmw[2], t->W), p.rmw[3] = std::min(rmw[3], t->H);
-        if (p.rmw[2] > p.rmw[0] && p.rmw[3] > p.rmw[1]) bytes += plane0_bytes(t, p.rmw[0], p.rmw[1], p.rmw[2], p.rmw[3]);
+        if (p.rmw[2] > p.rmw[0] && p.rmw[3] > p.rmw[1]) bytes += plane0_bytes(g, p.rmw[0], p.rmw[1], p.rmw[2], p.rmw[3]);
         else p.has_rmw = false;
     }
     if (bytes * 2 > t->frame_bytes) return;  // not worth the extra copies
     p.whole = false, p.n_win = k, p.bytes = bytes;
 }
 
-static vt_status do_upload(vt_tracker* t, const uint8_t* frame, size_t len, const UploadPlan& p, bool device_src, cudaStream_t stream) {
+// g: the geometry of the frame (the cfg one; vt_tracker_init: the slot's)
+static vt_status do_upload(vt_tracker* t, const StreamGeom& g, const uint8_t* frame, size_t len, const UploadPlan& p, bool device_src,
+                           cudaStream_t stream) {
     if (!stream) stream = t->stream;
-    size_t n = std::min(len, t->frame_bytes);
-    t->frame_valid = len >= fmt_valid_bytes(t->fmt, t->W, t->H);
-    if (!t->frame_valid && t->fmt == VT_FMT_NV12) n = 0;  // src/nv12_convert.rs:48-50 -> black image
+    const size_t frame_bytes = g.bytes();
+    size_t n = std::min(len, frame_bytes);
+    t->frame_valid = len >= fmt_valid_bytes(g.fmt, g.W, g.H);
+    if (!t->frame_valid && g.fmt == VT_FMT_NV12) n = 0;  // src/nv12_convert.rs:48-50 -> black image
     if (n == 0) return VT_OK;
     const cudaMemcpyKind kind = device_src ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
     if (!p.whole) {
         for (int i = 0; i < p.n_win; ++i) {
             const int* w = p.win[i];
             if (w[2] == w[0] || w[3] == w[1]) continue;
-            vt_status st = copy_window(t, t->d_frame, frame, w, true, kind, stream);
+            vt_status st = copy_window(g, t->d_frame, frame, w, true, kind, stream);
             if (st != VT_OK) return st;
         }
         if (p.has_rmw) {  // plane 0 only (the luma background dim reads and writes Y)
-            vt_status st = copy_window(t, t->d_frame, frame, p.rmw, false, kind, stream);
+            vt_status st = copy_window(g, t->d_frame, frame, p.rmw, false, kind, stream);
             if (st != VT_OK) return st;
         }
         if (!device_src) t->h2d_bytes += p.bytes;
@@ -403,7 +407,7 @@ static vt_status do_upload(vt_tracker* t, const uint8_t* frame, size_t len, cons
         return VT_OK;
     }
     const bool pinned = device_src || is_pinned(frame);
-    t->d_frame_is_last_host_frame = !device_src && n >= t->frame_bytes;
+    t->d_frame_is_last_host_frame = !device_src && n >= frame_bytes;
     if (!device_src) t->h2d_bytes += n;
     if (pinned) {
         VT_CUDA(cudaMemcpyAsync(t->d_frame, frame, n, kind, stream));
@@ -525,24 +529,24 @@ static inline double now_us() {
 }
 
 // A full-length packed device frame d as a surface: {d, d + W * H}, {W, W} (RGB24 / GRAY8: one plane)
-static vt_surface packed_surface(const vt_tracker* t, const uint8_t* d) {
-    const bool nv12 = t->fmt == VT_FMT_NV12;
+static vt_surface packed_surface(const StreamGeom& g, const uint8_t* d) {
+    const bool nv12 = g.fmt == VT_FMT_NV12;
     vt_surface s;
-    s.planes[0] = const_cast<uint8_t*>(d), s.planes[1] = nv12 ? const_cast<uint8_t*>(d) + (size_t)t->W * t->H : nullptr;
-    s.pitch[0] = fmt_row_bytes(t->fmt, t->W), s.pitch[1] = nv12 ? (size_t)t->W : 0;
+    s.planes[0] = const_cast<uint8_t*>(d), s.planes[1] = nv12 ? const_cast<uint8_t*>(d) + (size_t)g.W * g.H : nullptr;
+    s.pitch[0] = fmt_row_bytes(g.fmt, g.W), s.pitch[1] = nv12 ? (size_t)g.W : 0;
     return s;
 }
 
 // The caller's surface (include/vt_tracker.h: vt_surface): every plane of the format present, a pitch that holds a row, and device (or
-// managed) memory of the handle's GPU.  `i` >= 0 names the surface of a stream group in the message.
-static vt_status check_surface(const vt_tracker* t, const vt_surface* s, const char* where, int i) {
+// managed) memory of the handle's GPU, for a frame of geometry g.  `i` >= 0 names the surface of a stream group in the message.
+static vt_status check_surface(const vt_tracker* t, const StreamGeom& g, const vt_surface* s, const char* where, int i) {
     if (!s) {
         set_error("%s: surface %d is null", where, i);
         return VT_ERR_INVALID;
     }
-    const int np = t->fmt == VT_FMT_NV12 ? 2 : 1;
+    const int np = g.fmt == VT_FMT_NV12 ? 2 : 1;
     for (int p = 0; p < np; ++p) {
-        const size_t row = fmt_row_bytes(t->fmt, t->W);  // (NV12: the chroma rows are W bytes as well)
+        const size_t row = fmt_row_bytes(g.fmt, g.W);  // (NV12: the chroma rows are W bytes as well)
         if (!s->planes[p]) {
             set_error("%s: surface %d: plane %d is null", where, i, p);
             return VT_ERR_INVALID;
@@ -602,7 +606,7 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
     // device-resident frame: track (and draw the box) straight in the caller's device memory — no device->device copy.  A full-length
     // packed device frame is a surface like any other.
     vt_surface packed;
-    if (!surf && d_src && len >= t->frame_bytes) packed = packed_surface(t, d_src), surf = &packed;
+    if (!surf && d_src && len >= t->frame_bytes) packed = packed_surface(cfg_geom(t), d_src), surf = &packed;
     const bool in_place = surf != nullptr;
     if (!in_place) t->d_frame = t->d_frames[slot];  // the slot's own frame buffer: the other one may still be read by the frame in flight
     const bool lagging = t->q_count > 0;  // a frame is in flight: rect_mirror is one frame old, the windows are predictions
@@ -610,7 +614,7 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
     if (!in_place && !d_src) plan_upload(t, len, host_frame != nullptr, lagging, n_hud ? t->hud_next_rmw : nullptr, plan);
     if (!in_place && !d_src && lagging) {
         // pipelined host frame: upload on the copy stream while the frame in flight computes; the main stream picks it up through an event
-        vt_status st = do_upload(t, frame, len, plan, false, t->copy_stream);
+        vt_status st = do_upload(t, cfg_geom(t), frame, len, plan, false, t->copy_stream);
         if (st != VT_OK) return st;
         VT_CUDA(cudaEventRecord(t->ev_up[slot], t->copy_stream));
         VT_CUDA(cudaStreamWaitEvent(t->stream, t->ev_up[slot], 0));
@@ -635,10 +639,10 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
         t->frame_valid = 1;
         t->d_frame_is_last_host_frame = false;  // tracked in the caller's device memory: the internal buffer holds an older frame
     } else if (d_src) {  // short device frame: device->device copy of what there is (NV12: black frame, src/nv12_convert.rs:48-50)
-        vt_status st = do_upload(t, d_src, len, plan, true, nullptr);
+        vt_status st = do_upload(t, cfg_geom(t), d_src, len, plan, true, nullptr);
         if (st != VT_OK) return st;
     } else if (!lagging) {
-        vt_status st = do_upload(t, frame, len, plan, false, nullptr);  // the host mirror of rect_last is exact: the search windows suffice
+        vt_status st = do_upload(t, cfg_geom(t), frame, len, plan, false, nullptr);  // the host mirror of rect_last is exact: the search windows suffice
         if (st != VT_OK) return st;
     }
     const double hp1 = t->sw.hostprof ? now_us() : 0;
@@ -666,11 +670,12 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
     return VT_OK;
 }
 
-// Stream group: the n active targets of the handle are n independent video streams (one target each, same geometry), stepped together
-// through ONE batched forward (M = 320 n rows: from 1024 rows on the GEMMs run in their throughput forms).  frames[i] is the pinned
-// host frame of the i-th active target; each target's search window is uploaded into that target's own device frame and the box overlay
-// is mirrored into that target's host frame.  Or surfs[i] (frames / lens unused) is the i-th target's device surface, read and drawn
-// into in place.  Synchronous (rect_mirror is exact: the windows are the real search windows).
+// Stream group: the n active targets of the handle are n independent video streams (one target each, each of its slot's geometry),
+// stepped together through ONE batched forward (M = 320 n rows: from 1024 rows on the GEMMs run in their throughput forms).  frames[i] is
+// the pinned host frame of the i-th active target; each target's search window is uploaded into that target's own device frame and the
+// box overlay is mirrored into that target's host frame.  Or surfs[i] (frames / lens unused) is the i-th target's device surface, read
+// and drawn into in place.  Stream i's geometry travels in the control block (ctl.geom[i]), so one captured graph per stream count
+// serves any mix of sizes and formats.  Synchronous (rect_mirror is exact: the windows are the real search windows).
 static vt_status submit_streams(vt_tracker* t, uint8_t* const* frames, const size_t* lens, const vt_surface* surfs, int n) {
     const char* where = surfs ? "vt_tracker_update_streams_surface" : "vt_tracker_update_streams";
     if (t->q_count > 0 || t->hud_mode) {
@@ -682,11 +687,13 @@ static vt_status submit_streams(vt_tracker* t, uint8_t* const* frames, const siz
         return VT_ERR_INVALID;
     }
     for (int i = 0; i < n; ++i) {
+        const StreamGeom& g = slot_geom(t, t->active[i]);
         if (surfs) {
-            const vt_status st = check_surface(t, &surfs[i], where, i);
+            const vt_status st = check_surface(t, g, &surfs[i], where, i);
             if (st != VT_OK) return st;
-        } else if (!frames[i] || lens[i] < t->frame_bytes || !is_pinned(frames[i])) {
-            set_error("%s: frame %d must be a full frame in pinned host memory (vt_alloc_pinned)", where, i);
+        } else if (!frames[i] || lens[i] < g.bytes() || !is_pinned(frames[i])) {
+            set_error("%s: frame %d must be a full frame (%zu bytes for its %dx%d format %d, got %zu) in pinned host memory (vt_alloc_pinned)",
+                      where, i, g.bytes(), g.W, g.H, g.fmt, frames[i] ? lens[i] : (size_t)0);
             return VT_ERR_INVALID;
         }
     }
@@ -696,29 +703,34 @@ static vt_status submit_streams(vt_tracker* t, uint8_t* const* frames, const siz
     q.frame = surfs ? nullptr : frames[0], q.len = surfs ? 0 : lens[0], q.pageable = false, q.hud_bytes = 0, q.mirrored = !surfs;
     FrameCtl ctl;
     memset(&ctl, 0, sizeof(ctl));
-    const bool windows = t->cfg.upload_window && windows_allowed(t);
     for (int i = 0; i < n; ++i) {
+        const StreamGeom& g = slot_geom(t, t->active[i]);
+        ctl.geom[i][0] = g.fmt, ctl.geom[i][1] = g.W, ctl.geom[i][2] = g.H, ctl.geom[i][3] = 1;
         if (surfs) {  // in place: nothing to upload, the whole surface holds the frame
-            const bool nv12 = t->fmt == VT_FMT_NV12;
+            const bool nv12 = g.fmt == VT_FMT_NV12;
             ctl.frames[i] = surfs[i].planes[0], ctl.uvs[i] = nv12 ? surfs[i].planes[1] : nullptr;
             ctl.pitches[i][0] = surfs[i].pitch[0], ctl.pitches[i][1] = nv12 ? surfs[i].pitch[1] : 0;
             continue;
         }
-        if (!t->d_sframes[i]) {
-            VT_CUDA(cudaMalloc(&t->d_sframes[i], t->frame_bytes + 256));
-            VT_CUDA(cudaMemsetAsync(t->d_sframes[i], 0, t->frame_bytes + 256, t->stream));
+        const size_t fb = g.bytes();
+        if (t->d_sframe_bytes[i] < fb + 256) {  // (synchronous groups: nothing in flight reads the old buffer)
+            if (t->d_sframes[i]) VT_CUDA(cudaFree(t->d_sframes[i]));
+            t->d_sframes[i] = nullptr, t->d_sframe_bytes[i] = 0;
+            VT_CUDA(cudaMalloc(&t->d_sframes[i], fb + 256));
+            VT_CUDA(cudaMemsetAsync(t->d_sframes[i], 0, fb + 256, t->stream));
+            t->d_sframe_bytes[i] = fb + 256;
         }
         uint8_t* dst = t->d_sframes[i];
         const uint8_t* src = frames[i];
         int* w = ctl.win[i];
-        if (!windows) {
-            VT_CUDA(cudaMemcpyAsync(dst, src, t->frame_bytes, cudaMemcpyHostToDevice, t->stream));
-            t->h2d_bytes += t->frame_bytes;
-            w[0] = w[1] = 0, w[2] = t->W, w[3] = t->H;
-        } else if (search_window(t, t->rect_mirror[t->active[i]], 0, w[0], w[1], w[2], w[3])) {
-            vt_status st = copy_window(t, dst, src, w, true, cudaMemcpyHostToDevice, t->stream);
+        if (!t->cfg.upload_window || !windows_allowed(g)) {
+            VT_CUDA(cudaMemcpyAsync(dst, src, fb, cudaMemcpyHostToDevice, t->stream));
+            t->h2d_bytes += fb;
+            w[0] = w[1] = 0, w[2] = g.W, w[3] = g.H;
+        } else if (search_window(g, t->rect_mirror[t->active[i]], 0, w[0], w[1], w[2], w[3])) {
+            vt_status st = copy_window(g, dst, src, w, true, cudaMemcpyHostToDevice, t->stream);
             if (st != VT_OK) return st;
-            t->h2d_bytes += window_bytes(t, w);
+            t->h2d_bytes += window_bytes(g, w);
         } else {
             w[0] = w[1] = w[2] = w[3] = 0;  // the window misses the frame: the crop kernel flags it
         }
@@ -864,7 +876,7 @@ vt_status tracker_set_hud(vt_tracker* t, const HudCmd* cmds, int n) {
 }
 
 // The template window must intersect the frame (cv2 raises an ROI assertion otherwise, App. A.1)
-static vt_status check_template_window(const vt_tracker* t, vt_bbox box, const char* where) {
+static vt_status check_template_window(const vt_tracker* t, const StreamGeom& g, vt_bbox box, const char* where) {
     if (box.width <= 0 || box.height <= 0) {
         set_error("%s: empty box", where);
         return VT_ERR_CROP_OUTSIDE;
@@ -872,7 +884,7 @@ static vt_status check_template_window(const vt_tracker* t, vt_bbox box, const c
     const int c = (int)ceil(sqrt((double)((long long)box.width * box.height)) * 2.0);
     const int x1 = box.x + (box.width - c) / 2, y1 = box.y + (box.height - c) / 2;
     const int pp = t->cfg.pad_plus1;
-    const int pl = std::max(0, -x1), pt = std::max(0, -y1), pr = std::max(x1 + c - t->W + pp, 0), pb = std::max(y1 + c - t->H + pp, 0);
+    const int pl = std::max(0, -x1), pt = std::max(0, -y1), pr = std::max(x1 + c - g.W + pp, 0), pb = std::max(y1 + c - g.H + pp, 0);
     if (c - pl - pr <= 0 || c - pt - pb <= 0) {
         set_error("%s: template window lies outside the frame", where);
         return VT_ERR_CROP_OUTSIDE;
@@ -916,6 +928,35 @@ static vt_status init_template(vt_tracker* t, int32_t target, vt_bbox box, const
     return sync_slots(t);
 }
 
+vt_status check_uniform_geometry(const vt_tracker* t, const char* where) {
+    for (int s = 0; s < t->maxT; ++s)
+        if (!(slot_geom(t, s) == cfg_geom(t))) {
+            set_error("%s: slot %d has a stream geometry of its own (vt_tracker_set_stream_geometry): this handle takes frames through the "
+                      "stream-group calls only", where, s);
+            return VT_ERR_INVALID;
+        }
+    return VT_OK;
+}
+
+// d_frames[0..1] and h_stage hold any frame vt_tracker_init is given: the largest of the cfg and the slot geometries
+static vt_status grow_frame_buffers(vt_tracker* t, size_t bytes) {
+    if (bytes <= t->h_stage_bytes) return VT_OK;
+    VT_CUDA(cudaStreamSynchronize(t->stream));
+    for (uint8_t*& f : t->d_frames) {
+        VT_CUDA(cudaFree(f));
+        f = nullptr;
+    }
+    VT_CUDA(cudaFreeHost(t->h_stage));
+    t->h_stage = nullptr, t->h_stage_bytes = 0, t->d_frame = nullptr, t->d_frame_is_last_host_frame = false;
+    for (uint8_t*& f : t->d_frames) {
+        VT_CUDA(cudaMalloc(&f, bytes));
+        VT_CUDA(cudaMemset(f, 0, bytes));
+    }
+    VT_CUDA(cudaHostAlloc(&t->h_stage, bytes, cudaHostAllocDefault));
+    t->h_stage_bytes = bytes, t->d_frame = t->d_frames[0];
+    return VT_OK;
+}
+
 }  // namespace vt
 
 using namespace vt;
@@ -932,11 +973,12 @@ vt_status vt_tracker_init(vt_tracker* t, int32_t target, const uint8_t* frame, s
         return VT_ERR_INVALID;
     }
     VT_CUDA(cudaSetDevice(t->cfg.device));
-    vt_status st = check_template_window(t, box, "vt_tracker_init");
+    const StreamGeom& g = slot_geom(t, target);
+    vt_status st = check_template_window(t, g, box, "vt_tracker_init");
     if (st != VT_OK) return st;
-    st = do_upload(t, frame, len, UploadPlan(), false, nullptr);  // the whole frame
+    st = do_upload(t, g, frame, len, UploadPlan(), false, nullptr);  // the whole frame
     if (st != VT_OK) return st;
-    return init_template(t, target, box, FrameDesc{t->d_frame, nullptr, {0, 0}, t->W, t->H, t->fmt, t->frame_valid, nullptr, t->cfg.pad_plus1});
+    return init_template(t, target, box, FrameDesc{t->d_frame, nullptr, {0, 0}, g.W, g.H, g.fmt, t->frame_valid, nullptr, t->cfg.pad_plus1});
 }
 
 vt_status vt_tracker_init_surface(vt_tracker* t, int32_t target, const vt_surface* s, vt_bbox box) {
@@ -949,12 +991,53 @@ vt_status vt_tracker_init_surface(vt_tracker* t, int32_t target, const vt_surfac
         return VT_ERR_INVALID;
     }
     vt_status st = surface_call(t, "vt_tracker_init_surface", true);
-    if (st == VT_OK) st = check_surface(t, s, "vt_tracker_init_surface", 0);
-    if (st == VT_OK) st = check_template_window(t, box, "vt_tracker_init_surface");
+    if (st == VT_OK) st = check_surface(t, slot_geom(t, target), s, "vt_tracker_init_surface", 0);
+    const StreamGeom& g = slot_geom(t, target);
+    if (st == VT_OK) st = check_template_window(t, g, box, "vt_tracker_init_surface");
     if (st != VT_OK) return st;
-    const bool nv12 = t->fmt == VT_FMT_NV12;
-    return init_template(t, target, box, FrameDesc{s->planes[0], nv12 ? s->planes[1] : nullptr, {s->pitch[0], nv12 ? s->pitch[1] : 0}, t->W, t->H,
-                                                   t->fmt, 1, nullptr, t->cfg.pad_plus1});
+    const bool nv12 = g.fmt == VT_FMT_NV12;
+    return init_template(t, target, box, FrameDesc{s->planes[0], nv12 ? s->planes[1] : nullptr, {s->pitch[0], nv12 ? s->pitch[1] : 0}, g.W, g.H,
+                                                   g.fmt, 1, nullptr, t->cfg.pad_plus1});
+}
+
+vt_status vt_tracker_set_stream_geometry(vt_tracker* t, int32_t target, const vt_stream_geometry* g) {
+    if (!t || target < 0 || target >= t->maxT) {
+        set_error("vt_tracker_set_stream_geometry: invalid handle or target slot");
+        return VT_ERR_INVALID;
+    }
+    if (t->hud_mode) {
+        set_error("vt_tracker_set_stream_geometry: a probe (HUD) handle tracks one stream of the handle's geometry");
+        return VT_ERR_INVALID;
+    }
+    if (t->in_flight) {
+        set_error("vt_tracker_set_stream_geometry: frames are in flight (submit/wait); drain them first");
+        return VT_ERR_INVALID;
+    }
+    if (t->inited[target]) {
+        set_error("vt_tracker_set_stream_geometry: slot %d is initialised; vt_tracker_drop it first", target);
+        return VT_ERR_INVALID;
+    }
+    const StreamGeom ng = g ? StreamGeom{g->format, g->width, g->height} : cfg_geom(t);
+    if (g && (!geometry_ok(ng.fmt, ng.W, ng.H) || g->reserved != 0)) {
+        set_error("vt_tracker_set_stream_geometry: format %d, %d x %d (reserved %d) is not a frame geometry (a vt_format, width and height > 0, "
+                  "reserved 0)", g->format, g->width, g->height, g->reserved);
+        return VT_ERR_INVALID;
+    }
+    VT_CUDA(cudaSetDevice(t->cfg.device));
+    const vt_status st = grow_frame_buffers(t, ng.bytes() + 256);
+    if (st != VT_OK) return st;
+    t->geom[target] = ng;
+    return VT_OK;
+}
+
+vt_status vt_tracker_get_stream_geometry(const vt_tracker* t, int32_t target, vt_stream_geometry* out) {
+    if (!t || !out || target < 0 || target >= t->maxT) {
+        set_error("vt_tracker_get_stream_geometry: invalid argument");
+        return VT_ERR_INVALID;
+    }
+    const StreamGeom& g = slot_geom(t, target);
+    out->format = g.fmt, out->width = g.W, out->height = g.H, out->reserved = 0;
+    return VT_OK;
 }
 
 vt_status vt_tracker_drop(vt_tracker* t, int32_t target) {
@@ -970,6 +1053,8 @@ vt_status vt_tracker_drop(vt_tracker* t, int32_t target) {
 
 vt_status vt_tracker_submit(vt_tracker* t, uint8_t* frame, size_t len) {
     if (!t || !frame) return VT_ERR_INVALID;
+    vt_status st = check_uniform_geometry(t, "vt_tracker_submit");
+    if (st != VT_OK) return st;
     VT_CUDA(cudaSetDevice(t->cfg.device));
     return submit_common(t, frame, nullptr, len);
 }
@@ -986,6 +1071,8 @@ extern "C" {
 
 vt_status vt_tracker_submit_device(vt_tracker* t, uint8_t* d_frame, size_t len) {
     if (!t || !d_frame) return VT_ERR_INVALID;
+    vt_status st = check_uniform_geometry(t, "vt_tracker_submit_device");
+    if (st != VT_OK) return st;
     VT_CUDA(cudaSetDevice(t->cfg.device));
     return submit_common(t, nullptr, d_frame, len);
 }
@@ -998,12 +1085,14 @@ vt_status vt_tracker_wait(vt_tracker* t, vt_result* results) {
 
 vt_status vt_tracker_update(vt_tracker* t, uint8_t* frame, size_t len, vt_result* results) {
     if (!t || !frame) return VT_ERR_INVALID;
+    vt_status st = check_uniform_geometry(t, "vt_tracker_update");
+    if (st != VT_OK) return st;
     VT_CUDA(cudaSetDevice(t->cfg.device));
     if (t->q_count) {
         set_error("vt_tracker_update: frames are in flight (submit/wait); drain them first");
         return VT_ERR_INVALID;
     }
-    vt_status st = submit_common(t, frame, nullptr, len);
+    st = submit_common(t, frame, nullptr, len);
     if (st != VT_OK) return st;
     return wait_common(t, results);
 }
@@ -1018,20 +1107,23 @@ vt_status vt_tracker_update_streams(vt_tracker* t, uint8_t* const* frames, const
 
 vt_status vt_tracker_update_device(vt_tracker* t, uint8_t* d_frame, size_t len, vt_result* results) {
     if (!t || !d_frame) return VT_ERR_INVALID;
+    vt_status st = check_uniform_geometry(t, "vt_tracker_update_device");
+    if (st != VT_OK) return st;
     VT_CUDA(cudaSetDevice(t->cfg.device));
     if (t->q_count) {
         set_error("vt_tracker_update_device: frames are in flight (submit/wait); drain them first");
         return VT_ERR_INVALID;
     }
-    vt_status st = submit_common(t, nullptr, d_frame, len);
+    st = submit_common(t, nullptr, d_frame, len);
     if (st != VT_OK) return st;
     return wait_common(t, results);
 }
 
 vt_status vt_tracker_update_surface(vt_tracker* t, const vt_surface* s, vt_result* results) {
     if (!t || !s) return VT_ERR_INVALID;
-    vt_status st = surface_call(t, "vt_tracker_update_surface", true);
-    if (st == VT_OK) st = check_surface(t, s, "vt_tracker_update_surface", 0);
+    vt_status st = check_uniform_geometry(t, "vt_tracker_update_surface");
+    if (st == VT_OK) st = surface_call(t, "vt_tracker_update_surface", true);
+    if (st == VT_OK) st = check_surface(t, cfg_geom(t), s, "vt_tracker_update_surface", 0);
     if (st == VT_OK) st = submit_common(t, nullptr, nullptr, 0, true, s);
     if (st != VT_OK) return st;
     return wait_common(t, results);
@@ -1039,8 +1131,9 @@ vt_status vt_tracker_update_surface(vt_tracker* t, const vt_surface* s, vt_resul
 
 vt_status vt_tracker_submit_surface(vt_tracker* t, const vt_surface* s) {
     if (!t || !s) return VT_ERR_INVALID;
-    vt_status st = surface_call(t, "vt_tracker_submit_surface", false);
-    if (st == VT_OK) st = check_surface(t, s, "vt_tracker_submit_surface", 0);
+    vt_status st = check_uniform_geometry(t, "vt_tracker_submit_surface");
+    if (st == VT_OK) st = surface_call(t, "vt_tracker_submit_surface", false);
+    if (st == VT_OK) st = check_surface(t, cfg_geom(t), s, "vt_tracker_submit_surface", 0);
     if (st != VT_OK) return st;
     return submit_common(t, nullptr, nullptr, 0, true, s);
 }
@@ -1064,6 +1157,7 @@ vt_status vt_tracker_run_ring(vt_tracker* t, uint8_t* frames, size_t stride, siz
         set_error("vt_tracker_run_ring: frames are in flight; drain them first");
         return VT_ERR_INVALID;
     }
+    if (check_uniform_geometry(t, "vt_tracker_run_ring") != VT_OK) return VT_ERR_INVALID;
     VT_CUDA(cudaSetDevice(t->cfg.device));
     const bool device = mode >= VT_RUN_DEVICE_SYNC, pipelined = mode == VT_RUN_HOST_PIPELINED || mode == VT_RUN_DEVICE_PIPELINED;
     std::vector<vt_result> res((size_t)t->maxT);
@@ -1126,8 +1220,9 @@ vt_status vt_tracker_run_streams_ring(vt_tracker* t, uint8_t* const* rings, int3
         if (st == VT_OK && pristine && t->cfg.box_overlay)  // undo what the box overlays drew: the rings are replayed on clean frames
             for (int k = 0; k < n_streams && k < (int)t->active.size(); ++k) {
                 const vt_result& r = res[t->active[k]];
+                const StreamGeom& g = slot_geom(t, t->active[k]);
                 if (pristine[k] && r.status == VT_OK && r.success && r.score > t->cfg.overlay_gate)
-                    restore_box_region(fr[k], pristine[k] + off, t->fmt, t->W, t->H, r.bbox);
+                    restore_box_region(fr[k], pristine[k] + off, g.fmt, g.W, g.H, r.bbox);
             }
     }
     if (last && st == VT_OK && n > 0) memcpy(last, res.data(), sizeof(vt_result) * (size_t)t->maxT);

@@ -94,7 +94,8 @@ struct vt_tracker {
 
     // frame + state
     uint8_t* d_frame = nullptr;
-    uint8_t* d_sframes[kMaxWin] = {};  // stream groups: one device frame per target slot (allocated on first use)
+    uint8_t* d_sframes[kMaxWin] = {};  // stream groups: one device frame per stream (allocated on first use, grown with its geometry)
+    size_t d_sframe_bytes[kMaxWin] = {};
     uint8_t* d_frames[2] = {nullptr, nullptr};  // double buffer: d_frame points at the one most recently filled (queue slot s uses [s])
     cudaStream_t copy_stream = nullptr;          // uploads of pipelined host frames overlap the in-flight frame's kernels
     cudaEvent_t ev_up[2] = {nullptr, nullptr};
@@ -105,7 +106,7 @@ struct vt_tracker {
     int4* d_rsz_taps = nullptr;          // resize taps of the last geometry: [dw] column taps then [dh] row taps
     int rsz_geom[4] = {0, 0, 0, 0};      // sw, sh, dw, dh they were built for
     uint8_t* h_stage = nullptr;  // pinned staging for non-pinned callers
-    size_t h_stage_bytes = 0;
+    size_t h_stage_bytes = 0;    // bytes of h_stage and of each d_frames[i]: the largest frame of the cfg and the slot geometries, + 256
     int frame_valid = 1;
     // what the device frame buffer t->d_frame holds: the whole host frame most recently given to update()/submit()/init() (what
     // vt_overlay_current draws on), or something else (search windows only, a convert / overlay scratch upload, nothing: the last frame
@@ -133,6 +134,7 @@ struct vt_tracker {
     std::vector<int> active;          // slot indices, ascending
     std::vector<vt_bbox> rect_mirror; // host mirror of rect_last (valid after wait)
     std::vector<int> inited;
+    std::vector<StreamGeom> geom;     // per slot: the geometry of its stream's frames (the cfg one unless vt_tracker_set_stream_geometry)
 
     // activations
     float *patches_x = nullptr, *patches_z = nullptr, *Zemb = nullptr, *X = nullptr, *QKV = nullptr, *ATT = nullptr, *HID = nullptr,
@@ -195,6 +197,12 @@ struct vt_tracker {
 namespace vt {
 
 bool is_pinned(const void* p);
+// The one home of the geometry decision: the handle's own (cfg) geometry, and the geometry of target slot `slot`'s frames, which every
+// site that reads, uploads, checks or draws into a slot's frames goes through.  A uniform handle is one whose slots all hold the cfg one.
+inline StreamGeom cfg_geom(const vt_tracker* t) { return StreamGeom{t->fmt, t->W, t->H}; }
+inline const StreamGeom& slot_geom(const vt_tracker* t, int slot) { return t->geom[slot]; }
+// VT_ERR_INVALID (with a message naming `where`) on a handle where a slot's geometry differs from cfg: single-frame entry points
+vt_status check_uniform_geometry(const vt_tracker* t, const char* where);
 // vt_overlay_cmd -> device form (glyph rows resolved); VT_ERR_GLYPH for an unknown character in strict mode
 vt_status fill_cmd_dev(const vt_overlay_cmd& c, OverlayCmdDev& d);
 void bind_slot(vt_tracker* t, int slot);

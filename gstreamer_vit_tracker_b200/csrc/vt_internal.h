@@ -48,6 +48,17 @@ __host__ __device__ inline size_t fmt_frame_bytes(int fmt, int W, int H) {
 __host__ __device__ inline size_t fmt_valid_bytes(int fmt, int W, int H) {
     return fmt == VT_FMT_NV12 ? (size_t)W * H * 3 / 2 : fmt_frame_bytes(fmt, W, H);
 }
+// Geometry of the frames of one stream: the handle's (cfg.format / width / height), or a target slot's own in a stream group of mixed
+// cameras (vt_tracker_set_stream_geometry)
+struct StreamGeom {
+    int32_t fmt, W, H;
+    size_t bytes() const { return fmt_frame_bytes(fmt, W, H); }
+    bool operator==(const StreamGeom& o) const { return fmt == o.fmt && W == o.W && H == o.H; }
+};
+// the formats and sizes a handle's frames may have (vt_tracker_create's cfg, vt_tracker_set_stream_geometry)
+inline bool geometry_ok(int fmt, int W, int H) {
+    return W > 0 && H > 0 && (fmt == VT_FMT_NV12 || fmt == VT_FMT_RGB24 || fmt == VT_FMT_GRAY8 || fmt == VT_FMT_YUY2);
+}
 // the bytes [*o0, *o1) of a plane-0 row that hold the pixels x0 .. x1 - 1 (YUY2: the whole words of those pixels)
 __host__ __device__ inline void fmt_col_span(int fmt, long long x0, long long x1, size_t* o0, size_t* o1) {
     if (fmt == VT_FMT_YUY2) *o0 = (size_t)(2 * (x0 & ~1LL)), *o1 = (size_t)(4 * ((x1 + 1) / 2));
@@ -160,6 +171,8 @@ struct FrameCtl {
     const uint8_t* uvs[kMaxWin];          // chroma plane and row pitches of frames[i], as `uv` / `pitch` of `frame`
     size_t pitches[kMaxWin][2];
     uint8_t* host_frames[kMaxWin];
+    alignas(16) int32_t geom[kMaxWin][4]; // {format, width, height, valid} of frames[i]: the crop and the box overlay take them over FrameDesc's
+                                          // (a group may mix cameras; the captured graph does not change with the mix)
     int32_t bg_on_device;      // the region a leading HUD background dim reads was uploaded with the windows: read it from the device frame
     int32_t bg_ready;          // set by the host-pass CTA of the overlay kernel once its copy of that region is in registers (reset per frame)
 };

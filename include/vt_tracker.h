@@ -149,14 +149,29 @@ vt_status vt_tracker_submit(vt_tracker* t, uint8_t* frame, size_t len);
 vt_status vt_tracker_submit_device(vt_tracker* t, uint8_t* d_frame, size_t len);  /* frame already in device memory, tracked in place */
 vt_status vt_tracker_wait(vt_tracker* t, vt_result* results);
 
-/* Stream group: the handle's n active targets are n independent video streams of the same geometry — ≙ n TrackerContexts
- * (src/pipeline.rs:55: one per pipeline) stepped together.  frames[i] (pinned host memory, a full frame) belongs to the i-th active
- * target (ascending slot order); every stream's search window is uploaded into its own device frame, all n targets go through ONE
- * batched ViT forward (from 4 streams on the GEMMs run in their many-row throughput forms), and with cfg.box_overlay each stream's
- * box is drawn into ITS frame.  results[slot] as in update().  Each target is initialised on a frame of its own stream with
- * vt_tracker_init(t, slot, frame_of_that_stream, len, box).  Results equal those of n single-target handles (boxes equal, scores
- * within the re-association noise of the kernel forms, <= 1e-5). */
+/* Stream group: the handle's n active targets are n independent video streams — ≙ n TrackerContexts (src/pipeline.rs:55: one per
+ * pipeline) stepped together.  frames[i] (pinned host memory, a full frame: lens[i] >= the frame bytes of stream i's geometry) belongs
+ * to the i-th active target (ascending slot order); every stream's search window is uploaded into its own device frame, all n targets
+ * go through ONE batched ViT forward (from 4 streams on the GEMMs run in their many-row throughput forms), and with cfg.box_overlay
+ * each stream's box is drawn into ITS frame.  results[slot] as in update().  Each target is initialised on a frame of its own stream
+ * with vt_tracker_init(t, slot, frame_of_that_stream, len, box).  Results equal those of n single-target handles of the streams'
+ * geometries (boxes equal, scores within the re-association noise of the kernel forms, <= 1e-5).
+ * Every stream has the handle's geometry (cfg.format / width / height) unless its slot was given one of its own with
+ * vt_tracker_set_stream_geometry: one group may mix cameras of different sizes and formats (e.g. a 1920x1080 NV12 visible camera and a
+ * 640x512 YUY2 IR camera, src/pipeline.rs:26-36 / src/pipeline_ir.rs:27-56) in the same batched forward. */
 vt_status vt_tracker_update_streams(vt_tracker* t, uint8_t* const* frames, const size_t* lens, int32_t n, vt_result* results);
+
+/* Stream groups of mixed cameras: target slot `target` takes frames of its own format and size instead of cfg.format / width / height.
+ * Once set, every call that handles that slot's frames uses it: vt_tracker_init / vt_tracker_init_surface on the slot (template crop,
+ * length, pitch and template-window checks) and, for the stream of that slot, vt_tracker_update_streams, vt_tracker_update_streams_surface
+ * and vt_tracker_run_streams_ring.  Everything else stays per handle (pad_plus1, decode / window switches, normalisation, box_overlay,
+ * overlay_gate, upload_window).  VT_ERR_INVALID (and vt_last_error()) for: an initialised slot (vt_tracker_drop it first), frames in
+ * flight, a probe (HUD) handle, an unknown format, or a width or height <= 0.  g == NULL: the slot goes back to the cfg geometry.
+ * On a handle where any slot's geometry differs from cfg the single-frame entry points (update, submit, *_device, update_surface,
+ * submit_surface, run_ring, vt_overlay_current) are VT_ERR_INVALID: one frame of the handle's geometry cannot serve every target. */
+typedef struct { int32_t format, width, height, reserved; } vt_stream_geometry;  /* format: vt_format; reserved: 0 */
+vt_status vt_tracker_set_stream_geometry(vt_tracker* t, int32_t target, const vt_stream_geometry* g);
+vt_status vt_tracker_get_stream_geometry(const vt_tracker* t, int32_t target, vt_stream_geometry* out);
 
 /* Same as update() but the frame is already in device memory (bench `value` leg, NVDEC/NVMM producers): the tracker reads the
  * caller's frame in place (no copy) and, with cfg.box_overlay, draws the box INTO it — the in-place semantics of the reference's
@@ -179,7 +194,8 @@ vt_status vt_tracker_init_surface(vt_tracker* t, int32_t target, const vt_surfac
 vt_status vt_tracker_update_surface(vt_tracker* t, const vt_surface* s, vt_result* results);         /* ≙ vt_tracker_update_device */
 vt_status vt_tracker_submit_surface(vt_tracker* t, const vt_surface* s);                             /* ≙ vt_tracker_submit_device; then wait() */
 /* ≙ vt_tracker_update_streams: surfaces[i] belongs to the i-th active target (n = the number of active targets, at most 16); each stream's
- * box is drawn into its own surface.  Streams may have different pitches and plane offsets. */
+ * box is drawn into its own surface.  Streams may have different pitches and plane offsets, and each surface is checked against the row
+ * bytes and plane count of its own stream's geometry (vt_tracker_set_stream_geometry). */
 vt_status vt_tracker_update_streams_surface(vt_tracker* t, const vt_surface* surfaces, int32_t n, vt_result* results);
 
 /* The per-buffer loop of a streaming thread, run natively (≙ the GStreamer streaming thread invoking the probe once per buffer,
@@ -194,7 +210,8 @@ typedef enum { VT_RUN_HOST_SYNC = 0, VT_RUN_HOST_PIPELINED = 1, VT_RUN_DEVICE_SY
 vt_status vt_tracker_run_ring(vt_tracker* t, uint8_t* frames, size_t stride, size_t frame_len, int32_t ring, int32_t first, int32_t n,
                               int32_t mode, const uint8_t* pristine, vt_result* last, double* latency_us);
 /* The same loop for a stream group (vt_tracker_update_streams per step): rings[i] = ring of stream i (pinned host memory), pristine[i]
- * (nullable array / entries) = its clean copy. */
+ * (nullable array / entries) = its clean copy.  In a group of mixed geometries frame_len and stride cover the largest stream's frame;
+ * each stream reads (and restores) only the bytes of its own geometry. */
 vt_status vt_tracker_run_streams_ring(vt_tracker* t, uint8_t* const* rings, int32_t n_streams, size_t stride, size_t frame_len, int32_t ring,
                                       int32_t first, int32_t n, const uint8_t* const* pristine, vt_result* last, double* latency_us);
 
