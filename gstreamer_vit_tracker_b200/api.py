@@ -610,10 +610,19 @@ class TrackerContext:
     def new(cls, model_path: str, width: int, height: int, **kw) -> "TrackerContext":
         return cls(make_config(model_path, width, height, **kw))
 
+    @classmethod
+    def _member(cls, handle: C.c_void_p, cfg: vt_config, width: int, height: int) -> "TrackerContext":
+        """A non-owning view of a probe group's member context (close() leaves it to the group)."""
+        self = cls.__new__(cls)
+        self._h, self._cfg, self._owned = handle, cfg, False
+        self.frame_width, self.frame_height = width, height
+        self.tracker = VitTrack(cfg, _handle=C.c_void_p(lib().vt_context_tracker(handle)), _owned=False)
+        return self
+
     def close(self):
-        if getattr(self, "_h", None):
+        if getattr(self, "_h", None) and getattr(self, "_owned", True):
             lib().vt_context_destroy(self._h)
-            self._h = None
+        self._h = None
 
     def __del__(self):
         try:
@@ -709,3 +718,67 @@ class TimingStats:
 
     def avg_track_ms(self) -> float:
         return lib().vt_timing_stats_avg_track_ms(self._s) if self._s else self._t.timing().avg_track_ms
+
+
+class ProbeGroup:
+    """Probe groups (vt_probe_group_*): the drop-in probe for up to 16 cameras in one batched forward.  Stream i behaves exactly like a
+    TrackerContext of its own geometry probing the same frames with the same commands; one step runs ONE batched forward over the streams
+    whose state machine calls VitTrack on that frame and draws every stream's HUD in place, with one synchronisation.
+
+    `contexts[i]` is a non-owning TrackerContext view of stream i (commands, state, score, box, selection; its `tracker` is the group's
+    shared tracker, on which stream i is target i); `tracker` is that shared tracker."""
+
+    def __init__(self, cfg: vt_config, cams: Sequence[Tuple[int, int, str]]):
+        n = len(cams)
+        geoms = (vt_stream_geometry * max(n, 1))(*[vt_stream_geometry(FORMATS[f], int(w), int(h), 0) for (w, h, f) in cams])
+        cfg.max_targets = max(n, 1)  # (the group's tracker has one target slot per stream)
+        h = C.c_void_p()
+        check(lib().vt_probe_group_create(C.byref(cfg), n, geoms, C.byref(h)), "vt_probe_group_create")
+        self._h, self._cfg = h, cfg
+        self.cams = [(int(w), int(h_), f) for (w, h_, f) in cams]
+        self.contexts = [TrackerContext._member(C.c_void_p(lib().vt_probe_group_context(h, i)), cfg, w, h_) for i, (w, h_, _) in enumerate(self.cams)]
+        self.tracker = self.contexts[0].tracker if n else None
+
+    @classmethod
+    def new(cls, model_path: str, cams: Sequence[Tuple[int, int, str]], **kw) -> "ProbeGroup":
+        """cams = [(width, height, fmt), ...] (1..16 streams); kw: make_config's (the format / size there default to cams[0]'s)."""
+        w, h, f = cams[0] if cams else (1920, 1080, "nv12")
+        kw.setdefault("fmt", f)
+        return cls(make_config(model_path, w, h, **kw), cams)
+
+    def __len__(self) -> int:
+        return lib().vt_probe_group_size(self._h) if self._h else 0
+
+    def close(self):
+        if getattr(self, "_h", None):
+            for c in self.contexts:
+                c._h = None
+            self.tracker = None
+            lib().vt_probe_group_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def probe(self, frames: Sequence[np.ndarray], hud: Optional[Tuple[str, str]] = None) -> None:
+        """One step: frames[i] — a full frame of stream i in pinned host memory (PinnedBuffer) — probed and drawn on in place."""
+        n = len(frames)
+        ptrs = (C.c_void_p * n)(*[_ptr(f).value for f in frames])
+        lens = (C.c_size_t * n)(*[f.size for f in frames])
+        arr = (C.c_char_p * 2)(hud[0].encode(), hud[1].encode()) if hud is not None else None
+        check(lib().vt_probe_group_frame(self._h, ptrs, lens, arr), "vt_probe_group_frame")
+
+    def run_ring(self, ring_ptrs: Sequence[int], stride: int, frame_len: int, ring: int, first: int, n: int,
+                 hud: Optional[Tuple[str, str]] = None, pristine_ptrs: Optional[Sequence[int]] = None, want_latency: bool = False):
+        """n steps over per-stream host rings (pinned) in one native call (vt_probe_group_run_ring); returns the step latencies (us)."""
+        k = len(ring_ptrs)
+        rings = (C.c_void_p * k)(*ring_ptrs)
+        pr = (C.c_void_p * k)(*pristine_ptrs) if pristine_ptrs is not None else None
+        arr = (C.c_char_p * 2)(hud[0].encode(), hud[1].encode()) if hud is not None else None
+        lat = np.empty(n, np.float64) if want_latency else None
+        check(lib().vt_probe_group_run_ring(self._h, rings, stride, frame_len, ring, first, n, arr, pr,
+                                            lat.ctypes.data_as(C.POINTER(C.c_double)) if want_latency else None), "vt_probe_group_run_ring")
+        return lat

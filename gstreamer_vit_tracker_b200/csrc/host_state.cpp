@@ -78,8 +78,28 @@ struct vt_context {
     uint64_t frame_num = 0;
     bool have_last = false;
     std::chrono::steady_clock::time_point last_time;
+    vt_probe_group* group = nullptr;  // member of a probe group: borrowed (the group owns it and the tracker), frames go through the group
     vt_context(int w, int h) : selection(w, h), frame_width(w), frame_height(h) {}
 };
+
+// ≙ n TrackerContexts (one per pipeline, src/pipeline.rs:55) sharing one tracker handle: stream i = member i = target slot i
+struct vt_probe_group {
+    vt_tracker* tracker = nullptr;
+    std::vector<vt_context*> members;
+    // probe state of the group step (one interval per step: every stream is probed once per step)
+    uint64_t frame_num = 0;
+    bool have_last = false;
+    std::chrono::steady_clock::time_point last_time;
+};
+
+namespace {
+// the single-context frame entry points refuse a group member
+bool member_refused(const vt_context* c, const char* where) {
+    if (!c || !c->group) return false;
+    vt::set_error("%s: this context is a member of a probe group; its frames go through vt_probe_group_frame / vt_probe_group_run_ring", where);
+    return true;
+}
+}  // namespace
 
 extern "C" {
 
@@ -113,7 +133,7 @@ vt_status vt_context_create(const vt_config* cfg, vt_context** out) {
 }
 
 void vt_context_destroy(vt_context* c) {
-    if (!c) return;
+    if (!c || c->group) return;  // (a group member is destroyed with its group)
     if (c->tracker) vt_tracker_destroy(c->tracker);
     delete c;
 }
@@ -232,7 +252,7 @@ void process_frame_core(vt_context* c, InitUpdate init_and_update, Update update
 extern "C" {
 
 vt_status vt_context_process_frame(vt_context* c, uint8_t* frame, size_t len, int32_t* has_bbox, vt_bbox* bbox) {
-    if (!c || !c->tracker || !frame || !has_bbox || !bbox) return VT_ERR_INVALID;
+    if (!c || !c->tracker || !frame || !has_bbox || !bbox || member_refused(c, "vt_context_process_frame")) return VT_ERR_INVALID;
     c->frame_on_device = false;
     auto upd = [&]() {
         UpdateOutcome o;
@@ -466,7 +486,8 @@ static vt_status probe_one_sync(vt_context* c, uint8_t* frame, size_t len, const
 // ≙ the streaming thread invoking the probe once per buffer (src/pipeline.rs:65-67): n frames of a host ring through vt_probe_frame
 vt_status vt_context_run_ring(vt_context* c, uint8_t* frames, size_t stride, size_t frame_len, int32_t ring, int32_t first, int32_t n,
                               const char* const* hud_override, const uint8_t* pristine, double* latency_us) {
-    if (!c || !c->tracker || !frames || ring <= 0 || first < 0 || n < 0 || frame_len > stride) return VT_ERR_INVALID;
+    if (!c || !c->tracker || !frames || ring <= 0 || first < 0 || n < 0 || frame_len > stride || member_refused(c, "vt_context_run_ring"))
+        return VT_ERR_INVALID;
     const int fmt = c->cfg.format, W = c->frame_width, H = c->frame_height;
     for (int i = 0; i < n; ++i) {
         uint8_t* fr = frames + (size_t)((first + i) % ring) * stride;
@@ -486,7 +507,7 @@ vt_status vt_context_run_ring(vt_context* c, uint8_t* frames, size_t stride, siz
 
 // ≙ the pad-probe closure body: src/pipeline.rs:67-184 (NV12) / src/pipeline_ir.rs:100-228 (RGB24)
 vt_status vt_probe_frame(vt_context* c, uint8_t* frame, size_t len, const char* const* hud_override) {
-    if (!c || !c->tracker || !frame) return VT_ERR_INVALID;
+    if (!c || !c->tracker || !frame || member_refused(c, "vt_probe_frame")) return VT_ERR_INVALID;
     vt_tracker* t = c->tracker;
     const bool nv12 = vt::format_is_luma(c->cfg.format);  // GRAY8 / YUY2 frames take the luma-plane HUD of src/pipeline.rs:125-174
     // interval timing, src/pipeline.rs:69-79
@@ -499,6 +520,178 @@ vt_status vt_probe_frame(vt_context* c, uint8_t* frame, size_t len, const char* 
                                                                                 : probe_two_step(c, frame, len, hud_override, nv12);
     if (st != VT_OK) return st;
     probe_log(c, nv12, num);
+    return VT_OK;
+}
+
+// ---- probe groups: n cameras, one batched forward and one synchronisation per step (include/vt_tracker.h) ----------------------
+vt_status vt_probe_group_create(const vt_config* cfg, int32_t n_streams, const vt_stream_geometry* geoms, vt_probe_group** out) {
+    if (out) *out = nullptr;
+    if (!cfg || !out) {
+        vt::set_error("vt_probe_group_create: null config or output");
+        return VT_ERR_INVALID;
+    }
+    if (n_streams < 1 || n_streams > vt::kMaxWin) {
+        vt::set_error("vt_probe_group_create: %d streams (a group has 1..%d)", n_streams, vt::kMaxWin);
+        return VT_ERR_INVALID;
+    }
+    vt_config c;
+    vt_status st = vt::resolve_config(cfg, &c);
+    if (st != VT_OK) return st;
+    for (int i = 0; geoms && i < n_streams; ++i)  // (the rule of vt_tracker_set_stream_geometry, checked before anything is allocated)
+        if (!vt::geometry_ok(geoms[i].format, geoms[i].width, geoms[i].height) || geoms[i].reserved != 0) {
+            vt::set_error("vt_probe_group_create: stream %d: format %d, %d x %d (reserved %d) is not a frame geometry", i, geoms[i].format,
+                          geoms[i].width, geoms[i].height, geoms[i].reserved);
+            return VT_ERR_INVALID;
+        }
+    c.max_targets = n_streams;  // one VitTrack per TrackerContext: one target slot per stream
+    c.box_overlay = 0;          // the probe queues explicit overlay commands (the box is one of them)
+    vt_tracker* t = nullptr;
+    if ((st = vt_tracker_create(&c, &t)) != VT_OK) return st;
+    for (int i = 0; geoms && i < n_streams && st == VT_OK; ++i) st = vt_tracker_set_stream_geometry(t, i, &geoms[i]);  // before HUD mode
+    if (st == VT_OK) st = vt::tracker_make_group(t, n_streams);
+    if (st != VT_OK) {
+        vt_tracker_destroy(t);
+        return st;
+    }
+    vt_probe_group* g = new vt_probe_group();
+    g->tracker = t;
+    for (int i = 0; i < n_streams; ++i) {
+        vt_stream_geometry sg;
+        vt_tracker_get_stream_geometry(t, i, &sg);
+        vt_context* ctx = new vt_context(sg.width, sg.height);
+        ctx->tracker = t, ctx->group = g;
+        ctx->cfg = c;
+        ctx->cfg.weights_path = nullptr, ctx->cfg.format = sg.format, ctx->cfg.width = sg.width, ctx->cfg.height = sg.height, ctx->cfg.max_targets = 1;
+        g->members.push_back(ctx);
+    }
+    *out = g;
+    return VT_OK;
+}
+
+void vt_probe_group_destroy(vt_probe_group* g) {
+    if (!g) return;
+    if (g->tracker) vt_tracker_destroy(g->tracker);
+    for (vt_context* c : g->members) delete c;
+    delete g;
+}
+
+int32_t vt_probe_group_size(const vt_probe_group* g) { return g ? (int32_t)g->members.size() : VT_ERR_INVALID; }
+
+vt_context* vt_probe_group_context(vt_probe_group* g, int32_t stream) {
+    return g && stream >= 0 && stream < (int32_t)g->members.size() ? g->members[(size_t)stream] : nullptr;
+}
+
+// ≙ probe_one_sync for every stream of the group at once: each stream predicts whether its state machine calls VitTrack on this frame
+// (TRACKING: update; SELECT END with a pending confirm: init on this stream's frame into its slot, then update).  The others step their
+// state machines on the host first and queue their final HUD; those that take part queue the HUD of both outcomes, and the step's last
+// kernel picks per stream by that stream's own result.  A stream that leaves TRACKING, or whose confirm fails the gate, gives up its slot:
+// LOST and SELECT never call update, and tracking resumes only through a fresh init.
+vt_status vt_probe_group_frame(vt_probe_group* g, uint8_t* const* frames, const size_t* lens, const char* const* hud_override) {
+    if (!g || !g->tracker || !frames || !lens) {
+        vt::set_error("vt_probe_group_frame: null group, frames or lengths");
+        return VT_ERR_INVALID;
+    }
+    vt_tracker* t = g->tracker;
+    const int n = (int)g->members.size();
+    for (int i = 0; i < n; ++i) {
+        const vt_context* c = g->members[(size_t)i];
+        const size_t need = vt::fmt_frame_bytes(c->cfg.format, c->frame_width, c->frame_height);
+        if (!frames[i] || lens[i] < need || !vt::frame_is_pinned(frames[i])) {
+            vt::set_error("vt_probe_group_frame: frame %d must be a full frame (%zu bytes for its %dx%d format %d, got %zu) in pinned host memory "
+                          "(vt_alloc_pinned)", i, need, c->frame_width, c->frame_height, c->cfg.format, frames[i] ? lens[i] : (size_t)0);
+            return VT_ERR_INVALID;
+        }
+    }
+    const auto now = std::chrono::steady_clock::now();  // interval timing, src/pipeline.rs:69-79 (one probe per stream and step)
+    if (g->have_last) vt_timing_add_interval(t, (uint64_t)std::chrono::duration_cast<std::chrono::microseconds>(now - g->last_time).count());
+    g->last_time = now, g->have_last = true;
+    const uint64_t num = g->frame_num++;
+    const auto t1 = std::chrono::steady_clock::now();
+    std::vector<bool> part((size_t)n, false);
+    std::vector<vt::HudCmd> hud;
+    vt_status st;
+    bool any = false;
+    for (int i = 0; i < n; ++i) {
+        vt_context* c = g->members[(size_t)i];
+        const bool nv12 = vt::format_is_luma(c->cfg.format);
+        HudText h;
+        hud_text(c, nv12, hud_override, h);
+        // what process_frame will do with this frame (src/tracker_context.rs:64-155)
+        const bool init_update = c->state == AppState::Selecting && c->pending_confirm && c->selection.phase == 1;
+        const bool update = c->state == AppState::Tracking;
+        part[(size_t)i] = init_update || update;
+        any = any || part[(size_t)i];
+        hud.clear();
+        if (nv12) hud.push_back(vt::HudCmd{make_cmd(VT_OV_BACKGROUND, 10, 10, 400, 80, 150, 0, 0, 0), vt::VT_HUD_ALWAYS, vt::VT_HUD_GIVEN});
+        int32_t has = 0;
+        vt_bbox bb{0, 0, 0, 0};
+        if (!part[(size_t)i]) {
+            // no tracker call on this frame: the state machine steps on the host first, the HUD shows the new state; a slot still held
+            // (Cancel while tracking) leaves the forward
+            if (vt::tracker_group_active(t, i) && (st = vt::tracker_group_drop(t, i)) != VT_OK) return st;
+            process_frame_core(c, [&](vt_bbox) { return UpdateOutcome{false, vt_result{}}; }, [&]() { return UpdateOutcome{false, vt_result{}}; }, &has, &bb);
+            hud_commands(c, nv12, vt_context_state(c), h, false, bb, c->current_score, vt::VT_HUD_ALWAYS, false, hud);
+        } else {
+            if (init_update) vt::tracker_group_init(t, i, frames[i], lens[i], c->selection.get_bbox());  // return value ignored (:88)
+            // both outcomes: gate passed -> TRACKING + score + box; failed -> LOST (tracking frame) / SELECT START, selection reset (confirm)
+            hud_commands(c, nv12, VT_STATE_TRACKING, h, true, bb, 0.f, vt::VT_HUD_IF_PASS, true, hud);
+            hud_commands(c, nv12, update ? VT_STATE_LOST : VT_STATE_SELECT_START, h, false, bb, 0.f, vt::VT_HUD_IF_FAIL, false, hud);
+        }
+        if ((st = vt::tracker_set_hud(t, hud.data(), (int)hud.size(), i)) != VT_OK) return st;
+    }
+    std::vector<vt_result> res((size_t)n);
+    memset(res.data(), 0, sizeof(vt_result) * res.size());
+    st = vt::tracker_submit_group(t, frames, lens);
+    if (st == VT_OK) st = vt_tracker_wait(t, res.data());
+    if (st != VT_OK && !any) return st;  // (nothing was drawn; with streams in the forward a failed step is their Err, as in probe_one_sync)
+    for (int i = 0; i < n; ++i) {
+        if (!part[(size_t)i]) continue;
+        vt_context* c = g->members[(size_t)i];
+        UpdateOutcome o;
+        o.r = res[(size_t)i];
+        o.ok = st == VT_OK && o.r.status == VT_OK;
+        c->frame_on_device = st == VT_OK;
+        int32_t has = 0;
+        vt_bbox bb{0, 0, 0, 0};
+        // the state machine consumes the outcome exactly as in process_frame (the device applied the same gate to the same fp32 score)
+        process_frame_core(c, [&](vt_bbox) { return o; }, [&]() { return o; }, &has, &bb);
+        if (c->state != AppState::Tracking && vt::tracker_group_active(t, i)) vt::tracker_group_drop(t, i);
+    }
+    const uint64_t track_us = (uint64_t)std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t1).count();
+    vt_timing tm;
+    vt_timing_get(t, &tm);
+    vt_timing_add_times(t, any && st == VT_OK ? (uint64_t)(tm.preprocess_ms * 1000.f) : 0, track_us);
+    for (vt_context* c : g->members) probe_log(c, vt::format_is_luma(c->cfg.format), num);  // one line per stream, with its state
+    return VT_OK;
+}
+
+// ≙ vt_context_run_ring for a group: n steps, stream i's frames from its own ring
+vt_status vt_probe_group_run_ring(vt_probe_group* g, uint8_t* const* rings, size_t stride, size_t frame_len, int32_t ring, int32_t first,
+                                  int32_t n, const char* const* hud_override, const uint8_t* const* pristine, double* latency_us) {
+    if (!g || !g->tracker || !rings || ring <= 0 || first < 0 || n < 0 || frame_len > stride) {
+        vt::set_error("vt_probe_group_run_ring: invalid argument");
+        return VT_ERR_INVALID;
+    }
+    const int ns = (int)g->members.size();
+    std::vector<uint8_t*> fr((size_t)ns);
+    std::vector<size_t> lens((size_t)ns, frame_len);
+    for (int i = 0; i < n; ++i) {
+        const size_t off = (size_t)((first + i) % ring) * stride;
+        for (int k = 0; k < ns; ++k) fr[(size_t)k] = rings[k] + off;
+        const auto t0 = std::chrono::steady_clock::now();
+        const vt_status st = vt_probe_group_frame(g, fr.data(), lens.data(), hud_override);
+        if (latency_us) latency_us[i] = std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now() - t0).count();
+        if (st != VT_OK) return st;
+        for (int k = 0; pristine && k < ns; ++k) {  // what vt_context_run_ring restores, per stream
+            const vt_context* c = g->members[(size_t)k];
+            if (!pristine[k]) continue;
+            const uint8_t* clean = pristine[k] + off;
+            const int fmt = c->cfg.format, W = c->frame_width, H = c->frame_height;
+            vt::restore_rect_region(fr[(size_t)k], clean, fmt, W, H, 10, 10, 412, 92);
+            if (c->state == AppState::Tracking && c->has_bbox) vt::restore_box_region(fr[(size_t)k], clean, fmt, W, H, c->current_bbox);
+            else if (c->state == AppState::Selecting) vt::restore_rect_region(fr[(size_t)k], clean, fmt, W, H, 0, 0, W, H);
+        }
+    }
     return VT_OK;
 }
 

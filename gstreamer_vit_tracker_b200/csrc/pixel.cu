@@ -978,24 +978,31 @@ __device__ __forceinline__ uint32_t dim4(uint32_t v, unsigned factor, int step) 
     return step == 2 ? (d & 0x00ff00ffu) | (v & 0xff00ff00u) : d;
 }
 
-__global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int W, int H, int fmt, const DeviceResult* __restrict__ res,
-                                                                 const int32_t* __restrict__ slots, int n, float gate, const FrameCtl* ctl,
-                                                                 unsigned long long* stamp_end, const uint32_t* __restrict__ blk, int blk_words,
-                                                                 int draw_box) {
-    __shared__ OverlayCmdDev s_cmd[kMaxCmds];
+// The body of both last-kernel forms.  kGroup = false: box_overlay_kernel — CTA x draws the box of active target x (stream group: into
+// that target's own frame), CTA 0 also runs the frame's HUD list.  kGroup = true: probe_group_overlay_kernel — CTA pair x draws stream x
+// of a probe group (ProbeGroupCtl::s[x]: its frames, geometry, slot or -1, HUD list and background-dim handshake), whether or not the
+// stream took part in the forward.  (Two instances of one body rather than one kernel with a runtime switch: the per-stream addressing
+// stays out of the single probe's last kernel, whose size and register use are what they were.)
+template <bool kGroup>
+__device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int fmt, const DeviceResult* __restrict__ res,
+                                                 const int32_t* __restrict__ slots, int n, float gate, const FrameCtl* ctl,
+                                                 unsigned long long* stamp_end, const uint32_t* __restrict__ blk, int blk_words, int draw_box,
+                                                 OverlayCmdDev* s_cmd) {
     // the control block was written at the start of the frame (complete long before the kernel ahead of this one): every thread fetches
     // what it needs in one batch, and the HUD list comes out of pinned host memory, BEFORE the dependency wait: only the decode result
     // waits for the preceding kernel
-    const bool own = blockIdx.x < (unsigned)kMaxWin && ctl->frames[blockIdx.x] != nullptr;  // stream group: block i draws into stream i's frame
+    const ProbeStreamCtl* const e = kGroup ? &reinterpret_cast<const ProbeGroupCtl*>(ctl)->s[blockIdx.x] : nullptr;
+    // stream group: block i draws into stream i's frame; probe group: pair x into stream x's
+    const bool own = kGroup || (blockIdx.x < (unsigned)kMaxWin && ctl->frames[blockIdx.x] != nullptr);
     if (own) {  // ... with stream i's format and size: nothing is written outside its plane 0
-        const int4 g = *reinterpret_cast<const int4*>(ctl->geom[blockIdx.x]);
+        const int4 g = *reinterpret_cast<const int4*>(kGroup ? e->geom : ctl->geom[blockIdx.x]);
         fmt = g.x, W = g.y, H = g.z, len = fmt_frame_bytes(fmt, W, H);
     }
     // HUD mode runs two CTAs per target (gridDim.y = 2): y = 0 draws on the device frame (and publishes), y = 1 on the pinned host frame —
     // the two passes over the command list (~8 us each on one CTA) run side by side
     const bool split = gridDim.y > 1;
-    uint8_t* const frame0 = const_cast<uint8_t*>(own ? ctl->frames[blockIdx.x] : ctl->frame);
-    uint8_t* const host0 = own ? ctl->host_frames[blockIdx.x] : ctl->host_frame;
+    uint8_t* const frame0 = kGroup ? e->frame : const_cast<uint8_t*>(own ? ctl->frames[blockIdx.x] : ctl->frame);
+    uint8_t* const host0 = kGroup ? e->host_frame : own ? ctl->host_frames[blockIdx.x] : ctl->host_frame;
     if (split && blockIdx.y == 1 && !host0) return;       // nothing to mirror into
     uint8_t* const frame = frame0;
     uint8_t* const host = host0;
@@ -1003,13 +1010,16 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
     // below address packed rows: HUD handles take packed frames only.)  fmt is the frame's format: drawn with the overlay semantics of ofmt
     const size_t row = fmt_row_bytes(fmt, W);
     const int ofmt = overlay_format(fmt), step = fmt_px_step(fmt);
-    const size_t fpitch0 = own ? ctl->pitches[blockIdx.x][0] : ctl->pitch[0];
+    const size_t fpitch0 = kGroup ? 0 : own ? ctl->pitches[blockIdx.x][0] : ctl->pitch[0];
     const size_t fpitch = fpitch0 ? fpitch0 : row;
     const bool do_dev = !split || blockIdx.y == 0, do_host = host != nullptr && (!split || blockIdx.y == 1);
-    int n_hud = blockIdx.x == 0 ? ctl->n_hud : 0;
+    // this CTA's HUD list and background-dim flags: the frame's (CTA 0), or its stream's (probe group)
+    const int32_t* const bg_on_dev = kGroup ? &e->bg_on_device : &ctl->bg_on_device;
+    const int32_t* const bg_ready = kGroup ? &e->bg_ready : &ctl->bg_ready;
+    int n_hud = kGroup ? e->n_hud : blockIdx.x == 0 ? ctl->n_hud : 0;
     if (n_hud > kMaxCmds) n_hud = kMaxCmds;
     if (n_hud > 0) {
-        const uint32_t* src = reinterpret_cast<const uint32_t*>(ctl->hud);
+        const uint32_t* src = reinterpret_cast<const uint32_t*>(kGroup ? e->hud : ctl->hud);
         uint32_t* dst = reinterpret_cast<uint32_t*>(s_cmd);
         for (int i = threadIdx.x; i < n_hud * (int)(sizeof(OverlayCmdDev) / 4); i += blockDim.x) dst[i] = src[i];
         __syncthreads();
@@ -1026,8 +1036,8 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
         if (((reinterpret_cast<uintptr_t>(host) | reinterpret_cast<uintptr_t>(frame)) & 3) != 0) bg.wpr = 0;  // bytewise
         // source of the region: the device frame when it was uploaded with the windows (a copy-engine transfer ahead of the graph; an L2 hit
         // here), else the pinned host frame (PCIe reads: ~12 us for the 260 x 90 block, on the critical path of a short frame)
-        const uint8_t* bsrc = (host && !ctl->bg_on_device) ? host : frame;
-        bg_pre = (host || ctl->bg_on_device) && bg.wpr > 0 && rows * bg.wpr <= (long long)kBgWords * kOvThreads && (size_t)bg.y1 * row <= len;
+        const uint8_t* bsrc = (host && !*bg_on_dev) ? host : frame;
+        bg_pre = (host || *bg_on_dev) && bg.wpr > 0 && rows * bg.wpr <= (long long)kBgWords * kOvThreads && (size_t)bg.y1 * row <= len;
         if (bg_pre) {
             const int total = (int)rows * bg.wpr;
 #pragma unroll
@@ -1054,7 +1064,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
     }
     // two CTAs, both prefetched the region from the DEVICE frame: the device-pass CTA may only dim it there once the host-pass CTA holds
     // its copy (the loads are consumed below before the flag is raised)
-    const bool bg_handshake = split && host != nullptr && bg_pre && ctl->bg_on_device;
+    const bool bg_handshake = split && host != nullptr && bg_pre && *bg_on_dev;
     if (bg_handshake && blockIdx.y == 1) {
         uint32_t acc = 0;
 #pragma unroll
@@ -1065,10 +1075,10 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
         __syncthreads();
         if (threadIdx.x == 0) {
             __threadfence();
-            atomicExch(const_cast<int32_t*>(&ctl->bg_ready), 1);
+            atomicExch(const_cast<int32_t*>(bg_ready), 1);
         }
     }
-    const int slot = (int)blockIdx.x < n ? slots[blockIdx.x] : -1;
+    const int slot = kGroup ? e->slot : (int)blockIdx.x < n ? slots[blockIdx.x] : -1;
     if (stamp_end && threadIdx.x == 0 && blockIdx.x == 0 && blockIdx.y == 0) stamp_end[1] = device_time_ns();  // diagnostics: prologue done
     asm volatile("griddepcontrol.wait;" ::: "memory");
     if (stamp_end && threadIdx.x == 0 && blockIdx.x == 0 && blockIdx.y == 0) stamp_end[2] = device_time_ns();  // diagnostics: dependency satisfied
@@ -1096,7 +1106,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
             __syncthreads();
         }
     }
-    if (blockIdx.x != 0) return;
+    if (!kGroup && blockIdx.x != 0) return;
     if (n_hud > 0) {
         // resolve the result-dependent commands once (shared copy), drop the ones of the other outcome
         if ((int)threadIdx.x < n_hud) {
@@ -1110,7 +1120,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
         int first = 0;
         if (bg_handshake && blockIdx.y == 0) {  // (bounded: a protocol error must not hang the GPU; the flag is normally long set)
             if (threadIdx.x == 0) {
-                const volatile int32_t* f = &ctl->bg_ready;
+                const volatile int32_t* f = bg_ready;
                 for (int i = 0; i < (1 << 18) && *f == 0; ++i) {}
             }
             __syncthreads();
@@ -1125,7 +1135,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
                         if (!bg_pre || base > 0) {  // not prefetched (no pinned frame, or a region larger than the register budget)
                             // (pinned frame: the region may not have been uploaded; a host-pass CTA always reads the host frame — the device
                             // frame's copy is being dimmed by the other CTA)
-                            const uint8_t* src = ((host && !ctl->bg_on_device) || (split && do_host)) ? host : frame;
+                            const uint8_t* src = ((host && !*bg_on_dev) || (split && do_host)) ? host : frame;
 #pragma unroll
                             for (int k = 0; k < kBgWords; ++k) {
                                 const long long i = base + threadIdx.x + (long long)k * kOvThreads;
@@ -1150,7 +1160,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
                 }
                 // columns outside the word interior (<= 3 + 3 per row; every column when rows are not word addressable)
                 const long long eh = bg.wpr > 0 ? bg.ax0 - bg.x0 : bg.x1 - bg.x0, et = bg.wpr > 0 ? bg.x1 - bg.ax1 : 0, ec = eh + et;
-                const bool edge_host = (host && !ctl->bg_on_device) || (split && do_host);
+                const bool edge_host = (host && !*bg_on_dev) || (split && do_host);
                 for (long long i = threadIdx.x, kk = 0; i < rows * ec; i += blockDim.x, ++kk) {
                     const uint32_t rq = (uint32_t)i / (uint32_t)ec;  // (rows * ec < 2^31)
                     const long long yy = bg.y0 + rq, k = i - (long long)rq * ec, xx = k < eh ? bg.x0 + k : bg.ax1 + (k - eh);
@@ -1189,6 +1199,7 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
         }
     }
     if (split && blockIdx.y == 1) return;  // (the host waits for the whole grid: the mirrored pixels are complete when it reads the result)
+    if (kGroup && blockIdx.x != 0) return;  // (pair 0 publishes; the host waits for the whole grid, as above)
     if (stamp_end && threadIdx.x == 0) *stamp_end = device_time_ns();
     if (blk) {  // last kernel of the frame: publish the result block (see publish_kernel) — one kernel boundary less
         uint32_t* dst = ctl->hblk;
@@ -1197,6 +1208,27 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
         if (dst)
             for (int i = threadIdx.x; i < blk_words; i += blockDim.x) dst[i] = __ldcg(blk + i);
     }
+}
+
+__global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int W, int H, int fmt, const DeviceResult* __restrict__ res,
+                                                                 const int32_t* __restrict__ slots, int n, float gate, const FrameCtl* ctl,
+                                                                 unsigned long long* stamp_end, const uint32_t* __restrict__ blk, int blk_words,
+                                                                 int draw_box) {
+    __shared__ OverlayCmdDev s_cmd[kMaxCmds];
+    box_overlay_body<false>(len, W, H, fmt, res, slots, n, gate, ctl, stamp_end, blk, blk_words, draw_box, s_cmd);
+}
+
+__global__ void __launch_bounds__(kOvThreads) probe_group_overlay_kernel(const DeviceResult* __restrict__ res, float gate, const ProbeGroupCtl* ctl,
+                                                                         unsigned long long* stamp_end, const uint32_t* __restrict__ blk,
+                                                                         int blk_words) {
+    __shared__ OverlayCmdDev s_cmd[kMaxCmds];
+    box_overlay_body<true>(0, 0, 0, 0, res, nullptr, 0, gate, &ctl->f, stamp_end, blk, blk_words, 0, s_cmd);
+}
+
+cudaError_t launch_group_overlay(int n_streams, const DeviceResult* d_res, float gate, const ProbeGroupCtl* d_ctl, unsigned long long* stamp_end,
+                                 cudaStream_t s, bool pdl, const void* d_blk, size_t blk_bytes) {
+    return launch_ex(probe_group_overlay_kernel, dim3(n_streams, 2), dim3(kOvThreads), 0, s, pdl, 1, d_res, gate, d_ctl, stamp_end,
+                     (const uint32_t*)d_blk, (int)(blk_bytes / 4));
 }
 
 cudaError_t launch_box_overlay(size_t len, int width, int height, int format, const DeviceResult* d_res, const int32_t* d_slots, int n,
@@ -1236,6 +1268,16 @@ cudaError_t launch_stamp(unsigned long long* stamp, FrameCtl* d_ctl, const Frame
     } else {
         stamp_kernel<<<1, 96, 0, s>>>(stamp, d_ctl, ctl);
     }
+    return cudaGetLastError();
+}
+__global__ void stamp_group_kernel(unsigned long long* stamp, ProbeGroupCtl* dst, const ProbeGroupCtl val) {
+    if (threadIdx.x == 0) *stamp = device_time_ns();
+    const uint32_t* src = reinterpret_cast<const uint32_t*>(&val);
+    for (int i = threadIdx.x; i < (int)(sizeof(ProbeGroupCtl) / 4); i += blockDim.x) reinterpret_cast<uint32_t*>(dst)[i] = src[i];
+}
+cudaError_t launch_stamp_group(unsigned long long* stamp, ProbeGroupCtl* d_ctl, const ProbeGroupCtl& ctl, cudaStream_t s) {
+    static_assert(sizeof(ProbeGroupCtl) % 4 == 0 && sizeof(ProbeGroupCtl) + 2 * sizeof(void*) <= 32764, "stamp_group_kernel parameter block");
+    stamp_group_kernel<<<1, 256, 0, s>>>(stamp, d_ctl, ctl);
     return cudaGetLastError();
 }
 

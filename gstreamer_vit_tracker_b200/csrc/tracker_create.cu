@@ -241,6 +241,7 @@ void vt_tracker_destroy(vt_tracker* t) {
     for (auto& h : t->h_hud)
         if (h) cudaFreeHost(h);
     if (t->h_cmds) cudaFreeHost(t->h_cmds);
+    if (t->h_slots) cudaFreeHost(t->h_slots);
     if (t->stream) cudaStreamDestroy(t->stream);
     delete t;
 }

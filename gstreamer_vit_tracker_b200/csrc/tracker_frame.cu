@@ -241,7 +241,10 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const Forw
     else
         VT_LAUNCH(launch_decode(t->H1, C, t->h2_w, t->h2_b, t->d_hann, t->d_state, t->d_slots, n, t->threshold, t->d_res, t->d_maps, t->d_stamps, s,
                                 t->cfg.decode_window));
-    if (t->cfg.box_overlay || t->hud_mode)  // box overlay and / or the frame's HUD list, pinned-frame mirror, ... and publishes the result block
+    if (t->group_n)  // probe group: every stream's HUD (one CTA pair per stream of the group, not per target of the forward), mirror, publish
+        VT_LAUNCH(launch_group_overlay(t->group_n, t->d_res, t->cfg.overlay_gate, reinterpret_cast<const ProbeGroupCtl*>(t->d_ctl),
+                                       t->d_stamps + ST_OVL_END, s, f.pdl, t->d_res, t->res_block_bytes));
+    else if (t->cfg.box_overlay || t->hud_mode)  // box overlay and / or the frame's HUD list, pinned-frame mirror, ... and publishes the result block
         VT_LAUNCH(launch_box_overlay(t->frame_bytes, t->W, t->H, t->fmt, t->d_res, t->d_slots, n, t->cfg.overlay_gate, t->d_ctl,
                                      t->d_stamps + ST_OVL_END, s, f.pdl, t->d_res, t->res_block_bytes, t->cfg.box_overlay | (t->hud_mode ? 1 << 16 : 0)));
     else  // results, stage stamps and the error flag -> the pinned host block of this frame's queue slot
@@ -600,8 +603,8 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
     // the caller's pinned frame is device-mapped under UVA: zero-copy target of the overlay mirror, fall-back source of the crop kernel
     uint8_t* const host_frame = (frame && !d_src && !surf && pinned && len >= t->frame_bytes) ? frame : nullptr;
     // this frame's HUD list (staged by tracker_set_hud in this slot's pinned block)
-    const int n_hud = t->hud_mode ? t->hud_next_n : 0;
-    q.hud_bytes = n_hud ? t->hud_next_bytes : 0;
+    const int n_hud = t->hud_mode ? t->hud_next_n[0] : 0;
+    q.hud_bytes = n_hud ? t->hud_next_bytes[0] : 0;
     q.mirrored = host_frame && (t->cfg.box_overlay || n_hud > 0);
     // device-resident frame: track (and draw the box) straight in the caller's device memory — no device->device copy.  A full-length
     // packed device frame is a surface like any other.
@@ -611,7 +614,7 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
     if (!in_place) t->d_frame = t->d_frames[slot];  // the slot's own frame buffer: the other one may still be read by the frame in flight
     const bool lagging = t->q_count > 0;  // a frame is in flight: rect_mirror is one frame old, the windows are predictions
     UploadPlan plan;
-    if (!in_place && !d_src) plan_upload(t, len, host_frame != nullptr, lagging, n_hud ? t->hud_next_rmw : nullptr, plan);
+    if (!in_place && !d_src) plan_upload(t, len, host_frame != nullptr, lagging, n_hud ? t->hud_next_rmw[0] : nullptr, plan);
     if (!in_place && !d_src && lagging) {
         // pipelined host frame: upload on the copy stream while the frame in flight computes; the main stream picks it up through an event
         vt_status st = do_upload(t, cfg_geom(t), frame, len, plan, false, t->copy_stream);
@@ -632,7 +635,7 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
     ctl.n_win = plan.whole ? -1 : plan.n_win;
     if (!plan.whole) memcpy(ctl.win, plan.win, sizeof(ctl.win));
     ctl.bg_on_device = (n_hud && (in_place || d_src || plan.whole || plan.has_rmw)) ? 1 : 0;  // the dimmed region is in the device frame
-    t->hud_next_n = 0;
+    t->hud_next_n[0] = 0;
     VT_CUDA(launch_stamp(t->d_stamps + ST_SUBMIT, t->d_ctl, ctl, t->stream, hud_inline ? t->h_hud[slot] : nullptr, n_hud, t->d_hud[slot]));
     ++t->kernel_launches;
     if (in_place) {
@@ -829,20 +832,23 @@ void tracker_enable_hud(vt_tracker* t) {
     if (t && t->graphs.empty()) t->hud_mode = true;  // (the frame's last kernel is part of the captured graph)
 }
 
-// Stages the HUD list of the NEXT submit in the pinned block of the queue slot that submit will use.
-vt_status tracker_set_hud(vt_tracker* t, const HudCmd* cmds, int n) {
-    if (!t || !t->hud_mode || n < 0 || n > kMaxCmds || (n > 0 && !cmds)) {
-        set_error("tracker_set_hud: invalid argument (HUD mode %d, %d commands)", t ? (int)t->hud_mode : -1, n);
+// Stages the HUD list of the NEXT submit in the pinned block of the queue slot that submit will use.  A probe group's block holds one
+// list of up to kMaxCmds commands per stream: stream i's at [i * kMaxCmds], drawn on stream i's frame (its geometry).
+vt_status tracker_set_hud(vt_tracker* t, const HudCmd* cmds, int n, int stream) {
+    if (!t || !t->hud_mode || n < 0 || n > kMaxCmds || (n > 0 && !cmds) || stream < 0 || stream >= std::max(t->group_n, 1)) {
+        set_error("tracker_set_hud: invalid argument (HUD mode %d, %d commands, stream %d)", t ? (int)t->hud_mode : -1, n, stream);
         return VT_ERR_INVALID;
     }
     VT_CUDA(cudaSetDevice(t->cfg.device));
     const int slot = (t->q_head + t->q_count) % vt_tracker::kQueue;
-    if (!t->h_hud[slot]) VT_CUDA(cudaHostAlloc(&t->h_hud[slot], sizeof(OverlayCmdDev) * kMaxCmds, cudaHostAllocDefault));
-    if (!t->d_hud[slot]) VT_CUDA(cudaMalloc(&t->d_hud[slot], sizeof(OverlayCmdDev) * kHudInline));
+    if (!t->h_hud[slot])
+        VT_CUDA(cudaHostAlloc(&t->h_hud[slot], sizeof(OverlayCmdDev) * kMaxCmds * std::max(t->group_n, 1), cudaHostAllocDefault));
+    if (!t->d_hud[slot] && !t->group_n) VT_CUDA(cudaMalloc(&t->d_hud[slot], sizeof(OverlayCmdDev) * kHudInline));
+    const StreamGeom& g = slot_geom(t, stream);  // (a single probe: the cfg geometry)
     int rmw[4] = {0, 0, 0, 0};
     size_t bytes = 0;
     for (int i = 0; i < n; ++i) {
-        OverlayCmdDev& d = t->h_hud[slot][i];
+        OverlayCmdDev& d = t->h_hud[slot][stream * kMaxCmds + i];
         const vt_overlay_cmd& c = cmds[i].cmd;
         vt_status st = fill_cmd_dev(c, d);
         if (st != VT_OK) return st;
@@ -858,9 +864,9 @@ vt_status tracker_set_hud(vt_tracker* t, const HudCmd* cmds, int n) {
                 if (vt_glyph_rows(ch, rows) == 0) d.known[kHudDigitSlot + k] = 1, memcpy(d.glyph[kHudDigitSlot + k], rows, 7);
             }
         }
-        if (c.kind == VT_OV_BACKGROUND && format_is_luma(t->fmt) && c.x >= 0 && c.y >= 0 && c.w > 0 && c.h > 0) {
+        if (c.kind == VT_OV_BACKGROUND && format_is_luma(g.fmt) && c.x >= 0 && c.y >= 0 && c.w > 0 && c.h > 0) {
             // the luma background dim reads before it writes (src/nv12_convert.rs:324-343): that region must be on the device
-            const int x1 = (int)std::min<long long>((long long)c.x + c.w, t->W), y1 = (int)std::min<long long>((long long)c.y + c.h, t->H);
+            const int x1 = (int)std::min<long long>((long long)c.x + c.w, g.W), y1 = (int)std::min<long long>((long long)c.y + c.h, g.H);
             if (rmw[2] <= rmw[0]) rmw[0] = c.x, rmw[1] = c.y, rmw[2] = x1, rmw[3] = y1;
             else rmw[0] = std::min(rmw[0], c.x), rmw[1] = std::min(rmw[1], c.y), rmw[2] = std::max(rmw[2], x1), rmw[3] = std::max(rmw[3], y1);
             bytes += (size_t)std::max(0, x1 - c.x) * std::max(0, y1 - c.y);
@@ -870,8 +876,8 @@ vt_status tracker_set_hud(vt_tracker* t, const HudCmd* cmds, int n) {
             bytes += 1024;  // rect / crosshair / cursor / selection outlines
         }
     }
-    t->hud_next_n = n, t->hud_next_bytes = bytes;
-    memcpy(t->hud_next_rmw, rmw, sizeof(rmw));
+    t->hud_next_n[stream] = n, t->hud_next_bytes[stream] = bytes;
+    memcpy(t->hud_next_rmw[stream], rmw, sizeof(rmw));
     return VT_OK;
 }
 
@@ -957,6 +963,24 @@ static vt_status grow_frame_buffers(vt_tracker* t, size_t bytes) {
     return VT_OK;
 }
 
+// VitTrack::init of `target` on a host frame of the slot's geometry (the whole frame is uploaded)
+static vt_status init_from_host(vt_tracker* t, int32_t target, const uint8_t* frame, size_t len, vt_bbox box) {
+    VT_CUDA(cudaSetDevice(t->cfg.device));
+    const StreamGeom& g = slot_geom(t, target);
+    vt_status st = check_template_window(t, g, box, "vt_tracker_init");
+    if (st != VT_OK) return st;
+    st = do_upload(t, g, frame, len, UploadPlan(), false, nullptr);  // the whole frame
+    if (st != VT_OK) return st;
+    return init_template(t, target, box, FrameDesc{t->d_frame, nullptr, {0, 0}, g.W, g.H, g.fmt, t->frame_valid, nullptr, t->cfg.pad_plus1});
+}
+
+// The tracker of a probe group steps its streams through vt_probe_group_frame only: every public frame entry point refuses it.
+static bool group_refused(const vt_tracker* t, const char* where) {
+    if (!t->group_n) return false;
+    set_error("%s: this handle is the tracker of a probe group; its frames go through vt_probe_group_frame / vt_probe_group_run_ring", where);
+    return true;
+}
+
 }  // namespace vt
 
 using namespace vt;
@@ -972,13 +996,8 @@ vt_status vt_tracker_init(vt_tracker* t, int32_t target, const uint8_t* frame, s
         set_error("vt_tracker_init: a frame is in flight");
         return VT_ERR_INVALID;
     }
-    VT_CUDA(cudaSetDevice(t->cfg.device));
-    const StreamGeom& g = slot_geom(t, target);
-    vt_status st = check_template_window(t, g, box, "vt_tracker_init");
-    if (st != VT_OK) return st;
-    st = do_upload(t, g, frame, len, UploadPlan(), false, nullptr);  // the whole frame
-    if (st != VT_OK) return st;
-    return init_template(t, target, box, FrameDesc{t->d_frame, nullptr, {0, 0}, g.W, g.H, g.fmt, t->frame_valid, nullptr, t->cfg.pad_plus1});
+    if (group_refused(t, "vt_tracker_init")) return VT_ERR_INVALID;
+    return init_from_host(t, target, frame, len, box);
 }
 
 vt_status vt_tracker_init_surface(vt_tracker* t, int32_t target, const vt_surface* s, vt_bbox box) {
@@ -990,6 +1009,7 @@ vt_status vt_tracker_init_surface(vt_tracker* t, int32_t target, const vt_surfac
         set_error("vt_tracker_init_surface: a frame is in flight");
         return VT_ERR_INVALID;
     }
+    if (group_refused(t, "vt_tracker_init_surface")) return VT_ERR_INVALID;
     vt_status st = surface_call(t, "vt_tracker_init_surface", true);
     if (st == VT_OK) st = check_surface(t, slot_geom(t, target), s, "vt_tracker_init_surface", 0);
     const StreamGeom& g = slot_geom(t, target);
@@ -1053,6 +1073,7 @@ vt_status vt_tracker_drop(vt_tracker* t, int32_t target) {
 
 vt_status vt_tracker_submit(vt_tracker* t, uint8_t* frame, size_t len) {
     if (!t || !frame) return VT_ERR_INVALID;
+    if (group_refused(t, "vt_tracker_submit")) return VT_ERR_INVALID;
     vt_status st = check_uniform_geometry(t, "vt_tracker_submit");
     if (st != VT_OK) return st;
     VT_CUDA(cudaSetDevice(t->cfg.device));
@@ -1066,11 +1087,147 @@ vt_status tracker_submit_hud_only(vt_tracker* t, uint8_t* frame, size_t len) {
     VT_CUDA(cudaSetDevice(t->cfg.device));
     return submit_common(t, frame, nullptr, len, false);
 }
+
+vt_status tracker_make_group(vt_tracker* t, int n) {
+    if (!t || n < 1 || n > kMaxWin || n != t->maxT || !t->graphs.empty() || t->q_count || t->group_n) {
+        set_error("tracker_make_group: needs a fresh handle with max_targets = %d (1..%d)", n, kMaxWin);
+        return VT_ERR_INVALID;
+    }
+    VT_CUDA(cudaSetDevice(t->cfg.device));
+    VT_CUDA(cudaFree(t->d_ctl));
+    t->d_ctl = nullptr;
+    VT_CUDA(cudaMalloc(&t->d_ctl, sizeof(ProbeGroupCtl)));
+    VT_CUDA(cudaMemset(t->d_ctl, 0, sizeof(ProbeGroupCtl)));
+    VT_CUDA(cudaHostAlloc(&t->h_slots, sizeof(int32_t) * kMaxWin, cudaHostAllocDefault));
+    for (int i = 0; i < n; ++i) {  // one device frame per stream, of its geometry
+        const size_t fb = slot_geom(t, i).bytes() + 256;
+        VT_CUDA(cudaMalloc(&t->d_sframes[i], fb));
+        VT_CUDA(cudaMemset(t->d_sframes[i], 0, fb));
+        t->d_sframe_bytes[i] = fb;
+    }
+    tracker_enable_hud(t);
+    t->group_n = n;
+    return VT_OK;
+}
+
+vt_status tracker_group_init(vt_tracker* t, int stream, const uint8_t* frame, size_t len, vt_bbox box) {
+    if (!t || !t->group_n || stream < 0 || stream >= t->group_n || !frame || t->in_flight) {
+        set_error("tracker_group_init: invalid argument");
+        return VT_ERR_INVALID;
+    }
+    return init_from_host(t, stream, frame, len, box);
+}
+
+vt_status tracker_group_drop(vt_tracker* t, int stream) {
+    if (!t || !t->group_n || stream < 0 || stream >= t->group_n || t->in_flight) {
+        set_error("tracker_group_drop: invalid argument");
+        return VT_ERR_INVALID;
+    }
+    if (t->inited[stream]) {
+        t->inited[stream] = 0;
+        t->active.erase(std::remove(t->active.begin(), t->active.end(), stream), t->active.end());
+        VT_CUDA(cudaSetDevice(t->cfg.device));
+        VT_CUDA(cudaMemsetAsync(t->d_state + stream, 0, sizeof(TargetState), t->stream));
+    }
+    return VT_OK;
+}
+
+bool tracker_group_active(const vt_tracker* t, int stream) { return t && stream >= 0 && stream < t->group_n && t->inited[stream]; }
+
+// One probe-group step.  The streams whose slot is active (stream i = slot i, ascending) run ONE batched forward: each one's search window
+// is uploaded into its own device frame and the crop addresses them by active-target index, as in a stream group.  The step's last kernel
+// runs one CTA pair per stream of the group: the stream's HUD list (both outcomes for a stream in the forward, picked by its own result),
+// drawn on its device frame and mirrored into its pinned host frame.  With no stream in the forward that kernel is the whole step.
+// Every luma stream's HUD region is uploaded with the windows, so that — as in the single probe — the device pass dims its own copy of the
+// region while the host pass reads the pinned frame.  Synchronous (rect_mirror is exact: the windows are the real search windows).
+vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size_t* lens) {
+    const int n = t ? t->group_n : 0;
+    if (!n || t->q_count) {
+        set_error("tracker_submit_group: not the tracker of a probe group, or a step is in flight");
+        return VT_ERR_INVALID;
+    }
+    VT_CUDA(cudaSetDevice(t->cfg.device));
+    const int slot = t->q_head;
+    vt_tracker::Slot& q = t->q[slot];
+    q.t_submit = std::chrono::steady_clock::now();
+    q.frame = frames[0], q.len = lens[0], q.pageable = false, q.mirrored = true, q.hud_bytes = 0;
+    ProbeGroupCtl ctl;
+    memset(&ctl, 0, sizeof(ctl));
+    const int k_act = (int)t->active.size();
+    std::vector<bool> whole((size_t)n, false);
+    for (int k = 0; k < k_act; ++k) {  // the forward's targets, by active-target index
+        const int i = t->active[k];
+        const StreamGeom& g = slot_geom(t, i);
+        ctl.f.geom[k][0] = g.fmt, ctl.f.geom[k][1] = g.W, ctl.f.geom[k][2] = g.H, ctl.f.geom[k][3] = 1;
+        int* w = ctl.f.win[k];
+        if (!t->cfg.upload_window || !windows_allowed(g)) {
+            VT_CUDA(cudaMemcpyAsync(t->d_sframes[i], frames[i], g.bytes(), cudaMemcpyHostToDevice, t->stream));
+            t->h2d_bytes += g.bytes();
+            w[0] = w[1] = 0, w[2] = g.W, w[3] = g.H;
+            whole[i] = true;
+        } else if (search_window(g, t->rect_mirror[i], 0, w[0], w[1], w[2], w[3])) {
+            vt_status st = copy_window(g, t->d_sframes[i], frames[i], w, true, cudaMemcpyHostToDevice, t->stream);
+            if (st != VT_OK) return st;
+            t->h2d_bytes += window_bytes(g, w);
+        } else {
+            w[0] = w[1] = w[2] = w[3] = 0;  // the window misses the frame: the crop kernel flags it
+        }
+        ctl.f.frames[k] = t->d_sframes[i], ctl.f.host_frames[k] = frames[i];
+    }
+    for (int i = 0; i < n; ++i) {  // every stream of the group, by stream index
+        const StreamGeom& g = slot_geom(t, i);
+        ProbeStreamCtl& e = ctl.s[i];
+        e.frame = t->d_sframes[i], e.host_frame = frames[i];
+        e.geom[0] = g.fmt, e.geom[1] = g.W, e.geom[2] = g.H, e.geom[3] = 1;
+        e.n_hud = t->hud_next_n[i];
+        e.hud = e.n_hud ? t->h_hud[slot] + (size_t)i * kMaxCmds : nullptr;
+        e.slot = t->inited[i] ? i : -1;
+        const int* r = t->hud_next_rmw[i];
+        int w[4] = {std::max(r[0], 0), std::max(r[1], 0), std::min(r[2], g.W), std::min(r[3], g.H)};
+        if (e.n_hud && whole[i]) {
+            e.bg_on_device = 1;
+        } else if (e.n_hud && w[2] > w[0] && w[3] > w[1]) {  // plane 0 only (the luma background dim reads and writes Y)
+            vt_status st = copy_window(g, t->d_sframes[i], frames[i], w, false, cudaMemcpyHostToDevice, t->stream);
+            if (st != VT_OK) return st;
+            t->h2d_bytes += plane0_bytes(g, w[0], w[1], w[2], w[3]);
+            e.bg_on_device = 1;
+        }
+        if (e.n_hud) q.hud_bytes += t->hud_next_bytes[i];
+        t->hud_next_n[i] = 0;
+    }
+    ctl.f.frame = ctl.f.frames[0], ctl.f.host_frame = ctl.f.host_frames[0], ctl.f.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
+    ctl.f.n_win = k_act;
+    if (k_act) {  // (drops since the last step changed the list: it reaches the device ahead of the step's kernels)
+        memcpy(t->h_slots, t->active.data(), sizeof(int32_t) * (size_t)k_act);
+        VT_CUDA(cudaMemcpyAsync(t->d_slots, t->h_slots, sizeof(int32_t) * (size_t)k_act, cudaMemcpyHostToDevice, t->stream));
+    }
+    t->frame_valid = 1, t->d_frame_is_last_host_frame = false;
+    VT_CUDA(launch_stamp_group(t->d_stamps + ST_SUBMIT, reinterpret_cast<ProbeGroupCtl*>(t->d_ctl), ctl, t->stream));
+    ++t->kernel_launches;
+    if (k_act) {
+        vt_status st = run_forward(t);
+        if (st != VT_OK) return st;
+    } else {  // no stream in the forward: every stream's HUD in one launch
+        cudaError_t e = launch_group_overlay(n, t->d_res, t->cfg.overlay_gate, reinterpret_cast<const ProbeGroupCtl*>(t->d_ctl),
+                                             t->d_stamps + ST_OVL_END, t->stream, false, t->d_res, t->res_block_bytes);
+        if (e != cudaSuccess) {
+            set_error("probe group overlay launch failed: %s", cudaGetErrorString(e));
+            return VT_ERR_CUDA;
+        }
+        ++t->kernel_launches;
+    }
+    VT_CUDA(cudaEventRecord(t->q_done[slot], t->stream));
+    t->d2h_bytes += t->res_block_bytes;
+    ++t->q_count;
+    t->in_flight = true;
+    return VT_OK;
+}
 }  // namespace vt
 extern "C" {
 
 vt_status vt_tracker_submit_device(vt_tracker* t, uint8_t* d_frame, size_t len) {
     if (!t || !d_frame) return VT_ERR_INVALID;
+    if (group_refused(t, "vt_tracker_submit_device")) return VT_ERR_INVALID;
     vt_status st = check_uniform_geometry(t, "vt_tracker_submit_device");
     if (st != VT_OK) return st;
     VT_CUDA(cudaSetDevice(t->cfg.device));
@@ -1085,6 +1242,7 @@ vt_status vt_tracker_wait(vt_tracker* t, vt_result* results) {
 
 vt_status vt_tracker_update(vt_tracker* t, uint8_t* frame, size_t len, vt_result* results) {
     if (!t || !frame) return VT_ERR_INVALID;
+    if (group_refused(t, "vt_tracker_update")) return VT_ERR_INVALID;
     vt_status st = check_uniform_geometry(t, "vt_tracker_update");
     if (st != VT_OK) return st;
     VT_CUDA(cudaSetDevice(t->cfg.device));
@@ -1099,6 +1257,7 @@ vt_status vt_tracker_update(vt_tracker* t, uint8_t* frame, size_t len, vt_result
 
 vt_status vt_tracker_update_streams(vt_tracker* t, uint8_t* const* frames, const size_t* lens, int32_t n, vt_result* results) {
     if (!t || !frames || !lens) return VT_ERR_INVALID;
+    if (group_refused(t, "vt_tracker_update_streams")) return VT_ERR_INVALID;
     VT_CUDA(cudaSetDevice(t->cfg.device));
     vt_status st = submit_streams(t, frames, lens, nullptr, n);
     if (st != VT_OK) return st;
@@ -1107,6 +1266,7 @@ vt_status vt_tracker_update_streams(vt_tracker* t, uint8_t* const* frames, const
 
 vt_status vt_tracker_update_device(vt_tracker* t, uint8_t* d_frame, size_t len, vt_result* results) {
     if (!t || !d_frame) return VT_ERR_INVALID;
+    if (group_refused(t, "vt_tracker_update_device")) return VT_ERR_INVALID;
     vt_status st = check_uniform_geometry(t, "vt_tracker_update_device");
     if (st != VT_OK) return st;
     VT_CUDA(cudaSetDevice(t->cfg.device));
@@ -1121,6 +1281,7 @@ vt_status vt_tracker_update_device(vt_tracker* t, uint8_t* d_frame, size_t len, 
 
 vt_status vt_tracker_update_surface(vt_tracker* t, const vt_surface* s, vt_result* results) {
     if (!t || !s) return VT_ERR_INVALID;
+    if (group_refused(t, "vt_tracker_update_surface")) return VT_ERR_INVALID;
     vt_status st = check_uniform_geometry(t, "vt_tracker_update_surface");
     if (st == VT_OK) st = surface_call(t, "vt_tracker_update_surface", true);
     if (st == VT_OK) st = check_surface(t, cfg_geom(t), s, "vt_tracker_update_surface", 0);
@@ -1131,6 +1292,7 @@ vt_status vt_tracker_update_surface(vt_tracker* t, const vt_surface* s, vt_resul
 
 vt_status vt_tracker_submit_surface(vt_tracker* t, const vt_surface* s) {
     if (!t || !s) return VT_ERR_INVALID;
+    if (group_refused(t, "vt_tracker_submit_surface")) return VT_ERR_INVALID;
     vt_status st = check_uniform_geometry(t, "vt_tracker_submit_surface");
     if (st == VT_OK) st = surface_call(t, "vt_tracker_submit_surface", false);
     if (st == VT_OK) st = check_surface(t, cfg_geom(t), s, "vt_tracker_submit_surface", 0);
@@ -1140,6 +1302,7 @@ vt_status vt_tracker_submit_surface(vt_tracker* t, const vt_surface* s) {
 
 vt_status vt_tracker_update_streams_surface(vt_tracker* t, const vt_surface* surfaces, int32_t n, vt_result* results) {
     if (!t || !surfaces) return VT_ERR_INVALID;
+    if (group_refused(t, "vt_tracker_update_streams_surface")) return VT_ERR_INVALID;
     VT_CUDA(cudaSetDevice(t->cfg.device));
     vt_status st = submit_streams(t, nullptr, nullptr, surfaces, n);
     if (st != VT_OK) return st;
@@ -1157,6 +1320,7 @@ vt_status vt_tracker_run_ring(vt_tracker* t, uint8_t* frames, size_t stride, siz
         set_error("vt_tracker_run_ring: frames are in flight; drain them first");
         return VT_ERR_INVALID;
     }
+    if (group_refused(t, "vt_tracker_run_ring")) return VT_ERR_INVALID;
     if (check_uniform_geometry(t, "vt_tracker_run_ring") != VT_OK) return VT_ERR_INVALID;
     VT_CUDA(cudaSetDevice(t->cfg.device));
     const bool device = mode >= VT_RUN_DEVICE_SYNC, pipelined = mode == VT_RUN_HOST_PIPELINED || mode == VT_RUN_DEVICE_PIPELINED;
@@ -1205,6 +1369,7 @@ vt_status vt_tracker_run_streams_ring(vt_tracker* t, uint8_t* const* rings, int3
         set_error("vt_tracker_run_streams_ring: invalid argument");
         return VT_ERR_INVALID;
     }
+    if (group_refused(t, "vt_tracker_run_streams_ring")) return VT_ERR_INVALID;
     VT_CUDA(cudaSetDevice(t->cfg.device));
     std::vector<vt_result> res((size_t)t->maxT);
     uint8_t* fr[kMaxWin];

@@ -125,9 +125,14 @@ struct vt_tracker {
     bool hud_mode = false;
     OverlayCmdDev* h_hud[2] = {nullptr, nullptr};
     OverlayCmdDev* d_hud[2] = {nullptr, nullptr};  // device copies of the lists (written by the stamp kernel from its parameter block)
-    int hud_next_n = 0;
-    int hud_next_rmw[4] = {0, 0, 0, 0};  // region the list reads before it writes (NV12 background dim): x0, y0, x1, y1; empty = none
-    size_t hud_next_bytes = 0;            // pixels the list touches (device -> host accounting)
+    // (per stream of a probe group; [0] on every other handle)
+    int hud_next_n[kMaxWin] = {};
+    int hud_next_rmw[kMaxWin][4] = {};  // region the list reads before it writes (NV12 background dim): x0, y0, x1, y1; empty = none
+    size_t hud_next_bytes[kMaxWin] = {};  // pixels the list touches (device -> host accounting)
+    // probe group of group_n streams (vt_probe_group, tracker_make_group): stream i = target slot i; d_ctl is a ProbeGroupCtl; the public
+    // frame entry points are refused
+    int group_n = 0;
+    int32_t* h_slots = nullptr;  // pinned: the active slot list of the next group step (uploaded ahead of the step's kernels)
     bool inflight_mirrored = false;
     float* d_maps = nullptr;
     OverlayCmdDev *d_cmds = nullptr, *h_cmds = nullptr;

@@ -176,11 +176,30 @@ struct FrameCtl {
     int32_t bg_on_device;      // the region a leading HUD background dim reads was uploaded with the windows: read it from the device frame
     int32_t bg_ready;          // set by the host-pass CTA of the overlay kernel once its copy of that region is in registers (reset per frame)
 };
+// Probe groups (vt_probe_group_frame): the control block of a group's handle.  Its FrameCtl part addresses the streams that take part in
+// the step's forward by active-target index, as for a stream group (the crop reads it); the per-stream table addresses EVERY stream of the
+// group by its index, which is also its target slot: CTA pair x of the step's last kernel (probe_group_overlay_kernel) draws stream x.
+struct ProbeStreamCtl {
+    uint8_t* frame;              // the stream's device frame (its search window, if it takes part, and its HUD region uploaded this step)
+    uint8_t* host_frame;         // its pinned host frame: zero-copy target of the overlay mirror
+    const OverlayCmdDev* hud;    // its HUD list in the pinned block of the step's queue slot, n_hud entries
+    alignas(16) int32_t geom[4]; // {format, width, height, 1}
+    int32_t n_hud;
+    int32_t slot;                // its target slot when it takes part in this step's forward, else -1 (the HUD of a stream without result)
+    int32_t bg_on_device;        // as FrameCtl::bg_on_device, for this stream
+    int32_t bg_ready;            // as FrameCtl::bg_ready, for this stream's pair of CTAs (reset per step)
+};
+struct ProbeGroupCtl {
+    FrameCtl f;                  // first: every kernel of the forward reads it through the same pointer
+    ProbeStreamCtl s[kMaxWin];
+};
 // h_list / n / d_list (optional): the frame's HUD list travels in the kernel's parameter block and is written to d_list, so the overlay
 // kernel reads it from device memory (from the pinned block it was a PCIe round trip at the head of the frame's last kernel)
 constexpr int kHudInline = 12;
 cudaError_t launch_stamp(unsigned long long* stamp, FrameCtl* d_ctl, const FrameCtl& ctl, cudaStream_t s, const OverlayCmdDev* h_list = nullptr,
                          int n = 0, OverlayCmdDev* d_list = nullptr);
+// the same for a probe group's control block (its HUD lists stay in the pinned block: each CTA pair reads its stream's list there)
+cudaError_t launch_stamp_group(unsigned long long* stamp, ProbeGroupCtl* d_ctl, const ProbeGroupCtl& ctl, cudaStream_t s);
 // last kernel of a frame: result block -> the pinned host block ctl->hblk (zero-copy stores)
 cudaError_t launch_publish(const void* d_blk, const FrameCtl* d_ctl, size_t bytes, cudaStream_t s, bool pdl);
 
@@ -243,6 +262,10 @@ cudaError_t launch_overlay(uint8_t* d_frame, size_t len, int width, int height, 
 cudaError_t launch_box_overlay(size_t len, int width, int height, int format, const DeviceResult* d_res, const int32_t* d_slots, int n,
                                float gate, const FrameCtl* d_ctl, unsigned long long* stamp_end, cudaStream_t s, bool pdl, const void* d_blk,
                                size_t blk_bytes, int draw_box);
+// the last kernel of a probe group's step: the same drawing as launch_box_overlay in HUD mode, one CTA pair per stream of the group
+// (n_streams, whether or not the stream took part in the forward), each with its stream's frames, geometry, slot and HUD list from d_ctl
+cudaError_t launch_group_overlay(int n_streams, const DeviceResult* d_res, float gate, const ProbeGroupCtl* d_ctl, unsigned long long* stamp_end,
+                                 cudaStream_t s, bool pdl, const void* d_blk, size_t blk_bytes);
 
 // ---- live handles per GPU across processes (handle_registry.cpp) ----------------------------------------------------------------
 void registry_add(int device, int delta);
@@ -258,9 +281,21 @@ struct HudCmd {
     uint8_t from_result;  // VT_HUD_GIVEN / VT_HUD_RESULT_RECT / VT_HUD_RESULT_CROSS / VT_HUD_SCORE_TEXT
 };
 void tracker_enable_hud(vt_tracker* t);                                   // before the handle's first frame
-vt_status tracker_set_hud(vt_tracker* t, const HudCmd* cmds, int n);      // the list of the NEXT submit on this handle
+// the list of the NEXT submit on this handle (probe groups: of stream `stream` in the next group step)
+vt_status tracker_set_hud(vt_tracker* t, const HudCmd* cmds, int n, int stream = 0);
 // a frame on which no tracker runs (SELECT / LOST states): upload what the list reads, draw, mirror, publish — then vt_tracker_wait
 vt_status tracker_submit_hud_only(vt_tracker* t, uint8_t* frame, size_t len);
+// Probe groups (host_state.cpp: vt_probe_group).  tracker_make_group turns a fresh handle (max_targets = n, slot geometries set) into the
+// tracker of a group of n streams: HUD mode, a ProbeGroupCtl, and every public frame entry point refused.  Stream i is target slot i.
+vt_status tracker_make_group(vt_tracker* t, int n);
+// VitTrack::init of stream i's target on its full pinned frame (no public-entry-point check); the slot joins the next step's forward
+vt_status tracker_group_init(vt_tracker* t, int stream, const uint8_t* frame, size_t len, vt_bbox box);
+// takes the stream's target out of the forward (device state cleared; the slot list reaches the device with the next step)
+vt_status tracker_group_drop(vt_tracker* t, int stream);
+bool tracker_group_active(const vt_tracker* t, int stream);
+// one group step: frames[i] (pinned, full length: checked by the caller) of every stream, the HUD lists staged with tracker_set_hud; the
+// streams whose slot is active run one batched forward, and the step's last kernel draws every stream's HUD — then vt_tracker_wait
+vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size_t* lens);
 bool frame_is_pinned(const void* p);
 // copies the region of a frame that a box overlay (rect thickness 3 + crosshair 15) / the probe HUD touched back from a clean copy
 void restore_box_region(uint8_t* frame, const uint8_t* clean, int fmt, int W, int H, const vt_bbox& b);

@@ -383,6 +383,35 @@ vt_status vt_probe_frame(vt_context* c, uint8_t* frame, size_t len, const char* 
 vt_status vt_context_run_ring(vt_context* c, uint8_t* frames, size_t stride, size_t frame_len, int32_t ring, int32_t first, int32_t n,
                               const char* const* hud_override, const uint8_t* pristine, double* latency_us);
 
+/* ---- probe groups: the drop-in probe for up to 16 cameras in one batched forward (additive; VT_ABI_VERSION stays 2) ----------------
+ * ≙ n TrackerContext::new (one per pipeline, src/pipeline.rs:55) sharing ONE tracker handle with max_targets = n_streams (1..16): stream i
+ * is member context i and target slot i.  Each stream behaves exactly like a single vt_context probing the same frames with the same
+ * commands, but one group step runs ONE batched forward over the streams whose state machine calls VitTrack on that frame (TRACKING:
+ * update; SELECT END with a pending confirm: init on that stream's frame, then update) and draws every stream's HUD, cursor / selection and
+ * box in place — each with the HUD style of its format (luma: NV12 / GRAY8 / YUY2; RGB24) — with ONE synchronisation for the whole step.
+ * A stream that leaves TRACKING, or whose confirm fails the gate, gives up its slot (tracking resumes only through a fresh init).
+ * Timing: the group keeps one TimingStats (on its tracker) and every stream is probed once per step, so every stream's FPS / conv / trk
+ * HUD line shows the group's step figures. */
+typedef struct vt_probe_group vt_probe_group;
+/* geoms: NULL = every stream has cfg's format / width / height; else n_streams entries (validated as vt_tracker_set_stream_geometry). */
+vt_status vt_probe_group_create(const vt_config* cfg, int32_t n_streams, const vt_stream_geometry* geoms, vt_probe_group** out);
+void vt_probe_group_destroy(vt_probe_group* g);
+int32_t vt_probe_group_size(const vt_probe_group* g);  /* VT_ERR_INVALID for NULL */
+/* The borrowed member context of stream i (NULL when out of range): vt_context_handle_command and every read accessor (state, state_name,
+ * current_score, current_bbox, selection, lost_frames, vt_context_tracker) work on it; the frame entry points (vt_probe_frame,
+ * vt_context_process_frame, vt_context_run_ring) are VT_ERR_INVALID on a member; vt_context_destroy on a member does nothing.
+ * The shared tracker (vt_context_tracker of any member) refuses every frame entry point (init / update / submit / stream-group / ring
+ * calls); vt_tracker_get_rect / set_rect (stream i = target i), vt_tracker_debug_read, vt_timing_get and vt_tracker_stream stay usable. */
+vt_context* vt_probe_group_context(vt_probe_group* g, int32_t stream);
+/* ≙ the n pad-probe closures each invoked once for one buffer of its camera.  frames[i]: pinned host frame of stream i (vt_alloc_pinned),
+ * full length for its geometry (lens[i] >= its frame bytes); a pageable, short or NULL frame is VT_ERR_INVALID with a message.
+ * hud_override as in vt_probe_frame, for every stream. */
+vt_status vt_probe_group_frame(vt_probe_group* g, uint8_t* const* frames, const size_t* lens, const char* const* hud_override);
+/* ≙ vt_context_run_ring for a group: n steps, stream i's frames from rings[i] (pinned host memory; `ring` frames, `stride` apart, frame_len
+ * bytes each), pristine[i] (nullable; pristine itself nullable) restores what each step drew, latency_us[step] (nullable). */
+vt_status vt_probe_group_run_ring(vt_probe_group* g, uint8_t* const* rings, size_t stride, size_t frame_len, int32_t ring, int32_t first,
+                                  int32_t n, const char* const* hud_override, const uint8_t* const* pristine, double* latency_us);
+
 #ifdef __cplusplus
 }
 #endif
