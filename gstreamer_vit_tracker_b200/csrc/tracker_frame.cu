@@ -181,7 +181,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const Forw
             r.P = t->Pbuf, r.np = f.patch_slices, r.p_stride = (int64_t)t->maxT * kNTx * D, r.bias = t->patch_b, r.add = t->pos_x, r.add_period = kNTx;
             r.X = t->X, r.M = n * kNTx, r.D = D, r.period = kNTx, r.x_rows = kNTok, r.x_row_off = kNTz;
             r.ln_g = t->blk[0].ln1_g, r.ln_b = t->blk[0].ln1_b, r.ln_hi = t->ln_hi, r.ln_lo = LO(t->ln_lo), r.ln_rows = kNTok, r.ln_row_off = kNTz;
-            VT_LAUNCH(launch_reduce_ln(r, s, f.pdl));
+            VT_LAUNCH(launch_reduce_ln(r, s, f.pdl, f.spread));
         }
         if (t->debug_capture) VT_CUDA(cudaMemcpyAsync(t->d_dbg, t->X, sizeof(float) * M * D, cudaMemcpyDeviceToDevice, s));
         for (int l = 0; l < t->depth; ++l) {
@@ -201,7 +201,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const Forw
                 r.P = t->Pbuf, r.np = t->heads, r.p_stride = (int64_t)t->maxT * kNTok * D, r.bias = b.proj_b, r.add = t->X, r.add_period = 0;
                 r.X = t->X, r.M = M, r.D = D, r.period = kNTok, r.x_rows = kNTok, r.x_row_off = 0;
                 r.ln_g = b.ln2_g, r.ln_b = b.ln2_b, r.ln_hi = t->ln_hi, r.ln_lo = LO(t->ln_lo), r.ln_rows = kNTok, r.ln_row_off = 0;
-                VT_LAUNCH(launch_reduce_ln(r, s, f.pdl));
+                VT_LAUNCH(launch_reduce_ln(r, s, f.pdl, f.spread));
             } else {  // fused: + LN2
                 VT_LAUNCH(tc_gemm_launch(p.proj, M, ns, s, f.pdl && f.att != kAttSimt, f.spread));
             }
@@ -222,7 +222,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const Forw
                 r.ln_g = last ? t->lnf_g : t->blk[l + 1].ln1_g, r.ln_b = last ? t->lnf_b : t->blk[l + 1].ln1_b;
                 r.ln_hi = last ? t->yf_hi : t->ln_hi, r.ln_lo = LO(last ? t->yf_lo : t->ln_lo);
                 r.ln_rows = last ? kNTx : kNTok, r.ln_row_off = last ? -kNTz : 0;
-                VT_LAUNCH(launch_reduce_ln(r, s, f.pdl));
+                VT_LAUNCH(launch_reduce_ln(r, s, f.pdl, f.spread));
             } else {
                 VT_LAUNCH(tc_gemm_launch(p.fc2, M, ns, s, f.pdl));  // fused: + LN1 of the next block / the final LN of the search rows
             }
@@ -237,7 +237,7 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const Forw
     if (f.head_planes)
         VT_LAUNCH(launch_head_decode(t->Phead, f.head_planes, (int64_t)t->maxT * kNTx * C, C, t->h1_b, t->h2_w, t->h2_b, t->d_hann, t->d_state, t->d_slots,
                                      n, t->threshold, t->d_res, t->d_maps, t->d_cand, t->d_counters, t->d_stamps, s, f.pdl, t->cfg.decode_window,
-                                     t->d_tc_err));
+                                     t->d_tc_err, f.spread));
     else
         VT_LAUNCH(launch_decode(t->H1, C, t->h2_w, t->h2_b, t->d_hann, t->d_state, t->d_slots, n, t->threshold, t->d_res, t->d_maps, t->d_stamps, s,
                                 t->cfg.decode_window));

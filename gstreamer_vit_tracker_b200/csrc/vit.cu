@@ -235,7 +235,9 @@ cudaError_t launch_layernorm_split(const float* x, int64_t ldx, const float* g, 
 // Rows (= warps) per CTA.  (Measured: 2 rows per CTA — 160 CTAs instead of 40 for one target — changes nothing; the kernel is bound by
 // the L2 round trips of its dependent loads, not by the per-SM read rate.)
 constexpr int kReduceRows = 8;
-template <int NPAIR, int NP>  // D / 64 column pairs per lane; number of partials (0 = runtime np, batches of 4)
+// FRONT (latency mode: the GPU is otherwise idle): every partial-plane load ahead of the first add, see below.  Not in throughput mode:
+// there the 110 registers per thread of the 12-plane form cost more resident CTAs than the shorter latency gains (cfg5 -2 %).
+template <int NPAIR, int NP, bool FRONT>  // D / 64 column pairs per lane; number of partials (0 = runtime np, batches of 4)
 __global__ void __launch_bounds__(32 * kReduceRows) reduce_ln_kernel(const ReduceLnArgs a) {
     constexpr int D = NPAIR * 64;
     const int m = blockIdx.x * kReduceRows + (threadIdx.x >> 5), lane = threadIdx.x & 31;
@@ -261,6 +263,10 @@ __global__ void __launch_bounds__(32 * kReduceRows) reduce_ln_kernel(const Reduc
         for (int j = 0; j < NP; ++j)
 #pragma unroll
             for (int i = 0; i < NPAIR; ++i) v[j][i] = __ldcg(pr + j * ps + lane + 32 * i);  // L2 loads: the partials were written by other SMs a moment ago
+        // The fence keeps every load above ahead of the first add (ptxas may not sink a load below it).  Without it ptxas (40
+        // registers) interleaves the loads with the in-order adds and has only ~12 of the 48 loads of the 12-plane reduce in flight:
+        // several dependent L2 round trips instead of one.  (The adds need every load anyway, so waiting for them at the fence costs nothing.)
+        if (FRONT) __threadfence_block();
 #pragma unroll
         for (int i = 0; i < NPAIR; ++i) acc[i].x = x2[i].x + acc[i].x, acc[i].y = x2[i].y + acc[i].y;  // (x + bias) first, as before
 #pragma unroll
@@ -317,10 +323,11 @@ __global__ void __launch_bounds__(32 * kReduceRows) reduce_ln_kernel(const Reduc
     }
 }
 
-cudaError_t launch_reduce_ln(const ReduceLnArgs& a, cudaStream_t s, bool pdl) {
+cudaError_t launch_reduce_ln(const ReduceLnArgs& a, cudaStream_t s, bool pdl, bool front) {
     if (a.M <= 0) return cudaSuccess;
     const dim3 grid((a.M + kReduceRows - 1) / kReduceRows), block(32 * kReduceRows);
-#define VT_RL(NPAIR_, NP_) return launch_ex(reduce_ln_kernel<NPAIR_, NP_>, grid, block, 0, s, pdl, 1, a)
+#define VT_RL(NPAIR_, NP_) return front ? launch_ex(reduce_ln_kernel<NPAIR_, NP_, true>, grid, block, 0, s, pdl, 1, a) \
+                                   : launch_ex(reduce_ln_kernel<NPAIR_, NP_, false>, grid, block, 0, s, pdl, 1, a)
     switch (a.D / 64) {
         case 1:
             if (a.np == 4) VT_RL(1, 4);
@@ -556,7 +563,7 @@ template <int N> struct VecOf;
 template <> struct VecOf<4> { typedef float4 type; };
 template <> struct VecOf<2> { typedef float2 type; };
 constexpr int kCandStride = 8;  // floats per row candidate: value, index, off_x, off_y, size_w, size_h
-template <int CPL, int NP>  // channels per lane: head_ch / 32; taps (0 = runtime np, three in flight)
+template <int CPL, int NP, bool FRONT>  // channels per lane: head_ch / 32; taps (0 = runtime np, three in flight); FRONT: as reduce_ln_kernel
 __global__ void __launch_bounds__(256) head_decode_kernel(const float* __restrict__ P, int np, int64_t p_stride, const float* __restrict__ b1,
                                                           const float* __restrict__ w2, const float* __restrict__ b2,
                                                           const float* __restrict__ hann, TargetState* __restrict__ state,
@@ -595,6 +602,7 @@ __global__ void __launch_bounds__(256) head_decode_kernel(const float* __restric
 #pragma unroll
             for (int j = 0; j < NP; ++j) v[cc][j] = *reinterpret_cast<const Vec*>(pr + (int64_t)j * p_stride);
         }
+        if (FRONT) __threadfence_block();  // every tap load ahead of the first add (as in reduce_ln_kernel)
 #pragma unroll
         for (int cc = 0; cc < 2; ++cc) {
 #pragma unroll
@@ -682,17 +690,19 @@ __global__ void __launch_bounds__(256) head_decode_kernel(const float* __restric
 cudaError_t launch_head_decode(const float* P, int np, int64_t p_stride, int head_ch, const float* b1, const float* w2, const float* b2,
                                const float* hann, TargetState* d_state, const int32_t* d_slots, int n, float threshold, DeviceResult* d_res,
                                float* d_maps, float* d_cand, unsigned* d_counters, unsigned long long* stamps, cudaStream_t s, bool pdl,
-                               int decode_window, const int* tc_err) {
+                               int decode_window, const int* tc_err, bool front) {
     if (n <= 0) return cudaSuccess;
     const dim3 grid(kMap, n), block(256);
+    if (front && head_ch == 128 && np == 9)
+        return launch_ex(head_decode_kernel<4, 9, true>, grid, block, 0, s, pdl, 1, P, np, p_stride, b1, w2, b2, hann, d_state, d_slots, threshold, d_res, d_maps, d_cand, d_counters, stamps, decode_window, tc_err);
     if (head_ch == 128 && np == 9)
-        return launch_ex(head_decode_kernel<4, 9>, grid, block, 0, s, pdl, 1, P, np, p_stride, b1, w2, b2, hann, d_state, d_slots, threshold, d_res, d_maps, d_cand, d_counters, stamps, decode_window, tc_err);
+        return launch_ex(head_decode_kernel<4, 9, false>, grid, block, 0, s, pdl, 1, P, np, p_stride, b1, w2, b2, hann, d_state, d_slots, threshold, d_res, d_maps, d_cand, d_counters, stamps, decode_window, tc_err);
     if (head_ch == 64 && np == 9)
-        return launch_ex(head_decode_kernel<2, 9>, grid, block, 0, s, pdl, 1, P, np, p_stride, b1, w2, b2, hann, d_state, d_slots, threshold, d_res, d_maps, d_cand, d_counters, stamps, decode_window, tc_err);
+        return launch_ex(head_decode_kernel<2, 9, false>, grid, block, 0, s, pdl, 1, P, np, p_stride, b1, w2, b2, hann, d_state, d_slots, threshold, d_res, d_maps, d_cand, d_counters, stamps, decode_window, tc_err);
     if (head_ch == 128)
-        return launch_ex(head_decode_kernel<4, 0>, grid, block, 0, s, pdl, 1, P, np, p_stride, b1, w2, b2, hann, d_state, d_slots, threshold, d_res, d_maps, d_cand, d_counters, stamps, decode_window, tc_err);
+        return launch_ex(head_decode_kernel<4, 0, false>, grid, block, 0, s, pdl, 1, P, np, p_stride, b1, w2, b2, hann, d_state, d_slots, threshold, d_res, d_maps, d_cand, d_counters, stamps, decode_window, tc_err);
     if (head_ch == 64)
-        return launch_ex(head_decode_kernel<2, 0>, grid, block, 0, s, pdl, 1, P, np, p_stride, b1, w2, b2, hann, d_state, d_slots, threshold, d_res, d_maps, d_cand, d_counters, stamps, decode_window, tc_err);
+        return launch_ex(head_decode_kernel<2, 0, false>, grid, block, 0, s, pdl, 1, P, np, p_stride, b1, w2, b2, hann, d_state, d_slots, threshold, d_res, d_maps, d_cand, d_counters, stamps, decode_window, tc_err);
     return cudaErrorInvalidValue;
 }
 

@@ -354,13 +354,14 @@ struct ReduceLnArgs {
     __nv_bfloat16 *ln_hi, *ln_lo;
     int ln_rows, ln_row_off;
 };
-cudaError_t launch_reduce_ln(const ReduceLnArgs& a, cudaStream_t s, bool pdl);
+// front: latency mode (reduce_ln_kernel FRONT)
+cudaError_t launch_reduce_ln(const ReduceLnArgs& a, cudaStream_t s, bool pdl, bool front = false);
 // 3x3 head conv partials (one per tap) -> + bias, ReLU -> 1x1 conv -> sigmoid / hann / arg-max / bbox decode (App. A.5-A.6).
 // 16 CTAs per target (one map row each); the last one to finish merges the 16 row candidates and updates rect_last.
 cudaError_t launch_head_decode(const float* P, int np, int64_t p_stride, int head_ch, const float* b1, const float* w2, const float* b2,
                                const float* hann, TargetState* d_state, const int32_t* d_slots, int n, float threshold, DeviceResult* d_res,
                                float* d_maps, float* d_cand, unsigned* d_counters, unsigned long long* stamps, cudaStream_t s, bool pdl,
-                               int decode_window = 0, const int* tc_err = nullptr);
+                               int decode_window = 0, const int* tc_err = nullptr, bool front = false);
 // qkv: [B*320, 3D]; out: [B*320, D] fp32 (nullable) and/or bf16 split (nullable)
 cudaError_t launch_attention(const float* qkv, float* out, __nv_bfloat16* out_hi, __nv_bfloat16* out_lo, int B, int D, int heads,
                              cudaStream_t s);
