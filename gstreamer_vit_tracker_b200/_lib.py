@@ -155,11 +155,13 @@ SYMBOLS = {
     "vt_context_lost_frames": (C.c_uint64, [_vp]),
     "vt_context_tracker": (_vp, [_vp]),
     "vt_probe_frame": (C.c_int32, [_vp, _vp, C.c_size_t, C.POINTER(C.c_char_p)]),
+    "vt_probe_frame_surface": (C.c_int32, [_vp, C.POINTER(vt_surface), C.POINTER(C.c_char_p)]),
     "vt_probe_group_create": (C.c_int32, [C.POINTER(vt_config), C.c_int32, C.POINTER(vt_stream_geometry), C.POINTER(_vp)]),
     "vt_probe_group_destroy": (None, [_vp]),
     "vt_probe_group_size": (C.c_int32, [_vp]),
     "vt_probe_group_context": (_vp, [_vp, C.c_int32]),
     "vt_probe_group_frame": (C.c_int32, [_vp, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.POINTER(C.c_char_p)]),
+    "vt_probe_group_frame_surface": (C.c_int32, [_vp, C.POINTER(vt_surface), C.c_int32, C.POINTER(C.c_char_p)]),
     "vt_probe_group_run_ring": (C.c_int32, [_vp, C.POINTER(C.c_void_p), C.c_size_t, C.c_size_t, C.c_int32, C.c_int32, C.c_int32,
                                             C.POINTER(C.c_char_p), C.POINTER(C.c_void_p), C.POINTER(C.c_double)]),
 }

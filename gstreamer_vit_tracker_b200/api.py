@@ -678,6 +678,13 @@ class TrackerContext:
             arr = (C.c_char_p * 2)(hud[0].encode(), hud[1].encode())
         check(lib().vt_probe_frame(self._h, _ptr(frame), frame.size, arr), "vt_probe_frame")
 
+    def probe_surface(self, surface: Surface, hud: Optional[Tuple[str, str]] = None) -> None:
+        """probe() on a pitched device surface of the context's geometry (PitchedFrame.surface, a decoder's output): HUD, cursor /
+        selection and box drawn in place into its plane 0 (vt_probe_frame_surface)."""
+        arr = (C.c_char_p * 2)(hud[0].encode(), hud[1].encode()) if hud is not None else None
+        s = _surface(surface)
+        check(lib().vt_probe_frame_surface(self._h, C.byref(s), arr), "vt_probe_frame_surface")
+
 
 class TimingStats:
     """≙ TimingStats (src/timing_stats.rs): free-standing (TimingStats.new()) or bound to a tracker handle's windows."""
@@ -770,6 +777,14 @@ class ProbeGroup:
         lens = (C.c_size_t * n)(*[f.size for f in frames])
         arr = (C.c_char_p * 2)(hud[0].encode(), hud[1].encode()) if hud is not None else None
         check(lib().vt_probe_group_frame(self._h, ptrs, lens, arr), "vt_probe_group_frame")
+
+    def probe_surfaces(self, surfaces: Sequence[Surface], hud: Optional[Tuple[str, str]] = None) -> None:
+        """One step on device surfaces: surfaces[i] — stream i's current frame, of its geometry — probed and drawn on in place
+        (vt_probe_group_frame_surface)."""
+        n = len(surfaces)
+        arr_s = (vt_surface * max(n, 1))(*[_surface(s) for s in surfaces])
+        arr = (C.c_char_p * 2)(hud[0].encode(), hud[1].encode()) if hud is not None else None
+        check(lib().vt_probe_group_frame_surface(self._h, arr_s, n, arr), "vt_probe_group_frame_surface")
 
     def run_ring(self, ring_ptrs: Sequence[int], stride: int, frame_len: int, ring: int, first: int, n: int,
                  hud: Optional[Tuple[str, str]] = None, pristine_ptrs: Optional[Sequence[int]] = None, want_latency: bool = False):

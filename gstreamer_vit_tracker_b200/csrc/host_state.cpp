@@ -433,13 +433,14 @@ static vt_status probe_two_step(vt_context* c, uint8_t* frame, size_t len, const
                               : vt_overlay(t, frame, len, cmds.data(), (int32_t)cmds.size());
 }
 
-// Pinned frames: ONE synchronisation per probed frame.  Everything in the HUD except score / box / the state after the gate is known
-// before the frame runs; the list carries the commands of both outcomes and the frame's last kernel picks by the gate, renders the
-// score digits and the box from the device-side result and mirrors the touched pixels into the pinned frame.  The timing line shows
-// the rolling means up to the PREVIOUS frame (this frame's own conv / track times exist only once it has completed; the text is
-// timing dependent and not part of pixel parity, SURVEY.md §8 a16).
-static vt_status probe_one_sync(vt_context* c, uint8_t* frame, size_t len, const char* const* hud_override, bool nv12) {
+// Pinned frames and device surfaces: ONE synchronisation per probed frame.  Everything in the HUD except score / box / the state after
+// the gate is known before the frame runs; the list carries the commands of both outcomes and the frame's last kernel picks by the gate,
+// renders the score digits and the box from the device-side result and mirrors the touched pixels into the pinned frame (a surface,
+// surf != null, is drawn in place: frame / len unused).  The timing line shows the rolling means up to the PREVIOUS frame (this frame's
+// own conv / track times exist only once it has completed; the text is timing dependent and not part of pixel parity, SURVEY.md §8 a16).
+static vt_status probe_one_sync(vt_context* c, uint8_t* frame, size_t len, const vt_surface* surf, const char* const* hud_override, bool nv12) {
     vt_tracker* t = c->tracker;
+    static const char* const where = "vt_probe_frame_surface";
     const auto t1 = std::chrono::steady_clock::now();
     HudText h;
     hud_text(c, nv12, hud_override, h);
@@ -456,21 +457,24 @@ static vt_status probe_one_sync(vt_context* c, uint8_t* frame, size_t len, const
         process_frame_core(c, [&](vt_bbox) { return UpdateOutcome{false, vt_result{}}; }, [&]() { return UpdateOutcome{false, vt_result{}}; }, &has, &bb);
         hud_commands(c, nv12, vt_context_state(c), h, false, bb, c->current_score, vt::VT_HUD_ALWAYS, false, hud);
         if ((st = vt::tracker_set_hud(t, hud.data(), (int)hud.size())) != VT_OK) return st;
-        if ((st = vt::tracker_submit_hud_only(t, frame, len)) != VT_OK) return st;
+        if ((st = surf ? vt::tracker_submit_surface(t, surf, false, where) : vt::tracker_submit_hud_only(t, frame, len)) != VT_OK) return st;
         vt_result r;
         st = vt_tracker_wait(t, &r);
         if (st != VT_OK) return st;
         vt_timing_add_times(t, 0, (uint64_t)std::chrono::duration_cast<std::chrono::microseconds>(std::chrono::steady_clock::now() - t1).count());
         return VT_OK;
     }
-    if (init_update) vt_tracker_init(t, 0, frame, len, c->selection.get_bbox());  // return value ignored, like the reference (:88)
+    if (init_update) {  // return value ignored, like the reference (:88)
+        if (surf) vt::tracker_init_surface(t, 0, surf, c->selection.get_bbox(), where);
+        else vt_tracker_init(t, 0, frame, len, c->selection.get_bbox());
+    }
     // both outcomes: gate passed -> TRACKING + score + box; failed -> LOST (tracking frame) / SELECT START with the selection reset (confirm frame)
     hud_commands(c, nv12, VT_STATE_TRACKING, h, true, bb, 0.f, vt::VT_HUD_IF_PASS, true, hud);
     hud_commands(c, nv12, update ? VT_STATE_LOST : VT_STATE_SELECT_START, h, false, bb, 0.f, vt::VT_HUD_IF_FAIL, false, hud);
     if ((st = vt::tracker_set_hud(t, hud.data(), (int)hud.size())) != VT_OK) return st;
     UpdateOutcome o;
     memset(&o.r, 0, sizeof(o.r));
-    st = vt_tracker_submit(t, frame, len);
+    st = surf ? vt::tracker_submit_surface(t, surf, true, where) : vt_tracker_submit(t, frame, len);
     if (st == VT_OK) st = vt_tracker_wait(t, &o.r);
     o.ok = st == VT_OK && o.r.status == VT_OK;
     c->frame_on_device = st == VT_OK;
@@ -505,9 +509,10 @@ vt_status vt_context_run_ring(vt_context* c, uint8_t* frames, size_t stride, siz
     return VT_OK;
 }
 
-// ≙ the pad-probe closure body: src/pipeline.rs:67-184 (NV12) / src/pipeline_ir.rs:100-228 (RGB24)
-vt_status vt_probe_frame(vt_context* c, uint8_t* frame, size_t len, const char* const* hud_override) {
-    if (!c || !c->tracker || !frame || member_refused(c, "vt_probe_frame")) return VT_ERR_INVALID;
+}  // extern "C"
+
+// ≙ the pad-probe closure body: src/pipeline.rs:67-184 (NV12) / src/pipeline_ir.rs:100-228 (RGB24), on a host frame or a checked surface
+static vt_status probe_frame(vt_context* c, uint8_t* frame, size_t len, const vt_surface* surf, const char* const* hud_override) {
     vt_tracker* t = c->tracker;
     const bool nv12 = vt::format_is_luma(c->cfg.format);  // GRAY8 / YUY2 frames take the luma-plane HUD of src/pipeline.rs:125-174
     // interval timing, src/pipeline.rs:69-79
@@ -516,11 +521,29 @@ vt_status vt_probe_frame(vt_context* c, uint8_t* frame, size_t len, const char* 
     c->last_time = now, c->have_last = true;
     const uint64_t num = c->frame_num++;
     const size_t need = vt::fmt_valid_bytes(c->cfg.format, c->frame_width, c->frame_height);
-    const vt_status st = (len >= need && vt::frame_is_pinned(frame)) ? probe_one_sync(c, frame, len, hud_override, nv12)
-                                                                                : probe_two_step(c, frame, len, hud_override, nv12);
+    const vt_status st = (surf || (len >= need && vt::frame_is_pinned(frame))) ? probe_one_sync(c, frame, len, surf, hud_override, nv12)
+                                                                                         : probe_two_step(c, frame, len, hud_override, nv12);
     if (st != VT_OK) return st;
     probe_log(c, nv12, num);
     return VT_OK;
+}
+
+extern "C" {
+
+vt_status vt_probe_frame(vt_context* c, uint8_t* frame, size_t len, const char* const* hud_override) {
+    if (!c || !c->tracker || !frame || member_refused(c, "vt_probe_frame")) return VT_ERR_INVALID;
+    return probe_frame(c, frame, len, nullptr, hud_override);
+}
+
+vt_status vt_probe_frame_surface(vt_context* c, const vt_surface* s, const char* const* hud_override) {
+    if (!c || !c->tracker || !s) {
+        vt::set_error("vt_probe_frame_surface: null context (or a context without a tracker) or surface");
+        return VT_ERR_INVALID;
+    }
+    if (member_refused(c, "vt_probe_frame_surface")) return VT_ERR_INVALID;
+    const vt_status st = vt::tracker_check_surface(c->tracker, 0, s, "vt_probe_frame_surface");  // before the state machine steps
+    if (st != VT_OK) return st;
+    return probe_frame(c, nullptr, 0, s, hud_override);
 }
 
 // ---- probe groups: n cameras, one batched forward and one synchronisation per step (include/vt_tracker.h) ----------------------
@@ -586,22 +609,11 @@ vt_context* vt_probe_group_context(vt_probe_group* g, int32_t stream) {
 // state machines on the host first and queue their final HUD; those that take part queue the HUD of both outcomes, and the step's last
 // kernel picks per stream by that stream's own result.  A stream that leaves TRACKING, or whose confirm fails the gate, gives up its slot:
 // LOST and SELECT never call update, and tracking resumes only through a fresh init.
-vt_status vt_probe_group_frame(vt_probe_group* g, uint8_t* const* frames, const size_t* lens, const char* const* hud_override) {
-    if (!g || !g->tracker || !frames || !lens) {
-        vt::set_error("vt_probe_group_frame: null group, frames or lengths");
-        return VT_ERR_INVALID;
-    }
+// frames / lens: every stream's pinned frame, or surfs: every stream's device surface (checked by the caller)
+static vt_status probe_group_step(vt_probe_group* g, uint8_t* const* frames, const size_t* lens, const vt_surface* surfs,
+                                  const char* const* hud_override) {
     vt_tracker* t = g->tracker;
     const int n = (int)g->members.size();
-    for (int i = 0; i < n; ++i) {
-        const vt_context* c = g->members[(size_t)i];
-        const size_t need = vt::fmt_frame_bytes(c->cfg.format, c->frame_width, c->frame_height);
-        if (!frames[i] || lens[i] < need || !vt::frame_is_pinned(frames[i])) {
-            vt::set_error("vt_probe_group_frame: frame %d must be a full frame (%zu bytes for its %dx%d format %d, got %zu) in pinned host memory "
-                          "(vt_alloc_pinned)", i, need, c->frame_width, c->frame_height, c->cfg.format, frames[i] ? lens[i] : (size_t)0);
-            return VT_ERR_INVALID;
-        }
-    }
     const auto now = std::chrono::steady_clock::now();  // interval timing, src/pipeline.rs:69-79 (one probe per stream and step)
     if (g->have_last) vt_timing_add_interval(t, (uint64_t)std::chrono::duration_cast<std::chrono::microseconds>(now - g->last_time).count());
     g->last_time = now, g->have_last = true;
@@ -632,7 +644,10 @@ vt_status vt_probe_group_frame(vt_probe_group* g, uint8_t* const* frames, const 
             process_frame_core(c, [&](vt_bbox) { return UpdateOutcome{false, vt_result{}}; }, [&]() { return UpdateOutcome{false, vt_result{}}; }, &has, &bb);
             hud_commands(c, nv12, vt_context_state(c), h, false, bb, c->current_score, vt::VT_HUD_ALWAYS, false, hud);
         } else {
-            if (init_update) vt::tracker_group_init(t, i, frames[i], lens[i], c->selection.get_bbox());  // return value ignored (:88)
+            if (init_update && surfs)  // return value ignored (:88)
+                vt::tracker_init_surface(t, i, &surfs[i], c->selection.get_bbox(), "vt_probe_group_frame_surface");
+            else if (init_update)
+                vt::tracker_group_init(t, i, frames[i], lens[i], c->selection.get_bbox());
             // both outcomes: gate passed -> TRACKING + score + box; failed -> LOST (tracking frame) / SELECT START, selection reset (confirm)
             hud_commands(c, nv12, VT_STATE_TRACKING, h, true, bb, 0.f, vt::VT_HUD_IF_PASS, true, hud);
             hud_commands(c, nv12, update ? VT_STATE_LOST : VT_STATE_SELECT_START, h, false, bb, 0.f, vt::VT_HUD_IF_FAIL, false, hud);
@@ -641,7 +656,7 @@ vt_status vt_probe_group_frame(vt_probe_group* g, uint8_t* const* frames, const 
     }
     std::vector<vt_result> res((size_t)n);
     memset(res.data(), 0, sizeof(vt_result) * res.size());
-    st = vt::tracker_submit_group(t, frames, lens);
+    st = vt::tracker_submit_group(t, frames, lens, surfs);
     if (st == VT_OK) st = vt_tracker_wait(t, res.data());
     if (st != VT_OK && !any) return st;  // (nothing was drawn; with streams in the forward a failed step is their Err, as in probe_one_sync)
     for (int i = 0; i < n; ++i) {
@@ -663,6 +678,40 @@ vt_status vt_probe_group_frame(vt_probe_group* g, uint8_t* const* frames, const 
     vt_timing_add_times(t, any && st == VT_OK ? (uint64_t)(tm.preprocess_ms * 1000.f) : 0, track_us);
     for (vt_context* c : g->members) probe_log(c, vt::format_is_luma(c->cfg.format), num);  // one line per stream, with its state
     return VT_OK;
+}
+
+vt_status vt_probe_group_frame(vt_probe_group* g, uint8_t* const* frames, const size_t* lens, const char* const* hud_override) {
+    if (!g || !g->tracker || !frames || !lens) {
+        vt::set_error("vt_probe_group_frame: null group, frames or lengths");
+        return VT_ERR_INVALID;
+    }
+    const int n = (int)g->members.size();
+    for (int i = 0; i < n; ++i) {
+        const vt_context* c = g->members[(size_t)i];
+        const size_t need = vt::fmt_frame_bytes(c->cfg.format, c->frame_width, c->frame_height);
+        if (!frames[i] || lens[i] < need || !vt::frame_is_pinned(frames[i])) {
+            vt::set_error("vt_probe_group_frame: frame %d must be a full frame (%zu bytes for its %dx%d format %d, got %zu) in pinned host memory "
+                          "(vt_alloc_pinned)", i, need, c->frame_width, c->frame_height, c->cfg.format, frames[i] ? lens[i] : (size_t)0);
+            return VT_ERR_INVALID;
+        }
+    }
+    return probe_group_step(g, frames, lens, nullptr, hud_override);
+}
+
+vt_status vt_probe_group_frame_surface(vt_probe_group* g, const vt_surface* surfaces, int32_t n, const char* const* hud_override) {
+    if (!g || !g->tracker || !surfaces) {
+        vt::set_error("vt_probe_group_frame_surface: null group or surfaces");
+        return VT_ERR_INVALID;
+    }
+    if (n != (int32_t)g->members.size()) {
+        vt::set_error("vt_probe_group_frame_surface: %d surfaces for a group of %d streams (one per stream)", n, (int)g->members.size());
+        return VT_ERR_INVALID;
+    }
+    for (int i = 0; i < n; ++i) {  // each against its stream's geometry, before any state machine steps
+        const vt_status st = vt::tracker_check_surface(g->tracker, i, &surfaces[i], "vt_probe_group_frame_surface");
+        if (st != VT_OK) return st;
+    }
+    return probe_group_step(g, nullptr, nullptr, surfaces, hud_override);
 }
 
 // ≙ vt_context_run_ring for a group: n steps, stream i's frames from its own ring

@@ -959,14 +959,15 @@ struct BgRegion {
     long long x0, y0, x1, y1;  // clipped pixel rectangle (usize arithmetic of the reference), empty when x1 <= x0
     long long ax0, ax1;        // word-aligned interior of a row in pixels: [ax0, ax1), ax0 >= x0, ax1 <= x1
     int wpr;                   // words per row
-    bool vec;                  // rows are word addressable (row bytes % 4 == 0)
+    bool vec;                  // rows are word addressable (pitch % 4 == 0)
 };
-__device__ BgRegion bg_region(const OverlayCmdDev& c, int W, int H, size_t row, int step) {
+// pitch: bytes between the rows of the plane the region is read from and written to
+__device__ BgRegion bg_region(const OverlayCmdDev& c, int W, int H, size_t pitch, int step) {
     BgRegion g;
     const u64 x0 = (u64)c.x, y0 = (u64)c.y;
     const u64 x1 = umin64(x0 + (u64)c.w, (u64)W), y1 = umin64(y0 + (u64)c.h, (u64)H);
     g.x0 = (long long)x0, g.y0 = (long long)y0, g.x1 = x1 > x0 && y1 > y0 ? (long long)x1 : (long long)x0, g.y1 = (long long)y1;
-    g.vec = (row % 4) == 0;
+    g.vec = (pitch % 4) == 0;
     const long long ppw = 4 / step;  // pixels per word
     g.ax0 = (g.x0 + ppw - 1) & ~(ppw - 1), g.ax1 = g.x1 & ~(ppw - 1);
     g.wpr = g.vec && g.ax1 > g.ax0 ? (int)((g.ax1 - g.ax0) / ppw) : 0;
@@ -1006,12 +1007,15 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
     if (split && blockIdx.y == 1 && !host0) return;       // nothing to mirror into
     uint8_t* const frame = frame0;
     uint8_t* const host = host0;
-    // row pitch of the drawn plane: the caller's surface pitch for the device frame; the pinned host frame is packed.  (The HUD paths
-    // below address packed rows: HUD handles take packed frames only.)  fmt is the frame's format: drawn with the overlay semantics of ofmt
+    // row pitch of the drawn plane: the caller's surface pitch for the device frame; the pinned host frame is packed.  A host frame only
+    // ever goes with a packed device frame (the handle's own buffer, fpitch == row): a surface step has no host frame, so no host-pass CTA
+    // and no bg_ready handshake (host == nullptr above and below).  The background dim therefore addresses both frames by fpitch.
+    // fmt is the frame's format: drawn with the overlay semantics of ofmt
     const size_t row = fmt_row_bytes(fmt, W);
     const int ofmt = overlay_format(fmt), step = fmt_px_step(fmt);
-    const size_t fpitch0 = kGroup ? 0 : own ? ctl->pitches[blockIdx.x][0] : ctl->pitch[0];
+    const size_t fpitch0 = kGroup ? e->pitch : own ? ctl->pitches[blockIdx.x][0] : ctl->pitch[0];
     const size_t fpitch = fpitch0 ? fpitch0 : row;
+    const size_t plen = fpitch0 ? (size_t)(H - 1) * fpitch + row : len;  // bytes from the plane's first row to the end of its last
     const bool do_dev = !split || blockIdx.y == 0, do_host = host != nullptr && (!split || blockIdx.y == 1);
     // this CTA's HUD list and background-dim flags: the frame's (CTA 0), or its stream's (probe group)
     const int32_t* const bg_on_dev = kGroup ? &e->bg_on_device : &ctl->bg_on_device;
@@ -1024,26 +1028,27 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
         for (int i = threadIdx.x; i < n_hud * (int)(sizeof(OverlayCmdDev) / 4); i += blockDim.x) dst[i] = src[i];
         __syncthreads();
     }
-    // the luma background dim, if it leads the list unconditionally (the probe's HUD): prefetch its pixels from the host frame now
+    // the luma background dim, if it leads the list unconditionally (the probe's HUD): prefetch its pixels from the host frame now (or
+    // from the device frame: a surface too, which no earlier kernel of the frame writes)
     const bool bg_first = n_hud > 0 && ofmt == VT_FMT_NV12 && s_cmd[0].kind == VT_OV_BACKGROUND && s_cmd[0].cond == VT_HUD_ALWAYS;
     BgRegion bg{0, 0, 0, 0, 0, 0, 0, false};
     uint32_t bgw[kBgWords];
     uint8_t bge[kBgEdge];
     bool bg_pre = false, bg_edge_pre = false;
     if (bg_first) {
-        bg = bg_region(s_cmd[0], W, H, row, step);
+        bg = bg_region(s_cmd[0], W, H, fpitch, step);
         const long long rows = bg.y1 - bg.y0;
-        if (((reinterpret_cast<uintptr_t>(host) | reinterpret_cast<uintptr_t>(frame)) & 3) != 0) bg.wpr = 0;  // bytewise
+        if (((reinterpret_cast<uintptr_t>(host) | reinterpret_cast<uintptr_t>(frame)) & 3) != 0) bg.wpr = 0;  // bytewise (as a pitch % 4)
         // source of the region: the device frame when it was uploaded with the windows (a copy-engine transfer ahead of the graph; an L2 hit
         // here), else the pinned host frame (PCIe reads: ~12 us for the 260 x 90 block, on the critical path of a short frame)
         const uint8_t* bsrc = (host && !*bg_on_dev) ? host : frame;
-        bg_pre = (host || *bg_on_dev) && bg.wpr > 0 && rows * bg.wpr <= (long long)kBgWords * kOvThreads && (size_t)bg.y1 * row <= len;
+        bg_pre = (host || *bg_on_dev) && bg.wpr > 0 && rows * bg.wpr <= (long long)kBgWords * kOvThreads && (size_t)(bg.y1 - 1) * fpitch + row <= plen;
         if (bg_pre) {
             const int total = (int)rows * bg.wpr;
 #pragma unroll
             for (int k = 0; k < kBgWords; ++k) {
                 const int i = threadIdx.x + k * kOvThreads;
-                if (i < total) bgw[k] = *reinterpret_cast<const volatile uint32_t*>(bsrc + (size_t)(bg.y0 + i / bg.wpr) * row + bg.ax0 * step + 4 * (i % bg.wpr));
+                if (i < total) bgw[k] = *reinterpret_cast<const volatile uint32_t*>(bsrc + (size_t)(bg.y0 + i / bg.wpr) * fpitch + bg.ax0 * step + 4 * (i % bg.wpr));
             }
             // ... and the columns outside the word interior (<= 3 + 3 per row), so that nothing of the region is read after the dependency
             // wait: with two CTAs per target the other CTA dims the device frame's copy of the region after its own wait
@@ -1056,7 +1061,7 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
                     if (i < rows * ec) {
                         const uint32_t rq = (uint32_t)i / (uint32_t)ec;
                         const long long yy = bg.y0 + rq, kk = i - (long long)rq * ec, xx = kk < eh ? bg.x0 + kk : bg.ax1 + (kk - eh);
-                        bge[k] = *reinterpret_cast<const volatile uint8_t*>(bsrc + (size_t)yy * row + (size_t)xx * step);
+                        bge[k] = *reinterpret_cast<const volatile uint8_t*>(bsrc + (size_t)yy * fpitch + (size_t)xx * step);
                     }
                 }
             }
@@ -1128,7 +1133,7 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
         if (bg_first) {  // ---- the background dim: word interior from registers (or the device frame), ragged edges bytewise
             const unsigned factor = 255u - (unsigned)(uint8_t)s_cmd[0].a;
             const long long rows = bg.y1 - bg.y0;
-            if (bg.x1 > bg.x0 && (size_t)bg.y1 * row <= len) {
+            if (bg.x1 > bg.x0 && (size_t)(bg.y1 - 1) * fpitch + row <= plen) {
                 if (bg.wpr > 0) {
                     const long long total = rows * bg.wpr;
                     for (long long base = 0; base < total; base += (long long)kBgWords * kOvThreads) {
@@ -1141,7 +1146,7 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
                                 const long long i = base + threadIdx.x + (long long)k * kOvThreads;
                                 if (i < total) {
                                     const uint32_t rr = (uint32_t)i / (uint32_t)bg.wpr, cc = (uint32_t)i - rr * (uint32_t)bg.wpr;
-                                    bgw[k] = *reinterpret_cast<const uint32_t*>(src + (size_t)(bg.y0 + rr) * row + bg.ax0 * step + 4 * cc);
+                                    bgw[k] = *reinterpret_cast<const uint32_t*>(src + (size_t)(bg.y0 + rr) * fpitch + bg.ax0 * step + 4 * cc);
                                 }
                             }
                         }
@@ -1150,7 +1155,7 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
                             const long long i = base + threadIdx.x + (long long)k * kOvThreads;
                             if (i < total) {
                                 const uint32_t rr = (uint32_t)i / (uint32_t)bg.wpr, cc = (uint32_t)i - rr * (uint32_t)bg.wpr;
-                                const size_t o = (size_t)(bg.y0 + rr) * row + bg.ax0 * step + 4 * cc;
+                                const size_t o = (size_t)(bg.y0 + rr) * fpitch + bg.ax0 * step + 4 * cc;
                                 const uint32_t d = dim4(bgw[k], factor, step);
                                 if (do_dev) *reinterpret_cast<uint32_t*>(frame + o) = d;
                                 if (do_host) *reinterpret_cast<uint32_t*>(host + o) = d;
@@ -1164,7 +1169,7 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
                 for (long long i = threadIdx.x, kk = 0; i < rows * ec; i += blockDim.x, ++kk) {
                     const uint32_t rq = (uint32_t)i / (uint32_t)ec;  // (rows * ec < 2^31)
                     const long long yy = bg.y0 + rq, k = i - (long long)rq * ec, xx = k < eh ? bg.x0 + k : bg.ax1 + (k - eh);
-                    const size_t o = (size_t)yy * row + (size_t)xx * step;
+                    const size_t o = (size_t)yy * fpitch + (size_t)xx * step;
                     const unsigned v = (bg_edge_pre && bg.wpr > 0) ? (unsigned)bge[kk < kBgEdge ? kk : 0] : (unsigned)(edge_host ? host[o] : frame[o]);
                     const uint8_t d = (uint8_t)((v * factor) / 255u);
                     if (do_dev) frame[o] = d;
@@ -1185,7 +1190,7 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
                 if (c.kind < 0) continue;
                 if (p == 1 && c.kind == VT_OV_BACKGROUND && ofmt == VT_FMT_NV12 && !split) {  // (split: this CTA dims the host pixels itself)
                     // a dim that does not lead the list: the host copy takes the final pixels of the region from the device frame (the
-                    // later commands of this pass re-draw what lies on top of it)
+                    // later commands of this pass re-draw what lies on top of it; both packed, as every frame that has a host copy)
                     const BgRegion g = bg_region(c, W, H, row, step);
                     for (long long j = threadIdx.x; j < (g.y1 - g.y0) * (g.x1 - g.x0); j += blockDim.x) {
                         const size_t o = (size_t)(g.y0 + j / (g.x1 - g.x0)) * row + (size_t)(g.x0 + j % (g.x1 - g.x0)) * step;
@@ -1218,7 +1223,9 @@ __global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int
     box_overlay_body<false>(len, W, H, fmt, res, slots, n, gate, ctl, stamp_end, blk, blk_words, draw_box, s_cmd);
 }
 
-__global__ void __launch_bounds__(kOvThreads) probe_group_overlay_kernel(const DeviceResult* __restrict__ res, float gate, const ProbeGroupCtl* ctl,
+// (minimum of one CTA per SM stated: without it ptxas holds this instance to 64 registers and spills the background-dim prefetch; the grid
+// is one CTA pair per stream, at most 32 CTAs)
+__global__ void __launch_bounds__(kOvThreads, 1) probe_group_overlay_kernel(const DeviceResult* __restrict__ res, float gate, const ProbeGroupCtl* ctl,
                                                                          unsigned long long* stamp_end, const uint32_t* __restrict__ blk,
                                                                          int blk_words) {
     __shared__ OverlayCmdDev s_cmd[kMaxCmds];

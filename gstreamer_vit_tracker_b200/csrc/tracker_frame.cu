@@ -569,13 +569,8 @@ static vt_status check_surface(const vt_tracker* t, const StreamGeom& g, const v
     return VT_OK;
 }
 
-// Checks shared by the surface entry points: a probe (HUD) handle draws its command lists with packed-row addressing, and a synchronous
-// call finds no frame in flight.
+// Checks shared by the surface entry points: a synchronous call finds no frame in flight.
 static vt_status surface_call(vt_tracker* t, const char* where, bool sync) {
-    if (t->hud_mode) {
-        set_error("%s: a probe (HUD) handle takes packed frames only", where);
-        return VT_ERR_INVALID;
-    }
     if (sync && t->q_count) {
         set_error("%s: frames are in flight (submit/wait); drain them first", where);
         return VT_ERR_INVALID;
@@ -981,6 +976,41 @@ static bool group_refused(const vt_tracker* t, const char* where) {
     return true;
 }
 
+// The public surface calls refuse a probe (HUD) handle: the probe's state machine stages a HUD list for every frame of that handle, so
+// its surfaces go through vt_probe_frame_surface / vt_probe_group_frame_surface (tracker_init_surface / tracker_submit_surface below).
+static bool hud_refused(const vt_tracker* t, const char* where) {
+    if (!t->hud_mode) return false;
+    set_error("%s: a probe (HUD) handle takes surfaces through vt_probe_frame_surface / vt_probe_group_frame_surface only", where);
+    return true;
+}
+
+vt_status tracker_check_surface(const vt_tracker* t, int stream, const vt_surface* s, const char* where) {
+    return check_surface(t, slot_geom(t, stream), s, where, stream);
+}
+
+// VitTrack::init of `target` on a surface of the slot's geometry, read in place
+vt_status tracker_init_surface(vt_tracker* t, int32_t target, const vt_surface* s, vt_bbox box, const char* where) {
+    if (t->in_flight) {
+        set_error("%s: a frame is in flight", where);
+        return VT_ERR_INVALID;
+    }
+    vt_status st = surface_call(t, where, true);
+    if (st == VT_OK) st = check_surface(t, slot_geom(t, target), s, where, 0);
+    const StreamGeom& g = slot_geom(t, target);
+    if (st == VT_OK) st = check_template_window(t, g, box, where);
+    if (st != VT_OK) return st;
+    const bool nv12 = g.fmt == VT_FMT_NV12;
+    return init_template(t, target, box, FrameDesc{s->planes[0], nv12 ? s->planes[1] : nullptr, {s->pitch[0], nv12 ? s->pitch[1] : 0}, g.W, g.H,
+                                                   g.fmt, 1, nullptr, t->cfg.pad_plus1});
+}
+
+vt_status tracker_submit_surface(vt_tracker* t, const vt_surface* s, bool forward, const char* where) {
+    vt_status st = surface_call(t, where, false);
+    if (st == VT_OK) st = check_surface(t, cfg_geom(t), s, where, 0);
+    if (st != VT_OK) return st;
+    return submit_common(t, nullptr, nullptr, 0, forward, s);
+}
+
 }  // namespace vt
 
 using namespace vt;
@@ -1005,19 +1035,8 @@ vt_status vt_tracker_init_surface(vt_tracker* t, int32_t target, const vt_surfac
         set_error("vt_tracker_init_surface: invalid argument");
         return VT_ERR_INVALID;
     }
-    if (t->in_flight) {
-        set_error("vt_tracker_init_surface: a frame is in flight");
-        return VT_ERR_INVALID;
-    }
-    if (group_refused(t, "vt_tracker_init_surface")) return VT_ERR_INVALID;
-    vt_status st = surface_call(t, "vt_tracker_init_surface", true);
-    if (st == VT_OK) st = check_surface(t, slot_geom(t, target), s, "vt_tracker_init_surface", 0);
-    const StreamGeom& g = slot_geom(t, target);
-    if (st == VT_OK) st = check_template_window(t, g, box, "vt_tracker_init_surface");
-    if (st != VT_OK) return st;
-    const bool nv12 = g.fmt == VT_FMT_NV12;
-    return init_template(t, target, box, FrameDesc{s->planes[0], nv12 ? s->planes[1] : nullptr, {s->pitch[0], nv12 ? s->pitch[1] : 0}, g.W, g.H,
-                                                   g.fmt, 1, nullptr, t->cfg.pad_plus1});
+    if (group_refused(t, "vt_tracker_init_surface") || hud_refused(t, "vt_tracker_init_surface")) return VT_ERR_INVALID;
+    return tracker_init_surface(t, target, s, box, "vt_tracker_init_surface");
 }
 
 vt_status vt_tracker_set_stream_geometry(vt_tracker* t, int32_t target, const vt_stream_geometry* g) {
@@ -1139,8 +1158,10 @@ bool tracker_group_active(const vt_tracker* t, int stream) { return t && stream 
 // runs one CTA pair per stream of the group: the stream's HUD list (both outcomes for a stream in the forward, picked by its own result),
 // drawn on its device frame and mirrored into its pinned host frame.  With no stream in the forward that kernel is the whole step.
 // Every luma stream's HUD region is uploaded with the windows, so that — as in the single probe — the device pass dims its own copy of the
-// region while the host pass reads the pinned frame.  Synchronous (rect_mirror is exact: the windows are the real search windows).
-vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size_t* lens) {
+// region while the host pass reads the pinned frame.  Or surfs[i] (frames / lens unused; checked by the caller) is stream i's device
+// surface: read and drawn into in place, nothing uploaded and nothing mirrored.  Synchronous (rect_mirror is exact: the windows are the
+// real search windows).
+vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size_t* lens, const vt_surface* surfs) {
     const int n = t ? t->group_n : 0;
     if (!n || t->q_count) {
         set_error("tracker_submit_group: not the tracker of a probe group, or a step is in flight");
@@ -1150,7 +1171,7 @@ vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size
     const int slot = t->q_head;
     vt_tracker::Slot& q = t->q[slot];
     q.t_submit = std::chrono::steady_clock::now();
-    q.frame = frames[0], q.len = lens[0], q.pageable = false, q.mirrored = true, q.hud_bytes = 0;
+    q.frame = surfs ? nullptr : frames[0], q.len = surfs ? 0 : lens[0], q.pageable = false, q.mirrored = !surfs, q.hud_bytes = 0;
     ProbeGroupCtl ctl;
     memset(&ctl, 0, sizeof(ctl));
     const int k_act = (int)t->active.size();
@@ -1159,6 +1180,12 @@ vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size
         const int i = t->active[k];
         const StreamGeom& g = slot_geom(t, i);
         ctl.f.geom[k][0] = g.fmt, ctl.f.geom[k][1] = g.W, ctl.f.geom[k][2] = g.H, ctl.f.geom[k][3] = 1;
+        if (surfs) {  // in place: the whole surface holds the frame
+            const bool nv12 = g.fmt == VT_FMT_NV12;
+            ctl.f.frames[k] = surfs[i].planes[0], ctl.f.uvs[k] = nv12 ? surfs[i].planes[1] : nullptr;
+            ctl.f.pitches[k][0] = surfs[i].pitch[0], ctl.f.pitches[k][1] = nv12 ? surfs[i].pitch[1] : 0;
+            continue;
+        }
         int* w = ctl.f.win[k];
         if (!t->cfg.upload_window || !windows_allowed(g)) {
             VT_CUDA(cudaMemcpyAsync(t->d_sframes[i], frames[i], g.bytes(), cudaMemcpyHostToDevice, t->stream));
@@ -1177,14 +1204,15 @@ vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size
     for (int i = 0; i < n; ++i) {  // every stream of the group, by stream index
         const StreamGeom& g = slot_geom(t, i);
         ProbeStreamCtl& e = ctl.s[i];
-        e.frame = t->d_sframes[i], e.host_frame = frames[i];
+        e.frame = surfs ? surfs[i].planes[0] : t->d_sframes[i], e.host_frame = surfs ? nullptr : frames[i];
+        e.pitch = surfs ? surfs[i].pitch[0] : 0;
         e.geom[0] = g.fmt, e.geom[1] = g.W, e.geom[2] = g.H, e.geom[3] = 1;
         e.n_hud = t->hud_next_n[i];
         e.hud = e.n_hud ? t->h_hud[slot] + (size_t)i * kMaxCmds : nullptr;
         e.slot = t->inited[i] ? i : -1;
         const int* r = t->hud_next_rmw[i];
         int w[4] = {std::max(r[0], 0), std::max(r[1], 0), std::min(r[2], g.W), std::min(r[3], g.H)};
-        if (e.n_hud && whole[i]) {
+        if (e.n_hud && (surfs || whole[i])) {
             e.bg_on_device = 1;
         } else if (e.n_hud && w[2] > w[0] && w[3] > w[1]) {  // plane 0 only (the luma background dim reads and writes Y)
             vt_status st = copy_window(g, t->d_sframes[i], frames[i], w, false, cudaMemcpyHostToDevice, t->stream);
@@ -1196,7 +1224,7 @@ vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size
         t->hud_next_n[i] = 0;
     }
     ctl.f.frame = ctl.f.frames[0], ctl.f.host_frame = ctl.f.host_frames[0], ctl.f.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
-    ctl.f.n_win = k_act;
+    ctl.f.n_win = surfs ? -1 : k_act;
     if (k_act) {  // (drops since the last step changed the list: it reaches the device ahead of the step's kernels)
         memcpy(t->h_slots, t->active.data(), sizeof(int32_t) * (size_t)k_act);
         VT_CUDA(cudaMemcpyAsync(t->d_slots, t->h_slots, sizeof(int32_t) * (size_t)k_act, cudaMemcpyHostToDevice, t->stream));
@@ -1282,6 +1310,7 @@ vt_status vt_tracker_update_device(vt_tracker* t, uint8_t* d_frame, size_t len, 
 vt_status vt_tracker_update_surface(vt_tracker* t, const vt_surface* s, vt_result* results) {
     if (!t || !s) return VT_ERR_INVALID;
     if (group_refused(t, "vt_tracker_update_surface")) return VT_ERR_INVALID;
+    if (hud_refused(t, "vt_tracker_update_surface")) return VT_ERR_INVALID;
     vt_status st = check_uniform_geometry(t, "vt_tracker_update_surface");
     if (st == VT_OK) st = surface_call(t, "vt_tracker_update_surface", true);
     if (st == VT_OK) st = check_surface(t, cfg_geom(t), s, "vt_tracker_update_surface", 0);
@@ -1293,11 +1322,10 @@ vt_status vt_tracker_update_surface(vt_tracker* t, const vt_surface* s, vt_resul
 vt_status vt_tracker_submit_surface(vt_tracker* t, const vt_surface* s) {
     if (!t || !s) return VT_ERR_INVALID;
     if (group_refused(t, "vt_tracker_submit_surface")) return VT_ERR_INVALID;
+    if (hud_refused(t, "vt_tracker_submit_surface")) return VT_ERR_INVALID;
     vt_status st = check_uniform_geometry(t, "vt_tracker_submit_surface");
-    if (st == VT_OK) st = surface_call(t, "vt_tracker_submit_surface", false);
-    if (st == VT_OK) st = check_surface(t, cfg_geom(t), s, "vt_tracker_submit_surface", 0);
     if (st != VT_OK) return st;
-    return submit_common(t, nullptr, nullptr, 0, true, s);
+    return tracker_submit_surface(t, s, true, "vt_tracker_submit_surface");
 }
 
 vt_status vt_tracker_update_streams_surface(vt_tracker* t, const vt_surface* surfaces, int32_t n, vt_result* results) {

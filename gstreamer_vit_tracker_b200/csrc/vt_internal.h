@@ -180,9 +180,11 @@ struct FrameCtl {
 // the step's forward by active-target index, as for a stream group (the crop reads it); the per-stream table addresses EVERY stream of the
 // group by its index, which is also its target slot: CTA pair x of the step's last kernel (probe_group_overlay_kernel) draws stream x.
 struct ProbeStreamCtl {
-    uint8_t* frame;              // the stream's device frame (its search window, if it takes part, and its HUD region uploaded this step)
-    uint8_t* host_frame;         // its pinned host frame: zero-copy target of the overlay mirror
+    uint8_t* frame;              // the stream's device frame (its search window, if it takes part, and its HUD region uploaded this step),
+                                 // or plane 0 of its surface (vt_probe_group_frame_surface: drawn in place)
+    uint8_t* host_frame;         // its pinned host frame: zero-copy target of the overlay mirror (null for a surface)
     const OverlayCmdDev* hud;    // its HUD list in the pinned block of the step's queue slot, n_hud entries
+    size_t pitch;                // row pitch of `frame` in bytes; 0: packed rows
     alignas(16) int32_t geom[4]; // {format, width, height, 1}
     int32_t n_hud;
     int32_t slot;                // its target slot when it takes part in this step's forward, else -1 (the HUD of a stream without result)
@@ -294,8 +296,16 @@ vt_status tracker_group_init(vt_tracker* t, int stream, const uint8_t* frame, si
 vt_status tracker_group_drop(vt_tracker* t, int stream);
 bool tracker_group_active(const vt_tracker* t, int stream);
 // one group step: frames[i] (pinned, full length: checked by the caller) of every stream, the HUD lists staged with tracker_set_hud; the
-// streams whose slot is active run one batched forward, and the step's last kernel draws every stream's HUD — then vt_tracker_wait
-vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size_t* lens);
+// streams whose slot is active run one batched forward, and the step's last kernel draws every stream's HUD — then vt_tracker_wait.
+// surfs (else null): surfs[i] is stream i's device surface (checked by the caller), tracked and drawn into in place
+vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size_t* lens, const vt_surface* surfs = nullptr);
+// Probe (HUD) handles on the caller's device surfaces (vt_probe_frame_surface, vt_probe_group_frame_surface); the public surface calls
+// refuse those handles.  tracker_check_surface: the vt_surface rules for a frame of slot `stream`'s geometry (a single probe: 0).
+vt_status tracker_check_surface(const vt_tracker* t, int stream, const vt_surface* s, const char* where);
+// VitTrack::init of `target` on the surface (no public-entry-point checks; a probe group's stream i is target i)
+vt_status tracker_init_surface(vt_tracker* t, int32_t target, const vt_surface* s, vt_bbox box, const char* where);
+// a single probe's frame on the surface with the staged HUD list: forward = false for a frame on which no tracker runs — then vt_tracker_wait
+vt_status tracker_submit_surface(vt_tracker* t, const vt_surface* s, bool forward, const char* where);
 bool frame_is_pinned(const void* p);
 // copies the region of a frame that a box overlay (rect thickness 3 + crosshair 15) / the probe HUD touched back from a clean copy
 void restore_box_region(uint8_t* frame, const uint8_t* clean, int fmt, int W, int H, const vt_bbox& b);

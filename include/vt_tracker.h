@@ -188,7 +188,8 @@ vt_status vt_tracker_update_device(vt_tracker* t, uint8_t* d_frame, size_t len, 
  * planes[0] (the Y plane for NV12 / GRAY8, the Y samples for YUY2, the image for RGB24) with the reference's clamping, so nothing is
  * written into the pitch padding, the UV plane or the YUY2 chroma bytes.  The surface must stay valid until the call returns (submit: until the matching wait()).
  * VT_ERR_INVALID (and vt_last_error()) for a NULL surface or plane, a pitch below the plane's row bytes, a plane that is not device or
- * managed memory of cfg.device, a probe (HUD) handle, and — synchronous calls — frames in flight. */
+ * managed memory of cfg.device, and — synchronous calls — frames in flight.  These four vt_tracker_*_surface calls are also
+ * VT_ERR_INVALID on the tracker of a probe (HUD) handle, whose surfaces go through vt_probe_frame_surface / vt_probe_group_frame_surface. */
 typedef struct { uint8_t* planes[2]; size_t pitch[2]; } vt_surface;
 vt_status vt_tracker_init_surface(vt_tracker* t, int32_t target, const vt_surface* s, vt_bbox box);  /* ≙ vt_tracker_init */
 vt_status vt_tracker_update_surface(vt_tracker* t, const vt_surface* s, vt_result* results);         /* ≙ vt_tracker_update_device */
@@ -377,6 +378,12 @@ vt_tracker* vt_context_tracker(vt_context* c);
  * NULL) replaces the timing-dependent HUD strings so that pixel parity is testable:
  * {fps_line, timing_line}. */
 vt_status vt_probe_frame(vt_context* c, uint8_t* frame, size_t len, const char* const* hud_override);
+/* ≙ vt_probe_frame on a pitched device surface of the context's geometry (vt_surface rules above): the probe's HUD, cursor / selection
+ * and box are drawn in place into the surface's plane 0 (Y / RGB / the Y samples of YUY2), never into pitch padding, the UV plane or
+ * YUY2 chroma bytes; nothing is copied between host and device but the result block.  A confirm frame initialises the tracker on this
+ * surface.  VT_ERR_INVALID (and vt_last_error()) for a NULL surface, a surface that fails the vt_surface checks, or a probe-group member.
+ * A context may take host frames on one call and surfaces on the next. */
+vt_status vt_probe_frame_surface(vt_context* c, const vt_surface* s, const char* const* hud_override);
 
 /* The same loop over vt_probe_frame (the drop-in call): n frames of a host ring through the context, HUD drawn into every frame.
  * `pristine` (nullable): after each probe the HUD region and the box of that frame are restored from it. */
@@ -407,6 +414,10 @@ vt_context* vt_probe_group_context(vt_probe_group* g, int32_t stream);
  * full length for its geometry (lens[i] >= its frame bytes); a pageable, short or NULL frame is VT_ERR_INVALID with a message.
  * hud_override as in vt_probe_frame, for every stream. */
 vt_status vt_probe_group_frame(vt_probe_group* g, uint8_t* const* frames, const size_t* lens, const char* const* hud_override);
+/* ≙ vt_probe_group_frame with surfaces[i] the current surface of stream i (n = vt_probe_group_size(g)); each checked against stream i's
+ * geometry; one batched forward, one synchronisation, every stream's HUD drawn into its own surface.  VT_ERR_INVALID (and
+ * vt_last_error()) for a NULL group or array, n != the group's size, or a surface that fails the vt_surface checks for its stream. */
+vt_status vt_probe_group_frame_surface(vt_probe_group* g, const vt_surface* surfaces, int32_t n, const char* const* hud_override);
 /* ≙ vt_context_run_ring for a group: n steps, stream i's frames from rings[i] (pinned host memory; `ring` frames, `stride` apart, frame_len
  * bytes each), pristine[i] (nullable; pristine itself nullable) restores what each step drew, latency_us[step] (nullable). */
 vt_status vt_probe_group_run_ring(vt_probe_group* g, uint8_t* const* rings, size_t stride, size_t frame_len, int32_t ring, int32_t first,
