@@ -438,14 +438,15 @@ struct PixelSrc {
     size_t pitch, uv_pitch;       // their row pitches
     const uint8_t* host;          // null: everything is on the device
     int x0, y0, x1, y1;           // valid window of the device frame (even-aligned, so a pixel and its chroma pair sit on the same side)
-    bool dev_words, host_words;   // YUY2: the plane's pixel-pair words are 4-byte aligned (base and pitch), one 32-bit load each
+    bool dev_words, host_words;   // YUY2 / RGBA / BGRA: the plane's words (pixel pairs, pixels) are 4-byte aligned (base and pitch), one
+                                  // 32-bit load each
     int format;                   // vt_format of this target's frame
     int xlim, ylim;               // pixels [0, xlim) x [0, ylim) are read, the rest is border (0 x 0 for a short frame)
 };
 
-// the Y0 U Y1 V word of pixel fx in a YUY2 row: one 32-bit load when aligned, else four byte loads (surfaces may have any pitch)
-__device__ __forceinline__ uint32_t yuy2_word(const uint8_t* row, int fx, bool aligned) {
-    const uint8_t* q = row + 4 * (fx >> 1);
+// the 4 bytes at q (a YUY2 Y0 U Y1 V word, an RGBA / BGRA pixel): one 32-bit load when aligned, else four byte loads (surfaces may have
+// any pitch)
+__device__ __forceinline__ uint32_t plane_word(const uint8_t* q, bool aligned) {
     if (aligned) return *reinterpret_cast<const uint32_t*>(q);
     return (uint32_t)q[0] | ((uint32_t)q[1] << 8) | ((uint32_t)q[2] << 16) | ((uint32_t)q[3] << 24);
 }
@@ -462,9 +463,13 @@ __device__ __forceinline__ void frame_rgb(const PixelSrc& ps, int fx, int fy, in
     } else if (ps.format == VT_FMT_GRAY8) {
         r = g = b = data[(size_t)fy * ps.pitch + fx];
     } else if (ps.format == VT_FMT_YUY2) {
-        const uint32_t w = yuy2_word(data + (size_t)fy * ps.pitch, fx, host ? ps.host_words : ps.dev_words);
+        const uint32_t w = plane_word(data + (size_t)fy * ps.pitch + 4 * (fx >> 1), host ? ps.host_words : ps.dev_words);
         const Chroma c = chroma_terms((int)((w >> 8) & 0xff), (int)(w >> 24));
         yuv_px((int)((w >> ((fx & 1) * 16)) & 0xff), c, r, g, b);
+    } else if (format_is_rgb32(ps.format)) {  // byte 3 is loaded with the word but never used
+        const uint32_t w = plane_word(data + (size_t)fy * ps.pitch + 4 * (size_t)fx, host ? ps.host_words : ps.dev_words);
+        const RgbOffsets o = fmt_rgb_offsets(ps.format);
+        r = (int)((w >> (8 * o.r)) & 0xff), g = (int)((w >> (8 * o.g)) & 0xff), b = (int)((w >> (8 * o.b)) & 0xff);
     } else {
         const int yv = data[(size_t)fy * ps.pitch + fx];
         const uint8_t* uv = host ? ps.host + (ps.dev_uv - ps.dev) : ps.dev_uv;
@@ -504,7 +509,7 @@ __global__ void __launch_bounds__(256) crop_resize_norm_kernel(FrameDesc f, Targ
     if (!ps.dev_uv) ps.dev_uv = ps.dev + (size_t)f.width * f.height;
     if (!ps.uv_pitch) ps.uv_pitch = (size_t)f.width;
     ps.dev_words = ((reinterpret_cast<uintptr_t>(ps.dev) | ps.pitch) & 3) == 0;
-    ps.host_words = (reinterpret_cast<uintptr_t>(ps.host) & 3) == 0;  // (packed YUY2 rows are whole words)
+    ps.host_words = (reinterpret_cast<uintptr_t>(ps.host) & 3) == 0;  // (packed YUY2 / RGBA / BGRA rows are whole words)
     ps.format = f.format;
     // pad_plus1 (App. A.7, older OpenCV): a crop that reaches the right / bottom edge pads one pixel more, i.e. the last column / row of
     // the frame reads as border; a crop that stays inside never addresses it, so the bound can move unconditionally
@@ -733,17 +738,20 @@ struct Surface {
     size_t len;            // bytes of the drawn plane (RGB writes are bounds-checked against it)
     int W, H, fmt;
     size_t pitch;          // row pitch of the drawn plane in bytes (Y plane / RGB image)
-    int step;              // luma formats: bytes between the Y samples of a row (1; YUY2: 2, the chroma bytes in between are never written)
+    int step;              // bytes between the pixels of a row: luma formats, between the Y samples (1; YUY2: 2, the chroma bytes in
+                           // between are never written); RGB formats, the pixel size (RGB24: 3; RGBA / BGRA: 4, byte 3 is never written)
+    RgbOffsets ch;         // RGB formats: the bytes of R, G, B within a pixel
 };
 __device__ __forceinline__ Surface make_surface(uint8_t* d, size_t len, int W, int H, int fmt, size_t pitch) {
-    return Surface{d, len, W, H, overlay_format(fmt), pitch, fmt_px_step(fmt)};
+    return Surface{d, len, W, H, overlay_format(fmt), pitch, fmt_px_step(fmt), fmt_rgb_offsets(fmt)};
 }
-// NV12: luma write (Y plane). RGB: bounds-checked colour write (src/drawing_rgb.rs:18-28).
+// NV12: luma write (Y plane). RGB: bounds-checked colour write (src/drawing_rgb.rs:18-28); the pixel's last colour byte is byte 2 in
+// every RGB format.
 __device__ __forceinline__ void put_y(const Surface& s, u64 x, u64 y, uint8_t v) { s.d[y * (u64)s.pitch + x * (u64)s.step] = v; }
 __device__ __forceinline__ void put_rgb(const Surface& s, int x, int y, uint8_t r, uint8_t g, uint8_t b) {
     if (x < 0 || y < 0 || x >= s.W || y >= s.H) return;
-    const size_t off = (size_t)y * s.pitch + (size_t)x * 3;
-    if (off + 2 < s.len) s.d[off] = r, s.d[off + 1] = g, s.d[off + 2] = b;
+    const size_t off = (size_t)y * s.pitch + (size_t)x * s.step;
+    if (off + 2 < s.len) s.d[off + s.ch.r] = r, s.d[off + s.ch.g] = g, s.d[off + s.ch.b] = b;
 }
 
 __device__ void ov_rect_nv12(const Surface& s, int x, int y, int w, int h, int thickness, uint8_t v) {  // src/nv12_convert.rs:172-213
@@ -841,11 +849,12 @@ __device__ void ov_background(const Surface& s, const OverlayCmdDev& c) {
         const u64 xs = (u64)max(c.x, 0), xe = umin64(i32_as_usize((int)((unsigned)c.x + (unsigned)c.w)), (u64)s.W);
         const u64 ys = (u64)max(c.y, 0), ye = umin64(i32_as_usize((int)((unsigned)c.y + (unsigned)c.h)), (u64)s.H);
         if (xe <= xs || ye <= ys) return;
-        const u64 rb = (xe - xs) * 3, n = rb * (ye - ys);
+        // (every colour byte of the row span; of a 32-bit pixel, byte 3 is skipped)
+        const u64 rb = (xe - xs) * (u64)s.step, n = rb * (ye - ys);
         for (u64 i = threadIdx.x; i < n; i += blockDim.x) {
-            const u64 row = ys + i / rb;
-            const u64 off = row * (u64)s.pitch + xs * 3;
-            if (off + rb <= s.len) s.d[off + i % rb] = 30;
+            const u64 row = ys + i / rb, col = i % rb;
+            const u64 off = row * (u64)s.pitch + xs * (u64)s.step;
+            if (off + rb <= s.len && (s.step != 4 || (col & 3) != 3)) s.d[off + col] = 30;
         }
     }
 }

@@ -306,7 +306,7 @@ static vt_status build_cmds(vt_tracker* t, const vt_overlay_cmd* cmds, int n, st
             case VT_OV_TEXT: r0 = c.y, r1 = (long long)c.y + 7LL * std::max(c.a, 0); break;
             case VT_OV_BACKGROUND:
                 r0 = c.y, r1 = (long long)c.y + c.h;
-                if (t->fmt == VT_FMT_RGB24 && (long long)c.y + c.h < 0) r0 = 0, r1 = H - 1;  // (y+bh) as usize wraps, src/drawing_rgb.rs:45
+                if (!format_is_luma(t->fmt) && (long long)c.y + c.h < 0) r0 = 0, r1 = H - 1;  // (y+bh) as usize wraps, src/drawing_rgb.rs:45
                 break;
             case VT_OV_CURSOR: {
                 const long long yc = std::max(0LL, std::min<long long>(c.y, H - 1));  // src/drawing.rs:7 clamps, the RGB path does not
@@ -324,9 +324,10 @@ static vt_status build_cmds(vt_tracker* t, const vt_overlay_cmd* cmds, int n, st
 static vt_status overlay_impl(vt_tracker* t, uint8_t* frame, size_t len, const vt_overlay_cmd* cmds, int32_t n, bool upload) {
     if (!t || !frame || (n > 0 && !cmds) || t->in_flight) return VT_ERR_INVALID;
     VT_CUDA(cudaSetDevice(t->cfg.device));
-    const size_t need = format_is_luma(t->fmt) ? fmt_row_bytes(t->fmt, t->W) * t->H : 0;
+    // RGBA / BGRA: a full frame, so that every drawn pixel is whole (RGB24 writes are bounds-checked per pixel against len instead)
+    const size_t need = format_is_luma(t->fmt) || format_is_rgb32(t->fmt) ? fmt_row_bytes(t->fmt, t->W) * t->H : 0;
     if (len < need) {
-        set_error("vt_overlay: frame shorter than its Y plane (YUY2: than the packed frame)");
+        set_error("vt_overlay: frame shorter than its Y plane (YUY2 / RGBA / BGRA: than the packed frame)");
         return VT_ERR_INVALID;
     }
     std::vector<std::pair<int, int>> spans;

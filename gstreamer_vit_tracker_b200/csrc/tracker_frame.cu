@@ -326,9 +326,10 @@ struct UploadPlan {
     size_t bytes = 0;
 };
 // Window uploads need windows whose pixels carry their own chroma: even x0 (NV12 chroma pairs, YUY2 words) and, for NV12, even y0.
-// YUY2 takes any W and H: a window that ends on an odd last column copies that column's whole word, and chroma is per row.
+// YUY2 takes any W and H: a window that ends on an odd last column copies that column's whole word, and chroma is per row.  RGBA / BGRA
+// take any W and H: a window is whole 4-byte pixels, each with its own colour.
 static bool windows_allowed(const StreamGeom& g) {
-    return g.fmt == VT_FMT_YUY2 || (!(g.W % 2) && !((g.H % 2) && g.fmt == VT_FMT_NV12));
+    return g.fmt == VT_FMT_YUY2 || format_is_rgb32(g.fmt) || (!(g.W % 2) && !((g.H % 2) && g.fmt == VT_FMT_NV12));
 }
 // bytes of plane 0 that hold the pixels [x0, x1) x [y0, y1) of a packed frame (YUY2: whole words)
 static size_t plane0_bytes(const StreamGeom& g, int x0, int y0, int x1, int y1) {
@@ -483,7 +484,7 @@ void merge_spans(std::vector<std::pair<int, int>>& spans) {
     spans.swap(out);
 }
 
-// device -> host copy of whole rows [r0, r1] of the drawable plane (Y plane for NV12, the image for RGB24)
+// device -> host copy of whole rows [r0, r1] of the drawable plane (Y plane for NV12, the image for RGB24 / RGBA / BGRA)
 vt_status download_rows(vt_tracker* t, uint8_t* frame, size_t len, const std::vector<std::pair<int, int>>& spans, bool* staged) {
     const size_t pitch = fmt_row_bytes(t->fmt, t->W);
     const bool pinned = is_pinned(frame);
@@ -801,7 +802,7 @@ static vt_status wait_common(vt_tracker* t, vt_result* results) {
 
 // ---- ring replay support ----------------------------------------------------------------------------------------------------------
 // [x0, x1) x [y0, y1) of the drawable plane (Y plane / luma for NV12 and GRAY8, the RGB image for RGB24, the whole pixel-pair words
-// for YUY2), clipped to the frame
+// for YUY2, the whole 4-byte pixels for RGBA / BGRA), clipped to the frame
 void restore_rect_region(uint8_t* frame, const uint8_t* clean, int fmt, int W, int H, long long x0, long long y0, long long x1, long long y1) {
     x0 = std::max(x0, 0LL), y0 = std::max(y0, 0LL), x1 = std::min<long long>(x1, W), y1 = std::min<long long>(y1, H);
     if (x1 <= x0 || y1 <= y0) return;

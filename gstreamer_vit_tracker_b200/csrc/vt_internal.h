@@ -32,10 +32,22 @@ vt_status resolve_config(const vt_config* in, vt_config* out);
 // overlay semantics
 __host__ __device__ inline int overlay_format(int fmt) { return fmt == VT_FMT_GRAY8 || fmt == VT_FMT_YUY2 ? VT_FMT_NV12 : fmt; }
 __host__ __device__ inline bool format_is_luma(int fmt) { return fmt == VT_FMT_NV12 || fmt == VT_FMT_GRAY8 || fmt == VT_FMT_YUY2; }
+// RGBA / BGRA: 32-bit pixels whose byte 3 (alpha or padding) is never read or written; tracked and drawn on as the RGB24 frame of their
+// colour bytes
+__host__ __device__ inline bool format_is_rgb32(int fmt) { return fmt == VT_FMT_RGBA || fmt == VT_FMT_BGRA; }
+// byte offsets of R, G and B within a pixel of an RGB format (RGB24 / RGBA: 0 1 2; BGRA: 2 1 0): every reader and writer of colour bytes
+// takes the channel order from here
+struct RgbOffsets {
+    int r, g, b;
+};
+__host__ __device__ inline RgbOffsets fmt_rgb_offsets(int fmt) { return fmt == VT_FMT_BGRA ? RgbOffsets{2, 1, 0} : RgbOffsets{0, 1, 2}; }
 
-// ---- plane geometry of a format: every site that addresses plane 0 (Y / RGB / gray / packed YUY2) goes through these ----------
-// bytes between horizontally adjacent pixels of plane 0: the RGB triple, the Y sample (YUY2: Y0 U Y1 V, every second byte)
-__host__ __device__ inline int fmt_px_step(int fmt) { return fmt == VT_FMT_RGB24 ? 3 : fmt == VT_FMT_YUY2 ? 2 : 1; }
+// ---- plane geometry of a format: every site that addresses plane 0 (Y / RGB / gray / packed YUY2 / RGBA / BGRA) goes through these
+// bytes between horizontally adjacent pixels of plane 0: the RGB triple, the 32-bit RGBA / BGRA pixel, the Y sample (YUY2: Y0 U Y1 V,
+// every second byte)
+__host__ __device__ inline int fmt_px_step(int fmt) {
+    return fmt == VT_FMT_RGB24 ? 3 : format_is_rgb32(fmt) ? 4 : fmt == VT_FMT_YUY2 ? 2 : 1;
+}
 // bytes of one packed row of plane 0 (YUY2: whole pixel-pair words, 4 * ceil(W / 2): odd widths pad the last word)
 __host__ __device__ inline size_t fmt_row_bytes(int fmt, int W) {
     return fmt == VT_FMT_YUY2 ? (size_t)4 * (size_t)((W + 1) / 2) : (size_t)W * (size_t)fmt_px_step(fmt);
@@ -57,7 +69,7 @@ struct StreamGeom {
 };
 // the formats and sizes a handle's frames may have (vt_tracker_create's cfg, vt_tracker_set_stream_geometry)
 inline bool geometry_ok(int fmt, int W, int H) {
-    return W > 0 && H > 0 && (fmt == VT_FMT_NV12 || fmt == VT_FMT_RGB24 || fmt == VT_FMT_GRAY8 || fmt == VT_FMT_YUY2);
+    return W > 0 && H > 0 && (fmt == VT_FMT_NV12 || fmt == VT_FMT_RGB24 || fmt == VT_FMT_GRAY8 || fmt == VT_FMT_YUY2 || format_is_rgb32(fmt));
 }
 // the bytes [*o0, *o1) of a plane-0 row that hold the pixels x0 .. x1 - 1 (YUY2: the whole words of those pixels)
 __host__ __device__ inline void fmt_col_span(int fmt, long long x0, long long x1, size_t* o0, size_t* o1) {

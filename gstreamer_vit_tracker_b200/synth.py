@@ -80,6 +80,25 @@ def rgb_to_yuy2(rgb: np.ndarray) -> np.ndarray:
     return out.reshape(-1)
 
 
+def _rgb_to_32(rgb: np.ndarray, pad, order) -> np.ndarray:
+    h, w, _ = rgb.shape
+    out = np.empty((h, w, 4), dtype=np.uint8)
+    out[..., :3] = np.asarray(rgb, dtype=np.uint8)[..., order]
+    out[..., 3] = np.broadcast_to(np.asarray(pad, dtype=np.uint8).reshape((h, w) if np.ndim(pad) else ()), (h, w))
+    return out.reshape(-1)
+
+
+def rgb_to_rgba(rgb: np.ndarray, pad=255) -> np.ndarray:
+    """RGB(HWC u8) -> packed RGBA bytes R G B A (rows of 4 * w bytes, len = 4 * w * h).  `pad` is byte 3 of every pixel: a constant
+    (255: an opaque alpha; any value: RGBx padding) or an array of h * w bytes."""
+    return _rgb_to_32(rgb, pad, [0, 1, 2])
+
+
+def rgb_to_bgra(rgb: np.ndarray, pad=255) -> np.ndarray:
+    """RGB(HWC u8) -> packed BGRA bytes B G R A (rows of 4 * w bytes, len = 4 * w * h); `pad` as in rgb_to_rgba."""
+    return _rgb_to_32(rgb, pad, [2, 1, 0])
+
+
 def smooth_background(seed: int, w: int, h: int, cell: int = 32) -> np.ndarray:
     """Integer bilinear up-sampling of a coarse hash-noise grid plus 4-bit fine grain."""
     gh, gw = h // cell + 2, w // cell + 2

@@ -50,7 +50,12 @@ enum {
  * of 4 * ceil(W/2) bytes, so a packed frame is 4 * ceil(W/2) * H bytes; odd W and odd H are allowed.  The tracker sees exactly the RGB
  * of vt_convert_yuy2_rgb (BT.601 integer arithmetic of src/nv12_convert.rs:24-30,124-126 on the pixel's word); the overlays follow the
  * NV12 luma-plane semantics and write only the Y samples (byte 2x of row y), never the U / V bytes. */
-typedef enum { VT_FMT_NV12 = 0, VT_FMT_RGB24 = 1, VT_FMT_GRAY8 = 2, VT_FMT_YUY2 = 3 } vt_format;
+/* VT_FMT_RGBA / VT_FMT_BGRA: one plane of 32-bit pixels, bytes R G B A resp. B G R A (GStreamer RGBA / RGBx resp. BGRA / BGRx;
+ * DeepStream NVBUF_COLOR_FORMAT_RGBA resp. NVBUF_COLOR_FORMAT_BGRx), rows of 4W bytes, so a packed frame is 4 * W * H bytes; any W and H.
+ * The tracker sees exactly the RGB24 frame made of bytes 0, 1, 2 (RGBA) resp. 2, 1, 0 (BGRA) of every pixel; the overlays follow the
+ * RGB24 semantics and write each colour into its channel's byte.  Byte 3 (alpha or padding) is never read and never written.
+ * vt_overlay[_current] on such a handle needs a full frame (len >= 4 * W * H).  (Values 4 and 7 are not formats.) */
+typedef enum { VT_FMT_NV12 = 0, VT_FMT_RGB24 = 1, VT_FMT_GRAY8 = 2, VT_FMT_YUY2 = 3, VT_FMT_RGBA = 5, VT_FMT_BGRA = 6 } vt_format;
 /* BF16X3 (default): bf16 hi + lo operands, three products per K-step, scores within ~1e-5 of the fp32 oracle.  BF16 / FP16: single-pass
  * operands, 17 % faster, score error ~1e-3 / ~3e-4 — opt-in (near-tie arg-max flips are possible at that error). */
 typedef enum { VT_GEMM_FP32_SIMT = 0, VT_GEMM_TCGEN05_BF16X3 = 1, VT_GEMM_TCGEN05_BF16 = 2, VT_GEMM_TCGEN05_FP16 = 3 } vt_gemm_mode;
@@ -128,7 +133,7 @@ void vt_tracker_destroy(vt_tracker* t);
 
 /* ≙ VitTrack::init(&frame, bbox) (src/tracker_context.rs:88).  `frame` is host memory in the
  * handle's format, tightly packed (NV12: w*h*3/2 bytes, src/nv12_convert.rs:48; RGB24: h*w*3,
- * src/pipeline_ir.rs:142).  A short NV12 buffer is treated as an all-black image
+ * src/pipeline_ir.rs:142; RGBA / BGRA: h*w*4).  A short NV12 buffer is treated as an all-black image
  * (src/nv12_convert.rs:48-50). */
 vt_status vt_tracker_init(vt_tracker* t, int32_t target, const uint8_t* frame, size_t len, vt_bbox box);
 
@@ -179,14 +184,15 @@ vt_status vt_tracker_get_stream_geometry(const vt_tracker* t, int32_t target, vt
 vt_status vt_tracker_update_device(vt_tracker* t, uint8_t* d_frame, size_t len, vt_result* results);
 
 /* A frame in device memory on the handle's GPU, in the handle's format, with any row pitch (decoder surfaces: NVDEC, NvBufSurface).
- * NV12: planes[0] = Y (H rows), planes[1] = interleaved UV ((H+1)/2 rows); RGB24 / GRAY8 / YUY2: planes[0] only, planes[1] ignored.
- * pitch[i] >= the plane's row bytes (W for Y / UV / GRAY8, 3W for RGB24, 4 * ceil(W/2) for YUY2); planes may be separate allocations
+ * NV12: planes[0] = Y (H rows), planes[1] = interleaved UV ((H+1)/2 rows); RGB24 / GRAY8 / YUY2 / RGBA / BGRA: planes[0] only, planes[1]
+ * ignored.  pitch[i] >= the plane's row bytes (W for Y / UV / GRAY8, 3W for RGB24, 4 * ceil(W/2) for YUY2, 4W for RGBA / BGRA: a
+ * DeepStream NvBufSurface gives planes[0] = dataPtr + planeParams.offset[0], pitch[0] = planeParams.pitch[0]); planes may be separate allocations
  * and need no alignment.  A tightly packed frame d is the surface {d, d + W*H}, {W, W} (RGB24: {d, NULL}, {3W, 0}).
  *
  * The surface entry points below are additive (VT_ABI_VERSION stays 2): each behaves like the entry point it names, except that the
  * frame is a surface.  The tracker reads the surface in place (nothing is copied), and with cfg.box_overlay draws the box into it: into
- * planes[0] (the Y plane for NV12 / GRAY8, the Y samples for YUY2, the image for RGB24) with the reference's clamping, so nothing is
- * written into the pitch padding, the UV plane or the YUY2 chroma bytes.  The surface must stay valid until the call returns (submit: until the matching wait()).
+ * planes[0] (the Y plane for NV12 / GRAY8, the Y samples for YUY2, the image for RGB24, the colour bytes for RGBA / BGRA) with the
+ * reference's clamping, so nothing is written into the pitch padding, the UV plane, the YUY2 chroma bytes or byte 3 of a 32-bit pixel.  The surface must stay valid until the call returns (submit: until the matching wait()).
  * VT_ERR_INVALID (and vt_last_error()) for a NULL surface or plane, a pitch below the plane's row bytes, a plane that is not device or
  * managed memory of cfg.device, and — synchronous calls — frames in flight.  These four vt_tracker_*_surface calls are also
  * VT_ERR_INVALID on the tracker of a probe (HUD) handle, whose surfaces go through vt_probe_frame_surface / vt_probe_group_frame_surface. */
@@ -372,15 +378,15 @@ uint64_t vt_context_lost_frames(const vt_context* c);
 vt_tracker* vt_context_tracker(vt_context* c);
 
 /* ≙ the body of the pad-probe closure, src/pipeline.rs:67-184 (NV12) / src/pipeline_ir.rs:100-228
- * (RGB24, chosen by cfg.format): interval timing, process_frame, HUD + cursor/selection + box
+ * (RGB24 / RGBA / BGRA, chosen by cfg.format): interval timing, process_frame, HUD + cursor/selection + box
  * overlay written in place into `frame`.  Commands are delivered beforehand with
  * vt_context_handle_command (≙ draining cmd_rx, src/pipeline.rs:84-88).  hud_override (may be
  * NULL) replaces the timing-dependent HUD strings so that pixel parity is testable:
  * {fps_line, timing_line}. */
 vt_status vt_probe_frame(vt_context* c, uint8_t* frame, size_t len, const char* const* hud_override);
 /* ≙ vt_probe_frame on a pitched device surface of the context's geometry (vt_surface rules above): the probe's HUD, cursor / selection
- * and box are drawn in place into the surface's plane 0 (Y / RGB / the Y samples of YUY2), never into pitch padding, the UV plane or
- * YUY2 chroma bytes; nothing is copied between host and device but the result block.  A confirm frame initialises the tracker on this
+ * and box are drawn in place into the surface's plane 0 (Y / RGB / the Y samples of YUY2 / the colour bytes of RGBA / BGRA), never into
+ * pitch padding, the UV plane, YUY2 chroma bytes or byte 3 of a 32-bit pixel; nothing is copied between host and device but the result block.  A confirm frame initialises the tracker on this
  * surface.  VT_ERR_INVALID (and vt_last_error()) for a NULL surface, a surface that fails the vt_surface checks, or a probe-group member.
  * A context may take host frames on one call and surfaces on the next. */
 vt_status vt_probe_frame_surface(vt_context* c, const vt_surface* s, const char* const* hud_override);
@@ -395,7 +401,7 @@ vt_status vt_context_run_ring(vt_context* c, uint8_t* frames, size_t stride, siz
  * is member context i and target slot i.  Each stream behaves exactly like a single vt_context probing the same frames with the same
  * commands, but one group step runs ONE batched forward over the streams whose state machine calls VitTrack on that frame (TRACKING:
  * update; SELECT END with a pending confirm: init on that stream's frame, then update) and draws every stream's HUD, cursor / selection and
- * box in place — each with the HUD style of its format (luma: NV12 / GRAY8 / YUY2; RGB24) — with ONE synchronisation for the whole step.
+ * box in place — each with the HUD style of its format (luma: NV12 / GRAY8 / YUY2; RGB: RGB24 / RGBA / BGRA) — with ONE synchronisation for the whole step.
  * A stream that leaves TRACKING, or whose confirm fails the gate, gives up its slot (tracking resumes only through a fresh init).
  * Timing: the group keeps one TimingStats (on its tracker) and every stream is probed once per step, so every stream's FPS / conv / trk
  * HUD line shows the group's step figures. */
