@@ -431,13 +431,13 @@ __device__ __forceinline__ Tap lin_tap(int i, int s, int d, bool clamp_frac) {
 
 // Where the pixels of this frame live: the device frame inside the valid window (the part that was uploaded this frame), the
 // caller's pinned host frame (zero-copy loads over PCIe) outside of it.  With whole-frame uploads the window is the frame.  The device
-// frame may be a pitched surface (planes and pitches from the control block or the frame descriptor); the host frame is always packed,
-// and only exists beside a packed device frame of the same geometry (window uploads): it has the device frame's pitches and plane offset.
+// frame may be a pitched surface; the host frame has the device frame's pitches and plane offset (see FrameRef).
 struct PixelSrc {
     const uint8_t *dev, *dev_uv;  // device planes: Y / RGB / gray, NV12 chroma
     size_t pitch, uv_pitch;       // their row pitches
     const uint8_t* host;          // null: everything is on the device
-    int x0, y0, x1, y1;           // valid window of the device frame (even-aligned, so a pixel and its chroma pair sit on the same side)
+    int x0, y0, x1, y1;           // valid window of the device frame (even-aligned, so a pixel and its chroma pair sit on the same side;
+                                  // x1 >= x0, y1 >= y0)
     bool dev_words, host_words;   // YUY2 / RGBA / BGRA: the plane's words (pixel pairs, pixels) are 4-byte aligned (base and pitch), one
                                   // 32-bit load each
     int format;                   // vt_format of this target's frame
@@ -455,7 +455,7 @@ __device__ __forceinline__ uint32_t plane_word(const uint8_t* q, bool aligned) {
 __device__ __forceinline__ void frame_rgb(const PixelSrc& ps, int fx, int fy, int& r, int& g, int& b) {
     r = g = b = 0;
     if (fx < 0 || fy < 0 || fx >= ps.xlim || fy >= ps.ylim) return;
-    const bool host = ps.host && (fx < ps.x0 || fx >= ps.x1 || fy < ps.y0 || fy >= ps.y1);
+    const bool host = ps.host && ((unsigned)(fx - ps.x0) >= (unsigned)(ps.x1 - ps.x0) || (unsigned)(fy - ps.y0) >= (unsigned)(ps.y1 - ps.y0));
     const uint8_t* data = host ? ps.host : ps.dev;  // (same pitches: see PixelSrc)
     if (ps.format == VT_FMT_RGB24) {
         const uint8_t* p = data + (size_t)fy * ps.pitch + (size_t)fx * 3;
@@ -479,7 +479,8 @@ __device__ __forceinline__ void frame_rgb(const PixelSrc& ps, int fx, int fy, in
     }
 }
 
-__global__ void __launch_bounds__(256) crop_resize_norm_kernel(FrameDesc f, TargetState* __restrict__ state,
+// (minimum of 8 CTAs per SM stated: without it ptxas takes 40 registers, 6 CTAs of 256 per SM)
+__global__ void __launch_bounds__(256, 8) crop_resize_norm_kernel(FrameDesc f, TargetState* __restrict__ state,
                                                                const int32_t* __restrict__ slots, int factor, int S,
                                                                const float* __restrict__ lut, float* __restrict__ patches,
                                                                size_t patches_stride, __nv_bfloat16* __restrict__ p_hi,
@@ -487,33 +488,23 @@ __global__ void __launch_bounds__(256) crop_resize_norm_kernel(FrameDesc f, Targ
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");  // the template gather behind this kernel does not depend on it
     if (stamp && threadIdx.x == 0 && blockIdx.x == 0 && blockIdx.y == 0) *stamp = device_time_ns();
     const int bi = blockIdx.y;
-    PixelSrc ps{f.data, f.uv, f.pitch[0], f.pitch[1], nullptr, 0, 0, f.width, f.height, false, false, f.format, 0, 0};
-    if (f.ctl) {  // per-frame control block: frame planes, and which part of the device frame holds this frame's pixels
-        const bool own = bi < kMaxWin && f.ctl->frames[bi] != nullptr;  // stream group: this target has its own frame
-        if (own) {  // ... of its own format and size (one target per blockIdx.y: the format branch varies between CTAs, never within one)
-            const int4 g = *reinterpret_cast<const int4*>(f.ctl->geom[bi]);
-            f.format = g.x, f.width = g.y, f.height = g.z, f.valid = g.w;
-        }
-        ps.dev = own ? f.ctl->frames[bi] : f.ctl->frame;
-        ps.dev_uv = own ? f.ctl->uvs[bi] : f.ctl->uv;
-        ps.pitch = own ? f.ctl->pitches[bi][0] : f.ctl->pitch[0];
-        ps.uv_pitch = own ? f.ctl->pitches[bi][1] : f.ctl->pitch[1];
+    // this target's frame (one target per blockIdx.y: the format branch varies between CTAs, never within one), and with a control block
+    // which part of the device frame holds this frame's pixels
+    const FrameRef& fr = f.ctl ? target_frame(*f.ctl, bi) : f.frame;
+    const int4 g = *reinterpret_cast<const int4*>(fr.geom);
+    const int format = g.x, width = g.y, height = g.z, valid = g.w;
+    PixelSrc ps{fr.plane[0], fr.plane[1], fr.pitch[0], fr.pitch[1], nullptr, 0, 0, width, height, false, false, format, 0, 0};
+    if (f.ctl && f.ctl->n_win >= 0) {
         const int nw = f.ctl->n_win;
-        if (nw >= 0) {
-            ps.host = own ? f.ctl->host_frames[bi] : f.ctl->host_frame;
-            if (bi < nw) ps.x0 = f.ctl->win[bi][0], ps.y0 = f.ctl->win[bi][1], ps.x1 = f.ctl->win[bi][2], ps.y1 = f.ctl->win[bi][3];
-            else ps.x1 = ps.y1 = 0;  // nothing of this target was uploaded
-        }
+        ps.host = fr.host;
+        if (bi < nw) ps.x0 = f.ctl->win[bi][0], ps.y0 = f.ctl->win[bi][1], ps.x1 = f.ctl->win[bi][2], ps.y1 = f.ctl->win[bi][3];
+        else ps.x1 = ps.y1 = 0;  // nothing of this target was uploaded
     }
-    if (!ps.pitch) ps.pitch = fmt_row_bytes(f.format, f.width);  // packed frame
-    if (!ps.dev_uv) ps.dev_uv = ps.dev + (size_t)f.width * f.height;
-    if (!ps.uv_pitch) ps.uv_pitch = (size_t)f.width;
     ps.dev_words = ((reinterpret_cast<uintptr_t>(ps.dev) | ps.pitch) & 3) == 0;
     ps.host_words = (reinterpret_cast<uintptr_t>(ps.host) & 3) == 0;  // (packed YUY2 / RGBA / BGRA rows are whole words)
-    ps.format = f.format;
     // pad_plus1 (App. A.7, older OpenCV): a crop that reaches the right / bottom edge pads one pixel more, i.e. the last column / row of
     // the frame reads as border; a crop that stays inside never addresses it, so the bound can move unconditionally
-    ps.xlim = f.valid ? f.width - f.pad_plus1 : 0, ps.ylim = f.valid ? f.height - f.pad_plus1 : 0;
+    ps.xlim = valid ? width - f.pad_plus1 : 0, ps.ylim = valid ? height - f.pad_plus1 : 0;
     const int slot = slots[bi];
     TargetState* st = state + slot;
     const int bx = st->rect[0], by = st->rect[1], bw = st->rect[2], bh = st->rect[3];
@@ -523,7 +514,7 @@ __global__ void __launch_bounds__(256) crop_resize_norm_kernel(FrameDesc f, Targ
     if (bw > 0 && bh > 0) c = (int)ceil(__dmul_rn(sqrt((double)(int)area), (double)factor));
     const int x1 = bx + (bw - c) / 2, y1 = by + (bh - c) / 2;
     const int pl = max(0, -x1), pt = max(0, -y1);
-    const int pr = max(x1 + c - f.width + f.pad_plus1, 0), pb = max(y1 + c - f.height + f.pad_plus1, 0);
+    const int pr = max(x1 + c - width + f.pad_plus1, 0), pb = max(y1 + c - height + f.pad_plus1, 0);
     const bool outside = (c <= 0) || (c - pl - pr <= 0) || (c - pt - pb <= 0);
     if (threadIdx.x == 0 && blockIdx.x == 0 && factor == 4) st->crop_err = outside ? 1 : 0;
     if (outside) return;
@@ -934,7 +925,7 @@ cudaError_t launch_overlay(uint8_t* d_frame, size_t len, int width, int height, 
 // (probe: ≙ src/pipeline.rs:125-174 / src/pipeline_ir.rs:165-202), CTA 0: the list holds the commands of BOTH outcomes of the frame
 // and the kernel picks by the gate (status ok && success && score > gate, src/tracker_context.rs:93,122), takes the box geometry and
 // the score digits from the decode result — the host queued it before the frame's result existed, so the whole probe needs ONE
-// synchronisation.  (c) With a pinned caller frame (ctl->host_frame) the touched pixels are also written straight into the host frame
+// synchronisation.  (c) With a pinned caller frame (FrameRef::host) the touched pixels are also written straight into the host frame
 // (zero-copy stores over PCIe; the dimmed background is copied out of the device frame), so no device->host row copy and no second
 // synchronisation is needed to hand the overlaid frame back.  (d) The result block is published into the pinned host block.
 __device__ void hud_score_glyphs(OverlayCmdDev& c, float score) {  // "score: " + "{:.0}%" of score*100 (src/pipeline.rs:146-156)
@@ -994,45 +985,41 @@ __device__ __forceinline__ uint32_t dim4(uint32_t v, unsigned factor, int step) 
 // stream took part in the forward.  (Two instances of one body rather than one kernel with a runtime switch: the per-stream addressing
 // stays out of the single probe's last kernel, whose size and register use are what they were.)
 template <bool kGroup>
-__device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int fmt, const DeviceResult* __restrict__ res,
-                                                 const int32_t* __restrict__ slots, int n, float gate, const FrameCtl* ctl,
-                                                 unsigned long long* stamp_end, const uint32_t* __restrict__ blk, int blk_words, int draw_box,
-                                                 OverlayCmdDev* s_cmd) {
+__device__ __forceinline__ void box_overlay_body(const DeviceResult* __restrict__ res, const int32_t* __restrict__ slots, int n, float gate,
+                                                 const FrameCtl* ctl, unsigned long long* stamp_end, const uint32_t* __restrict__ blk,
+                                                 int blk_words, int draw_box, OverlayCmdDev* s_cmd) {
     // the control block was written at the start of the frame (complete long before the kernel ahead of this one): every thread fetches
     // what it needs in one batch, and the HUD list comes out of pinned host memory, BEFORE the dependency wait: only the decode result
     // waits for the preceding kernel
     const ProbeStreamCtl* const e = kGroup ? &reinterpret_cast<const ProbeGroupCtl*>(ctl)->s[blockIdx.x] : nullptr;
-    // stream group: block i draws into stream i's frame; probe group: pair x into stream x's
-    const bool own = kGroup || (blockIdx.x < (unsigned)kMaxWin && ctl->frames[blockIdx.x] != nullptr);
-    if (own) {  // ... with stream i's format and size: nothing is written outside its plane 0
-        const int4 g = *reinterpret_cast<const int4*>(kGroup ? e->geom : ctl->geom[blockIdx.x]);
-        fmt = g.x, W = g.y, H = g.z, len = fmt_frame_bytes(fmt, W, H);
-    }
+    // the frame this CTA draws into — block i: target i's (stream group: stream i's own frame); probe group: pair x, stream x's — with its
+    // format and size (nothing is written outside its plane 0), and its HUD list and background-dim flags: the frame's (CTA 0), or its
+    // stream's (probe group)
+    const FrameRef* const fr = kGroup ? &e->frame : &target_frame(*ctl, blockIdx.x);
+    const HudCtl* const hud = kGroup ? &e->hud : &ctl->hud;
+    const int4 g = *reinterpret_cast<const int4*>(fr->geom);
+    const int fmt = g.x, W = g.y, H = g.z;
     // HUD mode runs two CTAs per target (gridDim.y = 2): y = 0 draws on the device frame (and publishes), y = 1 on the pinned host frame —
     // the two passes over the command list (~8 us each on one CTA) run side by side
     const bool split = gridDim.y > 1;
-    uint8_t* const frame0 = kGroup ? e->frame : const_cast<uint8_t*>(own ? ctl->frames[blockIdx.x] : ctl->frame);
-    uint8_t* const host0 = kGroup ? e->host_frame : own ? ctl->host_frames[blockIdx.x] : ctl->host_frame;
-    if (split && blockIdx.y == 1 && !host0) return;       // nothing to mirror into
-    uint8_t* const frame = frame0;
-    uint8_t* const host = host0;
-    // row pitch of the drawn plane: the caller's surface pitch for the device frame; the pinned host frame is packed.  A host frame only
-    // ever goes with a packed device frame (the handle's own buffer, fpitch == row): a surface step has no host frame, so no host-pass CTA
-    // and no bg_ready handshake (host == nullptr above and below).  The background dim therefore addresses both frames by fpitch.
+    uint8_t* const frame = const_cast<uint8_t*>(fr->plane[0]);
+    uint8_t* const host = fr->host;
+    if (split && blockIdx.y == 1 && !host) return;  // nothing to mirror into
+    // row pitch of the drawn plane: the caller's surface pitch for the device frame; the pinned host frame is packed, and only ever goes
+    // with a packed device frame (fpitch == row, see FrameRef): a surface step has no host frame, so no host-pass CTA and no bg_ready
+    // handshake (host == nullptr above and below).  The background dim therefore addresses both frames by fpitch.
     // fmt is the frame's format: drawn with the overlay semantics of ofmt
     const size_t row = fmt_row_bytes(fmt, W);
     const int ofmt = overlay_format(fmt), step = fmt_px_step(fmt);
-    const size_t fpitch0 = kGroup ? e->pitch : own ? ctl->pitches[blockIdx.x][0] : ctl->pitch[0];
-    const size_t fpitch = fpitch0 ? fpitch0 : row;
-    const size_t plen = fpitch0 ? (size_t)(H - 1) * fpitch + row : len;  // bytes from the plane's first row to the end of its last
+    const size_t fpitch = fr->pitch[0];
+    const size_t plen = (size_t)(H - 1) * fpitch + row;  // bytes from the plane's first row to the end of its last
     const bool do_dev = !split || blockIdx.y == 0, do_host = host != nullptr && (!split || blockIdx.y == 1);
-    // this CTA's HUD list and background-dim flags: the frame's (CTA 0), or its stream's (probe group)
-    const int32_t* const bg_on_dev = kGroup ? &e->bg_on_device : &ctl->bg_on_device;
-    const int32_t* const bg_ready = kGroup ? &e->bg_ready : &ctl->bg_ready;
-    int n_hud = kGroup ? e->n_hud : blockIdx.x == 0 ? ctl->n_hud : 0;
+    const int32_t* const bg_on_dev = &hud->bg_on_device;
+    const int32_t* const bg_ready = &hud->bg_ready;
+    int n_hud = kGroup || blockIdx.x == 0 ? hud->n : 0;
     if (n_hud > kMaxCmds) n_hud = kMaxCmds;
     if (n_hud > 0) {
-        const uint32_t* src = reinterpret_cast<const uint32_t*>(kGroup ? e->hud : ctl->hud);
+        const uint32_t* src = reinterpret_cast<const uint32_t*>(hud->list);
         uint32_t* dst = reinterpret_cast<uint32_t*>(s_cmd);
         for (int i = threadIdx.x; i < n_hud * (int)(sizeof(OverlayCmdDev) / 4); i += blockDim.x) dst[i] = src[i];
         __syncthreads();
@@ -1107,7 +1094,7 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
             if (!dst) break;
             if ((p == 0 && !do_dev) || (p == 1 && !do_host)) continue;
             const size_t pitch = p == 0 ? fpitch : row;
-            const Surface s = make_surface(dst, pitch * H, W, H, fmt, pitch);
+            const Surface s = make_surface(dst, plen, W, H, fmt, pitch);
             if (ofmt == VT_FMT_NV12) {
                 ov_rect_nv12(s, x, y, w, h, 3, 255);
                 __syncthreads();
@@ -1193,7 +1180,7 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
             if (!dst) break;
             if ((p == 0 && !do_dev) || (p == 1 && !do_host)) continue;
             const size_t pitch = p == 0 ? fpitch : row;
-            const Surface s = make_surface(dst, pitch * H, W, H, fmt, pitch);
+            const Surface s = make_surface(dst, plen, W, H, fmt, pitch);
             for (int i = first; i < n_hud; ++i) {
                 const OverlayCmdDev& c = s_cmd[i];
                 if (c.kind < 0) continue;
@@ -1203,7 +1190,7 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
                     const BgRegion g = bg_region(c, W, H, row, step);
                     for (long long j = threadIdx.x; j < (g.y1 - g.y0) * (g.x1 - g.x0); j += blockDim.x) {
                         const size_t o = (size_t)(g.y0 + j / (g.x1 - g.x0)) * row + (size_t)(g.x0 + j % (g.x1 - g.x0)) * step;
-                        if (o < len) host[o] = frame[o];
+                        if (o < plen) host[o] = frame[o];
                     }
                 } else {
                     ov_dispatch(s, c);
@@ -1224,12 +1211,11 @@ __device__ __forceinline__ void box_overlay_body(size_t len, int W, int H, int f
     }
 }
 
-__global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(size_t len, int W, int H, int fmt, const DeviceResult* __restrict__ res,
-                                                                 const int32_t* __restrict__ slots, int n, float gate, const FrameCtl* ctl,
-                                                                 unsigned long long* stamp_end, const uint32_t* __restrict__ blk, int blk_words,
-                                                                 int draw_box) {
+__global__ void __launch_bounds__(kOvThreads) box_overlay_kernel(const DeviceResult* __restrict__ res, const int32_t* __restrict__ slots, int n,
+                                                                 float gate, const FrameCtl* ctl, unsigned long long* stamp_end,
+                                                                 const uint32_t* __restrict__ blk, int blk_words, int draw_box) {
     __shared__ OverlayCmdDev s_cmd[kMaxCmds];
-    box_overlay_body<false>(len, W, H, fmt, res, slots, n, gate, ctl, stamp_end, blk, blk_words, draw_box, s_cmd);
+    box_overlay_body<false>(res, slots, n, gate, ctl, stamp_end, blk, blk_words, draw_box, s_cmd);
 }
 
 // (minimum of one CTA per SM stated: without it ptxas holds this instance to 64 registers and spills the background-dim prefetch; the grid
@@ -1238,7 +1224,7 @@ __global__ void __launch_bounds__(kOvThreads, 1) probe_group_overlay_kernel(cons
                                                                          unsigned long long* stamp_end, const uint32_t* __restrict__ blk,
                                                                          int blk_words) {
     __shared__ OverlayCmdDev s_cmd[kMaxCmds];
-    box_overlay_body<true>(0, 0, 0, 0, res, nullptr, 0, gate, &ctl->f, stamp_end, blk, blk_words, 0, s_cmd);
+    box_overlay_body<true>(res, nullptr, 0, gate, &ctl->f, stamp_end, blk, blk_words, 0, s_cmd);
 }
 
 cudaError_t launch_group_overlay(int n_streams, const DeviceResult* d_res, float gate, const ProbeGroupCtl* d_ctl, unsigned long long* stamp_end,
@@ -1247,12 +1233,11 @@ cudaError_t launch_group_overlay(int n_streams, const DeviceResult* d_res, float
                      (const uint32_t*)d_blk, (int)(blk_bytes / 4));
 }
 
-cudaError_t launch_box_overlay(size_t len, int width, int height, int format, const DeviceResult* d_res, const int32_t* d_slots, int n,
-                               float gate, const FrameCtl* d_ctl, unsigned long long* stamp_end, cudaStream_t s, bool pdl, const void* d_blk,
-                               size_t blk_bytes, int draw_box) {
+cudaError_t launch_box_overlay(const DeviceResult* d_res, const int32_t* d_slots, int n, float gate, const FrameCtl* d_ctl,
+                               unsigned long long* stamp_end, cudaStream_t s, bool pdl, const void* d_blk, size_t blk_bytes, int draw_box) {
     const bool split = (draw_box >> 16) != 0;  // HUD mode: device pass and host pass in two CTAs
-    return launch_ex(box_overlay_kernel, dim3(n > 0 ? n : 1, split ? 2 : 1), dim3(kOvThreads), 0, s, pdl, 1, len, width, height, format, d_res, d_slots, n,
-                     gate, d_ctl, stamp_end, (const uint32_t*)d_blk, (int)(blk_bytes / 4), draw_box & 0xffff);
+    return launch_ex(box_overlay_kernel, dim3(n > 0 ? n : 1, split ? 2 : 1), dim3(kOvThreads), 0, s, pdl, 1, d_res, d_slots, n, gate, d_ctl,
+                     stamp_end, (const uint32_t*)d_blk, (int)(blk_bytes / 4), draw_box & 0xffff);
 }
 
 // per-frame, outside the graph: submit stamp + the control block (addresses and parameters that change from frame to frame)

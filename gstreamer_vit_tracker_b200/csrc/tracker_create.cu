@@ -363,7 +363,8 @@ vt_status vt_tracker_create(const vt_config* cfg_in, vt_tracker** out) {
     {
         FrameCtl ctl;
         memset(&ctl, 0, sizeof(ctl));
-        ctl.frame = t->d_frame, ctl.n_win = -1;
+        ctl.frames[0] = packed_ref(cfg_geom(t), t->d_frame, nullptr, true);
+        ctl.n_frames = 1, ctl.n_win = -1;
         VT_TRY(cudaMalloc(&t->d_ctl, sizeof(FrameCtl)));
         VT_TRY(cudaMemcpy(t->d_ctl, &ctl, sizeof(ctl), cudaMemcpyHostToDevice));
     }

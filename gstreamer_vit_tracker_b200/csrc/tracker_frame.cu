@@ -45,7 +45,7 @@ static GemmArgs gemm_args(const float* A, int64_t lda, const float* W, const flo
 }
 
 // The kernel forms of one forward, a function of the handle, n and spread (latency mode: few live handles on the GPU, run_forward):
-// the graph key (n, frame_valid, spread) determines them.
+// the graph key (n, spread) determines them.
 constexpr int kAttSimt = -1;  // ForwardForms::att: launch_attention (else a VT_ATT_* form of tc_attention_launch)
 struct ForwardForms {
     int patch_slices = 0;      // patch-embed K-slices summed by reduce_ln: 0 (unsplit), 4, or 2 (merged, from kUnchainTargets targets)
@@ -116,7 +116,7 @@ static ForwardForms forward_forms(const vt_tracker* t, int n, bool spread) {
 static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const ForwardForms& f) {
     const int D = t->D, Hd = t->hidden, C = t->head_ch;
     cudaStream_t s = t->stream;
-    FrameDesc fd{t->d_frame, nullptr, {0, 0}, t->W, t->H, t->fmt, t->frame_valid, t->d_ctl, t->cfg.pad_plus1};  // planes from d_ctl
+    const FrameDesc fd{FrameRef{}, t->d_ctl, t->cfg.pad_plus1};  // the frames from d_ctl
     auto LO = [&](__nv_bfloat16* p) { return t->f16 ? nullptr : p; };  // fp16 mode: "hi only" (see vt_internal.h: operand_bits)
     VT_LAUNCH(launch_crop_resize_norm(fd, t->d_state, t->d_slots, n, 4, kSearch, t->d_lut, t->patches_x, (size_t)kNTx * kPatchK, t->px_hi,
                                       LO(t->px_lo), s, t->d_stamps + ST_PRE));
@@ -245,8 +245,8 @@ static vt_status enqueue_forward(vt_tracker* t, int n, int& launches, const Forw
         VT_LAUNCH(launch_group_overlay(t->group_n, t->d_res, t->cfg.overlay_gate, reinterpret_cast<const ProbeGroupCtl*>(t->d_ctl),
                                        t->d_stamps + ST_OVL_END, s, f.pdl, t->d_res, t->res_block_bytes));
     else if (t->cfg.box_overlay || t->hud_mode)  // box overlay and / or the frame's HUD list, pinned-frame mirror, ... and publishes the result block
-        VT_LAUNCH(launch_box_overlay(t->frame_bytes, t->W, t->H, t->fmt, t->d_res, t->d_slots, n, t->cfg.overlay_gate, t->d_ctl,
-                                     t->d_stamps + ST_OVL_END, s, f.pdl, t->d_res, t->res_block_bytes, t->cfg.box_overlay | (t->hud_mode ? 1 << 16 : 0)));
+        VT_LAUNCH(launch_box_overlay(t->d_res, t->d_slots, n, t->cfg.overlay_gate, t->d_ctl, t->d_stamps + ST_OVL_END, s, f.pdl, t->d_res,
+                                     t->res_block_bytes, t->cfg.box_overlay | (t->hud_mode ? 1 << 16 : 0)));
     else  // results, stage stamps and the error flag -> the pinned host block of this frame's queue slot
         VT_LAUNCH(launch_publish(t->d_res, t->d_ctl, t->res_block_bytes, s, f.pdl));
     return VT_OK;
@@ -265,7 +265,7 @@ static vt_status run_forward(vt_tracker* t) {
         t->kernels_per_frame = launches;
         return st;
     }
-    const int key = (n * 2 + (t->frame_valid ? 1 : 0)) * 2 + (spread ? 1 : 0);  // frame_valid is a kernel parameter baked into the graph
+    const int key = n * 2 + (spread ? 1 : 0);
     auto it = t->graphs.find(key);
     if (it == t->graphs.end()) {
         cudaGraph_t graph = nullptr;
@@ -391,8 +391,7 @@ static vt_status do_upload(vt_tracker* t, const StreamGeom& g, const uint8_t* fr
     if (!stream) stream = t->stream;
     const size_t frame_bytes = g.bytes();
     size_t n = std::min(len, frame_bytes);
-    t->frame_valid = len >= fmt_valid_bytes(g.fmt, g.W, g.H);
-    if (!t->frame_valid && g.fmt == VT_FMT_NV12) n = 0;  // src/nv12_convert.rs:48-50 -> black image
+    if (len < fmt_valid_bytes(g.fmt, g.W, g.H) && g.fmt == VT_FMT_NV12) n = 0;  // src/nv12_convert.rs:48-50 -> black image
     if (n == 0) return VT_OK;
     const cudaMemcpyKind kind = device_src ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
     if (!p.whole) {
@@ -532,13 +531,17 @@ static inline double now_us() {
     return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
 
-// A full-length packed device frame d as a surface: {d, d + W * H}, {W, W} (RGB24 / GRAY8: one plane)
-static vt_surface packed_surface(const StreamGeom& g, const uint8_t* d) {
+// The two constructors of a FrameRef.  A packed frame of geometry g at `base` (NV12: the chroma plane right behind the Y plane), beside
+// the caller's pinned host frame `host` (or null); valid = false: the buffer was short, the crop reads a black image.
+FrameRef packed_ref(const StreamGeom& g, const uint8_t* base, uint8_t* host, bool valid) {
     const bool nv12 = g.fmt == VT_FMT_NV12;
-    vt_surface s;
-    s.planes[0] = const_cast<uint8_t*>(d), s.planes[1] = nv12 ? const_cast<uint8_t*>(d) + (size_t)g.W * g.H : nullptr;
-    s.pitch[0] = fmt_row_bytes(g.fmt, g.W), s.pitch[1] = nv12 ? (size_t)g.W : 0;
-    return s;
+    return FrameRef{{base, nv12 ? base + (size_t)g.W * g.H : nullptr}, {fmt_row_bytes(g.fmt, g.W), nv12 ? (size_t)g.W : 0}, host,
+                    {g.fmt, g.W, g.H, valid ? 1 : 0}};
+}
+// the caller's surface s (checked by check_surface), read and drawn into in place
+static FrameRef surface_ref(const StreamGeom& g, const vt_surface& s) {
+    const bool nv12 = g.fmt == VT_FMT_NV12;
+    return FrameRef{{s.planes[0], nv12 ? s.planes[1] : nullptr}, {s.pitch[0], nv12 ? s.pitch[1] : 0}, nullptr, {g.fmt, g.W, g.H, 1}};
 }
 
 // The caller's surface (include/vt_tracker.h: vt_surface): every plane of the format present, a pitch that holds a row, and device (or
@@ -580,6 +583,15 @@ static vt_status surface_call(vt_tracker* t, const char* where, bool sync) {
     return VT_OK;
 }
 
+// The end of every submit: the queue slot's completion event, the result block's device -> host bytes, one more frame in flight
+static vt_status finish_submit(vt_tracker* t, int slot) {
+    VT_CUDA(cudaEventRecord(t->q_done[slot], t->stream));
+    t->d2h_bytes += t->res_block_bytes;
+    ++t->q_count;
+    t->in_flight = true;
+    return VT_OK;
+}
+
 // surf: a pitched device surface tracked in place (frame / d_src unused)
 static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_src, size_t len, bool forward = true, const vt_surface* surf = nullptr) {
     if (t->q_count >= vt_tracker::kQueue) {
@@ -603,45 +615,40 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
     q.hud_bytes = n_hud ? t->hud_next_bytes[0] : 0;
     q.mirrored = host_frame && (t->cfg.box_overlay || n_hud > 0);
     // device-resident frame: track (and draw the box) straight in the caller's device memory — no device->device copy.  A full-length
-    // packed device frame is a surface like any other.
-    vt_surface packed;
-    if (!surf && d_src && len >= t->frame_bytes) packed = packed_surface(cfg_geom(t), d_src), surf = &packed;
-    const bool in_place = surf != nullptr;
+    // packed device frame is tracked in place like a surface.
+    const StreamGeom g = cfg_geom(t);
+    const bool in_place = surf || (d_src && len >= t->frame_bytes);
     if (!in_place) t->d_frame = t->d_frames[slot];  // the slot's own frame buffer: the other one may still be read by the frame in flight
     const bool lagging = t->q_count > 0;  // a frame is in flight: rect_mirror is one frame old, the windows are predictions
     UploadPlan plan;
     if (!in_place && !d_src) plan_upload(t, len, host_frame != nullptr, lagging, n_hud ? t->hud_next_rmw[0] : nullptr, plan);
     if (!in_place && !d_src && lagging) {
         // pipelined host frame: upload on the copy stream while the frame in flight computes; the main stream picks it up through an event
-        vt_status st = do_upload(t, cfg_geom(t), frame, len, plan, false, t->copy_stream);
+        vt_status st = do_upload(t, g, frame, len, plan, false, t->copy_stream);
         if (st != VT_OK) return st;
         VT_CUDA(cudaEventRecord(t->ev_up[slot], t->copy_stream));
         VT_CUDA(cudaStreamWaitEvent(t->stream, t->ev_up[slot], 0));
     }
     FrameCtl ctl;
     memset(&ctl, 0, sizeof(ctl));
-    ctl.frame = in_place ? surf->planes[0] : t->d_frame, ctl.host_frame = host_frame, ctl.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
-    if (in_place) {
-        const bool nv12 = t->fmt == VT_FMT_NV12;
-        ctl.uv = nv12 ? surf->planes[1] : nullptr, ctl.pitch[0] = surf->pitch[0], ctl.pitch[1] = nv12 ? surf->pitch[1] : 0;
-    }
-    ctl.hud = n_hud ? t->h_hud[slot] : nullptr, ctl.n_hud = n_hud;
+    ctl.frames[0] = surf ? surface_ref(g, *surf) : packed_ref(g, in_place ? d_src : t->d_frame, host_frame, len >= fmt_valid_bytes(g.fmt, g.W, g.H));
+    ctl.n_frames = 1, ctl.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
+    ctl.hud.list = n_hud ? t->h_hud[slot] : nullptr, ctl.hud.n = n_hud;
     const bool hud_inline = n_hud > 0 && n_hud <= kHudInline && t->d_hud[slot] != nullptr;
-    if (hud_inline) ctl.hud = t->d_hud[slot];
+    if (hud_inline) ctl.hud.list = t->d_hud[slot];
     ctl.n_win = plan.whole ? -1 : plan.n_win;
     if (!plan.whole) memcpy(ctl.win, plan.win, sizeof(ctl.win));
-    ctl.bg_on_device = (n_hud && (in_place || d_src || plan.whole || plan.has_rmw)) ? 1 : 0;  // the dimmed region is in the device frame
+    ctl.hud.bg_on_device = (n_hud && (in_place || d_src || plan.whole || plan.has_rmw)) ? 1 : 0;  // the dimmed region is in the device frame
     t->hud_next_n[0] = 0;
     VT_CUDA(launch_stamp(t->d_stamps + ST_SUBMIT, t->d_ctl, ctl, t->stream, hud_inline ? t->h_hud[slot] : nullptr, n_hud, t->d_hud[slot]));
     ++t->kernel_launches;
     if (in_place) {
-        t->frame_valid = 1;
         t->d_frame_is_last_host_frame = false;  // tracked in the caller's device memory: the internal buffer holds an older frame
     } else if (d_src) {  // short device frame: device->device copy of what there is (NV12: black frame, src/nv12_convert.rs:48-50)
-        vt_status st = do_upload(t, cfg_geom(t), d_src, len, plan, true, nullptr);
+        vt_status st = do_upload(t, g, d_src, len, plan, true, nullptr);
         if (st != VT_OK) return st;
     } else if (!lagging) {
-        vt_status st = do_upload(t, cfg_geom(t), frame, len, plan, false, nullptr);  // the host mirror of rect_last is exact: the search windows suffice
+        vt_status st = do_upload(t, g, frame, len, plan, false, nullptr);  // the host mirror of rect_last is exact: the search windows suffice
         if (st != VT_OK) return st;
     }
     const double hp1 = t->sw.hostprof ? now_us() : 0;
@@ -650,8 +657,8 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
         vt_status st = run_forward(t);
         if (st != VT_OK) return st;
     } else if (n_hud > 0) {  // no tracker runs on this frame (SELECT / LOST states of the probe): HUD list + publish only
-        cudaError_t e = launch_box_overlay(t->frame_bytes, t->W, t->H, t->fmt, t->d_res, t->d_slots, 0, t->cfg.overlay_gate, t->d_ctl,
-                                           t->d_stamps + ST_OVL_END, t->stream, false, t->d_res, t->res_block_bytes, 0);
+        cudaError_t e = launch_box_overlay(t->d_res, t->d_slots, 0, t->cfg.overlay_gate, t->d_ctl, t->d_stamps + ST_OVL_END, t->stream, false,
+                                           t->d_res, t->res_block_bytes, 0);
         if (e != cudaSuccess) {
             set_error("overlay launch failed: %s", cudaGetErrorString(e));
             return VT_ERR_CUDA;
@@ -661,11 +668,45 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
     const double hp2 = t->sw.hostprof ? now_us() : 0;
     // the result block reaches t->h_blk[slot] through the last kernel of the frame; nothing ran: copy it
     if (!ran && n_hud == 0) VT_CUDA(cudaMemcpyAsync(t->h_blk[slot], t->d_res, t->res_block_bytes, cudaMemcpyDeviceToHost, t->stream));
-    VT_CUDA(cudaEventRecord(t->q_done[slot], t->stream));
-    t->d2h_bytes += t->res_block_bytes;
-    if (t->sw.hostprof) t->hp[0] += hp1 - hp0, t->hp[1] += hp2 - hp1, t->hp[2] += now_us() - hp2;
-    ++t->q_count;
-    t->in_flight = true;
+    const vt_status st = finish_submit(t, slot);
+    if (st == VT_OK && t->sw.hostprof) t->hp[0] += hp1 - hp0, t->hp[1] += hp2 - hp1, t->hp[2] += now_us() - hp2;
+    return st;
+}
+
+// Stream i's device frame d_sframes[i] holds a frame of `bytes` (+ 256), grown only between synchronous group steps: nothing in flight
+// reads the old buffer
+static vt_status ensure_stream_frame(vt_tracker* t, int i, size_t bytes) {
+    if (t->d_sframe_bytes[i] >= bytes + 256) return VT_OK;
+    if (t->d_sframes[i]) VT_CUDA(cudaFree(t->d_sframes[i]));
+    t->d_sframes[i] = nullptr, t->d_sframe_bytes[i] = 0;
+    VT_CUDA(cudaMalloc(&t->d_sframes[i], bytes + 256));
+    VT_CUDA(cudaMemsetAsync(t->d_sframes[i], 0, bytes + 256, t->stream));
+    t->d_sframe_bytes[i] = bytes + 256;
+    return VT_OK;
+}
+
+// One stream of a group step that takes part in the forward: its full pinned host frame `frame`, of target slot `slot`'s geometry, goes
+// into the device frame d_sframes[buf] — whole (and *whole = true), or with cfg.upload_window only the search window around the slot's
+// rect_last.  win: the uploaded window (empty: the window misses the frame, the crop kernel flags it); *ref: the stream's frame.
+static vt_status stage_stream(vt_tracker* t, int buf, int slot, uint8_t* frame, int* win, FrameRef* ref, bool* whole) {
+    const StreamGeom& g = slot_geom(t, slot);
+    vt_status st = ensure_stream_frame(t, buf, g.bytes());
+    if (st != VT_OK) return st;
+    uint8_t* dst = t->d_sframes[buf];
+    const bool all = !t->cfg.upload_window || !windows_allowed(g);
+    if (all) {
+        VT_CUDA(cudaMemcpyAsync(dst, frame, g.bytes(), cudaMemcpyHostToDevice, t->stream));
+        t->h2d_bytes += g.bytes();
+        win[0] = win[1] = 0, win[2] = g.W, win[3] = g.H;
+    } else if (search_window(g, t->rect_mirror[slot], 0, win[0], win[1], win[2], win[3])) {
+        st = copy_window(g, dst, frame, win, true, cudaMemcpyHostToDevice, t->stream);
+        if (st != VT_OK) return st;
+        t->h2d_bytes += window_bytes(g, win);
+    } else {
+        win[0] = win[1] = win[2] = win[3] = 0;
+    }
+    *ref = packed_ref(g, dst, frame, true);
+    if (whole) *whole = all;
     return VT_OK;
 }
 
@@ -673,7 +714,7 @@ static vt_status submit_common(vt_tracker* t, uint8_t* frame, const uint8_t* d_s
 // stepped together through ONE batched forward (M = 320 n rows: from 1024 rows on the GEMMs run in their throughput forms).  frames[i] is
 // the pinned host frame of the i-th active target; each target's search window is uploaded into that target's own device frame and the
 // box overlay is mirrored into that target's host frame.  Or surfs[i] (frames / lens unused) is the i-th target's device surface, read
-// and drawn into in place.  Stream i's geometry travels in the control block (ctl.geom[i]), so one captured graph per stream count
+// and drawn into in place.  Stream i's geometry travels in the control block (ctl.frames[i]), so one captured graph per stream count
 // serves any mix of sizes and formats.  Synchronous (rect_mirror is exact: the windows are the real search windows).
 static vt_status submit_streams(vt_tracker* t, uint8_t* const* frames, const size_t* lens, const vt_surface* surfs, int n) {
     const char* where = surfs ? "vt_tracker_update_streams_surface" : "vt_tracker_update_streams";
@@ -703,51 +744,21 @@ static vt_status submit_streams(vt_tracker* t, uint8_t* const* frames, const siz
     FrameCtl ctl;
     memset(&ctl, 0, sizeof(ctl));
     for (int i = 0; i < n; ++i) {
-        const StreamGeom& g = slot_geom(t, t->active[i]);
-        ctl.geom[i][0] = g.fmt, ctl.geom[i][1] = g.W, ctl.geom[i][2] = g.H, ctl.geom[i][3] = 1;
         if (surfs) {  // in place: nothing to upload, the whole surface holds the frame
-            const bool nv12 = g.fmt == VT_FMT_NV12;
-            ctl.frames[i] = surfs[i].planes[0], ctl.uvs[i] = nv12 ? surfs[i].planes[1] : nullptr;
-            ctl.pitches[i][0] = surfs[i].pitch[0], ctl.pitches[i][1] = nv12 ? surfs[i].pitch[1] : 0;
+            ctl.frames[i] = surface_ref(slot_geom(t, t->active[i]), surfs[i]);
             continue;
         }
-        const size_t fb = g.bytes();
-        if (t->d_sframe_bytes[i] < fb + 256) {  // (synchronous groups: nothing in flight reads the old buffer)
-            if (t->d_sframes[i]) VT_CUDA(cudaFree(t->d_sframes[i]));
-            t->d_sframes[i] = nullptr, t->d_sframe_bytes[i] = 0;
-            VT_CUDA(cudaMalloc(&t->d_sframes[i], fb + 256));
-            VT_CUDA(cudaMemsetAsync(t->d_sframes[i], 0, fb + 256, t->stream));
-            t->d_sframe_bytes[i] = fb + 256;
-        }
-        uint8_t* dst = t->d_sframes[i];
-        const uint8_t* src = frames[i];
-        int* w = ctl.win[i];
-        if (!t->cfg.upload_window || !windows_allowed(g)) {
-            VT_CUDA(cudaMemcpyAsync(dst, src, fb, cudaMemcpyHostToDevice, t->stream));
-            t->h2d_bytes += fb;
-            w[0] = w[1] = 0, w[2] = g.W, w[3] = g.H;
-        } else if (search_window(g, t->rect_mirror[t->active[i]], 0, w[0], w[1], w[2], w[3])) {
-            vt_status st = copy_window(g, dst, src, w, true, cudaMemcpyHostToDevice, t->stream);
-            if (st != VT_OK) return st;
-            t->h2d_bytes += window_bytes(g, w);
-        } else {
-            w[0] = w[1] = w[2] = w[3] = 0;  // the window misses the frame: the crop kernel flags it
-        }
-        ctl.frames[i] = dst, ctl.host_frames[i] = frames[i];
+        vt_status st = stage_stream(t, i, t->active[i], frames[i], ctl.win[i], &ctl.frames[i], nullptr);
+        if (st != VT_OK) return st;
     }
-    ctl.frame = ctl.frames[0], ctl.uv = ctl.uvs[0], ctl.pitch[0] = ctl.pitches[0][0], ctl.pitch[1] = ctl.pitches[0][1];
-    ctl.host_frame = ctl.host_frames[0], ctl.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
+    ctl.n_frames = n, ctl.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
     ctl.n_win = surfs ? -1 : n;
-    t->frame_valid = 1, t->d_frame_is_last_host_frame = false;
+    t->d_frame_is_last_host_frame = false;
     VT_CUDA(launch_stamp(t->d_stamps + ST_SUBMIT, t->d_ctl, ctl, t->stream));
     ++t->kernel_launches;
     vt_status st = run_forward(t);
     if (st != VT_OK) return st;
-    VT_CUDA(cudaEventRecord(t->q_done[slot], t->stream));
-    t->d2h_bytes += t->res_block_bytes;
-    ++t->q_count;
-    t->in_flight = true;
-    return VT_OK;
+    return finish_submit(t, slot);
 }
 
 static vt_status wait_common(vt_tracker* t, vt_result* results) {
@@ -967,7 +978,8 @@ static vt_status init_from_host(vt_tracker* t, int32_t target, const uint8_t* fr
     if (st != VT_OK) return st;
     st = do_upload(t, g, frame, len, UploadPlan(), false, nullptr);  // the whole frame
     if (st != VT_OK) return st;
-    return init_template(t, target, box, FrameDesc{t->d_frame, nullptr, {0, 0}, g.W, g.H, g.fmt, t->frame_valid, nullptr, t->cfg.pad_plus1});
+    const bool valid = len >= fmt_valid_bytes(g.fmt, g.W, g.H);
+    return init_template(t, target, box, FrameDesc{packed_ref(g, t->d_frame, nullptr, valid), nullptr, t->cfg.pad_plus1});
 }
 
 // The tracker of a probe group steps its streams through vt_probe_group_frame only: every public frame entry point refuses it.
@@ -1000,9 +1012,7 @@ vt_status tracker_init_surface(vt_tracker* t, int32_t target, const vt_surface* 
     const StreamGeom& g = slot_geom(t, target);
     if (st == VT_OK) st = check_template_window(t, g, box, where);
     if (st != VT_OK) return st;
-    const bool nv12 = g.fmt == VT_FMT_NV12;
-    return init_template(t, target, box, FrameDesc{s->planes[0], nv12 ? s->planes[1] : nullptr, {s->pitch[0], nv12 ? s->pitch[1] : 0}, g.W, g.H,
-                                                   g.fmt, 1, nullptr, t->cfg.pad_plus1});
+    return init_template(t, target, box, FrameDesc{surface_ref(g, *s), nullptr, t->cfg.pad_plus1});
 }
 
 vt_status tracker_submit_surface(vt_tracker* t, const vt_surface* s, bool forward, const char* where) {
@@ -1119,11 +1129,9 @@ vt_status tracker_make_group(vt_tracker* t, int n) {
     VT_CUDA(cudaMalloc(&t->d_ctl, sizeof(ProbeGroupCtl)));
     VT_CUDA(cudaMemset(t->d_ctl, 0, sizeof(ProbeGroupCtl)));
     VT_CUDA(cudaHostAlloc(&t->h_slots, sizeof(int32_t) * kMaxWin, cudaHostAllocDefault));
-    for (int i = 0; i < n; ++i) {  // one device frame per stream, of its geometry
-        const size_t fb = slot_geom(t, i).bytes() + 256;
-        VT_CUDA(cudaMalloc(&t->d_sframes[i], fb));
-        VT_CUDA(cudaMemset(t->d_sframes[i], 0, fb));
-        t->d_sframe_bytes[i] = fb;
+    for (int i = 0; i < n; ++i) {  // one device frame per stream, of its geometry: every stream's HUD is drawn into it at every step
+        const vt_status st = ensure_stream_frame(t, i, slot_geom(t, i).bytes());
+        if (st != VT_OK) return st;
     }
     tracker_enable_hud(t);
     t->group_n = n;
@@ -1176,61 +1184,43 @@ vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size
     ProbeGroupCtl ctl;
     memset(&ctl, 0, sizeof(ctl));
     const int k_act = (int)t->active.size();
-    std::vector<bool> whole((size_t)n, false);
-    for (int k = 0; k < k_act; ++k) {  // the forward's targets, by active-target index
-        const int i = t->active[k];
-        const StreamGeom& g = slot_geom(t, i);
-        ctl.f.geom[k][0] = g.fmt, ctl.f.geom[k][1] = g.W, ctl.f.geom[k][2] = g.H, ctl.f.geom[k][3] = 1;
-        if (surfs) {  // in place: the whole surface holds the frame
-            const bool nv12 = g.fmt == VT_FMT_NV12;
-            ctl.f.frames[k] = surfs[i].planes[0], ctl.f.uvs[k] = nv12 ? surfs[i].planes[1] : nullptr;
-            ctl.f.pitches[k][0] = surfs[i].pitch[0], ctl.f.pitches[k][1] = nv12 ? surfs[i].pitch[1] : 0;
-            continue;
-        }
-        int* w = ctl.f.win[k];
-        if (!t->cfg.upload_window || !windows_allowed(g)) {
-            VT_CUDA(cudaMemcpyAsync(t->d_sframes[i], frames[i], g.bytes(), cudaMemcpyHostToDevice, t->stream));
-            t->h2d_bytes += g.bytes();
-            w[0] = w[1] = 0, w[2] = g.W, w[3] = g.H;
-            whole[i] = true;
-        } else if (search_window(g, t->rect_mirror[i], 0, w[0], w[1], w[2], w[3])) {
-            vt_status st = copy_window(g, t->d_sframes[i], frames[i], w, true, cudaMemcpyHostToDevice, t->stream);
-            if (st != VT_OK) return st;
-            t->h2d_bytes += window_bytes(g, w);
-        } else {
-            w[0] = w[1] = w[2] = w[3] = 0;  // the window misses the frame: the crop kernel flags it
-        }
-        ctl.f.frames[k] = t->d_sframes[i], ctl.f.host_frames[k] = frames[i];
-    }
-    for (int i = 0; i < n; ++i) {  // every stream of the group, by stream index
+    for (int i = 0, k = 0; i < n; ++i) {  // every stream of the group, by stream index; the forward's targets by active-target index k
         const StreamGeom& g = slot_geom(t, i);
         ProbeStreamCtl& e = ctl.s[i];
-        e.frame = surfs ? surfs[i].planes[0] : t->d_sframes[i], e.host_frame = surfs ? nullptr : frames[i];
-        e.pitch = surfs ? surfs[i].pitch[0] : 0;
-        e.geom[0] = g.fmt, e.geom[1] = g.W, e.geom[2] = g.H, e.geom[3] = 1;
-        e.n_hud = t->hud_next_n[i];
-        e.hud = e.n_hud ? t->h_hud[slot] + (size_t)i * kMaxCmds : nullptr;
+        const bool fwd = k < k_act && t->active[k] == i;  // (active is ascending)
+        bool whole = surfs != nullptr;  // in place: the whole surface holds the frame
+        if (surfs) {
+            e.frame = surface_ref(g, surfs[i]);
+        } else if (fwd) {
+            vt_status st = stage_stream(t, i, i, frames[i], ctl.f.win[k], &e.frame, &whole);
+            if (st != VT_OK) return st;
+        } else {
+            e.frame = packed_ref(g, t->d_sframes[i], frames[i], true);
+        }
+        if (fwd) ctl.f.frames[k++] = e.frame;
+        e.hud.n = t->hud_next_n[i];
+        e.hud.list = e.hud.n ? t->h_hud[slot] + (size_t)i * kMaxCmds : nullptr;
         e.slot = t->inited[i] ? i : -1;
         const int* r = t->hud_next_rmw[i];
         int w[4] = {std::max(r[0], 0), std::max(r[1], 0), std::min(r[2], g.W), std::min(r[3], g.H)};
-        if (e.n_hud && (surfs || whole[i])) {
-            e.bg_on_device = 1;
-        } else if (e.n_hud && w[2] > w[0] && w[3] > w[1]) {  // plane 0 only (the luma background dim reads and writes Y)
+        if (e.hud.n && whole) {
+            e.hud.bg_on_device = 1;
+        } else if (e.hud.n && w[2] > w[0] && w[3] > w[1]) {  // plane 0 only (the luma background dim reads and writes Y)
             vt_status st = copy_window(g, t->d_sframes[i], frames[i], w, false, cudaMemcpyHostToDevice, t->stream);
             if (st != VT_OK) return st;
             t->h2d_bytes += plane0_bytes(g, w[0], w[1], w[2], w[3]);
-            e.bg_on_device = 1;
+            e.hud.bg_on_device = 1;
         }
-        if (e.n_hud) q.hud_bytes += t->hud_next_bytes[i];
+        if (e.hud.n) q.hud_bytes += t->hud_next_bytes[i];
         t->hud_next_n[i] = 0;
     }
-    ctl.f.frame = ctl.f.frames[0], ctl.f.host_frame = ctl.f.host_frames[0], ctl.f.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
+    ctl.f.n_frames = k_act, ctl.f.hblk = reinterpret_cast<uint32_t*>(t->h_blk[slot]);
     ctl.f.n_win = surfs ? -1 : k_act;
     if (k_act) {  // (drops since the last step changed the list: it reaches the device ahead of the step's kernels)
         memcpy(t->h_slots, t->active.data(), sizeof(int32_t) * (size_t)k_act);
         VT_CUDA(cudaMemcpyAsync(t->d_slots, t->h_slots, sizeof(int32_t) * (size_t)k_act, cudaMemcpyHostToDevice, t->stream));
     }
-    t->frame_valid = 1, t->d_frame_is_last_host_frame = false;
+    t->d_frame_is_last_host_frame = false;
     VT_CUDA(launch_stamp_group(t->d_stamps + ST_SUBMIT, reinterpret_cast<ProbeGroupCtl*>(t->d_ctl), ctl, t->stream));
     ++t->kernel_launches;
     if (k_act) {
@@ -1245,11 +1235,7 @@ vt_status tracker_submit_group(vt_tracker* t, uint8_t* const* frames, const size
         }
         ++t->kernel_launches;
     }
-    VT_CUDA(cudaEventRecord(t->q_done[slot], t->stream));
-    t->d2h_bytes += t->res_block_bytes;
-    ++t->q_count;
-    t->in_flight = true;
-    return VT_OK;
+    return finish_submit(t, slot);
 }
 }  // namespace vt
 extern "C" {

@@ -107,7 +107,6 @@ struct vt_tracker {
     int rsz_geom[4] = {0, 0, 0, 0};      // sw, sh, dw, dh they were built for
     uint8_t* h_stage = nullptr;  // pinned staging for non-pinned callers
     size_t h_stage_bytes = 0;    // bytes of h_stage and of each d_frames[i]: the largest frame of the cfg and the slot geometries, + 256
-    int frame_valid = 1;
     // what the device frame buffer t->d_frame holds: the whole host frame most recently given to update()/submit()/init() (what
     // vt_overlay_current draws on), or something else (search windows only, a convert / overlay scratch upload, nothing: the last frame
     // was tracked in place in the caller's device memory)
@@ -119,7 +118,7 @@ struct vt_tracker {
     size_t res_block_bytes = 0;
     unsigned long long *d_stamps = nullptr, *h_stamps = nullptr;
     int* h_tc_err = nullptr;
-    FrameCtl* d_ctl = nullptr;         // per-frame control block (frame / host frame / result block addresses, valid windows, HUD list)
+    FrameCtl* d_ctl = nullptr;         // per-frame control block (frames, result block address, valid windows, HUD list)
     // probe HUD (host_state.cpp): the frame's last kernel runs a per-frame command list; the list of the NEXT submit is staged in the
     // pinned block of that submit's queue slot by tracker_set_hud()
     bool hud_mode = false;
@@ -206,6 +205,9 @@ bool is_pinned(const void* p);
 // site that reads, uploads, checks or draws into a slot's frames goes through.  A uniform handle is one whose slots all hold the cfg one.
 inline StreamGeom cfg_geom(const vt_tracker* t) { return StreamGeom{t->fmt, t->W, t->H}; }
 inline const StreamGeom& slot_geom(const vt_tracker* t, int slot) { return t->geom[slot]; }
+// A packed frame of geometry g at `base` as the kernels read it, beside the caller's pinned host frame `host` (or null); valid = false:
+// the buffer was short (tracker_frame.cu, with surface_ref the only constructors of a FrameRef)
+FrameRef packed_ref(const StreamGeom& g, const uint8_t* base, uint8_t* host, bool valid);
 // VT_ERR_INVALID (with a message naming `where`) on a handle where a slot's geometry differs from cfg: single-frame entry points
 vt_status check_uniform_geometry(const vt_tracker* t, const char* where);
 // vt_overlay_cmd -> device form (glyph rows resolved); VT_ERR_GLYPH for an unknown character in strict mode

@@ -163,45 +163,49 @@ __device__ __forceinline__ unsigned long long device_time_ns() {
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)::"memory");
     return t;
 }
+// One frame as the kernels read and draw it, built on the host by packed_ref / surface_ref (tracker_frame.cu): always complete, the
+// kernels apply no defaults.  A host frame only ever goes with a PACKED device frame of the same layout (the handle's or a stream's own
+// buffer, into which windows of the host frame are uploaded), so the crop kernel's fall-back and the overlay mirror address the host
+// frame with the device frame's pitches and chroma offset; a surface or a device frame tracked in place has none.
+struct FrameRef {
+    const uint8_t* plane[2];      // plane 0 (Y / RGB / gray / YUY2 / RGBA / BGRA); NV12 chroma plane, else null
+    size_t pitch[2];              // their row pitches in bytes (packed frames: fmt_row_bytes, W)
+    uint8_t* host;                // the caller's PINNED host frame (device-mapped under UVA) or null: zero-copy target of the overlay mirror
+                                  // and the crop kernel's fall-back source for pixels outside the uploaded windows
+    alignas(16) int32_t geom[4];  // {format, width, height, valid}; valid 0: the buffer was short -> black image (src/nv12_convert.rs:48-50)
+};
+// A frame's (or a probe-group stream's) HUD: the overlay command list of the probe and the background-dim handshake
+struct OverlayCmdDev;
+struct HudCtl {
+    const OverlayCmdDev* list;  // in pinned host memory (or the device copy the stamp kernel wrote), n entries
+    int32_t n;
+    int32_t bg_on_device;       // the region a leading HUD background dim reads was uploaded with the windows: read it from the device frame
+    int32_t bg_ready;           // set by the host-pass CTA of the overlay kernel once its copy of that region is in registers (reset per frame)
+};
 // Per-frame control block in device memory: the addresses and parameters that change from frame to frame reach the kernels of the
 // (captured once, replayed) per-frame graph through it.  Written by stamp_kernel at the start of every frame, outside the graph.
-struct OverlayCmdDev;
 constexpr int kMaxWin = 16;
 struct FrameCtl {
-    const uint8_t* frame;      // device frame this step reads: the handle's own buffer, or the caller's device frame tracked in place
-    const uint8_t* uv;         // NV12 chroma plane of `frame`; null: packed behind the Y plane (frame + W * H)
-    size_t pitch[2];           // row pitch of `frame` / `uv` in bytes (pitched device surfaces); 0: packed rows
-    uint8_t* host_frame;       // the caller's PINNED host frame (device-mapped under UVA) or null: zero-copy target of the overlay mirror
-                               // and the crop kernel's fall-back source for pixels outside the uploaded windows
-    uint32_t* hblk;            // pinned host result block of the frame's queue slot
-    const OverlayCmdDev* hud;  // this frame's overlay command list (probe HUD) in pinned host memory, n_hud entries
-    int32_t n_hud;
+    // the frames this step reads and draws into: frames[0] for every target of a single-frame handle (n_frames = 1); active target i's
+    // OWN frame frames[i] in a stream group or the forward of a probe group (n_frames = n: a group may mix cameras, and the captured graph
+    // does not change with the mix).  target_frame() is the one reader of this rule.  (The scalars first: a kernel's first load of the
+    // block brings frames[0] into the same cache line.)
+    int32_t n_frames;
     int32_t n_win;             // -1: the whole device frame holds this frame; else win[i] = the region that does, for active target i
+    uint32_t* hblk;            // pinned host result block of the frame's queue slot
+    HudCtl hud;                // this frame's HUD (probe)
+    FrameRef frames[kMaxWin];
     int32_t win[kMaxWin][4];   // x0, y0, x1, y1 (exclusive), even-aligned
-    // stream groups (vt_tracker_update_streams): active target i reads — and is drawn into — its OWN frame; null = `frame` / `host_frame`
-    const uint8_t* frames[kMaxWin];
-    const uint8_t* uvs[kMaxWin];          // chroma plane and row pitches of frames[i], as `uv` / `pitch` of `frame`
-    size_t pitches[kMaxWin][2];
-    uint8_t* host_frames[kMaxWin];
-    alignas(16) int32_t geom[kMaxWin][4]; // {format, width, height, valid} of frames[i]: the crop and the box overlay take them over FrameDesc's
-                                          // (a group may mix cameras; the captured graph does not change with the mix)
-    int32_t bg_on_device;      // the region a leading HUD background dim reads was uploaded with the windows: read it from the device frame
-    int32_t bg_ready;          // set by the host-pass CTA of the overlay kernel once its copy of that region is in registers (reset per frame)
 };
+__host__ __device__ inline const FrameRef& target_frame(const FrameCtl& c, int i) { return c.frames[i < c.n_frames ? i : 0]; }
 // Probe groups (vt_probe_group_frame): the control block of a group's handle.  Its FrameCtl part addresses the streams that take part in
 // the step's forward by active-target index, as for a stream group (the crop reads it); the per-stream table addresses EVERY stream of the
 // group by its index, which is also its target slot: CTA pair x of the step's last kernel (probe_group_overlay_kernel) draws stream x.
 struct ProbeStreamCtl {
-    uint8_t* frame;              // the stream's device frame (its search window, if it takes part, and its HUD region uploaded this step),
-                                 // or plane 0 of its surface (vt_probe_group_frame_surface: drawn in place)
-    uint8_t* host_frame;         // its pinned host frame: zero-copy target of the overlay mirror (null for a surface)
-    const OverlayCmdDev* hud;    // its HUD list in the pinned block of the step's queue slot, n_hud entries
-    size_t pitch;                // row pitch of `frame` in bytes; 0: packed rows
-    alignas(16) int32_t geom[4]; // {format, width, height, 1}
-    int32_t n_hud;
-    int32_t slot;                // its target slot when it takes part in this step's forward, else -1 (the HUD of a stream without result)
-    int32_t bg_on_device;        // as FrameCtl::bg_on_device, for this stream
-    int32_t bg_ready;            // as FrameCtl::bg_ready, for this stream's pair of CTAs (reset per step)
+    FrameRef frame;  // the stream's device frame (its search window, if it takes part, and its HUD region uploaded this step) beside its
+                     // pinned host frame, or its surface (vt_probe_group_frame_surface: drawn in place)
+    HudCtl hud;      // its HUD list in the pinned block of the step's queue slot; the handshake of its pair of CTAs
+    int32_t slot;    // its target slot when it takes part in this step's forward, else -1 (the HUD of a stream without result)
 };
 struct ProbeGroupCtl {
     FrameCtl f;                  // first: every kernel of the forward reads it through the same pointer
@@ -219,15 +223,10 @@ cudaError_t launch_publish(const void* d_blk, const FrameCtl* d_ctl, size_t byte
 
 // ---- pixel kernels (pixel.cu) ------------------------------------------------------------------
 struct FrameDesc {
-    const uint8_t* data;   // device pointer: the frame (plane 0: Y / RGB / gray)
-    const uint8_t* uv;     // NV12 chroma plane; null: packed behind the Y plane (data + W * H)
-    size_t pitch[2];       // row pitch of data / uv in bytes; 0: packed rows
-    int32_t width, height;
-    int32_t format;        // vt_format
-    int32_t valid;         // 0: buffer was short -> black image (src/nv12_convert.rs:48-50)
-    // When non-null the frame address (and the valid windows / host fall-back) are read from this per-frame control block instead
-    // of `data`: the per-frame graph is captured once, while vt_tracker_update_device tracks straight out of the caller's device frame
-    // (no device->device copy) and window uploads change from frame to frame.
+    FrameRef frame;        // read only when ctl is null (the template pass of vt_tracker_init)
+    // When non-null the frames (and the valid windows / host fall-back) are read from this per-frame control block: the per-frame graph
+    // is captured once, while vt_tracker_update_device tracks straight out of the caller's device frame (no device->device copy) and
+    // window uploads change from frame to frame.
     const FrameCtl* ctl;
     int32_t pad_plus1;     // App. A.7: 1 = the crop treats the last column / row of the frame as padding (older OpenCV: padR = x2-W+1)
 };
@@ -269,13 +268,12 @@ constexpr int kHudDigitSlot = 37, kHudPercentSlot = 47;
 // (overlay kernels: `format` is the frame's vt_format; they draw with the semantics of overlay_format(format))
 cudaError_t launch_overlay(uint8_t* d_frame, size_t len, int width, int height, int format, const OverlayCmdDev* d_cmds, int n,
                            cudaStream_t s);
-// device-side box overlay straight from the decode result (rect thickness 3 + crosshair 15, src/pipeline.rs:165-168)
-// also the frame's last kernel: runs the per-frame HUD list of the control block (if any), mirrors the touched pixels into the pinned
-// host frame and publishes the result block.  draw_box = 0: HUD list only (probe: the box is part of the list).  n = 0 is legal with
-// a HUD list (frames on which no tracker ran).
-cudaError_t launch_box_overlay(size_t len, int width, int height, int format, const DeviceResult* d_res, const int32_t* d_slots, int n,
-                               float gate, const FrameCtl* d_ctl, unsigned long long* stamp_end, cudaStream_t s, bool pdl, const void* d_blk,
-                               size_t blk_bytes, int draw_box);
+// device-side box overlay straight from the decode result (rect thickness 3 + crosshair 15, src/pipeline.rs:165-168) into each target's
+// frame of the control block; also the frame's last kernel: runs the per-frame HUD list of the control block (if any), mirrors the
+// touched pixels into the pinned host frame and publishes the result block.  draw_box = 0: HUD list only (probe: the box is part of the
+// list).  n = 0 is legal with a HUD list (frames on which no tracker ran).
+cudaError_t launch_box_overlay(const DeviceResult* d_res, const int32_t* d_slots, int n, float gate, const FrameCtl* d_ctl,
+                               unsigned long long* stamp_end, cudaStream_t s, bool pdl, const void* d_blk, size_t blk_bytes, int draw_box);
 // the last kernel of a probe group's step: the same drawing as launch_box_overlay in HUD mode, one CTA pair per stream of the group
 // (n_streams, whether or not the stream took part in the forward), each with its stream's frames, geometry, slot and HUD list from d_ctl
 cudaError_t launch_group_overlay(int n_streams, const DeviceResult* d_res, float gate, const ProbeGroupCtl* d_ctl, unsigned long long* stamp_end,
