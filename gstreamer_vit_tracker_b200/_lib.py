@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("VT_B200_LIB") or os.path.join(_HERE, "libvittrack_b200.so")  # (override: A/B runs of two builds)
 
 VT_OK, VT_ERR_INVALID, VT_ERR_CUDA, VT_ERR_WEIGHTS, VT_ERR_CROP_OUTSIDE, VT_ERR_NOT_INIT, VT_ERR_GLYPH = 0, -1, -2, -3, -4, -5, -6
-VT_FMT_NV12, VT_FMT_RGB24, VT_FMT_GRAY8, VT_FMT_YUY2, VT_FMT_RGBA, VT_FMT_BGRA = 0, 1, 2, 3, 5, 6
+VT_FMT_NV12, VT_FMT_RGB24, VT_FMT_GRAY8, VT_FMT_YUY2, VT_FMT_RGBA, VT_FMT_BGRA, VT_FMT_I420 = 0, 1, 2, 3, 5, 6, 8
 VT_GEMM_FP32_SIMT, VT_GEMM_TCGEN05_BF16X3, VT_GEMM_TCGEN05_BF16, VT_GEMM_TCGEN05_FP16 = 0, 1, 2, 3
 VT_RUN_HOST_SYNC, VT_RUN_HOST_PIPELINED, VT_RUN_DEVICE_SYNC, VT_RUN_DEVICE_PIPELINED = range(4)
 VT_DECODE_CEIL4, VT_DECODE_4FLOOR = 0, 1

@@ -95,14 +95,16 @@ def _ptr(a: np.ndarray) -> C.c_void_p:
 
 
 FORMATS = {"nv12": L.VT_FMT_NV12, "rgb24": L.VT_FMT_RGB24, "gray8": L.VT_FMT_GRAY8, "yuy2": L.VT_FMT_YUY2, "rgba": L.VT_FMT_RGBA,
-           "bgra": L.VT_FMT_BGRA}
+           "bgra": L.VT_FMT_BGRA, "i420": L.VT_FMT_I420}
 
 
 def row_bytes(fmt: str, width: int) -> int:
     """Bytes of one packed row of plane 0 (the Y plane, the RGB / gray image, the packed YUY2 words: 4 * ceil(width / 2), the 32-bit
-    RGBA / BGRA pixels: 4 * width)."""
+    RGBA / BGRA pixels: 4 * width; I420: the Y stride of GStreamer's layout, width rounded up to a multiple of 4)."""
     if fmt == "yuy2":
         return 4 * ((width + 1) // 2)
+    if fmt == "i420":
+        return (width + 3) & ~3
     return width * {"rgb24": 3, "rgba": 4, "bgra": 4}.get(fmt, 1)
 
 
@@ -297,7 +299,7 @@ class VitTrack:
 
     def set_stream_geometry(self, target: int, width: Optional[int] = None, height: Optional[int] = None, fmt: Optional[str] = None) -> None:
         """Stream groups of mixed cameras (vt_tracker_set_stream_geometry): target slot `target` takes frames of `fmt` ("nv12", "rgb24",
-        "gray8", "yuy2", "rgba", "bgra") at width x height instead of the handle's geometry — init() on that slot and its stream in update_streams /
+        "gray8", "yuy2", "rgba", "bgra", "i420") at width x height instead of the handle's geometry — init() on that slot and its stream in update_streams /
         update_streams_surface / run_streams_ring.  Only a slot that is not initialised may change; no arguments: back to the handle's
         geometry.  A handle with a slot of its own geometry takes frames through the stream-group calls only."""
         if width is None and height is None and fmt is None:

@@ -433,7 +433,7 @@ __device__ __forceinline__ Tap lin_tap(int i, int s, int d, bool clamp_frac) {
 // caller's pinned host frame (zero-copy loads over PCIe) outside of it.  With whole-frame uploads the window is the frame.  The device
 // frame may be a pitched surface; the host frame has the device frame's pitches and plane offset (see FrameRef).
 struct PixelSrc {
-    const uint8_t *dev, *dev_uv;  // device planes: Y / RGB / gray, NV12 chroma
+    const uint8_t *dev, *dev_uv;  // device planes: Y / RGB / gray, NV12 chroma / I420 U
     size_t pitch, uv_pitch;       // their row pitches
     const uint8_t* host;          // null: everything is on the device
     int x0, y0, x1, y1;           // valid window of the device frame (even-aligned, so a pixel and its chroma pair sit on the same side;
@@ -451,8 +451,8 @@ __device__ __forceinline__ uint32_t plane_word(const uint8_t* q, bool aligned) {
     return (uint32_t)q[0] | ((uint32_t)q[1] << 8) | ((uint32_t)q[2] << 16) | ((uint32_t)q[3] << 24);
 }
 
-// RGB of the frame pixel (fx, fy); zero outside the frame (constant border of the crop).
-__device__ __forceinline__ void frame_rgb(const PixelSrc& ps, int fx, int fy, int& r, int& g, int& b) {
+// RGB of the frame pixel (fx, fy); zero outside the frame (constant border of the crop).  pad: the kernel's pad_plus1.
+__device__ __forceinline__ void frame_rgb(const PixelSrc& ps, int pad, int fx, int fy, int& r, int& g, int& b) {
     r = g = b = 0;
     if (fx < 0 || fy < 0 || fx >= ps.xlim || fy >= ps.ylim) return;
     const bool host = ps.host && ((unsigned)(fx - ps.x0) >= (unsigned)(ps.x1 - ps.x0) || (unsigned)(fy - ps.y0) >= (unsigned)(ps.y1 - ps.y0));
@@ -473,8 +473,18 @@ __device__ __forceinline__ void frame_rgb(const PixelSrc& ps, int fx, int fy, in
     } else {
         const int yv = data[(size_t)fy * ps.pitch + fx];
         const uint8_t* uv = host ? ps.host + (ps.dev_uv - ps.dev) : ps.dev_uv;
-        const size_t uvi = (size_t)(fy >> 1) * ps.uv_pitch + (fx & ~1);
-        const Chroma c = chroma_terms(uv[uvi], uv[uvi + 1]);
+        int u, v;
+        if (ps.format == VT_FMT_I420) {
+            // U of the pixel's 2x2 block in plane 1; V at the same place one chroma plane further, uv_pitch * ceil(H / 2): only packed
+            // frames are I420 (no surfaces), and a pixel is read only when the frame is valid, where H = ylim + pad.  (H is not kept in
+            // PixelSrc: one more live register would make ptxas spill at 32.)
+            const uint8_t* q = uv + (size_t)(fy >> 1) * ps.uv_pitch + (fx >> 1);
+            u = q[0], v = q[ps.uv_pitch * (size_t)((ps.ylim + pad + 1) >> 1)];
+        } else {
+            const size_t uvi = (size_t)(fy >> 1) * ps.uv_pitch + (fx & ~1);
+            u = uv[uvi], v = uv[uvi + 1];
+        }
+        const Chroma c = chroma_terms(u, v);
         yuv_px(yv, c, r, g, b);
     }
 }
@@ -526,19 +536,23 @@ __global__ void __launch_bounds__(256, 8) crop_resize_norm_kernel(FrameDesc f, T
     const Tap ty = lin_tap(dy, c, S, false);
     const int cx0 = tx.ofs, cx1 = min(tx.ofs + 1, c - 1);
     const int cy0 = min(max(ty.ofs, 0), c - 1), cy1 = min(max(ty.ofs + 1, 0), c - 1);
-    int p00[3], p01[3], p10[3], p11[3];
-    frame_rgb(ps, x1 + cx0, y1 + cy0, p00[0], p00[1], p00[2]);
-    frame_rgb(ps, x1 + cx1, y1 + cy0, p01[0], p01[1], p01[2]);
-    frame_rgb(ps, x1 + cx0, y1 + cy1, p10[0], p10[1], p10[2]);
-    frame_rgb(ps, x1 + cx1, y1 + cy1, p11[0], p11[1], p11[2]);
+    // each pair of horizontal taps is blended as soon as it is read (three sums stay live instead of six samples: with the I420 read in
+    // frame_rgb this keeps the kernel at 32 registers without spills; the arithmetic is unchanged)
+    int qa[3], qb[3], t0[3], t1[3];
+    frame_rgb(ps, f.pad_plus1, x1 + cx0, y1 + cy0, qa[0], qa[1], qa[2]);
+    frame_rgb(ps, f.pad_plus1, x1 + cx1, y1 + cy0, qb[0], qb[1], qb[2]);
+#pragma unroll
+    for (int ch = 0; ch < 3; ++ch) t0[ch] = qa[ch] * tx.a0 + qb[ch] * tx.a1;
+    frame_rgb(ps, f.pad_plus1, x1 + cx0, y1 + cy1, qa[0], qa[1], qa[2]);
+    frame_rgb(ps, f.pad_plus1, x1 + cx1, y1 + cy1, qb[0], qb[1], qb[2]);
+#pragma unroll
+    for (int ch = 0; ch < 3; ++ch) t1[ch] = qa[ch] * tx.a0 + qb[ch] * tx.a1;
     const int nt = S >> 4;
     const int token = (dy >> 4) * nt + (dx >> 4);
     const size_t off = (size_t)bi * patches_stride + (size_t)token * kPatchK + (dy & 15) * 16 + (dx & 15);
 #pragma unroll
     for (int ch = 0; ch < 3; ++ch) {
-        const int t0 = p00[ch] * tx.a0 + p01[ch] * tx.a1;
-        const int t1 = p10[ch] * tx.a0 + p11[ch] * tx.a1;
-        const int v = (((ty.a0 * (t0 >> 4)) >> 16) + ((ty.a1 * (t1 >> 4)) >> 16) + 2) >> 2;
+        const int v = (((ty.a0 * (t0[ch] >> 4)) >> 16) + ((ty.a1 * (t1[ch] >> 4)) >> 16) + 2) >> 2;
         const float val = lut[ch * 256 + (v & 255)];
         patches[off + ch * 256] = val;
         if (p_hi && !p_lo) {  // single-pass fp16 operands

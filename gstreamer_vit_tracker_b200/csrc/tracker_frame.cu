@@ -327,9 +327,14 @@ struct UploadPlan {
 };
 // Window uploads need windows whose pixels carry their own chroma: even x0 (NV12 chroma pairs, YUY2 words) and, for NV12, even y0.
 // YUY2 takes any W and H: a window that ends on an odd last column copies that column's whole word, and chroma is per row.  RGBA / BGRA
-// take any W and H: a window is whole 4-byte pixels, each with its own colour.
+// take any W and H: a window is whole 4-byte pixels, each with its own colour.  I420 takes any W and H: the chroma planes are copied
+// over the blocks [x0 / 2, ceil(x1 / 2)) x [y0 / 2, ceil(y1 / 2)), which hold the chroma of every pixel of the window.
 static bool windows_allowed(const StreamGeom& g) {
-    return g.fmt == VT_FMT_YUY2 || format_is_rgb32(g.fmt) || (!(g.W % 2) && !((g.H % 2) && g.fmt == VT_FMT_NV12));
+    return g.fmt == VT_FMT_YUY2 || format_is_rgb32(g.fmt) || g.fmt == VT_FMT_I420 || (!(g.W % 2) && !((g.H % 2) && g.fmt == VT_FMT_NV12));
+}
+// I420: the chroma blocks under the window w, [cx, cx + cw) x [cy, cy + ch), in each of the U and V planes
+static void i420_chroma_window(const int* w, size_t& cx, size_t& cy, size_t& cw, size_t& ch) {
+    cx = (size_t)(w[0] / 2), cy = (size_t)(w[1] / 2), cw = (size_t)((w[2] + 1) / 2) - cx, ch = (size_t)((w[3] + 1) / 2) - cy;
 }
 // bytes of plane 0 that hold the pixels [x0, x1) x [y0, y1) of a packed frame (YUY2: whole words)
 static size_t plane0_bytes(const StreamGeom& g, int x0, int y0, int x1, int y1) {
@@ -337,11 +342,17 @@ static size_t plane0_bytes(const StreamGeom& g, int x0, int y0, int x1, int y1) 
     fmt_col_span(g.fmt, x0, x1, &o0, &o1);
     return (o1 - o0) * (size_t)(y1 - y0);
 }
-// bytes of the window w = (x0, y0, x1, y1): plane 0 and, for NV12, the chroma rows under it
+// bytes of the window w = (x0, y0, x1, y1): plane 0 and, for NV12, the chroma rows under it (I420: the chroma blocks, in U and in V)
 static size_t window_bytes(const StreamGeom& g, const int* w) {
+    if (g.fmt == VT_FMT_I420) {
+        size_t cx, cy, cw, ch;
+        i420_chroma_window(w, cx, cy, cw, ch);
+        return plane0_bytes(g, w[0], w[1], w[2], w[3]) + 2 * cw * ch;
+    }
     return plane0_bytes(g, w[0], w[1], w[2], w[3]) + (g.fmt == VT_FMT_NV12 ? (size_t)(w[2] - w[0]) * ((w[3] - w[1]) / 2) : 0);
 }
-// one 2D copy of the window w of a packed frame out of plane 0 (+ one of the NV12 chroma rows under it when `chroma`)
+// one 2D copy of the window w of a packed frame out of plane 0 (+ one of the NV12 chroma rows under it when `chroma`; I420: one 3D copy
+// of depth 2, its slices the U and the V plane, so that a window costs two copy calls as for NV12)
 static vt_status copy_window(const StreamGeom& g, uint8_t* dst, const uint8_t* src, const int* w, bool chroma, cudaMemcpyKind kind,
                              cudaStream_t stream) {
     const size_t row = fmt_row_bytes(g.fmt, g.W), rows = (size_t)(w[3] - w[1]);
@@ -352,6 +363,17 @@ static vt_status copy_window(const StreamGeom& g, uint8_t* dst, const uint8_t* s
     if (chroma && g.fmt == VT_FMT_NV12) {
         const size_t W = (size_t)g.W, uvo = W * g.H + (size_t)(w[1] / 2) * W + w[0];
         VT_CUDA(cudaMemcpy2DAsync(dst + uvo, W, src + uvo, W, (size_t)(w[2] - w[0]), rows / 2, kind, stream));
+    } else if (chroma && g.fmt == VT_FMT_I420) {
+        size_t cx, cy, cw, ch;
+        i420_chroma_window(w, cx, cy, cw, ch);
+        const size_t cp = i420_chroma_pitch(g.W), crows = (size_t)((g.H + 1) / 2), uo = i420_u_offset(g.W, g.H);
+        cudaMemcpy3DParms p = {};
+        p.srcPtr = make_cudaPitchedPtr(const_cast<uint8_t*>(src + uo), cp, cp, crows);
+        p.dstPtr = make_cudaPitchedPtr(dst + uo, cp, cp, crows);
+        p.srcPos = p.dstPos = make_cudaPos(cx, cy, 0);
+        p.extent = make_cudaExtent(cw, ch, 2);
+        p.kind = kind;
+        VT_CUDA(cudaMemcpy3DAsync(&p, stream));
     }
     return VT_OK;
 }
@@ -531,12 +553,14 @@ static inline double now_us() {
     return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
 
-// The two constructors of a FrameRef.  A packed frame of geometry g at `base` (NV12: the chroma plane right behind the Y plane), beside
-// the caller's pinned host frame `host` (or null); valid = false: the buffer was short, the crop reads a black image.
+// The two constructors of a FrameRef.  A packed frame of geometry g at `base` (NV12: the chroma plane right behind the Y plane; I420:
+// plane 1 is the U plane, the V plane follows it), beside the caller's pinned host frame `host` (or null); valid = false: the buffer was
+// short, the crop reads a black image.
 FrameRef packed_ref(const StreamGeom& g, const uint8_t* base, uint8_t* host, bool valid) {
-    const bool nv12 = g.fmt == VT_FMT_NV12;
-    return FrameRef{{base, nv12 ? base + (size_t)g.W * g.H : nullptr}, {fmt_row_bytes(g.fmt, g.W), nv12 ? (size_t)g.W : 0}, host,
-                    {g.fmt, g.W, g.H, valid ? 1 : 0}};
+    const bool nv12 = g.fmt == VT_FMT_NV12, i420 = g.fmt == VT_FMT_I420;
+    const uint8_t* p1 = nv12 ? base + (size_t)g.W * g.H : i420 ? base + i420_u_offset(g.W, g.H) : nullptr;
+    const size_t pitch1 = nv12 ? (size_t)g.W : i420 ? i420_chroma_pitch(g.W) : 0;
+    return FrameRef{{base, p1}, {fmt_row_bytes(g.fmt, g.W), pitch1}, host, {g.fmt, g.W, g.H, valid ? 1 : 0}};
 }
 // the caller's surface s (checked by check_surface), read and drawn into in place
 static FrameRef surface_ref(const StreamGeom& g, const vt_surface& s) {
@@ -547,6 +571,11 @@ static FrameRef surface_ref(const StreamGeom& g, const vt_surface& s) {
 // The caller's surface (include/vt_tracker.h: vt_surface): every plane of the format present, a pitch that holds a row, and device (or
 // managed) memory of the handle's GPU, for a frame of geometry g.  `i` >= 0 names the surface of a stream group in the message.
 static vt_status check_surface(const vt_tracker* t, const StreamGeom& g, const vt_surface* s, const char* where, int i) {
+    if (g.fmt == VT_FMT_I420) {  // (three planes: a vt_surface has two, and the crop kernel addresses V by the packed layout)
+        set_error("%s: surface %d: I420 frames are not taken as surfaces (host frames or packed device frames only: "
+                  "vt_tracker_update_device / vt_tracker_submit_device)", where, i);
+        return VT_ERR_INVALID;
+    }
     if (!s) {
         set_error("%s: surface %d is null", where, i);
         return VT_ERR_INVALID;
@@ -812,8 +841,8 @@ static vt_status wait_common(vt_tracker* t, vt_result* results) {
 }
 
 // ---- ring replay support ----------------------------------------------------------------------------------------------------------
-// [x0, x1) x [y0, y1) of the drawable plane (Y plane / luma for NV12 and GRAY8, the RGB image for RGB24, the whole pixel-pair words
-// for YUY2, the whole 4-byte pixels for RGBA / BGRA), clipped to the frame
+// [x0, x1) x [y0, y1) of the drawable plane (Y plane / luma for NV12, I420 and GRAY8, the RGB image for RGB24, the whole pixel-pair
+// words for YUY2, the whole 4-byte pixels for RGBA / BGRA), clipped to the frame
 void restore_rect_region(uint8_t* frame, const uint8_t* clean, int fmt, int W, int H, long long x0, long long y0, long long x1, long long y1) {
     x0 = std::max(x0, 0LL), y0 = std::max(y0, 0LL), x1 = std::min<long long>(x1, W), y1 = std::min<long long>(y1, H);
     if (x1 <= x0 || y1 <= y0) return;

@@ -28,10 +28,12 @@ void set_error(const char* fmt, ...);
 // caller's vt_config (any struct_size the ABI ever had) -> the library's full struct with defaults for what the caller's header lacks
 vt_status resolve_config(const vt_config* in, vt_config* out);
 
-// GRAY8 frames are a bare luma plane and YUY2 frames carry one Y sample per pixel: both are drawn on with the NV12 (Y plane)
-// overlay semantics
-__host__ __device__ inline int overlay_format(int fmt) { return fmt == VT_FMT_GRAY8 || fmt == VT_FMT_YUY2 ? VT_FMT_NV12 : fmt; }
-__host__ __device__ inline bool format_is_luma(int fmt) { return fmt == VT_FMT_NV12 || fmt == VT_FMT_GRAY8 || fmt == VT_FMT_YUY2; }
+// GRAY8 frames are a bare luma plane, YUY2 frames carry one Y sample per pixel and I420 frames lead with a Y plane: all are drawn on
+// with the NV12 (Y plane) overlay semantics
+__host__ __device__ inline bool format_is_luma(int fmt) {
+    return fmt == VT_FMT_NV12 || fmt == VT_FMT_GRAY8 || fmt == VT_FMT_YUY2 || fmt == VT_FMT_I420;
+}
+__host__ __device__ inline int overlay_format(int fmt) { return format_is_luma(fmt) ? VT_FMT_NV12 : fmt; }
 // RGBA / BGRA: 32-bit pixels whose byte 3 (alpha or padding) is never read or written; tracked and drawn on as the RGB24 frame of their
 // colour bytes
 __host__ __device__ inline bool format_is_rgb32(int fmt) { return fmt == VT_FMT_RGBA || fmt == VT_FMT_BGRA; }
@@ -48,12 +50,22 @@ __host__ __device__ inline RgbOffsets fmt_rgb_offsets(int fmt) { return fmt == V
 __host__ __device__ inline int fmt_px_step(int fmt) {
     return fmt == VT_FMT_RGB24 ? 3 : format_is_rgb32(fmt) ? 4 : fmt == VT_FMT_YUY2 ? 2 : 1;
 }
-// bytes of one packed row of plane 0 (YUY2: whole pixel-pair words, 4 * ceil(W / 2): odd widths pad the last word)
+// bytes of one packed row of plane 0 (YUY2: whole pixel-pair words, 4 * ceil(W / 2): odd widths pad the last word; I420: the Y stride,
+// RU4(W), as GStreamer lays it out)
 __host__ __device__ inline size_t fmt_row_bytes(int fmt, int W) {
-    return fmt == VT_FMT_YUY2 ? (size_t)4 * (size_t)((W + 1) / 2) : (size_t)W * (size_t)fmt_px_step(fmt);
+    return fmt == VT_FMT_YUY2 ? (size_t)4 * (size_t)((W + 1) / 2)
+         : fmt == VT_FMT_I420 ? (size_t)((W + 3) & ~3)
+                              : (size_t)W * (size_t)fmt_px_step(fmt);
 }
+// I420 in GStreamer's default layout (include/vt_tracker.h): the Y plane of RU2(H) rows (odd H: one padding row), then the U plane,
+// then the V plane, each ceil(H / 2) rows of i420_chroma_pitch(W) = RU4(ceil(W / 2)) bytes.  These two and fmt_row_bytes are the one
+// place that knows that layout.
+__host__ __device__ inline size_t i420_chroma_pitch(int W) { return (size_t)(((W + 1) / 2 + 3) & ~3); }
+// the U plane's offset in the frame; the V plane starts i420_chroma_pitch(W) * ceil(H / 2) bytes after it
+__host__ __device__ inline size_t i420_u_offset(int W, int H) { return fmt_row_bytes(VT_FMT_I420, W) * (size_t)((H + 1) & ~1); }
 // bytes of a packed frame, every plane
 __host__ __device__ inline size_t fmt_frame_bytes(int fmt, int W, int H) {
+    if (fmt == VT_FMT_I420) return i420_u_offset(W, H) + 2 * i420_chroma_pitch(W) * (size_t)((H + 1) / 2);
     return fmt == VT_FMT_NV12 ? (size_t)W * H + (size_t)((H + 1) / 2) * W + (W & 1) : fmt_row_bytes(fmt, W) * (size_t)H;
 }
 // the shortest buffer that is a frame; anything shorter is an all-black image (NV12: src/nv12_convert.rs:48-50)
@@ -69,7 +81,7 @@ struct StreamGeom {
 };
 // the formats and sizes a handle's frames may have (vt_tracker_create's cfg, vt_tracker_set_stream_geometry)
 inline bool geometry_ok(int fmt, int W, int H) {
-    return W > 0 && H > 0 && (fmt == VT_FMT_NV12 || fmt == VT_FMT_RGB24 || fmt == VT_FMT_GRAY8 || fmt == VT_FMT_YUY2 || format_is_rgb32(fmt));
+    return W > 0 && H > 0 && (format_is_luma(fmt) || fmt == VT_FMT_RGB24 || format_is_rgb32(fmt));
 }
 // the bytes [*o0, *o1) of a plane-0 row that hold the pixels x0 .. x1 - 1 (YUY2: the whole words of those pixels)
 __host__ __device__ inline void fmt_col_span(int fmt, long long x0, long long x1, size_t* o0, size_t* o1) {
@@ -168,8 +180,9 @@ __device__ __forceinline__ unsigned long long device_time_ns() {
 // buffer, into which windows of the host frame are uploaded), so the crop kernel's fall-back and the overlay mirror address the host
 // frame with the device frame's pitches and chroma offset; a surface or a device frame tracked in place has none.
 struct FrameRef {
-    const uint8_t* plane[2];      // plane 0 (Y / RGB / gray / YUY2 / RGBA / BGRA); NV12 chroma plane, else null
-    size_t pitch[2];              // their row pitches in bytes (packed frames: fmt_row_bytes, W)
+    const uint8_t* plane[2];      // plane 0 (Y / RGB / gray / YUY2 / RGBA / BGRA); NV12 chroma plane, I420 U plane (always packed: the V
+                                  // plane follows it at pitch[1] * ceil(H / 2)), else null
+    size_t pitch[2];              // their row pitches in bytes (packed frames: fmt_row_bytes, W; I420: i420_chroma_pitch)
     uint8_t* host;                // the caller's PINNED host frame (device-mapped under UVA) or null: zero-copy target of the overlay mirror
                                   // and the crop kernel's fall-back source for pixels outside the uploaded windows
     alignas(16) int32_t geom[4];  // {format, width, height, valid}; valid 0: the buffer was short -> black image (src/nv12_convert.rs:48-50)

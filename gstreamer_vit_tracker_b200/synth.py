@@ -80,6 +80,33 @@ def rgb_to_yuy2(rgb: np.ndarray) -> np.ndarray:
     return out.reshape(-1)
 
 
+def i420_layout(w: int, h: int) -> Tuple[int, int, int, int, int]:
+    """GStreamer's default I420 layout: (Y stride, U / V stride, U offset, V offset, frame bytes)."""
+    s0, s1, ch = (w + 3) & ~3, ((w + 1) // 2 + 3) & ~3, (h + 1) // 2
+    u = s0 * (h + (h & 1))
+    return s0, s1, u, u + s1 * ch, u + 2 * s1 * ch
+
+
+def rgb_to_i420(rgb: np.ndarray) -> np.ndarray:
+    """BT.601 limited-range RGB(HWC u8) -> planar I420 bytes in GStreamer's default layout (i420_layout): Y, then U, then V.
+
+    Any width and height.  Luma and chroma as rgb_to_nv12 (the rounded 2x2 mean); at an odd size the last column / row is replicated
+    into the missing half of its 2x2 blocks.  Row padding and the Y padding row of an odd height are zero.
+    """
+    h, w, _ = rgb.shape
+    p = np.asarray(rgb, dtype=np.uint8)
+    p = np.pad(p, ((0, h & 1), (0, w & 1), (0, 0)), mode="edge")
+    nv = rgb_to_nv12(p)
+    H2, W2 = p.shape[0], p.shape[1]
+    s0, s1, uo, vo, n = i420_layout(w, h)
+    out = np.zeros(n, dtype=np.uint8)
+    out[: s0 * h].reshape(h, s0)[:, :w] = nv[: W2 * H2].reshape(H2, W2)[:h, :w]
+    uv = nv[W2 * H2:].reshape(H2 // 2, W2 // 2, 2)
+    out[uo: vo].reshape(H2 // 2, s1)[:, : W2 // 2] = uv[..., 0]
+    out[vo:].reshape(H2 // 2, s1)[:, : W2 // 2] = uv[..., 1]
+    return out
+
+
 def _rgb_to_32(rgb: np.ndarray, pad, order) -> np.ndarray:
     h, w, _ = rgb.shape
     out = np.empty((h, w, 4), dtype=np.uint8)

@@ -55,7 +55,20 @@ enum {
  * The tracker sees exactly the RGB24 frame made of bytes 0, 1, 2 (RGBA) resp. 2, 1, 0 (BGRA) of every pixel; the overlays follow the
  * RGB24 semantics and write each colour into its channel's byte.  Byte 3 (alpha or padding) is never read and never written.
  * vt_overlay[_current] on such a handle needs a full frame (len >= 4 * W * H).  (Values 4 and 7 are not formats.) */
-typedef enum { VT_FMT_NV12 = 0, VT_FMT_RGB24 = 1, VT_FMT_GRAY8 = 2, VT_FMT_YUY2 = 3, VT_FMT_RGBA = 5, VT_FMT_BGRA = 6 } vt_format;
+/* VT_FMT_I420: planar 4:2:0, the Y plane, then the U plane, then the V plane (GStreamer I420: avdec_h264 / avdec_h265, openh264dec,
+ * vp8dec / vp9dec, dav1ddec, jpegdec, videotestsrc), in GStreamer's default layout, so that a mapped buffer is handed over as it is at any
+ * W and H (RU4 / RU2: rounded up to a multiple of 4 / 2):
+ *   Y stride s0 = RU4(W), U / V stride s1 = RU4(ceil(W/2)),
+ *   U offset = s0 * RU2(H) (odd H: the Y plane has one padding row), V offset = U offset + s1 * ceil(H/2),
+ *   frame bytes = V offset + s1 * ceil(H/2)    (1920x1080: 3,110,400 = W*H*3/2; 641x481: 466,576).
+ * The tracker sees pixel (x, y) as the BT.601 integer RGB of Y[y][x], U[y/2][x/2], V[y/2][x/2] (the arithmetic of NV12): for even W,
+ * tracking an I420 frame equals tracking the NV12 frame of the same Y and interleaved UV.  A buffer shorter than the frame is an
+ * all-black image.  The overlays follow the NV12 luma-plane semantics: they write only the Y samples of the W x H image, never U, V, the
+ * Y row padding or the padding row.  I420 frames are host frames or packed device frames (vt_tracker_update_device); pitched I420
+ * surfaces are refused (see vt_surface). */
+typedef enum {
+    VT_FMT_NV12 = 0, VT_FMT_RGB24 = 1, VT_FMT_GRAY8 = 2, VT_FMT_YUY2 = 3, VT_FMT_RGBA = 5, VT_FMT_BGRA = 6, VT_FMT_I420 = 8
+} vt_format;
 /* BF16X3 (default): bf16 hi + lo operands, three products per K-step, scores within ~1e-5 of the fp32 oracle.  BF16 / FP16: single-pass
  * operands, 17 % faster, score error ~1e-3 / ~3e-4 — opt-in (near-tie arg-max flips are possible at that error). */
 typedef enum { VT_GEMM_FP32_SIMT = 0, VT_GEMM_TCGEN05_BF16X3 = 1, VT_GEMM_TCGEN05_BF16 = 2, VT_GEMM_TCGEN05_FP16 = 3 } vt_gemm_mode;
@@ -133,7 +146,7 @@ void vt_tracker_destroy(vt_tracker* t);
 
 /* ≙ VitTrack::init(&frame, bbox) (src/tracker_context.rs:88).  `frame` is host memory in the
  * handle's format, tightly packed (NV12: w*h*3/2 bytes, src/nv12_convert.rs:48; RGB24: h*w*3,
- * src/pipeline_ir.rs:142; RGBA / BGRA: h*w*4).  A short NV12 buffer is treated as an all-black image
+ * src/pipeline_ir.rs:142; RGBA / BGRA: h*w*4; I420: GStreamer's layout, see vt_format).  A short NV12 buffer is treated as an all-black image
  * (src/nv12_convert.rs:48-50). */
 vt_status vt_tracker_init(vt_tracker* t, int32_t target, const uint8_t* frame, size_t len, vt_bbox box);
 
@@ -188,6 +201,10 @@ vt_status vt_tracker_update_device(vt_tracker* t, uint8_t* d_frame, size_t len, 
  * ignored.  pitch[i] >= the plane's row bytes (W for Y / UV / GRAY8, 3W for RGB24, 4 * ceil(W/2) for YUY2, 4W for RGBA / BGRA: a
  * DeepStream NvBufSurface gives planes[0] = dataPtr + planeParams.offset[0], pitch[0] = planeParams.pitch[0]); planes may be separate allocations
  * and need no alignment.  A tightly packed frame d is the surface {d, d + W*H}, {W, W} (RGB24: {d, NULL}, {3W, 0}).
+ * There are no I420 surfaces: a vt_surface has two planes, and hardware decoders (NVDEC, nvv4l2decoder, nvh264dec) deliver NV12, while
+ * I420 comes from software decoders in host memory.  Every surface entry point (the vt_tracker_*_surface calls, vt_probe_frame_surface,
+ * vt_probe_group_frame_surface) is VT_ERR_INVALID, with vt_last_error() naming I420, for an I420 handle or stream slot; a packed I420
+ * device frame goes through vt_tracker_update_device / vt_tracker_submit_device.
  *
  * The surface entry points below are additive (VT_ABI_VERSION stays 2): each behaves like the entry point it names, except that the
  * frame is a surface.  The tracker reads the surface in place (nothing is copied), and with cfg.box_overlay draws the box into it: into
